@@ -2,6 +2,7 @@
 """Benchmark of the OpenPose hot path (BASELINE.json: body-pose frames/s at 720p, 4 scales).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--frames-per-step F]
+                    [--dump-outputs DIR]
 
 A step is one pass of the whole Body path (preprocess at 4 scales -> CNN -> upsample/average -> Gaussian+NMS ->
 PAF scoring / matching / assembly) over F synthetic 1280x720 frames on every rank, submitted as F/B batches of B
@@ -10,7 +11,8 @@ exchange data (weak scaling, no collective on the data path).  Rank 0 prints ONE
 JSON line.  `value` is measured with the frames already resident in HBM; `e2e` goes through the same public
 `Body` API with pinned HOST frames, the host->device copy of every frame and the device->host read of every
 result inside the timed region.  `--impl reference` times the CPU restatement of the reference (oracle/) on the
-host cores instead (the reference itself, /root/reference, does not exist on the GPU box)."""
+host cores instead.  `--dump-outputs DIR` writes the results of the last timed step (see dump_outputs); inputs and
+weights are seeded, so two builds run with the same arguments can be compared output for output."""
 import argparse
 import json
 import os
@@ -29,6 +31,8 @@ SCALES = (0.5, 1.0, 1.5, 2.0)
 METRIC = "body_pose_frames_per_sec_720p_4scale"
 GFLOP_PER_FRAME = 3634.8          # SURVEY.md 8d: algorithmic conv FLOPs of the body net at the four padded sizes
 POOL_FRAMES = 80                  # 80 x 2.76 MB = 221 MB of distinct inputs (> 126 MB L2)
+REF_POOL_FRAMES = 12              # distinct frames of the host-side reference leg, reused modulo the pool
+DUMP_LIMIT = 64 << 20             # bytes --dump-outputs may write
 
 
 def rank_info():
@@ -40,6 +44,32 @@ def synth_frames(n, seed):
     rng = np.random.default_rng(seed)
     base = rng.integers(0, 256, (n, H // 8, W // 8, 3), dtype=np.uint8)
     return np.ascontiguousarray(np.repeat(np.repeat(base, 8, 1), 8, 2))
+
+
+def dump_outputs(d, results):
+    """Writes one step's per-frame (candidate, subset) results, what Body hands its caller, as float64 .npy files:
+    candidate.npy (N, 4) and subset.npy (M, 20) hold the rows of all written frames in frame order, and
+    candidate_rows.npy / subset_rows.npy how many rows belong to each of them.  frame_index.npy names the frames of
+    the step that were written: all of them, or a fixed seeded sample when the whole step exceeds DUMP_LIMIT.
+    An array without rows is not written: its row counts, all zero, already say everything it holds (random-init
+    weights find candidates but assemble no person, so subset.npy is usually absent)."""
+    cands = [np.asarray(c, dtype=np.float64).reshape(-1, 4) for c, _ in results]
+    subs = [np.asarray(s, dtype=np.float64).reshape(-1, 20) for _, s in results]
+    n = len(results)
+    keep = np.arange(n)
+    nbytes = np.array([c.nbytes + s.nbytes + 3 * 8 for c, s in zip(cands, subs)])
+    if nbytes.sum() > DUMP_LIMIT:
+        perm = np.random.default_rng(0).permutation(n)
+        keep = np.sort(perm[:np.searchsorted(np.cumsum(nbytes[perm]), DUMP_LIMIT, side="right")])
+    os.makedirs(d, exist_ok=True)
+    arrays = {"candidate": np.concatenate([cands[i] for i in keep] or [np.empty((0, 4))]),
+              "subset": np.concatenate([subs[i] for i in keep] or [np.empty((0, 20))]),
+              "candidate_rows": np.array([len(cands[i]) for i in keep], dtype=np.float64),
+              "subset_rows": np.array([len(subs[i]) for i in keep], dtype=np.float64),
+              "frame_index": keep.astype(np.float64)}
+    for name, a in arrays.items():
+        if a.size:
+            np.save(os.path.join(d, name + ".npy"), a)
 
 
 class ClockSampler(object):
@@ -99,18 +129,19 @@ def measured_peaks():
 
 def cpu_reference_frames(n_frames, threads):
     """The reference's algorithm on the host cores: the oracle's Body.__call__ restatement, torch CPU fp32 convs,
-    cv2 resizes, scipy-exact Gaussian, Python PAF loops vectorised per limb.  Returns seconds per frame list."""
+    cv2 resizes, scipy-exact Gaussian, Python PAF loops vectorised per limb.  Returns the list of seconds per frame
+    and the (candidate, subset) of the last frame."""
     import torch
     from oracle import openpose_oracle as O
     torch.set_num_threads(threads)
     sd = O.make_weights("body", 0)
-    frames = synth_frames(max(n_frames, 1), 123)
-    times = []
+    frames = synth_frames(max(1, min(n_frames, REF_POOL_FRAMES)), 123)
+    times, out = [], None
     for i in range(n_frames):
         t0 = time.perf_counter()
-        O.body_call(frames[i % len(frames)], sd, SCALES, use_cv2=True)
+        out = O.body_call(frames[i % len(frames)], sd, SCALES, use_cv2=True)
         times.append(time.perf_counter() - t0)
-    return times
+    return times, out
 
 
 def run_reference(args):
@@ -118,20 +149,22 @@ def run_reference(args):
     if rank != 0:
         return
     threads = os.cpu_count() or 1
-    warm = min(args.warmup, 1)
-    steps = max(1, min(args.steps, 12))          # one 720p 4-scale frame is ~10 s of CPU work
-    times = cpu_reference_frames(warm + steps, threads)[warm:]
-    sec = float(np.sum(times))
+    warm = min(args.warmup, 1)                   # one 720p 4-scale frame is ~10 s of CPU work
+    steps = args.steps
+    times, last = cpu_reference_frames(warm + steps, threads)
+    sec = float(np.sum(times[warm:]))
     fps = steps / sec
     line = {"metric": METRIC, "value": fps, "unit": "frames/s", "n_gpus": args.gpus, "steps": steps, "warmup": warm,
             "ms_per_step": 1e3 * sec / steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic", "impl": "reference",
             "config": {"workload": "Body() 4-scale [0.5,1.0,1.5,2.0] on synthetic 1280x720 frames, random-init bodypose_model",
-                       "frames_per_step": 1, "note": "steps capped at 12 and warmup at 1: one frame is ~10 s on the host"},
+                       "frames_per_step": 1, "note": "warmup capped at 1: one frame is ~10 s on the host"},
             "cpu_baseline": {"value": fps, "unit": "frames/s", "cores": threads, "kind": "port",
                              "sample": "%d full frames (oracle restatement of src/body.py; the reference checkout is not on the GPU box)" % steps},
             "e2e": {"value": fps, "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [last])
     print(json.dumps(line), flush=True)
 
 
@@ -309,23 +342,24 @@ def run_ours(args):
     assert F % B == 0 and POOL_FRAMES % B == 0, "frames-per-step and the frame pool must be multiples of --batch"
 
     def step(step_idx, device_resident):
-        """F frames as F/B batches of B consecutive pool frames, round-robin over the sessions (streams)."""
-        inflight = [False] * len(sessions)
-        out = None
+        """F frames as F/B batches of B consecutive pool frames, round-robin over the sessions (streams).
+        Returns the (candidate, subset) of every frame, in frame order."""
+        pending = [None] * len(sessions)             # batch in flight on each session
+        results = [None] * (F // B)
         for b in range(F // B):
             si = b % len(sessions)
-            if inflight[si]:
-                out = body.collect_batch(sessions[si])
+            if pending[si] is not None:
+                results[pending[si]] = body.collect_batch(sessions[si])
             idx = (step_idx * F + b * B) % POOL_FRAMES
             if device_resident:
                 body.submit_batch((frames_dev[idx].data_ptr(), (B, H, W)), sessions[si], where=1)
             else:
                 body.submit_batch(host_np[idx:idx + B], sessions[si], where=2)
-            inflight[si] = True
-        for si, fl in enumerate(inflight):
-            if fl:
-                out = body.collect_batch(sessions[si])
-        return out
+            pending[si] = b
+        for si, b in enumerate(pending):
+            if b is not None:
+                results[b] = body.collect_batch(sessions[si])
+        return [r for batch in results for r in batch]
 
     def timed(device_resident):
         for w in range(Wm):
@@ -334,21 +368,21 @@ def run_ours(args):
         l0 = _lib.launch_count(local)
         sessions[0].mark(0)
         for k in range(K):
-            step(Wm + k, device_resident)
+            out = step(Wm + k, device_resident)
         for s in sessions:
             s.mark(1)
         torch.cuda.synchronize()
         ms = max(sessions[0].elapsed_ms(0, s, 1) for s in sessions)
         launches = _lib.launch_count(local) - l0
         barrier()
-        return max_over_ranks(ms), launches
+        return max_over_ranks(ms), launches, out
 
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms_dev, launches = timed(True)
+    ms_dev, launches, last = timed(True)
     clocks = sampler.stop() if rank == 0 else None
-    ms_e2e, _ = timed(False)
+    ms_e2e, _, _ = timed(False)
 
     # ---- roofline of the dominant kernel (tcgen05 implicit-GEMM conv), serialised profiled frames ----
     roof = None
@@ -420,7 +454,7 @@ def run_ours(args):
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:        # reported at N=1 only
         threads = os.cpu_count() or 1
-        t = cpu_reference_frames(2, threads)
+        t, _ = cpu_reference_frames(2, threads)
         cpu = {"value": 2.0 / float(np.sum(t)), "unit": "frames/s", "cores": threads, "kind": "port",
                "sample": "2 full 720p 4-scale frames through the oracle restatement of src/body.py (no warm-up)"}
 
@@ -479,6 +513,8 @@ def run_ours(args):
                            "note": "PAF values are sampled on demand (10 samples x 2 channels per candidate pair) from the net "
                                    "outputs: the 140 MB of full-resolution PAF planes per frame are never written"}
         line["stage_roofline"] = sr
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -497,7 +533,12 @@ def main():
     ap.add_argument("--no-grouping", action="store_true", help="skip the PAF-grouping leg (50-person scene)")
     ap.add_argument("--no-extras", action="store_true", help="skip the config-3 / config-4 / decode-inclusive legs")
     ap.add_argument("--layers", default=None, help="write the per-launch profile of one frame to this CSV")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the results of the last timed step to DIR/<name>.npy (float64, at most 64 MB; "
+                         "arrays without rows are left out)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -9,7 +9,7 @@ import pytest
 from oracle import reference_loader as RL
 from pytorch_openpose_b200 import extract as E
 
-live = pytest.mark.skipif(not RL.available(), reason="reference checkout not present")
+live = pytest.mark.skipif(not RL.available(), reason="needs a checkout of the original project (set OPENPOSE_REFERENCE_ROOT)")
 REC = [(20, 10), (150, 110)]                      # ROI [(x0, y0), (x1, y1)]
 
 

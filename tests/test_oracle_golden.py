@@ -5,7 +5,18 @@ import pytest
 import torch
 
 from oracle import openpose_oracle as O
-from oracle.make_golden import smooth_noise_maps
+from oracle.make_golden import THREADS, smooth_noise_maps
+
+
+@pytest.fixture(autouse=True, scope="module")
+def recorded_thread_count():
+    """oneDNN partitions the fp32 convolutions by the intra-op thread count, which reorders their sums and changes the
+    last bits of the network outputs: the oracle computes with the count the fixtures were recorded with
+    (make_golden.THREADS), whatever the host's core count."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(THREADS)
+    yield
+    torch.set_num_threads(n)
 
 
 def test_network_matches_reference_modules(golden):

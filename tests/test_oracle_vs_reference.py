@@ -7,7 +7,7 @@ import torch
 from oracle import openpose_oracle as O
 from oracle import reference_loader as RL
 
-pytestmark = pytest.mark.skipif(not RL.available(), reason="reference checkout not present")
+pytestmark = pytest.mark.skipif(not RL.available(), reason="needs a checkout of the original project (set OPENPOSE_REFERENCE_ROOT)")
 
 
 def test_weights_follow_reference_rng_stream():

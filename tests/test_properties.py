@@ -10,7 +10,7 @@ from oracle import openpose_oracle as O
 from oracle import reference_loader as RL
 from pytorch_openpose_b200 import util
 
-live = pytest.mark.skipif(not RL.available(), reason="reference checkout not present")
+live = pytest.mark.skipif(not RL.available(), reason="needs a checkout of the original project (set OPENPOSE_REFERENCE_ROOT)")
 
 
 @settings(max_examples=40, deadline=None)

@@ -157,6 +157,27 @@ int opb_batch_hand_submit(opb_session* s, const float* crops, int where, int n_c
 int opb_batch_body_submit_u8(opb_session* s, const uint8_t* frames_hwc, int where, int n_frames, int height, int width,
                              double g_scale);
 int opb_batch_hand_submit_u8(opb_session* s, const uint8_t* crops_hwc, int where, int n_crops, int height, int width);
+/* ---- Batch_hand_extraction (srcmx/Batch_motion_Estimation.py:19-63) on the device --------------------------------
+ * For n_frames ROI-cropped frames (n, height, width, 3) uint8 and their saved body poses (host, n x 18 x 3 float64, the
+ * track Batch_body_extraction writes): both hand boxes of every pose (HandImageDataset.__getitem__,
+ * srcmx/Batch_model.py:68-104 -- a joint is missing when x + y + score == 0, util.handDetect on the one person), the
+ * crops cv2.resize(crop, (boxsize, boxsize), INTER_CUBIC), the left one mirrored, a uniform 128 image where a hand is
+ * missing, Batch_hand on all 2n crops (as opb_batch_hand_submit_u8), and the key points moved back to ROI coordinates
+ * (Batch_motion_Estimation.py:41-56).  `where`: 0 pageable host, 1 device, 2 pinned host.  2 * n_frames <= 1024;
+ * boxsize a multiple of 8.  A box of width <= 0 (the reference's cv2.resize raises on it) counts as a missing hand.
+ * wait: HandMat n x 42 x 3 float64 (rows 0-20 left hand, 21-41 right hand; a coordinate of exactly 0 means "missing"
+ * -- a missing hand keeps the scores Batch_hand finds on its grey crop).  hand_s must not be used by other calls
+ * while a batch is in flight.                                                                             */
+int opb_hand_track_submit(opb_session* hand_s, const uint8_t* frames_bgr, int where, int n_frames, int height, int width,
+                          const double* host_poses, int boxsize);
+int opb_hand_track_wait(opb_session* hand_s, double* hand_mats);
+/* the 2n crops of the last hand-track batch, (2n, boxsize, boxsize, 3) uint8, slot 2f the left hand of frame f (parity
+ * tests); valid until the session runs other work.                                                   */
+int opb_hand_track_crops(opb_session* hand_s, uint8_t* host_crops);
+/* Host only (no device call): the two boxes of one pose (pose54 = 18 x 3) in a height x width frame, computed by the
+ * same function as the device -- boxes8 = [left, right] x [x, y, w, valid]; (0, 0, 0, 0) when a joint is missing.  */
+int opb_hand_track_boxes(const double* pose54, int height, int width, int* boxes8);
+
 /* blurred heat maps of the last batched-estimator call: (n, 19 | 22, height, width) planar fp32; the
  * un-blurred maps and the PAFs come from opb_body_maps / opb_hand_maps.                             */
 int opb_batch_maps(opb_session* s, float* host_blurred_heat);
@@ -225,8 +246,11 @@ int opb_wide_pool_weights(const float* weight, const float* bias, unsigned short
  *   clamped when used; 4 float32 coefficients per destination index) -- src/body.py:38,55,57.
  * opb_debug_composite_taps: the per-axis operator of "x8 cubic upsample, crop to n_resized, cubic resize to n_orig"
  *   (src/body.py:55-57) as first source index + 6 float32 weights per destination index.
- * opb_debug_resize_dsize: cv2's destination size for a scale factor (round half to even).                            */
+ * opb_debug_resize_dsize: cv2's destination size for a scale factor (round half to even).
+ * opb_debug_hand_track_taps: the taps opb_hand_track_submit's tables hold for a side x side crop resized to boxsize
+ *   (boxsize entries of first / coef4).                                                                             */
 int opb_debug_resize_taps(int src, int dst, double scale, int* first, float* coef4);
+int opb_debug_hand_track_taps(int side, int boxsize, int* first, float* coef4);
 int opb_debug_composite_taps(int n_net, int n_resized, int n_orig, int* first, float* w6);
 int opb_debug_resize_dsize(int n, double f);
 

@@ -22,6 +22,24 @@ def _as_frames_u8(frames, where):
     return arr.ctypes.data, arr, arr.shape[:3]
 
 
+def _as_track_frames(frames, where):
+    """-> (pointer, where, keepalive, (B, h, w)) of (B, h, w, 3) uint8 frames: torch CUDA tensors are read in place
+    (where=1), pinned CPU tensors straight from their pages (where=2); anything else as `where` says."""
+    if hasattr(frames, "detach"):
+        import torch
+        t = frames.detach()
+        if t.is_cuda or t.is_pinned():
+            if t.dtype != torch.uint8 or t.dim() != 4 or t.shape[3] != 3:
+                raise ValueError("expected (B, h, w, 3) uint8 frames")
+            t = t.contiguous()
+            if t.is_cuda:
+                torch.cuda.current_stream(t.device).synchronize()       # producer work is on torch's stream
+            return t.data_ptr(), (1 if t.is_cuda else 2), t, tuple(t.shape[:3])
+        frames = t.numpy()
+    ptr, keep, shape = _as_frames_u8(frames, where)
+    return ptr, where, keep, shape
+
+
 def _as_float_batch(batch):
     """-> (pointer, where, keepalive, shape).  torch CUDA tensors are read in place (where=1), pinned CPU tensors are
     copied straight from their pages (where=2); anything else goes through the library's pinned staging buffer."""
@@ -128,6 +146,45 @@ class Batch_hand(object):
         peaks = np.empty((s._n, 21, 3), dtype=np.float64)
         _lib.check(_lib.lib().opb_hand_wait(s.handle, peaks.ctypes.data))
         return peaks
+
+    TRACK_BATCH = MAX_BATCH // 2                      # frames per track submit: two crops each
+
+    def submit_track(self, frames_u8, poses, session=None, where=0, boxsize=368):
+        """One batch of `Batch_hand_extraction` (srcmx/Batch_motion_Estimation.py:19-63) on the device: ROI-cropped
+        (B, h, w, 3) uint8 frames and their saved (B, 18, 3) body poses -> both hand crops of every frame
+        (`extract.hand_crops_from_pose`), Batch_hand on them and the key points back in ROI coordinates
+        (`collect_track`).  where: 0 pageable, 1 device (a CUDA tensor is always read in place), 2 pinned."""
+        s = session or self._session
+        ptr, where, keep, (B, h, w) = _as_track_frames(frames_u8, where)
+        p = np.ascontiguousarray(poses, dtype=np.float64)
+        if p.shape != (B, 18, 3):
+            raise ValueError("expected (%d, 18, 3) poses for %d frames, got %s" % (B, B, p.shape))
+        if boxsize % 8:
+            raise ValueError("boxsize must be a multiple of 8 (srcmx/Batch_model.py:377)")
+        s._keepalive, s._track_n, s._track_box = (keep, p), B, int(boxsize)
+        _lib.check(_lib.lib().opb_hand_track_submit(s.handle, ptr, where, B, h, w, p.ctypes.data, int(boxsize)))
+
+    def collect_track(self, session=None):
+        """HandMat (B, 42, 3) float64 of the last `submit_track`: rows 0-20 left hand, 21-41 right hand."""
+        s = session or self._session
+        mats = np.empty((s._track_n, 42, 3), dtype=np.float64)
+        _lib.check(_lib.lib().opb_hand_track_wait(s.handle, mats.ctypes.data))
+        return mats
+
+    def track_crops(self, session=None):
+        """The (2B, boxsize, boxsize, 3) uint8 crops of the last `submit_track` (slot 2f: left hand of frame f)."""
+        s = session or self._session
+        crops = np.empty((2 * s._track_n, s._track_box, s._track_box, 3), dtype=np.uint8)
+        _lib.check(_lib.lib().opb_hand_track_crops(s.handle, crops.ctypes.data))
+        return crops
+
+    def track(self, frames, poses, boxsize=368):
+        """HandMat (B, 42, 3) of `Batch_hand_extraction` for frames (B, h, w, 3) uint8 and poses (B, 18, 3)."""
+        out = []
+        for lo in range(0, len(frames), self.TRACK_BATCH):
+            self.submit_track(frames[lo:lo + self.TRACK_BATCH], poses[lo:lo + self.TRACK_BATCH], boxsize=boxsize)
+            out.append(self.collect_track())
+        return np.concatenate(out, 0)
 
     def __call__(self, batch_imgs):
         out = []

@@ -83,24 +83,27 @@ struct U8Taps {
     short *xc, *yc;
     void relocate_to(uint8_t* b) { relocate(xf, b); relocate(yf, b); relocate(xc, b); relocate(yc, b); }
 };
+static std::vector<short> u8_coefs(const CubicTaps& t) {
+    std::vector<short> out(t.coef.size());
+    for (size_t i = 0; i < t.coef.size(); ++i) {
+        long v = lrintf(t.coef[i] * 2048.0f);           // saturate_cast<short>(coef * INTER_RESIZE_COEF_SCALE)
+        out[i] = (short)std::max(-32768l, std::min(32767l, v));
+    }
+    return out;
+}
 static U8Taps make_u8_taps(TableSlab& pool, int H, int W, const ScaleDims& d) {
-    auto conv = [&](const CubicTaps& t, std::vector<short>& out) {
-        out.resize(t.coef.size());
-        for (size_t i = 0; i < t.coef.size(); ++i) {
-            long v = lrintf(t.coef[i] * 2048.0f);       // saturate_cast<short>(coef * INTER_RESIZE_COEF_SCALE)
-            out[i] = (short)std::max(-32768l, std::min(32767l, v));
-        }
-    };
     const CubicTaps tx = cubic_taps(W, d.w, 1.0 / d.mult), ty = cubic_taps(H, d.h, 1.0 / d.mult);
-    std::vector<short> sx, sy;
-    conv(tx, sx);
-    conv(ty, sy);
     U8Taps u;
     u.xf = pool.add(tx.first);
     u.yf = pool.add(ty.first);
-    u.xc = pool.add(sx);
-    u.yc = pool.add(sy);
+    u.xc = pool.add(u8_coefs(tx));
+    u.yc = pool.add(u8_coefs(ty));
     return u;
+}
+// cv2.resize(crop, (boxsize, boxsize), INTER_CUBIC) of a side x side crop (srcmx/Batch_model.py:96-101): dsize mode,
+// inverse scale (double)boxsize / side, step = 1 / inverse scale
+static CubicTaps hand_track_taps(int side, int boxsize) {
+    return cubic_taps(side, boxsize, 1.0 / ((double)boxsize / side));
 }
 
 // Batch_body.calculate_size_pad (srcmx/Batch_model.py:340-345): truncating sizes, one scale; Batch_hand: no resize
@@ -243,9 +246,14 @@ struct FramePlan {
     cudaGraphExec_t pose_graph = nullptr;
     uint64_t pose_gen = 0;
     int pose_uses = 0;
+    // the same for the hand-track sequence of opb_hand_track_submit (a uint8 Batch_hand plan fed by the crop kernel)
+    cudaGraphExec_t track_graph = nullptr;
+    uint64_t track_gen = 0;
+    int track_uses = 0;
     ~FramePlan() {
         if (graph) cudaGraphExecDestroy(graph);
         if (pose_graph) cudaGraphExecDestroy(pose_graph);
+        if (track_graph) cudaGraphExecDestroy(track_graph);
     }
     std::vector<ScaleDims> dims;
     std::vector<U8Taps> u8taps;
@@ -374,6 +382,30 @@ struct opb_session {
         }
     };
     std::unique_ptr<PoseBuffers> pose;
+    // the batched hand job on saved poses (opb_hand_track_*), on a hand session: tap tables of every crop side for one
+    // boxsize, and per-batch buffers grown to the largest batch / frame seen
+    struct HandTrack {
+        DevPool table_pool;
+        RaggedTables tabs{};         // one "scale": crop side -> boxsize, preprocess entries only
+        int boxsize = 0;
+        DevPool pool, frame_pool;
+        int frames = 0;              // capacity of the per-frame buffers
+        size_t frame_bytes = 0;      // capacity of `frames_dev`
+        uint8_t* frames_dev = nullptr;   // the decoded (ROI-cropped) frames of the batch
+        double* poses = nullptr;     // [frames][18][3]
+        HandBox* boxes = nullptr;    // [frames][2]
+        double* mats = nullptr;      // [frames][42][3]
+        double* poses_host = nullptr;   // pinned
+        double* mats_host = nullptr;    // pinned
+        uint64_t gen = 1;            // bumped whenever a buffer, the tables or the frame size change
+        int H = 0, W = 0, n = 0;     // last batch
+        FramePlan* plan = nullptr;   // uint8 Batch_hand plan of the last batch (its input buffer holds the crops)
+        ~HandTrack() {
+            if (poses_host) cudaFreeHost(poses_host);
+            if (mats_host) cudaFreeHost(mats_host);
+        }
+    };
+    std::unique_ptr<HandTrack> track;
     opb_session* pose_hand = nullptr;    // hand session of the pose batch in flight
     std::vector<double> pose_hand_scales;
     bool pose_fixed = false;
@@ -616,17 +648,20 @@ static void run_or_replay(opb_session* s, FramePlan* fp, F&& enqueue) {
     run_or_replay_slot(s, GraphSlot{fp->graph, fp->graph_gen, fp->uses}, s->buffer_gen, enqueue);
 }
 
-static void upload_image(opb_session* s, FramePlan* fp, const uint8_t* img, int where, size_t bytes) {
+static void upload_bytes(opb_session* s, void* dst, const void* img, int where, size_t bytes) {
     if (where == 1) {                                    // already on the device
-        OPB_CUDA(cudaMemcpyAsync(fp->d_img, img, bytes, cudaMemcpyDeviceToDevice, s->stream));
+        OPB_CUDA(cudaMemcpyAsync(dst, img, bytes, cudaMemcpyDeviceToDevice, s->stream));
     } else if (where == 2) {                             // caller-owned pinned host memory
-        OPB_CUDA(cudaMemcpyAsync(fp->d_img, img, bytes, cudaMemcpyHostToDevice, s->stream));
+        OPB_CUDA(cudaMemcpyAsync(dst, img, bytes, cudaMemcpyHostToDevice, s->stream));
     } else {                                             // pageable host memory: stage through pinned
         ensure_staging(s, bytes);
         OPB_CUDA(cudaStreamSynchronize(s->stream));      // staging buffer may still feed the previous frame
         memcpy(s->staging, img, bytes);
-        OPB_CUDA(cudaMemcpyAsync(fp->d_img, s->staging, bytes, cudaMemcpyHostToDevice, s->stream));
+        OPB_CUDA(cudaMemcpyAsync(dst, s->staging, bytes, cudaMemcpyHostToDevice, s->stream));
     }
+}
+static void upload_image(opb_session* s, FramePlan* fp, const uint8_t* img, int where, size_t bytes) {
+    upload_bytes(s, fp->d_img, img, where, bytes);
 }
 
 static void run_front(opb_session* s, FramePlan* fp, int n, int H, int W) {
@@ -917,7 +952,19 @@ static void hand_submit(opb_session* s, const uint8_t* img, int where, int n, in
     finish_submit(s, fp);
 }
 
-// Batch_hand.__call__ (srcmx/Batch_model.py:366-406)
+// Batch_hand.__call__ (srcmx/Batch_model.py:366-406) on the crops already in the plan's input buffer: peaks of every
+// crop in fp->hb.peaks
+static void batch_hand_enqueue(opb_session* s, FramePlan* fp, int n, int H, int W) {
+    cudaStream_t st = s->stream;
+    run_front_f32(s, fp, n, H, W);
+    run_upsample(fp, false, n, 22, 24, H, W, fp->heat_avg, st);                                    // x8 bicubic, :377
+    s->prof.mark(st, "upsample_avg");
+    blur5_planar_launch(fp->heat_avg, fp->blurred, n * 22, H, W, st);                                     // :378
+    s->prof.mark(st, "blur5");
+    hand_peaks_blurred_launch(fp->blurred, n, 22, H, W, 0.035f, fp->hb, st);                       // thre, :361
+    s->prof.mark(st, "hand_peaks");
+}
+
 static void batch_hand_submit(opb_session* s, const void* crops, bool u8, int where, int n, int H, int W) {
     OPB_REQUIRE(s->net->kind == OPB_NET_HAND, "session was created on a body network");
     OPB_REQUIRE(n >= 1 && n <= 1024, "1..1024 crops per batch");
@@ -933,17 +980,97 @@ static void batch_hand_submit(opb_session* s, const void* crops, bool u8, int wh
     upload_image(s, fp, (const uint8_t*)crops, where, (size_t)n * H * W * 3 * (u8 ? 1 : sizeof(float)));
     s->prof.mark(st, "h2d");
     run_or_replay(s, fp, [&] {
-        run_front_f32(s, fp, n, H, W);
-        run_upsample(fp, false, n, 22, 24, H, W, fp->heat_avg, st);                                // x8 bicubic, :377
-        s->prof.mark(st, "upsample_avg");
-        blur5_planar_launch(fp->heat_avg, fp->blurred, n * 22, H, W, st);                                 // :378
-        s->prof.mark(st, "blur5");
-        hand_peaks_blurred_launch(fp->blurred, n, 22, H, W, 0.035f, fp->hb, st);                   // thre, :361
-        s->prof.mark(st, "hand_peaks");
+        batch_hand_enqueue(s, fp, n, H, W);
         OPB_CUDA(cudaMemcpyAsync(s->hand_host, fp->hb.peaks, (size_t)n * 63 * sizeof(double), cudaMemcpyDeviceToHost, st));
         s->prof.mark(st, "d2h");
     });
     finish_submit(s, fp);
+}
+
+// ------------------------------------------------------------------------------------------------
+// the batched hand job on the device: Batch_hand_extraction, srcmx/Batch_motion_Estimation.py:19-63
+// ------------------------------------------------------------------------------------------------
+// Tap tables of cv2.resize(crop, (boxsize, boxsize), INTER_CUBIC) for every crop side 1..wmax, in the RaggedTables layout
+// of the pose pipeline with one scale (only the preprocess entries are filled: the upsample runs on boxsize-square maps).
+static void build_track_tables(opb_session::HandTrack& t, int boxsize, int wmax) {
+    TableSlab slab;
+    std::vector<unsigned> index((size_t)(wmax + 1) * 5, 0u);
+    for (int w = 1; w <= wmax; ++w) {
+        const CubicTaps taps = hand_track_taps(w, boxsize);
+        index[(size_t)w * 5 + 0] = (unsigned)(size_t)slab.add(taps.first);
+        index[(size_t)w * 5 + 1] = (unsigned)(size_t)slab.add(u8_coefs(taps));
+    }
+    OPB_REQUIRE(slab.host.size() < (1ull << 32), "hand-track tables exceed 4 GB");
+    t.table_pool.release();
+    uint8_t* dev = (uint8_t*)t.table_pool.alloc(slab.host.size());
+    OPB_CUDA(cudaMemcpy(dev, slab.host.data(), slab.host.size(), cudaMemcpyHostToDevice));
+    t.tabs.slab = dev;
+    t.tabs.index = t.table_pool.upload(index);
+    t.tabs.n_scales = 1;
+    t.tabs.wmax = wmax;
+    t.boxsize = boxsize;
+    ++t.gen;
+}
+
+static void hand_track_submit(opb_session* s, const uint8_t* frames, int where, int n, int H, int W, const double* poses,
+                              int boxsize) {
+    OPB_REQUIRE(s->net->kind == OPB_NET_HAND, "session was created on a body network");
+    OPB_REQUIRE(n >= 1 && 2 * n <= 1024, "1..512 frames per batch (two crops each)");
+    OPB_REQUIRE(H >= 1 && W >= 1, "empty frame");
+    OPB_REQUIRE(boxsize >= 8 && boxsize % 8 == 0, "boxsize must be a positive multiple of 8 (srcmx/Batch_model.py:377)");
+    OPB_CUDA(cudaSetDevice(s->net->ctx->device));
+    cudaStream_t st = s->stream;
+    OPB_CUDA(cudaStreamSynchronize(st));          // the pinned buffers and the tables may still serve the previous batch
+    if (!s->track) s->track = std::make_unique<opb_session::HandTrack>();
+    opb_session::HandTrack& t = *s->track;
+    const int wmax = std::min(H, W);
+    if (t.boxsize != boxsize || t.tabs.wmax < wmax) build_track_tables(t, boxsize, wmax);
+    if (t.frames < n) {
+        t.pool.release();
+        if (t.poses_host) cudaFreeHost(t.poses_host);
+        if (t.mats_host) cudaFreeHost(t.mats_host);
+        t.poses_host = t.mats_host = nullptr;
+        t.frames = 0;
+        t.poses = t.pool.alloc_t<double>((size_t)n * 54);
+        t.boxes = t.pool.alloc_t<HandBox>((size_t)n * 2);
+        t.mats = t.pool.alloc_t<double>((size_t)n * 126);
+        OPB_CUDA(cudaMallocHost((void**)&t.poses_host, (size_t)n * 54 * sizeof(double)));
+        OPB_CUDA(cudaMallocHost((void**)&t.mats_host, (size_t)n * 126 * sizeof(double)));
+        t.frames = n;
+        ++t.gen;
+    }
+    const size_t bytes = (size_t)n * H * W * 3;
+    if (t.frame_bytes < bytes) {
+        t.frame_pool.release();
+        t.frames_dev = (uint8_t*)t.frame_pool.alloc(bytes);
+        t.frame_bytes = bytes;
+        ++t.gen;
+    }
+    if (t.H != H || t.W != W) ++t.gen;           // the captured launches carry the frame size
+    t.H = H;
+    t.W = W;
+    t.n = n;
+    memcpy(t.poses_host, poses, (size_t)n * 54 * sizeof(double));
+    // the crops go straight into the input buffer of the uint8 Batch_hand plan of 2n boxsize-square crops
+    const int slots = 2 * n;
+    const double one = 1.0;
+    FramePlan* fp = get_plan(s, slots, boxsize, boxsize, &one, 1, 2);
+    s->active = fp;
+    s->hand_crops = slots;
+    t.plan = fp;
+    s->prof.reset();
+    upload_bytes(s, t.frames_dev, frames, where, bytes);
+    const uint64_t gen = (s->buffer_gen << 32) ^ t.gen;
+    run_or_replay_slot(s, GraphSlot{fp->track_graph, fp->track_gen, fp->track_uses}, gen, [&] {
+        OPB_CUDA(cudaMemcpyAsync(t.poses, t.poses_host, (size_t)n * 54 * sizeof(double), cudaMemcpyHostToDevice, st));
+        hand_track_boxes_launch(t.poses, n, H, W, t.boxes, st);
+        preprocess_ragged_launch(t.frames_dev, H, W, t.boxes, slots, fp->d_img, boxsize, 0, t.tabs, st);
+        batch_hand_enqueue(s, fp, slots, boxsize, boxsize);
+        hand_track_finish_launch(t.boxes, fp->hb.peaks, n, boxsize, t.mats, st);
+        OPB_CUDA(cudaMemcpyAsync(t.mats_host, t.mats, (size_t)n * 126 * sizeof(double), cudaMemcpyDeviceToHost, st));
+    });
+    OPB_CUDA(cudaEventRecord(s->done, st));
+    s->net->ctx->launches += 3 /* boxes, crops, finish */ + fp->launches_per_frame;
 }
 
 
@@ -1350,6 +1477,54 @@ int opb_batch_maps(opb_session* s, float* host_blurred_heat) {
         }
         OPB_CUDA(cudaMemcpyAsync(host_blurred_heat, fp->blurred, px * C * 4, cudaMemcpyDeviceToHost, s->stream));
         OPB_CUDA(cudaStreamSynchronize(s->stream));
+    });
+}
+
+/* ---- the batched hand job on the device ------------------------------------------------------------------------- */
+int opb_hand_track_submit(opb_session* hand_s, const uint8_t* frames_bgr, int where, int n_frames, int height, int width,
+                          const double* host_poses, int boxsize) {
+    return guarded([&] {
+        OPB_REQUIRE(hand_s && frames_bgr && host_poses, "null argument");
+        OPB_REQUIRE(where >= 0 && where <= 2, "where: 0 pageable host, 1 device, 2 pinned host");
+        hand_track_submit(hand_s, frames_bgr, where, n_frames, height, width, host_poses, boxsize);
+    });
+}
+int opb_hand_track_wait(opb_session* hand_s, double* hand_mats) {
+    return guarded([&] {
+        OPB_REQUIRE(hand_s && hand_mats && hand_s->track && hand_s->track->n > 0, "no hand-track batch in flight");
+        OPB_CUDA(cudaEventSynchronize(hand_s->done));
+        memcpy(hand_mats, hand_s->track->mats_host, (size_t)hand_s->track->n * 126 * sizeof(double));
+    });
+}
+int opb_hand_track_crops(opb_session* hand_s, uint8_t* host_crops) {
+    return guarded([&] {
+        OPB_REQUIRE(hand_s && host_crops && hand_s->track && hand_s->track->plan && hand_s->active == hand_s->track->plan,
+                    "the session's last batch was not a hand-track batch");
+        OPB_CUDA(cudaSetDevice(hand_s->net->ctx->device));
+        OPB_CUDA(cudaEventSynchronize(hand_s->done));
+        const FramePlan* fp = hand_s->track->plan;
+        OPB_CUDA(cudaMemcpy(host_crops, fp->d_img, (size_t)fp->key.n * fp->key.H * fp->key.W * 3, cudaMemcpyDeviceToHost));
+    });
+}
+int opb_hand_track_boxes(const double* pose54, int height, int width, int* boxes8) {
+    return guarded([&] {
+        OPB_REQUIRE(pose54 && boxes8 && height >= 1 && width >= 1, "opb_hand_track_boxes: bad argument");
+        HandBox hb[2];
+        hand_track_boxes_host(pose54, height, width, hb);
+        for (int k = 0; k < 2; ++k) {
+            boxes8[k * 4 + 0] = hb[k].x;
+            boxes8[k * 4 + 1] = hb[k].y;
+            boxes8[k * 4 + 2] = hb[k].w;
+            boxes8[k * 4 + 3] = hb[k].valid;
+        }
+    });
+}
+int opb_debug_hand_track_taps(int side, int boxsize, int* first, float* coef4) {
+    return guarded([&] {
+        OPB_REQUIRE(first && coef4 && side >= 1 && boxsize >= 1, "opb_debug_hand_track_taps: bad argument");
+        const CubicTaps t = hand_track_taps(side, boxsize);
+        memcpy(first, t.first.data(), sizeof(int) * boxsize);
+        memcpy(coef4, t.coef.data(), sizeof(float) * 4 * boxsize);
     });
 }
 

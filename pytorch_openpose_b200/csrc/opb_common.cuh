@@ -295,6 +295,65 @@ struct HandBox {
     int left;                 // left hand: the crop is mirrored before the network, x un-mirrored afterwards
     int valid;                // 0: no box for this slot (no person, missing joints, empty box)
 };
+// float64 operations rounded once each, on the device and on the host (the units that include this file and call the
+// functions below are built without FMA contraction: --fmad=false on the device, baseline x86-64 on the host)
+__host__ __device__ inline double dadd_rn(double a, double b) {
+#ifdef __CUDA_ARCH__
+    return __dadd_rn(a, b);
+#else
+    return a + b;
+#endif
+}
+__host__ __device__ inline double dmul_rn(double a, double b) {
+#ifdef __CUDA_ARCH__
+    return __dmul_rn(a, b);
+#else
+    return a * b;
+#endif
+}
+// util.handDetect (src/util.py:133-201) for one arm of one person: shoulder (x1, y1), elbow (x2, y2), wrist (x3, y3) in
+// an H x W image -> square box (x, y, w); valid = w > 0 (the reference's crop of an empty box raises)
+__host__ __device__ inline void hand_detect_box(double x1, double y1, double x2, double y2, double x3, double y3, int H, int W,
+                                                HandBox& b) {
+    double x = dadd_rn(x3, dmul_rn(0.33, x3 - x2));
+    double y = dadd_rn(y3, dmul_rn(0.33, y3 - y2));
+    const double dwe = sqrt(dadd_rn(dmul_rn(x3 - x2, x3 - x2), dmul_rn(y3 - y2, y3 - y2)));
+    const double des = sqrt(dadd_rn(dmul_rn(x2 - x1, x2 - x1), dmul_rn(y2 - y1, y2 - y1)));
+    const double m = dmul_rn(0.9, des);
+    double width = dmul_rn(1.5, dwe > m ? dwe : m);          // max(a, b): a if a > b ... Python's max keeps the first on ties
+    x = dadd_rn(x, -(width / 2));
+    y = dadd_rn(y, -(width / 2));
+    if (x < 0) x = 0;
+    if (y < 0) y = 0;
+    double w1 = width, w2 = width;
+    if (dadd_rn(x, width) > (double)W) w1 = (double)W - x;
+    if (dadd_rn(y, width) > (double)H) w2 = (double)H - y;
+    width = w2 < w1 ? w2 : w1;                                 // min(width1, width2)
+    b.x = (int)x;
+    b.y = (int)y;
+    b.w = (int)width;
+    b.valid = b.w > 0;
+}
+// HandImageDataset.__getitem__ (srcmx/Batch_model.py:68-104) on a saved (18, 3) pose: joint i is missing when Python's
+// sum(pose[i, :]) -- 0 + x + y + score -- is 0; boxes[0] = left hand (joints 5, 6, 7), boxes[1] = right hand (2, 3, 4).
+// A hand with a missing joint gets the box (0, 0, 0), invalid.
+__host__ __device__ inline void pose_hand_boxes(const double* pose, int frame, int H, int W, HandBox* boxes) {
+    for (int k = 0; k < 2; ++k) {
+        HandBox& b = boxes[k];
+        b.frame = frame;
+        b.x = b.y = b.w = 0;
+        b.left = k == 0;
+        b.valid = 0;
+        const int j0 = k == 0 ? 5 : 2;
+        bool present = true;
+        for (int j = j0; j < j0 + 3; ++j)
+            present = present && dadd_rn(dadd_rn(dadd_rn(0.0, pose[j * 3]), pose[j * 3 + 1]), pose[j * 3 + 2]) != 0.0;
+        if (present)
+            hand_detect_box(pose[j0 * 3], pose[j0 * 3 + 1], pose[(j0 + 1) * 3], pose[(j0 + 1) * 3 + 1], pose[(j0 + 2) * 3],
+                            pose[(j0 + 2) * 3 + 1], H, W, b);
+    }
+}
+
 struct RaggedTables {
     const uint8_t* slab;      // all tables
     const unsigned* index;    // [(w * n_scales + s) * 5 + {0: pre first, 1: pre coef, 2: up first, 3: up x weights, 4: up y weights}] byte offsets
@@ -312,6 +371,11 @@ void pose_select_launch(const FramePost* frames_dev, int n_frames, int H, int W,
                         HandBox* boxes_dev, int* dims_dev, cudaStream_t stream);
 void pose_finish_launch(const HandBox* boxes_dev, const double* hand_peaks_dev, int n_frames, double* pose_dev,
                         cudaStream_t stream);
+// the batched hand job on saved poses (pose.cu): boxes (2 per frame, left first) and HandMat (n x 42 x 3) assembly
+void hand_track_boxes_launch(const double* poses_dev, int n_frames, int H, int W, HandBox* boxes_dev, cudaStream_t stream);
+void hand_track_boxes_host(const double* pose, int H, int W, HandBox* boxes);      // the same function on the host
+void hand_track_finish_launch(const HandBox* boxes_dev, const double* hand_peaks_dev, int n_frames, int boxsize,
+                              double* mats_dev, cudaStream_t stream);
 
 // ---- gaussian taps shared by peaks.cu / hand.cu: scipy.ndimage.gaussian_filter(sigma=3) uses
 // radius int(4*3+0.5) = 12 and weights exp(-x^2/18) / sum (src/body.py:75, src/hand.py:62).  The

@@ -61,24 +61,8 @@ __global__ void pose_select_kernel(const FramePost* __restrict__ frames, int n_f
             const double x1 = cand[(size_t)is * 4], y1 = cand[(size_t)is * 4 + 1];
             const double x2 = cand[(size_t)ie * 4], y2 = cand[(size_t)ie * 4 + 1];
             const double x3 = cand[(size_t)iw * 4], y3 = cand[(size_t)iw * 4 + 1];
-            double x = __dadd_rn(x3, __dmul_rn(0.33, x3 - x2));
-            double y = __dadd_rn(y3, __dmul_rn(0.33, y3 - y2));
-            const double dwe = sqrt(__dadd_rn(__dmul_rn(x3 - x2, x3 - x2), __dmul_rn(y3 - y2, y3 - y2)));
-            const double des = sqrt(__dadd_rn(__dmul_rn(x2 - x1, x2 - x1), __dmul_rn(y2 - y1, y2 - y1)));
-            const double m = __dmul_rn(0.9, des);
-            double width = __dmul_rn(1.5, dwe > m ? dwe : m);          // max(a, b): a if a > b ... Python's max keeps the first on ties
-            x = __dadd_rn(x, -(width / 2));
-            y = __dadd_rn(y, -(width / 2));
-            if (x < 0) x = 0;
-            if (y < 0) y = 0;
-            double w1 = width, w2 = width;
-            if (__dadd_rn(x, width) > (double)W) w1 = (double)W - x;
-            if (__dadd_rn(y, width) > (double)H) w2 = (double)H - y;
-            width = w2 < w1 ? w2 : w1;                                 // min(width1, width2)
-            hb[k].x = (int)x;
-            hb[k].y = (int)y;
-            hb[k].w = (int)width;
-            hb[k].valid = hb[k].w > 0;        // the reference's Hand divides by the crop height: an empty box raises there
+            // an empty box is invalid: the reference's Hand divides by the crop height, it raises there
+            hand_detect_box(x1, y1, x2, y2, x3, y3, H, W, hb[k]);
         }
     }
     if (fixed_boxes) {                        // benchmarks / tests: random weights find nobody
@@ -118,7 +102,51 @@ __global__ void pose_finish_kernel(const HandBox* __restrict__ boxes, const doub
     out[2] = p[2];
 }
 
+// ---- the batched hand job (srcmx/Batch_motion_Estimation.py:19-63) on saved body poses
+// one thread per frame: both hand boxes of poses[f] (n x 18 x 3) in an H x W frame
+__global__ void hand_track_boxes_kernel(const double* __restrict__ poses, int n_frames, int H, int W,
+                                        HandBox* __restrict__ boxes) {
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= n_frames) return;
+    HandBox hb[2];
+    pose_hand_boxes(poses + (size_t)f * 54, f, H, W, hb);
+    boxes[2 * f] = hb[0];
+    boxes[2 * f + 1] = hb[1];
+}
+
+// Batch_hand key points of slot (frame, k) -> HandMat rows (_box_to_roi, Batch_motion_Estimation.py:41-56): scaled by
+// w / boxsize, shifted by the box origin, x un-mirrored for left hands; a coordinate of exactly 0 stays 0.  A slot
+// without a box has the box (0, 0, 0): its coordinates become 0 but its scores -- Batch_hand on the grey crop -- stay.
+__global__ void hand_track_finish_kernel(const HandBox* __restrict__ boxes, const double* __restrict__ peaks, int boxsize,
+                                         double* __restrict__ mats) {
+    const int slot = blockIdx.x;
+    const int j = threadIdx.x;
+    if (j >= 21) return;
+    const HandBox b = boxes[slot];
+    const double bx = b.valid ? b.x : 0, by = b.valid ? b.y : 0, bw = b.valid ? b.w : 0;
+    const double* p = peaks + ((size_t)slot * 21 + j) * 3;
+    const double px = __ddiv_rn(__dmul_rn(p[0], bw), (double)boxsize);
+    const double py = __ddiv_rn(__dmul_rn(p[1], bw), (double)boxsize);
+    double* out = mats + (size_t)(slot >> 1) * 126 + (size_t)((b.left ? 0 : 21) + j) * 3;
+    out[0] = px == 0 ? px : (b.left ? __dadd_rn(__dsub_rn(__dsub_rn(bw, px), 1.0), bx) : __dadd_rn(px, bx));
+    out[1] = py == 0 ? py : __dadd_rn(py, by);
+    out[2] = p[2];
+}
+
 }  // namespace
+
+void hand_track_boxes_host(const double* pose, int H, int W, HandBox* boxes) { pose_hand_boxes(pose, 0, H, W, boxes); }
+
+void hand_track_boxes_launch(const double* poses_dev, int n_frames, int H, int W, HandBox* boxes_dev, cudaStream_t stream) {
+    hand_track_boxes_kernel<<<cdiv(n_frames, 64), 64, 0, stream>>>(poses_dev, n_frames, H, W, boxes_dev);
+    OPB_CUDA(cudaGetLastError());
+}
+
+void hand_track_finish_launch(const HandBox* boxes_dev, const double* hand_peaks_dev, int n_frames, int boxsize,
+                              double* mats_dev, cudaStream_t stream) {
+    hand_track_finish_kernel<<<n_frames * 2, 32, 0, stream>>>(boxes_dev, hand_peaks_dev, boxsize, mats_dev);
+    OPB_CUDA(cudaGetLastError());
+}
 
 void pose_select_launch(const FramePost* frames_dev, int n_frames, int H, int W, const int* fixed_boxes_dev, double* pose_dev,
                         HandBox* boxes_dev, int* dims_dev, cudaStream_t stream) {

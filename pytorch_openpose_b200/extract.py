@@ -416,16 +416,23 @@ def batch_body_extraction(videopath, outpath, batch_size, recpoint, batch_body_m
     return mat
 
 
-def hand_crops_from_pose(image, pose, boxsize=368):
-    """`HandImageDataset.__getitem__` (srcmx/Batch_model.py:68-104) for one ROI-cropped frame and its saved (18,3) pose:
-    -> (LeftHand, leftparams, RightHand, rightparams); images uint8 (boxsize, boxsize, 3), grey (128) when the hand
-    is missing, the left one mirrored; params = [x, y, w]."""
-    import cv2
+def pose_person(pose):
+    """The one-person (candidate (20, 4), subset (1, 20)) that HandImageDataset builds from a saved (18, 3) pose for
+    util.handDetect (srcmx/Batch_model.py:75-82): joint i is missing when Python's sum(pose[i, :]) is 0."""
     subset = np.zeros((1, 20))
     candidate = np.zeros((20, 4))
     for i in range(18):
         subset[0, i] = -1 if sum(pose[i, :]) == 0 else i
         candidate[i, :2] = pose[i, :2]
+    return candidate, subset
+
+
+def hand_crops_from_pose(image, pose, boxsize=368):
+    """`HandImageDataset.__getitem__` (srcmx/Batch_model.py:68-104) for one ROI-cropped frame and its saved (18,3) pose:
+    -> (LeftHand, leftparams, RightHand, rightparams); images uint8 (boxsize, boxsize, 3), grey (128) when the hand
+    is missing, the left one mirrored; params = [x, y, w]."""
+    import cv2
+    candidate, subset = pose_person(pose)
     left = np.zeros((boxsize, boxsize, 3), dtype=np.uint8) + 128
     right = np.zeros_like(left) + 128
     leftparams, rightparams = np.zeros((3,)), np.zeros((3,))
@@ -453,10 +460,21 @@ def _box_to_roi(peaks, box, boxsize, mirrored):
 
 
 def batch_hand_extraction(videopath, motiondata, recpoints, outpath, batch_hand_estimation, boxsize=368, batchsize=32,
-                          log=print):
+                          log=print, decode_workers=1, sessions=2):
     """`Batch_hand_extraction` (srcmx/Batch_motion_Estimation.py:19-63) -> HandMat (COUNTS, 42, 3): rows 0-20 left hand,
-    21-41 right hand, in ROI coordinates; a coordinate of exactly 0 means "missing" and is not offset."""
+    21-41 right hand, in ROI coordinates; a coordinate of exactly 0 means "missing" and is not offset.
+
+    With this package's `Batch_hand` the whole per-frame work -- boxes from the saved pose, crops, network, ROI
+    coordinates -- runs on the device (`Batch_hand.submit_track`): decoded frames go up as uint8 from a pinned ring,
+    batches are in flight on `sessions` sessions and HandMat rows are the only thing that comes back (batches of at
+    most 32 frames; `decode_workers` as in `batch_body_extraction`).  One deviation from the host path: a hand box of
+    width 0, on which the reference's cv2.resize raises, is treated as a missing hand.  OPB_HOST_HANDS=1, or any other
+    estimator, takes the host path: crops cut with cv2 and `batch_hand_estimation` called on ToTensor-ed batches."""
     import joblib
+    from .batch_model import Batch_hand
+    if type(batch_hand_estimation) is Batch_hand and os.environ.get("OPB_HOST_HANDS") is None:
+        return _batch_hand_on_device(videopath, motiondata, recpoints, outpath, batch_hand_estimation, boxsize,
+                                     min(batchsize, Batch_hand.TRACK_BATCH), log, decode_workers, sessions)
     src = FrameBatches(videopath, recpoints, batch=batchsize, depth=4, pinned=False)
     assert src.count == len(motiondata)
     mat = np.zeros((len(motiondata), 42, 3))
@@ -471,6 +489,45 @@ def batch_hand_extraction(videopath, motiondata, recpoints, outpath, batch_hand_
             count += 1
             if count % 1000 == 0:
                 log("%s-%d/%d" % (outpath, count, len(motiondata)))
+    joblib.dump(mat, outpath)
+    log("the %s file is saved" % outpath)
+    return mat
+
+
+def _batch_hand_on_device(videopath, motiondata, recpoints, outpath, est, boxsize, batchsize, log, decode_workers,
+                          sessions):
+    import joblib
+    src = FrameBatches(videopath, recpoints, batch=batchsize, depth=sessions + 3, pinned=True, workers=decode_workers,
+                       pad_last=True)
+    assert src.count == len(motiondata)
+    motiondata = np.asarray(motiondata, dtype=np.float64)
+    mat = np.zeros((len(motiondata), 42, 3))
+    ss = _job_sessions(est, sessions)
+    pending = []                                                   # (session, first, n_valid)
+    count = 0
+
+    def retire():
+        nonlocal count
+        s, first, nv = pending.pop(0)
+        hi = min(first + nv, len(mat))
+        mat[first:hi] = est.collect_track(s)[:hi - first]
+        for _ in range(hi - first):
+            count += 1
+            if count % 1000 == 0:
+                log("%s-%d/%d" % (outpath, count, len(motiondata)))
+
+    for frames, first, n_valid in src:
+        nv = max(0, min(n_valid, len(motiondata) - first))
+        poses = np.empty((len(frames), 18, 3))
+        poses[:nv] = motiondata[first:first + nv]
+        poses[nv:] = motiondata[first + nv - 1] if nv else 0         # padded frames: a copy of the last valid pose
+        if len(pending) == sessions:
+            retire()
+        s = next(c for c in ss if all(c is not p[0] for p in pending))
+        est.submit_track(frames, poses, s, where=2, boxsize=boxsize)
+        pending.append((s, first, nv))
+    while pending:
+        retire()
     joblib.dump(mat, outpath)
     log("the %s file is saved" % outpath)
     return mat

@@ -177,6 +177,25 @@ int opb_hand_track_crops(opb_session* hand_s, uint8_t* host_crops);
 /* Host only (no device call): the two boxes of one pose (pose54 = 18 x 3) in a height x width frame, computed by the
  * same function as the device -- boxes8 = [left, right] x [x, y, w, valid]; (0, 0, 0, 0) when a joint is missing.  */
 int opb_hand_track_boxes(const double* pose54, int height, int width, int* boxes8);
+/* ---- Batch_body_extraction + Batch_hand_extraction (srcmx/Batch_motion_Estimation.py:19-112) in one pass -----------
+ * For n_frames ROI-cropped frames (n, height, width, 3) uint8, uploaded once: Batch_body on them (as
+ * opb_batch_body_submit_u8 with g_scale), the person with the largest left-shoulder x and its 18 body rows (body_pose,
+ * :86-105), both hand boxes derived from those rows exactly as from the saved MotionMat (HandImageDataset.__getitem__,
+ * srcmx/Batch_model.py:68-104: a joint is missing when x + y + score == 0), the crops cv2.resize(crop, (boxsize,
+ * boxsize), INTER_CUBIC) cut from the frames already on the device -- the left one mirrored, a uniform 128 image where a
+ * hand is missing --, Batch_hand on all 2n crops and the key points moved back to ROI coordinates (:41-56).  Both tracks
+ * equal those of the two jobs run one after the other.  `where`: 0 pageable host, 1 device, 2 pinned host.
+ * 1 <= n_frames <= 64; boxsize a positive multiple of 8; body_s on a body network and hand_s on a hand network of the
+ * same context.  hand_s must not be used by other calls while a batch is in flight.
+ * wait: MotionMat n x 18 x 3 and HandMat n x 42 x 3 float64 (HandMat rows 0-20 left hand, 21-41 right hand; a
+ * coordinate of exactly 0 means "missing"; a missing hand -- a missing joint, or a box of width <= 0, on which the
+ * reference's cv2.resize raises -- keeps the scores Batch_hand finds on its grey crop).  frame_status (optional): n
+ * ints, OPB_OK or OPB_ERR_SUBSET_INDEX per frame; returns the first non-OK status like opb_body_wait_batch.
+ * opb_hand_track_crops(hand_s) returns the crops of the last batch.                                                  */
+int opb_batch_pose_submit(opb_session* body_s, opb_session* hand_s, const uint8_t* frames_bgr, int where, int n_frames,
+                          int height, int width, double g_scale, int boxsize);
+int opb_batch_pose_wait(opb_session* body_s, double* motion_mats /* n x 18 x 3 */, double* hand_mats /* n x 42 x 3 */,
+                        int* frame_status);
 
 /* blurred heat maps of the last batched-estimator call: (n, 19 | 22, height, width) planar fp32; the
  * un-blurred maps and the PAFs come from opb_body_maps / opb_hand_maps.                             */

@@ -2,7 +2,7 @@
 hand-written sm_100a kernels in libopenpose_b200.so.  See DESIGN.md / INTEGRATION.md."""
 from .body import Body            # noqa: F401
 from .hand import Hand            # noqa: F401
-from .batch_model import Batch_body, Batch_hand      # noqa: F401
+from .batch_model import Batch_body, Batch_hand, BatchPoseEstimator      # noqa: F401
 from . import util                # noqa: F401
 
 

@@ -200,3 +200,55 @@ class Batch_hand(object):
         blurred = np.empty((B, 22, h, w), dtype=np.float32)
         _lib.check(_lib.lib().opb_batch_maps(s.handle, blurred.ctypes.data))
         return np.ascontiguousarray(blurred.transpose(0, 2, 3, 1))
+
+
+class BatchPoseEstimator(object):
+    """`Batch_body_extraction` followed by `Batch_hand_extraction` (srcmx/Batch_motion_Estimation.py:19-112) for batches
+    of ROI-cropped frames in one device pass -- the batched counterpart of `motion.PoseEstimator`.  The frames go up
+    once; Batch_body, the person with the largest left-shoulder x, both hand boxes from its body rows (as
+    HandImageDataset derives them from the saved MotionMat), both crops cut from the frames in device memory, Batch_hand
+    on all of them and the key points in ROI coordinates all run as one launch sequence.  Only the two tracks come back,
+    equal to what the two jobs write: MotionMat (n, 18, 3) and HandMat (n, 42, 3).
+
+    `batch_body` / `batch_hand`: this package's `Batch_body` / `Batch_hand` (their scale_search, 0.5, is used).  A hand
+    box of width 0, on which the reference's cv2.resize raises, counts as a missing hand (as in `Batch_hand.track`)."""
+
+    MAX_BATCH = 32                                    # frames per submit: 64 hand crops, like Batch_hand.TRACK_BATCH
+
+    def __init__(self, batch_body, batch_hand):
+        self.body, self.hand = batch_body, batch_hand
+
+    def sessions(self, k):
+        """k (body session, hand session) pairs kept on the estimator (plans and buffers are expensive to warm up)."""
+        have = self.__dict__.setdefault("_session_pairs", [])
+        while len(have) < k:
+            have.append((self.body.net.session(), self.hand.net.session()))
+        return have[:k]
+
+    def submit(self, frames_u8, pair=None, where=0, boxsize=368):
+        """Enqueue one batch of (B, h, w, 3) uint8 frames (numpy, or a pinned / CUDA torch tensor read in place).
+        where: 0 pageable, 1 device, 2 pinned."""
+        bs, hs = pair or self.sessions(1)[0]
+        ptr, where, keep, (B, h, w) = _as_track_frames(frames_u8, where)
+        bs._keepalive, bs._batch = keep, B
+        _lib.check(_lib.lib().opb_batch_pose_submit(bs.handle, hs.handle, ptr, where, B, h, w,
+                                                    float(self.body.scale_search), int(boxsize)))
+
+    def collect(self, pair=None):
+        """-> (MotionMat (B, 18, 3), HandMat (B, 42, 3)) float64 of the last `submit` on `pair`.  Raises IndexError
+        where the reference's Batch_body would (src/body.py:173)."""
+        bs, hs = pair or self.sessions(1)[0]
+        motion = np.empty((bs._batch, 18, 3), dtype=np.float64)
+        hand = np.empty((bs._batch, 42, 3), dtype=np.float64)
+        status = (ctypes.c_int * bs._batch)()
+        _lib.check(_lib.lib().opb_batch_pose_wait(bs.handle, motion.ctypes.data, hand.ctypes.data, status))
+        return motion, hand
+
+    def __call__(self, frames, boxsize=368):
+        motion, hand = [], []
+        for lo in range(0, len(frames), self.MAX_BATCH):
+            self.submit(frames[lo:lo + self.MAX_BATCH], boxsize=boxsize)
+            m, h = self.collect()
+            motion.append(m)
+            hand.append(h)
+        return np.concatenate(motion, 0), np.concatenate(hand, 0)

@@ -5,6 +5,7 @@
 #include <cstring>
 #include <algorithm>
 #include <cmath>
+#include <initializer_list>
 #include <mutex>
 
 namespace opb {
@@ -250,10 +251,15 @@ struct FramePlan {
     cudaGraphExec_t track_graph = nullptr;
     uint64_t track_gen = 0;
     int track_uses = 0;
+    // the same for the one-pass body + hand sequence of opb_batch_pose_submit (on the Batch_body plan)
+    cudaGraphExec_t batch_pose_graph = nullptr;
+    uint64_t batch_pose_gen = 0;
+    int batch_pose_uses = 0;
     ~FramePlan() {
         if (graph) cudaGraphExecDestroy(graph);
         if (pose_graph) cudaGraphExecDestroy(pose_graph);
         if (track_graph) cudaGraphExecDestroy(track_graph);
+        if (batch_pose_graph) cudaGraphExecDestroy(batch_pose_graph);
     }
     std::vector<ScaleDims> dims;
     std::vector<U8Taps> u8taps;
@@ -409,6 +415,7 @@ struct opb_session {
     opb_session* pose_hand = nullptr;    // hand session of the pose batch in flight
     std::vector<double> pose_hand_scales;
     bool pose_fixed = false;
+    int batch_pose_box = 0;              // boxsize of the opb_batch_pose batch in flight; 0: an opb_pose batch
     ~opb_session() {
         plans.clear();
         net_plans.clear();
@@ -798,6 +805,10 @@ static bool grow_and_redo(opb_session* s, FramePlan* fp, int f, int appended, in
         cudaGraphExecDestroy(fp->pose_graph);
         fp->pose_graph = nullptr;
     }
+    if (fp->batch_pose_graph) {
+        cudaGraphExecDestroy(fp->batch_pose_graph);
+        fp->batch_pose_graph = nullptr;
+    }
     const bool prof = s->prof.on;
     s->prof.on = false;
     body_post_range(s, fp, f, 1, fp->key.H, fp->key.W);
@@ -1011,6 +1022,13 @@ static void build_track_tables(opb_session::HandTrack& t, int boxsize, int wmax)
     t.boxsize = boxsize;
     ++t.gen;
 }
+// the hand session's HandTrack with tables for `boxsize` and crops of up to wmax pixels (nothing may still use them)
+static opb_session::HandTrack& track_with_tables(opb_session* s, int boxsize, int wmax) {
+    if (!s->track) s->track = std::make_unique<opb_session::HandTrack>();
+    opb_session::HandTrack& t = *s->track;
+    if (t.boxsize != boxsize || t.tabs.wmax < wmax) build_track_tables(t, boxsize, wmax);
+    return t;
+}
 
 static void hand_track_submit(opb_session* s, const uint8_t* frames, int where, int n, int H, int W, const double* poses,
                               int boxsize) {
@@ -1021,10 +1039,7 @@ static void hand_track_submit(opb_session* s, const uint8_t* frames, int where, 
     OPB_CUDA(cudaSetDevice(s->net->ctx->device));
     cudaStream_t st = s->stream;
     OPB_CUDA(cudaStreamSynchronize(st));          // the pinned buffers and the tables may still serve the previous batch
-    if (!s->track) s->track = std::make_unique<opb_session::HandTrack>();
-    opb_session::HandTrack& t = *s->track;
-    const int wmax = std::min(H, W);
-    if (t.boxsize != boxsize || t.tabs.wmax < wmax) build_track_tables(t, boxsize, wmax);
+    opb_session::HandTrack& t = track_with_tables(s, boxsize, std::min(H, W));
     if (t.frames < n) {
         t.pool.release();
         if (t.poses_host) cudaFreeHost(t.poses_host);
@@ -1066,7 +1081,7 @@ static void hand_track_submit(opb_session* s, const uint8_t* frames, int where, 
         hand_track_boxes_launch(t.poses, n, H, W, t.boxes, st);
         preprocess_ragged_launch(t.frames_dev, H, W, t.boxes, slots, fp->d_img, boxsize, 0, t.tabs, st);
         batch_hand_enqueue(s, fp, slots, boxsize, boxsize);
-        hand_track_finish_launch(t.boxes, fp->hb.peaks, n, boxsize, t.mats, st);
+        hand_track_finish_launch(t.boxes, fp->hb.peaks, n, boxsize, t.mats, 126, st);
         OPB_CUDA(cudaMemcpyAsync(t.mats_host, t.mats, (size_t)n * 126 * sizeof(double), cudaMemcpyDeviceToHost, st));
     });
     OPB_CUDA(cudaEventRecord(s->done, st));
@@ -1114,6 +1129,21 @@ static void build_ragged_tables(opb_session* hs, const double* scales, int ns, i
     hs->ragged = std::move(r);
 }
 
+// per-batch [n][60][3] records, hand boxes and their pinned host copy on a body session, grown to the largest batch seen
+static void ensure_pose_buffers(opb_session* bs, int n) {
+    if (bs->pose && bs->pose->frames >= n) return;
+    OPB_CUDA(cudaStreamSynchronize(bs->stream));
+    auto pb = std::make_unique<opb_session::PoseBuffers>();
+    pb->frames = n;
+    pb->pose = pb->pool.alloc_t<double>((size_t)n * 180);
+    pb->boxes = pb->pool.alloc_t<HandBox>((size_t)n * 2);
+    pb->dims = pb->pool.alloc_t<int>((size_t)n * 2);
+    pb->fixed = pb->pool.alloc_t<int>((size_t)n * 6);
+    OPB_CUDA(cudaMallocHost((void**)&pb->host, (size_t)n * 180 * sizeof(double)));
+    OPB_CUDA(cudaMallocHost((void**)&pb->fixed_host, (size_t)n * 6 * sizeof(int)));
+    bs->pose = std::move(pb);
+}
+
 // the hand half of the pose pipeline, on the body session's stream: boxes from the body results (or the fixed ones already
 // in the pinned buffer), ragged crops -> hand CNN -> ragged post-processing -> PoseMat -> pinned host buffer
 static void pose_hand_enqueue(opb_session* bs, opb_session* hs, FramePlan* fp, FramePlan* hp, int n, int H, int W, bool fixed) {
@@ -1149,24 +1179,14 @@ static void pose_submit(opb_session* bs, opb_session* hs, const uint8_t* imgs, i
         build_ragged_tables(hs, hscales, nhs, wmax);
     }
     const int tw = hs->ragged->tabs.wmax;                       // plane pitch of the ragged buffers
-    if (!bs->pose || bs->pose->frames < n) {
-        OPB_CUDA(cudaStreamSynchronize(bs->stream));
-        auto pb = std::make_unique<opb_session::PoseBuffers>();
-        pb->frames = n;
-        pb->pose = pb->pool.alloc_t<double>((size_t)n * 180);
-        pb->boxes = pb->pool.alloc_t<HandBox>((size_t)n * 2);
-        pb->dims = pb->pool.alloc_t<int>((size_t)n * 2);
-        pb->fixed = pb->pool.alloc_t<int>((size_t)n * 6);
-        OPB_CUDA(cudaMallocHost((void**)&pb->host, (size_t)n * 180 * sizeof(double)));
-        OPB_CUDA(cudaMallocHost((void**)&pb->fixed_host, (size_t)n * 6 * sizeof(int)));
-        bs->pose = std::move(pb);
-    }
+    ensure_pose_buffers(bs, n);
     // body part: as opb_body_submit_batch
     FramePlan* fp = get_plan(bs, n, H, W, bscales, nbs);
     ensure_host(bs, n, 0);
     bs->active = fp;
     bs->n_frames = n;
     bs->pose_hand = hs;
+    bs->batch_pose_box = 0;
     cudaStream_t st = bs->stream;
     upload_image(bs, fp, imgs, where, (size_t)n * H * W * 3);
     // hand part on the same stream, with the hand session's CNN plan and work buffers (sized for the largest crop)
@@ -1193,6 +1213,104 @@ static void pose_submit(opb_session* bs, opb_session* hs, const uint8_t* imgs, i
     });
     OPB_CUDA(cudaEventRecord(bs->done, st));
     bs->net->ctx->launches += fp->launches_per_frame + nhs + hp->net->kernel_launches + (nhs + 1) + 6 + 2;
+}
+
+// the overflow check of a pose batch after its body results arrived: a frame that overflowed its peak / pair / connection
+// / person buffers gets larger ones and its body post-processing is repeated (like opb_body_wait_batch; `grew` tells the
+// caller to repeat the hand half of the batch).  Fills frame_status (optional) and returns the first non-OK status.
+static int pose_batch_status(opb_session* bs, int* frame_status, bool& grew) {
+    int rc = OPB_OK;
+    OPB_CUDA(cudaEventSynchronize(bs->done));
+    FramePlan* fp = bs->active;
+    for (int f = 0; f < bs->n_frames; ++f) {
+        const HostResults* h = bs->host + f;
+        for (int attempt = 0; attempt < 12; ++attempt) {
+            const FramePost& bp = fp->post[f];
+            if (h->counts[0] <= bp.pb.capacity && !(h->counts[21] & (kStPairOverflow | kStConnOverflow | kStSubsetOverflow))) break;
+            if (!grow_and_redo(bs, fp, f, h->counts[0], h->counts[21])) break;
+            grew = true;
+        }
+        const int status = h->counts[21];
+        if (h->counts[0] > fp->post[f].pb.capacity || (status & (kStPairOverflow | kStConnOverflow | kStSubsetOverflow)))
+            throw Error(OPB_ERR_CAPACITY, "a frame overflowed the body result buffers (status " + std::to_string(status) + ")");
+        const int st = (status & kStIndexError) ? OPB_ERR_SUBSET_INDEX : OPB_OK;
+        if (frame_status) frame_status[f] = st;
+        if (st != OPB_OK && rc == OPB_OK) rc = st;
+    }
+    if (rc == OPB_ERR_SUBSET_INDEX)
+        set_last_error("list assignment index out of range (three subset rows match one connection, src/body.py:173)");
+    return rc;
+}
+
+// ------------------------------------------------------------------------------------------------
+// the one-pass body + hand job: Batch_body_extraction and Batch_hand_extraction (srcmx/Batch_motion_Estimation.py:19-112)
+// on one upload of the decoded frames
+// ------------------------------------------------------------------------------------------------
+// The hand half, on the body session's stream: person, body rows and both hand boxes from the Batch_body results, both
+// crops cut from the frames still in the body plan's input buffer into the uint8 Batch_hand plan `hp` of the hand session,
+// Batch_hand on all 2n crops, HandMat into rows 18-59 of the records, one copy of the records into pinned host memory.
+static void batch_pose_hand_enqueue(opb_session* bs, opb_session* hs, FramePlan* fp, FramePlan* hp, int n, int boxsize) {
+    cudaStream_t st = bs->stream;
+    const int H = fp->key.H, W = fp->key.W, slots = 2 * n;
+    const opb_session::PoseBuffers& pb = *bs->pose;
+    batch_pose_select_launch(fp->post_dev, n, H, W, pb.pose, pb.boxes, st);
+    preprocess_ragged_launch(fp->d_img, H, W, pb.boxes, slots, hp->d_img, boxsize, 0, hs->track->tabs, st);
+    batch_hand_enqueue(bs, hp, slots, boxsize, boxsize);        // bs only lends its stream and profiler
+    hand_track_finish_launch(pb.boxes, hp->hb.peaks, n, boxsize, pb.pose + 54, 180, st);
+    OPB_CUDA(cudaMemcpyAsync(pb.host, pb.pose, (size_t)n * 180 * sizeof(double), cudaMemcpyDeviceToHost, st));
+}
+
+static uint64_t gen_key(std::initializer_list<uint64_t> parts) {      // FNV-1a over the words
+    uint64_t h = 14695981039346656037ull;
+    for (uint64_t v : parts) h = (h ^ v) * 1099511628211ull;
+    return h;
+}
+
+static void batch_pose_submit(opb_session* bs, opb_session* hs, const uint8_t* frames, int where, int n, int H, int W,
+                              double g_scale, int boxsize) {
+    OPB_REQUIRE(bs->net->kind == OPB_NET_BODY && hs->net->kind == OPB_NET_HAND,
+                "batch pose: a body session and a hand session");
+    OPB_REQUIRE(bs->net->ctx == hs->net->ctx, "batch pose: both networks must live on the same context");
+    OPB_REQUIRE(n >= 1 && n <= 64, "1..64 frames per batch");
+    OPB_REQUIRE(H >= 1 && W >= 1, "empty frame");
+    OPB_REQUIRE(g_scale > 0, "scale must be positive");
+    OPB_REQUIRE(boxsize >= 8 && boxsize % 8 == 0, "boxsize must be a positive multiple of 8 (srcmx/Batch_model.py:377)");
+    OPB_CUDA(cudaSetDevice(bs->net->ctx->device));
+    cudaStream_t st = bs->stream;
+    // the records, boxes and crop tables may still serve the previous batch of this pair, the hand plan work of the
+    // hand session's own stream
+    OPB_CUDA(cudaStreamSynchronize(st));
+    OPB_CUDA(cudaStreamSynchronize(hs->stream));
+    ensure_pose_buffers(bs, n);
+    opb_session::HandTrack& t = track_with_tables(hs, boxsize, std::min(H, W));
+    FramePlan* fp = get_plan(bs, n, H, W, &g_scale, 1, 2);          // Batch_body on uint8 frames
+    ensure_host(bs, n, 0);
+    bs->active = fp;
+    bs->n_frames = n;
+    bs->pose_hand = hs;
+    bs->batch_pose_box = boxsize;
+    const double one = 1.0;
+    FramePlan* hp = get_plan(hs, 2 * n, boxsize, boxsize, &one, 1, 2);      // uint8 Batch_hand on 2n crops
+    hs->active = hp;
+    hs->hand_crops = 2 * n;
+    t.plan = hp;
+    bs->prof.reset();
+    bs->prof.mark(st, "start");
+    upload_image(bs, fp, frames, where, (size_t)n * H * W * 3);
+    bs->prof.mark(st, "h2d");
+    // one launch sequence from the uploaded frames to the records copy, replayed as a CUDA graph from the third use on;
+    // re-captured when a buffer of either session, the hand plan, the crop tables, the records or the frame size change
+    const opb_session::PoseBuffers& pb = *bs->pose;
+    const uint64_t gen = gen_key({bs->buffer_gen, hs->buffer_gen, (uint64_t)(uintptr_t)hp, t.gen,
+                                  (uint64_t)(uintptr_t)pb.pose, (uint64_t)(uintptr_t)pb.boxes, (uint64_t)(uintptr_t)pb.host,
+                                  (uint64_t)H, (uint64_t)W, (uint64_t)boxsize});
+    run_or_replay_slot(bs, GraphSlot{fp->batch_pose_graph, fp->batch_pose_gen, fp->batch_pose_uses}, gen, [&] {
+        run_front_f32(bs, fp, n, H, W);
+        body_post_enqueue(bs, fp, n, H, W);
+        batch_pose_hand_enqueue(bs, hs, fp, hp, n, boxsize);
+    });
+    OPB_CUDA(cudaEventRecord(bs->done, st));
+    bs->net->ctx->launches += fp->launches_per_frame + 3 /* select, crops, finish */ + hp->launches_per_frame;
 }
 
 }  // namespace opb
@@ -1542,37 +1660,49 @@ int opb_pose_submit_batch(opb_session* body_s, opb_session* hand_s, const uint8_
 int opb_pose_wait(opb_session* body_s, double* pose_mats, int* frame_status) {
     int rc = OPB_OK;
     int g = guarded([&] {
-        OPB_REQUIRE(body_s && pose_mats && body_s->pose && body_s->active, "no pose batch in flight");
+        OPB_REQUIRE(body_s && pose_mats && body_s->pose && body_s->active && !body_s->batch_pose_box,
+                    "no pose batch in flight");
         // body results first: they report the overflow / IndexError conditions of every frame
-        std::vector<int> st(body_s->n_frames);
-        OPB_CUDA(cudaEventSynchronize(body_s->done));
-        FramePlan* fp = body_s->active;
         bool grew = false;
-        for (int f = 0; f < body_s->n_frames; ++f) {
-            const HostResults* h = body_s->host + f;
-            // a frame that overflowed its peak / pair / connection / person buffers gets larger ones and its body
-            // post-processing is repeated (like opb_body_wait_batch); the hand half is then repeated for the batch
-            for (int attempt = 0; attempt < 12; ++attempt) {
-                const FramePost& bp = fp->post[f];
-                if (h->counts[0] <= bp.pb.capacity && !(h->counts[21] & (kStPairOverflow | kStConnOverflow | kStSubsetOverflow))) break;
-                if (!grow_and_redo(body_s, fp, f, h->counts[0], h->counts[21])) break;
-                grew = true;
-            }
-            const int status = h->counts[21];
-            if (h->counts[0] > fp->post[f].pb.capacity || (status & (kStPairOverflow | kStConnOverflow | kStSubsetOverflow)))
-                throw Error(OPB_ERR_CAPACITY, "a frame overflowed the body result buffers (status " + std::to_string(status) + ")");
-            st[f] = (status & kStIndexError) ? OPB_ERR_SUBSET_INDEX : OPB_OK;
-            if (frame_status) frame_status[f] = st[f];
-            if (st[f] != OPB_OK && rc == OPB_OK) rc = st[f];
-        }
+        rc = pose_batch_status(body_s, frame_status, grew);
         if (grew) {
+            FramePlan* fp = body_s->active;
             opb_session* hs = body_s->pose_hand;
             pose_hand_enqueue(body_s, hs, fp, hs->active, body_s->n_frames, fp->key.H, fp->key.W, body_s->pose_fixed);
             OPB_CUDA(cudaStreamSynchronize(body_s->stream));
         }
         memcpy(pose_mats, body_s->pose->host, (size_t)body_s->n_frames * 180 * sizeof(double));
-        if (rc == OPB_ERR_SUBSET_INDEX)
-            set_last_error("list assignment index out of range (three subset rows match one connection, src/body.py:173)");
+    });
+    return g != OPB_OK ? g : rc;
+}
+
+/* ---- the one-pass body + hand job ------------------------------------------------------------------------------- */
+int opb_batch_pose_submit(opb_session* body_s, opb_session* hand_s, const uint8_t* frames_bgr, int where, int n_frames,
+                          int height, int width, double g_scale, int boxsize) {
+    return guarded([&] {
+        OPB_REQUIRE(body_s && hand_s && frames_bgr, "null argument");
+        OPB_REQUIRE(where >= 0 && where <= 2, "where: 0 pageable host, 1 device, 2 pinned host");
+        batch_pose_submit(body_s, hand_s, frames_bgr, where, n_frames, height, width, g_scale, boxsize);
+    });
+}
+int opb_batch_pose_wait(opb_session* body_s, double* motion_mats, double* hand_mats, int* frame_status) {
+    int rc = OPB_OK;
+    int g = guarded([&] {
+        OPB_REQUIRE(body_s && motion_mats && hand_mats && body_s->pose && body_s->active && body_s->batch_pose_box,
+                    "no batch-pose batch in flight");
+        OPB_CUDA(cudaSetDevice(body_s->net->ctx->device));
+        bool grew = false;
+        rc = pose_batch_status(body_s, frame_status, grew);
+        if (grew) {                                   // the hand half again, on the grown frames' new body results
+            opb_session* hs = body_s->pose_hand;
+            batch_pose_hand_enqueue(body_s, hs, body_s->active, hs->active, body_s->n_frames, body_s->batch_pose_box);
+            OPB_CUDA(cudaStreamSynchronize(body_s->stream));
+        }
+        const double* rec = body_s->pose->host;
+        for (int f = 0; f < body_s->n_frames; ++f) {
+            memcpy(motion_mats + (size_t)f * 54, rec + (size_t)f * 180, 54 * sizeof(double));
+            memcpy(hand_mats + (size_t)f * 126, rec + (size_t)f * 180 + 54, 126 * sizeof(double));
+        }
     });
     return g != OPB_OK ? g : rc;
 }

@@ -353,6 +353,38 @@ __host__ __device__ inline void pose_hand_boxes(const double* pose, int frame, i
                             pose[(j0 + 2) * 3 + 1], H, W, b);
     }
 }
+// the person with the largest left-shoulder x among the body results of one frame (srcmx/MotionEstimation.py:141-158,
+// srcmx/Batch_motion_Estimation.py:86-105): a missing shoulder (-1) indexes the LAST candidate, like candidate[-1];
+// np.argmax keeps the first maximum.  Writes the person's 18 body rows (x, y, score) into body54 -- rows of missing
+// joints are left as they are (the callers zero them first) -- and returns the chosen subset row, or null for nobody.
+__device__ inline const double* select_person_rows(const FramePost& fr, double* body54) {
+    const double* cand = fr.pb.candidates;
+    const int n_cand = fr.pb.part_begin[18];
+    const double* subset = fr.lb.subset;
+    const int n_sub = *fr.lb.subset_count;
+    int chosen = -1;
+    double best = 0.0;
+    for (int p = 0; p < n_sub; ++p) {
+        int idx = (int)subset[(size_t)p * 20 + 5];
+        if (idx < 0) idx += n_cand;
+        const double x = cand[(size_t)idx * 4];
+        if (chosen < 0 || x > best) {
+            chosen = p;
+            best = x;
+        }
+    }
+    if (chosen < 0) return nullptr;
+    const double* row = subset + (size_t)chosen * 20;
+    for (int k = 0; k < 18; ++k) {
+        const int idx = (int)row[k];
+        if (idx != -1) {
+            body54[k * 3 + 0] = cand[(size_t)idx * 4 + 0];
+            body54[k * 3 + 1] = cand[(size_t)idx * 4 + 1];
+            body54[k * 3 + 2] = cand[(size_t)idx * 4 + 2];
+        }
+    }
+    return row;
+}
 
 struct RaggedTables {
     const uint8_t* slab;      // all tables
@@ -374,8 +406,13 @@ void pose_finish_launch(const HandBox* boxes_dev, const double* hand_peaks_dev, 
 // the batched hand job on saved poses (pose.cu): boxes (2 per frame, left first) and HandMat (n x 42 x 3) assembly
 void hand_track_boxes_launch(const double* poses_dev, int n_frames, int H, int W, HandBox* boxes_dev, cudaStream_t stream);
 void hand_track_boxes_host(const double* pose, int H, int W, HandBox* boxes);      // the same function on the host
+// mats_dev: HandMat of frame f at mats_dev + f * frame_stride (126 for n x 42 x 3, 180 for rows 18-59 of n x 60 x 3)
 void hand_track_finish_launch(const HandBox* boxes_dev, const double* hand_peaks_dev, int n_frames, int boxsize,
-                              double* mats_dev, cudaStream_t stream);
+                              double* mats_dev, int frame_stride, cudaStream_t stream);
+// the one-pass body + hand job (pose.cu): from the results of a Batch_body batch, the body rows of a per-frame
+// [60][3] record (rows 18-59 zeroed) and both hand boxes derived from those rows as from a saved pose
+void batch_pose_select_launch(const FramePost* frames_dev, int n_frames, int H, int W, double* records_dev,
+                              HandBox* boxes_dev, cudaStream_t stream);
 
 // ---- gaussian taps shared by peaks.cu / hand.cu: scipy.ndimage.gaussian_filter(sigma=3) uses
 // radius int(4*3+0.5) = 12 and weights exp(-x^2/18) / sum (src/body.py:75, src/hand.py:62).  The

@@ -16,25 +16,11 @@ __global__ void pose_select_kernel(const FramePost* __restrict__ frames, int n_f
     if (f >= n_frames) return;
     const FramePost& fr = frames[f];
     const double* cand = fr.pb.candidates;
-    const int n_cand = fr.pb.part_begin[18];
-    const double* subset = fr.lb.subset;
-    const int n_sub = *fr.lb.subset_count;
     double* pm = pose + (size_t)f * 180;
     for (int i = 0; i < 180; ++i) pm[i] = 0.0;
 
-    // the person with the largest left-shoulder x (MotionEstimation.py:144-150); a missing shoulder (-1) indexes the
-    // LAST candidate, like candidate[-1]; np.argmax keeps the first maximum
-    int chosen = -1;
-    double best = 0.0;
-    for (int p = 0; p < n_sub; ++p) {
-        int idx = (int)subset[(size_t)p * 20 + 5];
-        if (idx < 0) idx += n_cand;
-        const double x = cand[(size_t)idx * 4];
-        if (chosen < 0 || x > best) {
-            chosen = p;
-            best = x;
-        }
-    }
+    // the person (MotionEstimation.py:144-158) and its body rows
+    const double* row = select_person_rows(fr, pm);
     HandBox hb[2];
     for (int k = 0; k < 2; ++k) {
         hb[k].frame = f;
@@ -42,16 +28,7 @@ __global__ void pose_select_kernel(const FramePost* __restrict__ frames, int n_f
         hb[k].left = k == 0;
         hb[k].valid = 0;
     }
-    if (chosen >= 0) {
-        const double* row = subset + (size_t)chosen * 20;
-        for (int k = 0; k < 18; ++k) {
-            const int idx = (int)row[k];
-            if (idx != -1) {
-                pm[k * 3 + 0] = cand[(size_t)idx * 4 + 0];
-                pm[k * 3 + 1] = cand[(size_t)idx * 4 + 1];
-                pm[k * 3 + 2] = cand[(size_t)idx * 4 + 2];
-            }
-        }
+    if (row) {
         // util.handDetect on the chosen person (the caller blanks all other rows first, MotionEstimation.py:160-162):
         // left hand from shoulder / elbow / wrist 5, 6, 7, right hand from 2, 3, 4
         for (int k = 0; k < 2; ++k) {
@@ -118,7 +95,7 @@ __global__ void hand_track_boxes_kernel(const double* __restrict__ poses, int n_
 // w / boxsize, shifted by the box origin, x un-mirrored for left hands; a coordinate of exactly 0 stays 0.  A slot
 // without a box has the box (0, 0, 0): its coordinates become 0 but its scores -- Batch_hand on the grey crop -- stay.
 __global__ void hand_track_finish_kernel(const HandBox* __restrict__ boxes, const double* __restrict__ peaks, int boxsize,
-                                         double* __restrict__ mats) {
+                                         double* __restrict__ mats, int frame_stride) {
     const int slot = blockIdx.x;
     const int j = threadIdx.x;
     if (j >= 21) return;
@@ -127,10 +104,28 @@ __global__ void hand_track_finish_kernel(const HandBox* __restrict__ boxes, cons
     const double* p = peaks + ((size_t)slot * 21 + j) * 3;
     const double px = __ddiv_rn(__dmul_rn(p[0], bw), (double)boxsize);
     const double py = __ddiv_rn(__dmul_rn(p[1], bw), (double)boxsize);
-    double* out = mats + (size_t)(slot >> 1) * 126 + (size_t)((b.left ? 0 : 21) + j) * 3;
+    double* out = mats + (size_t)(slot >> 1) * frame_stride + (size_t)((b.left ? 0 : 21) + j) * 3;
     out[0] = px == 0 ? px : (b.left ? __dadd_rn(__dsub_rn(__dsub_rn(bw, px), 1.0), bx) : __dadd_rn(px, bx));
     out[1] = py == 0 ? py : __dadd_rn(py, by);
     out[2] = p[2];
+}
+
+// ---- the one-pass body + hand job: Batch_body_extraction and Batch_hand_extraction (srcmx/Batch_motion_Estimation.py:
+// 19-112) on one decode.  One thread per frame of a Batch_body batch: the body rows MotionMat gets (as body_pose on the
+// fetched candidates / subset) go into rows 0-17 of records[f] (rows 18-59 zeroed, HandMat lands there later), and the
+// hand boxes are derived from exactly those doubles as Batch_hand_extraction derives them from the saved MotionMat
+// (HandImageDataset.__getitem__: a joint is missing when x + y + score == 0) -- so both tracks equal the two-pass job's.
+__global__ void batch_pose_select_kernel(const FramePost* __restrict__ frames, int n_frames, int H, int W,
+                                         double* __restrict__ records, HandBox* __restrict__ boxes) {
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= n_frames) return;
+    double* rec = records + (size_t)f * 180;
+    for (int i = 0; i < 180; ++i) rec[i] = 0.0;
+    select_person_rows(frames[f], rec);
+    HandBox hb[2];
+    pose_hand_boxes(rec, f, H, W, hb);
+    boxes[2 * f] = hb[0];
+    boxes[2 * f + 1] = hb[1];
 }
 
 }  // namespace
@@ -143,8 +138,14 @@ void hand_track_boxes_launch(const double* poses_dev, int n_frames, int H, int W
 }
 
 void hand_track_finish_launch(const HandBox* boxes_dev, const double* hand_peaks_dev, int n_frames, int boxsize,
-                              double* mats_dev, cudaStream_t stream) {
-    hand_track_finish_kernel<<<n_frames * 2, 32, 0, stream>>>(boxes_dev, hand_peaks_dev, boxsize, mats_dev);
+                              double* mats_dev, int frame_stride, cudaStream_t stream) {
+    hand_track_finish_kernel<<<n_frames * 2, 32, 0, stream>>>(boxes_dev, hand_peaks_dev, boxsize, mats_dev, frame_stride);
+    OPB_CUDA(cudaGetLastError());
+}
+
+void batch_pose_select_launch(const FramePost* frames_dev, int n_frames, int H, int W, double* records_dev,
+                              HandBox* boxes_dev, cudaStream_t stream) {
+    batch_pose_select_kernel<<<cdiv(n_frames, 64), 64, 0, stream>>>(frames_dev, n_frames, H, W, records_dev, boxes_dev);
     OPB_CUDA(cudaGetLastError());
 }
 

@@ -533,6 +533,85 @@ def _batch_hand_on_device(videopath, motiondata, recpoints, outpath, est, boxsiz
     return mat
 
 
+def batch_bodyhand_extraction(videopath, body_outpath, hand_outpath, batch_size, recpoint, batch_body_model,
+                              batch_hand_estimation, boxsize=368, log=print, decode_workers=1, sessions=2):
+    """`Batch_body_extraction` and then `Batch_hand_extraction` on its track (srcmx/Batch_motion_Estimation.py:19-112)
+    -> (MotionMat (COUNTS, 18, 3), HandMat (COUNTS, 42, 3)), written to `body_outpath` / `hand_outpath` with the same
+    shapes, dtypes and log lines as `batch_body_extraction` and `batch_hand_extraction`.
+
+    With this package's `Batch_body` and `Batch_hand` the video is decoded once: every batch of frames goes up once from
+    a pinned ring and `BatchPoseEstimator` runs body, person selection, hand boxes, crops and the hand network on it in
+    one launch sequence, with batches in flight on `sessions` (body, hand) session pairs (at most 32 frames per batch;
+    `decode_workers` as in `batch_body_extraction`).  Both tracks equal the two-pass job's bit for bit; a frame on which
+    Batch_body raises IndexError makes the job raise it before any file is written.  With any other estimators the two
+    jobs run one after the other on the same ROI.
+
+    From `run_body_job`, one video per call, writing the `-hand` track next to the body track:
+
+        def process_video(videopath, outpath):
+            batch_bodyhand_extraction(videopath, outpath, outpath.replace("-body.pkl", "-hand.pkl"), 32, recpoint,
+                                      Batch_body(body_model_path), Batch_hand(hand_model_path))
+        run_body_job(videofolder, datadir, recpoint, process_video)
+
+    (create the two estimators once, outside the closure: their sessions are kept across videos)."""
+    from .batch_model import Batch_body, Batch_hand, BatchPoseEstimator
+    if type(batch_body_model) is not Batch_body or type(batch_hand_estimation) is not Batch_hand:
+        motion = batch_body_extraction(videopath, body_outpath, batch_size, recpoint, batch_body_model, log=log,
+                                       decode_workers=decode_workers, sessions=sessions)
+        if motion is None:
+            return None
+        hand = batch_hand_extraction(videopath, motion, recpoint, hand_outpath, batch_hand_estimation, boxsize=boxsize,
+                                     batchsize=batch_size, log=log, decode_workers=decode_workers, sessions=sessions)
+        return motion, hand
+    import joblib
+    batch = min(batch_size, BatchPoseEstimator.MAX_BATCH)
+    try:
+        src = FrameBatches(videopath, recpoint, batch=batch, depth=sessions + 3, pinned=True, workers=decode_workers,
+                           pad_last=True)
+    except FileNotFoundError as e:
+        log(str(e))
+        return None
+    est = batch_body_model.__dict__.setdefault("_batch_pose_estimator", None)
+    if est is None or est.hand is not batch_hand_estimation:
+        est = batch_body_model.__dict__["_batch_pose_estimator"] = BatchPoseEstimator(batch_body_model,
+                                                                                      batch_hand_estimation)
+    pairs = est.sessions(sessions)
+    outname = os.path.split(body_outpath)[1]
+    motion = np.zeros((src.count, 18, 3))
+    hand = np.zeros((src.count, 42, 3))
+    pending = []                                                   # (pair, first, n_valid)
+    counts = [0, 0]                                                # frames retired: body job, hand job
+
+    def retire():
+        pair, first, nv = pending.pop(0)
+        m, h = est.collect(pair)
+        hi = min(first + nv, len(motion))
+        motion[first:hi] = m[:hi - first]
+        hand[first:hi] = h[:hi - first]
+        for f in range(nv):                                        # the progress lines of the two jobs
+            counts[0] += 1
+            if counts[0] % 1000 == 0:
+                log("%s-%d/%d" % (outname, counts[0], src.count))
+            if first + f < hi:
+                counts[1] += 1
+                if counts[1] % 1000 == 0:
+                    log("%s-%d/%d" % (hand_outpath, counts[1], src.count))
+
+    for frames, first, n_valid in src:
+        if len(pending) == len(pairs):
+            retire()
+        pair = next(c for c in pairs if all(c is not p[0] for p in pending))
+        est.submit(frames, pair, where=2, boxsize=boxsize)
+        pending.append((pair, first, n_valid))
+    while pending:
+        retire()
+    joblib.dump(motion, body_outpath)
+    log("the %s file is saved" % body_outpath)
+    joblib.dump(hand, hand_outpath)
+    log("the %s file is saved" % hand_outpath)
+    return motion, hand
+
+
 # ---- resume ledger (srcmx/utilmx.py:190-208) ----------------------------------------------------------------------
 class ExtractLedger(object):
     """`extract_ed_ing.txt` in the data directory: one output file name per line, appended BEFORE a video is processed

@@ -137,6 +137,25 @@ int opb_pose_submit_batch(opb_session* body_s, opb_session* hand_s, const uint8_
                           int height, int width, const double* body_scales, int n_body_scales,
                           const double* hand_scales, int n_hand_scales, const int* fixed_boxes);
 int opb_pose_wait(opb_session* body_s, double* pose_mats, int* frame_status);
+/* ---- every person of every frame ----------------------------------------------------------------------------------
+ * The caller's loop over everyone Body finds, for a batch of equally sized uint8 BGR frames: per frame, one 60 x 3
+ * float64 record per subset row, in subset order (rows 0-17 candidate[subset[p][k]][:3], zero where the index is -1),
+ * util.handDetect on every subset row (src/util.py:133-201), Hand on every box it returns -- the left crop mirrored --
+ * and the key points in frame coordinates in rows 18-38 (left) and 39-59 (right) of the box's person, as
+ * srcmx/MotionEstimation.py:185-194 computes them.  A hand with a missing joint gets zero rows and no crop; a box of
+ * width <= 0, on which the reference's Hand raises ZeroDivisionError, gives zero rows.  Arguments as
+ * opb_pose_submit_batch (1 <= n_frames <= 64, `where`: 0 pageable host, 1 device, 2 pinned host).  The hand crops run
+ * in fixed chunks of 8 through one hand plan, so memory does not depend on the number of persons.  hand_s must not be
+ * used by other calls while a batch is in flight.
+ * wait: runs the hand chunks, fills persons (n ints: records of each frame) and frame_status (optional: OPB_OK or
+ * OPB_ERR_SUBSET_INDEX per frame), returns the first non-OK status like opb_body_wait_batch.
+ * fetch: the records of the last wait, frame after frame (sum of persons x 60 x 3); rows = capacity of `records` in
+ * records.                                                                                                        */
+int opb_pose_every_submit(opb_session* body_s, opb_session* hand_s, const uint8_t* imgs_bgr, int where, int n_frames,
+                          int height, int width, const double* body_scales, int n_body_scales,
+                          const double* hand_scales, int n_hand_scales);
+int opb_pose_every_wait(opb_session* body_s, int* persons, int* frame_status);
+int opb_pose_every_fetch(opb_session* body_s, double* records, int rows);
 
 /* ---- batched estimators: srcmx/Batch_model.py (the reference author's throughput path) ---------- */
 /* Batch_body.__call__ (srcmx/Batch_model.py:142-204): `frames` = (n, 3, height, width) float32 planar in
@@ -240,6 +259,11 @@ int opb_bench_grouping(opb_context* ctx, const float* dev_heat, const float* dev
  * [x, y, w, valid]) -- the device kernel of the opb_pose_* pipeline, for parity tests.                 */
 int opb_pose_select(opb_context* ctx, const double* host_candidates, int n_candidates, const double* host_subset,
                     int n_subset, int height, int width, double* host_pose180, int* host_boxes8);
+/* The rows-and-boxes kernel of the opb_pose_every_* pipeline on host-provided body results of one frame (parity tests):
+ * host_records = n_subset x 60 x 3 (body rows, hand rows zero); host_boxes = 2 * n_subset x [x, y, w, is_left,
+ * record], the boxes util.handDetect returns in its order, rows past the box count all -1.                        */
+int opb_pose_every_select(opb_context* ctx, const double* host_candidates, int n_candidates, const double* host_subset,
+                          int n_subset, int height, int width, double* host_records, int* host_boxes);
 /* src/hand.py:59-75 on a planar (>=21, h, w) fp32 device map -> 21x3 float64 host array.            */
 int opb_hand_peaks(opb_context* ctx, const float* dev_heat, int height, int width, double thre, double* host_peaks);
 

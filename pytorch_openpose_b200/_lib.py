@@ -54,6 +54,11 @@ SIGNATURES = {
                                       POINTER(c_double), c_int, c_void_p]),
     "opb_pose_wait": (c_int, [c_void_p, c_void_p, POINTER(c_int)]),
     "opb_pose_select": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "opb_pose_every_submit": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, POINTER(c_double), c_int,
+                                      POINTER(c_double), c_int]),
+    "opb_pose_every_wait": (c_int, [c_void_p, POINTER(c_int), POINTER(c_int)]),
+    "opb_pose_every_fetch": (c_int, [c_void_p, c_void_p, c_int]),
+    "opb_pose_every_select": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
     "opb_body_maps": (c_int, [c_void_p, c_void_p, c_void_p]),
     "opb_hand_maps": (c_int, [c_void_p, c_void_p]),
     "opb_batch_body_submit": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_double]),

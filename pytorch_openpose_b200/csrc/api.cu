@@ -255,11 +255,21 @@ struct FramePlan {
     cudaGraphExec_t batch_pose_graph = nullptr;
     uint64_t batch_pose_gen = 0;
     int batch_pose_uses = 0;
+    // every person (opb_pose_every_*): the body sequence with the rows-and-boxes kernel, and one hand chunk (replayed
+    // once per kEveryChunk boxes) -- both on the body plan of the batch
+    cudaGraphExec_t every_graph = nullptr;
+    uint64_t every_gen = 0;
+    int every_uses = 0;
+    cudaGraphExec_t every_hand_graph = nullptr;
+    uint64_t every_hand_gen = 0;
+    int every_hand_uses = 0;
     ~FramePlan() {
         if (graph) cudaGraphExecDestroy(graph);
         if (pose_graph) cudaGraphExecDestroy(pose_graph);
         if (track_graph) cudaGraphExecDestroy(track_graph);
         if (batch_pose_graph) cudaGraphExecDestroy(batch_pose_graph);
+        if (every_graph) cudaGraphExecDestroy(every_graph);
+        if (every_hand_graph) cudaGraphExecDestroy(every_hand_graph);
     }
     std::vector<ScaleDims> dims;
     std::vector<U8Taps> u8taps;
@@ -416,6 +426,30 @@ struct opb_session {
     std::vector<double> pose_hand_scales;
     bool pose_fixed = false;
     int batch_pose_box = 0;              // boxsize of the opb_batch_pose batch in flight; 0: an opb_pose batch
+    // every person of a batch (opb_pose_every_*), on a body session: the records and the compacted hand boxes, grown to
+    // the largest person count seen, and the boxes of one hand chunk
+    struct EveryBuffers {
+        DevPool pool;
+        int cap = 0;                 // records; the box list holds 2 * cap
+        uint64_t gen = 0;            // unique per allocation (graph keys)
+        double* records = nullptr;   // [cap][60][3]
+        HandBox* list = nullptr;     // [2 cap] in util.handDetect's order
+        int* list_rec = nullptr;     // [2 cap] record of each box
+        int* counts = nullptr;       // [kEveryCounts] persons, boxes, chunk cursor
+        HandBox* chunk_boxes = nullptr;  // [kEveryChunk]
+        int* chunk_dims = nullptr;       // [kEveryChunk]
+        int* chunk_rec = nullptr;        // [kEveryChunk]
+        double* records_host = nullptr;  // pinned [cap][60][3]
+        int* counts_host = nullptr;      // pinned [kEveryCounts]
+        ~EveryBuffers() {
+            if (records_host) cudaFreeHost(records_host);
+            if (counts_host) cudaFreeHost(counts_host);
+        }
+    };
+    std::unique_ptr<EveryBuffers> every;
+    uint64_t every_allocs = 0;
+    bool every_batch = false;            // the batch in flight is an opb_pose_every batch
+    int every_persons = -1;              // persons of the last finished opb_pose_every batch; -1: none
     ~opb_session() {
         plans.clear();
         net_plans.clear();
@@ -809,6 +843,10 @@ static bool grow_and_redo(opb_session* s, FramePlan* fp, int f, int appended, in
         cudaGraphExecDestroy(fp->batch_pose_graph);
         fp->batch_pose_graph = nullptr;
     }
+    if (fp->every_graph) {
+        cudaGraphExecDestroy(fp->every_graph);
+        fp->every_graph = nullptr;
+    }
     const bool prof = s->prof.on;
     s->prof.on = false;
     body_post_range(s, fp, f, 1, fp->key.H, fp->key.W);
@@ -1129,6 +1167,17 @@ static void build_ragged_tables(opb_session* hs, const double* scales, int ns, i
     hs->ragged = std::move(r);
 }
 
+// the hand session's ragged tables cover every crop of an H x W frame at these scales; returns their crop side limit, the
+// plane pitch of the ragged buffers
+static int ensure_ragged_tables(opb_session* bs, opb_session* hs, int H, int W, const double* hscales, int nhs) {
+    const int wmax = std::min(H, W);
+    if (!hs->ragged || hs->ragged->tabs.wmax < wmax || hs->ragged->scales != std::vector<double>(hscales, hscales + nhs)) {
+        OPB_CUDA(cudaStreamSynchronize(bs->stream));
+        build_ragged_tables(hs, hscales, nhs, wmax);
+    }
+    return hs->ragged->tabs.wmax;
+}
+
 // per-batch [n][60][3] records, hand boxes and their pinned host copy on a body session, grown to the largest batch seen
 static void ensure_pose_buffers(opb_session* bs, int n) {
     if (bs->pose && bs->pose->frames >= n) return;
@@ -1144,25 +1193,33 @@ static void ensure_pose_buffers(opb_session* bs, int n) {
     bs->pose = std::move(pb);
 }
 
-// the hand half of the pose pipeline, on the body session's stream: boxes from the body results (or the fixed ones already
-// in the pinned buffer), ragged crops -> hand CNN -> ragged post-processing -> PoseMat -> pinned host buffer
-static void pose_hand_enqueue(opb_session* bs, opb_session* hs, FramePlan* fp, FramePlan* hp, int n, int H, int W, bool fixed) {
-    cudaStream_t st = bs->stream;
+// Hand on `slots` boxes (dims: side of each valid box, else 0) of the frames `fp` holds, as one ragged batch on the hand
+// plan `hp` of hs: crops cut -- the left ones mirrored -- from the frames -> hand CNN -> ragged post-processing, the
+// key points of slot i at hp->hb.peaks + i * 63
+static void ragged_hand_enqueue(cudaStream_t st, opb_session* hs, FramePlan* fp, FramePlan* hp, const HandBox* boxes,
+                                const int* dims, int slots) {
     const opb_session::Ragged& rg = *hs->ragged;
-    const int slots = 2 * n, tw = rg.tabs.wmax, nhs = rg.tabs.n_scales;
-    if (fixed)
-        OPB_CUDA(cudaMemcpyAsync(bs->pose->fixed, bs->pose->fixed_host, (size_t)n * 6 * sizeof(int), cudaMemcpyHostToDevice, st));
-    pose_select_launch(fp->post_dev, n, H, W, fixed ? bs->pose->fixed : nullptr, bs->pose->pose, bs->pose->boxes, bs->pose->dims, st);
+    const int tw = rg.tabs.wmax, nhs = rg.tabs.n_scales;
     const float* src[kMaxScales];
     int ho[kMaxScales], wo[kMaxScales];
     for (int s = 0; s < nhs; ++s) {
-        preprocess_ragged_launch(fp->d_img, H, W, bs->pose->boxes, slots, hp->net->in_u8[s], rg.net_side[s], s, rg.tabs, st);
+        preprocess_ragged_launch(fp->d_img, fp->key.H, fp->key.W, boxes, slots, hp->net->in_u8[s], rg.net_side[s], s, rg.tabs, st);
         src[s] = hp->net->out_heat[s];
         ho[s] = wo[s] = rg.net_side[s] / 8;
     }
     hp->net->run(st, nullptr);
-    upsample_ragged_launch(src, ho, wo, nhs, 24, 22, bs->pose->boxes, slots, rg.tabs, tw, hp->up_scratch, hp->heat_avg, st);
-    hand_peaks_ragged_launch(hp->heat_avg, slots, 22, bs->pose->dims, tw, 0.03, hp->hb, st);      // thre, src/hand.py:31
+    upsample_ragged_launch(src, ho, wo, nhs, 24, 22, boxes, slots, rg.tabs, tw, hp->up_scratch, hp->heat_avg, st);
+    hand_peaks_ragged_launch(hp->heat_avg, slots, 22, dims, tw, 0.03, hp->hb, st);      // thre, src/hand.py:31
+}
+
+// the hand half of the pose pipeline, on the body session's stream: boxes from the body results (or the fixed ones already
+// in the pinned buffer), ragged crops -> hand CNN -> ragged post-processing -> PoseMat -> pinned host buffer
+static void pose_hand_enqueue(opb_session* bs, opb_session* hs, FramePlan* fp, FramePlan* hp, int n, int H, int W, bool fixed) {
+    cudaStream_t st = bs->stream;
+    if (fixed)
+        OPB_CUDA(cudaMemcpyAsync(bs->pose->fixed, bs->pose->fixed_host, (size_t)n * 6 * sizeof(int), cudaMemcpyHostToDevice, st));
+    pose_select_launch(fp->post_dev, n, H, W, fixed ? bs->pose->fixed : nullptr, bs->pose->pose, bs->pose->boxes, bs->pose->dims, st);
+    ragged_hand_enqueue(st, hs, fp, hp, bs->pose->boxes, bs->pose->dims, 2 * n);
     pose_finish_launch(bs->pose->boxes, hp->hb.peaks, n, bs->pose->pose, st);
     OPB_CUDA(cudaMemcpyAsync(bs->pose->host, bs->pose->pose, (size_t)n * 180 * sizeof(double), cudaMemcpyDeviceToHost, st));
 }
@@ -1173,12 +1230,8 @@ static void pose_submit(opb_session* bs, opb_session* hs, const uint8_t* imgs, i
     OPB_REQUIRE(bs->net->ctx == hs->net->ctx, "pose: both networks must live on the same context");
     OPB_REQUIRE(n >= 1 && n <= 64, "1..64 frames per batch");
     OPB_CUDA(cudaSetDevice(bs->net->ctx->device));
-    const int wmax = std::min(H, W), slots = 2 * n;
-    if (!hs->ragged || hs->ragged->tabs.wmax < wmax || hs->ragged->scales != std::vector<double>(hscales, hscales + nhs)) {
-        OPB_CUDA(cudaStreamSynchronize(bs->stream));
-        build_ragged_tables(hs, hscales, nhs, wmax);
-    }
-    const int tw = hs->ragged->tabs.wmax;                       // plane pitch of the ragged buffers
+    const int slots = 2 * n;
+    const int tw = ensure_ragged_tables(bs, hs, H, W, hscales, nhs);
     ensure_pose_buffers(bs, n);
     // body part: as opb_body_submit_batch
     FramePlan* fp = get_plan(bs, n, H, W, bscales, nbs);
@@ -1187,6 +1240,7 @@ static void pose_submit(opb_session* bs, opb_session* hs, const uint8_t* imgs, i
     bs->n_frames = n;
     bs->pose_hand = hs;
     bs->batch_pose_box = 0;
+    bs->every_batch = false;
     cudaStream_t st = bs->stream;
     upload_image(bs, fp, imgs, where, (size_t)n * H * W * 3);
     // hand part on the same stream, with the hand session's CNN plan and work buffers (sized for the largest crop)
@@ -1289,6 +1343,7 @@ static void batch_pose_submit(opb_session* bs, opb_session* hs, const uint8_t* f
     bs->n_frames = n;
     bs->pose_hand = hs;
     bs->batch_pose_box = boxsize;
+    bs->every_batch = false;
     const double one = 1.0;
     FramePlan* hp = get_plan(hs, 2 * n, boxsize, boxsize, &one, 1, 2);      // uint8 Batch_hand on 2n crops
     hs->active = hp;
@@ -1311,6 +1366,129 @@ static void batch_pose_submit(opb_session* bs, opb_session* hs, const uint8_t* f
     });
     OPB_CUDA(cudaEventRecord(bs->done, st));
     bs->net->ctx->launches += fp->launches_per_frame + 3 /* select, crops, finish */ + hp->launches_per_frame;
+}
+
+// ------------------------------------------------------------------------------------------------
+// every person of every frame: Body, util.handDetect on every subset row (src/util.py:133-201), Hand on every box --
+// the caller's host loop on the reference's Body / Hand, with the PoseMat arithmetic of MotionEstimation.py:185-194
+// ------------------------------------------------------------------------------------------------
+// Hand slots per chunk.  The ragged hand buffers grow with slots x min(H, W)^2; 8 slots are half of what
+// opb_pose_submit_batch holds at 8 frames (16 slots).  The CNN runs on every slot of a chunk, the empty ones of the
+// last chunk too, so a smaller chunk wastes less on a batch with few hands.
+constexpr int kEveryChunk = 8;
+
+// records and box list for `persons` persons (grown by doubling; OPB_TEST_SMALL_BUFFERS starts tiny so that tests reach
+// the growth path of opb_pose_every_wait)
+static void ensure_every_buffers(opb_session* bs, int persons) {
+    if (bs->every && bs->every->cap >= persons) return;
+    static const bool tiny = getenv("OPB_TEST_SMALL_BUFFERS") != nullptr;
+    int cap = bs->every ? 2 * bs->every->cap : (tiny ? 2 : 512);
+    while (cap < persons) cap *= 2;
+    OPB_CUDA(cudaStreamSynchronize(bs->stream));
+    auto e = std::make_unique<opb_session::EveryBuffers>();
+    e->cap = cap;
+    e->gen = ++bs->every_allocs;
+    e->records = e->pool.alloc_t<double>((size_t)cap * 180);
+    e->list = e->pool.alloc_t<HandBox>((size_t)cap * 2);
+    e->list_rec = e->pool.alloc_t<int>((size_t)cap * 2);
+    e->counts = e->pool.alloc_t<int>(kEveryCounts, true);
+    e->chunk_boxes = e->pool.alloc_t<HandBox>(kEveryChunk);
+    e->chunk_dims = e->pool.alloc_t<int>(kEveryChunk);
+    e->chunk_rec = e->pool.alloc_t<int>(kEveryChunk);
+    OPB_CUDA(cudaMallocHost((void**)&e->records_host, (size_t)cap * 180 * sizeof(double)));
+    OPB_CUDA(cudaMallocHost((void**)&e->counts_host, kEveryCounts * sizeof(int)));
+    bs->every = std::move(e);
+}
+
+// rows and boxes of every person from the body results of the batch; the counts to pinned memory
+static void every_rows_enqueue(opb_session* bs, FramePlan* fp, int n) {
+    opb_session::EveryBuffers& e = *bs->every;
+    every_rows_launch(fp->post_dev, n, fp->key.H, fp->key.W, e.cap, e.records, e.list, e.list_rec, e.counts, bs->stream);
+    OPB_CUDA(cudaMemcpyAsync(e.counts_host, e.counts, kEveryCounts * sizeof(int), cudaMemcpyDeviceToHost, bs->stream));
+}
+
+// one chunk of the hand half: the next kEveryChunk boxes of the list (the cursor lives on the device, so the same launch
+// sequence -- one CUDA graph -- serves every chunk of every batch), Hand on them, key points into their records
+static void every_chunk_enqueue(opb_session* bs, opb_session* hs, FramePlan* fp, FramePlan* hp) {
+    cudaStream_t st = bs->stream;
+    opb_session::EveryBuffers& e = *bs->every;
+    every_stage_launch(e.list, e.list_rec, e.counts, kEveryChunk, e.chunk_boxes, e.chunk_dims, e.chunk_rec, st);
+    ragged_hand_enqueue(st, hs, fp, hp, e.chunk_boxes, e.chunk_dims, kEveryChunk);
+    every_finish_launch(e.chunk_boxes, e.chunk_rec, hp->hb.peaks, kEveryChunk, e.records, e.counts, st);
+}
+
+static void every_submit(opb_session* bs, opb_session* hs, const uint8_t* imgs, int where, int n, int H, int W,
+                         const double* bscales, int nbs, const double* hscales, int nhs) {
+    OPB_REQUIRE(bs->net->kind == OPB_NET_BODY && hs->net->kind == OPB_NET_HAND, "every person: a body session and a hand session");
+    OPB_REQUIRE(bs->net->ctx == hs->net->ctx, "every person: both networks must live on the same context");
+    OPB_REQUIRE(n >= 1 && n <= 64, "1..64 frames per batch");
+    OPB_REQUIRE(H >= 1 && W >= 1, "empty frame");
+    OPB_CUDA(cudaSetDevice(bs->net->ctx->device));
+    cudaStream_t st = bs->stream;
+    const int tw = ensure_ragged_tables(bs, hs, H, W, hscales, nhs);
+    ensure_every_buffers(bs, 0);
+    FramePlan* fp = get_plan(bs, n, H, W, bscales, nbs);
+    ensure_host(bs, n, 0);
+    bs->active = fp;
+    bs->n_frames = n;
+    bs->pose_hand = hs;
+    bs->batch_pose_box = 0;
+    bs->every_batch = true;
+    bs->every_persons = -1;
+    upload_image(bs, fp, imgs, where, (size_t)n * H * W * 3);
+    // the hand plan of the chunks, with the hand session's work buffers sized for the largest crop
+    OPB_CUDA(cudaStreamSynchronize(hs->stream));
+    FramePlan* hp = get_plan(hs, kEveryChunk, tw, tw, hscales, nhs);
+    hs->active = hp;
+    hs->hand_crops = kEveryChunk;
+    const uint64_t gen = gen_key({bs->buffer_gen, bs->every->gen});
+    run_or_replay_slot(bs, GraphSlot{fp->every_graph, fp->every_gen, fp->every_uses}, gen, [&] {
+        run_front(bs, fp, n, H, W);
+        body_post_enqueue(bs, fp, n, H, W);
+        every_rows_enqueue(bs, fp, n);
+    });
+    OPB_CUDA(cudaEventRecord(bs->done, st));
+    bs->net->ctx->launches += fp->launches_per_frame + 1;
+}
+
+// Body overflow check (frames that overflowed are grown and redone, then the rows-and-boxes kernel runs again), records
+// grown to the person count, ceil(V / kEveryChunk) hand chunks, one copy of the T records.  persons: n ints.
+static int every_wait(opb_session* bs, int* persons, int* frame_status) {
+    OPB_REQUIRE(bs->active && bs->every && bs->every_batch && bs->pose_hand, "no every-person batch in flight");
+    OPB_CUDA(cudaSetDevice(bs->net->ctx->device));
+    cudaStream_t st = bs->stream;
+    FramePlan* fp = bs->active;
+    const int n = bs->n_frames;
+    bool again = false;
+    const int rc = pose_batch_status(bs, frame_status, again);
+    for (;;) {
+        if (again) {
+            every_rows_enqueue(bs, fp, n);
+            OPB_CUDA(cudaStreamSynchronize(st));
+        }
+        if (bs->every->counts_host[0] <= bs->every->cap) break;
+        ensure_every_buffers(bs, bs->every->counts_host[0]);
+        again = true;
+    }
+    opb_session::EveryBuffers& e = *bs->every;
+    const int T = e.counts_host[0], V = e.counts_host[1];
+    if (V > 0) {
+        opb_session* hs = bs->pose_hand;
+        FramePlan* hp = hs->active;
+        const opb_session::Ragged& rg = *hs->ragged;
+        const uint64_t gen = gen_key({bs->buffer_gen, hs->buffer_gen, (uint64_t)(uintptr_t)hp, (uint64_t)(uintptr_t)rg.tabs.slab,
+                                      (uint64_t)rg.tabs.wmax, e.gen, (uint64_t)(uintptr_t)fp->d_img});
+        for (int base = 0; base < V; base += kEveryChunk)
+            run_or_replay_slot(bs, GraphSlot{fp->every_hand_graph, fp->every_hand_gen, fp->every_hand_uses}, gen,
+                               [&] { every_chunk_enqueue(bs, hs, fp, hp); });
+        const int nhs = rg.tabs.n_scales;
+        bs->net->ctx->launches += (int64_t)cdiv(V, kEveryChunk) * (1 + nhs + hp->net->kernel_launches + (nhs + 1) + 6 + 1);
+    }
+    if (T > 0) OPB_CUDA(cudaMemcpyAsync(e.records_host, e.records, (size_t)T * 180 * sizeof(double), cudaMemcpyDeviceToHost, st));
+    OPB_CUDA(cudaStreamSynchronize(st));
+    for (int f = 0; f < n; ++f) persons[f] = e.counts_host[kEveryFrameCounts + f];
+    bs->every_persons = T;
+    return rc;
 }
 
 }  // namespace opb
@@ -1660,7 +1838,7 @@ int opb_pose_submit_batch(opb_session* body_s, opb_session* hand_s, const uint8_
 int opb_pose_wait(opb_session* body_s, double* pose_mats, int* frame_status) {
     int rc = OPB_OK;
     int g = guarded([&] {
-        OPB_REQUIRE(body_s && pose_mats && body_s->pose && body_s->active && !body_s->batch_pose_box,
+        OPB_REQUIRE(body_s && pose_mats && body_s->pose && body_s->active && !body_s->batch_pose_box && !body_s->every_batch,
                     "no pose batch in flight");
         // body results first: they report the overflow / IndexError conditions of every frame
         bool grew = false;
@@ -1688,8 +1866,8 @@ int opb_batch_pose_submit(opb_session* body_s, opb_session* hand_s, const uint8_
 int opb_batch_pose_wait(opb_session* body_s, double* motion_mats, double* hand_mats, int* frame_status) {
     int rc = OPB_OK;
     int g = guarded([&] {
-        OPB_REQUIRE(body_s && motion_mats && hand_mats && body_s->pose && body_s->active && body_s->batch_pose_box,
-                    "no batch-pose batch in flight");
+        OPB_REQUIRE(body_s && motion_mats && hand_mats && body_s->pose && body_s->active && body_s->batch_pose_box &&
+                        !body_s->every_batch, "no batch-pose batch in flight");
         OPB_CUDA(cudaSetDevice(body_s->net->ctx->device));
         bool grew = false;
         rc = pose_batch_status(body_s, frame_status, grew);
@@ -1705,6 +1883,38 @@ int opb_batch_pose_wait(opb_session* body_s, double* motion_mats, double* hand_m
         }
     });
     return g != OPB_OK ? g : rc;
+}
+
+/* ---- every person of every frame ------------------------------------------------------------------------------- */
+int opb_pose_every_submit(opb_session* body_s, opb_session* hand_s, const uint8_t* imgs_bgr, int where, int n_frames,
+                          int height, int width, const double* body_scales, int n_body_scales, const double* hand_scales,
+                          int n_hand_scales) {
+    return guarded([&] {
+        OPB_REQUIRE(body_s && hand_s && imgs_bgr && body_scales && hand_scales, "null argument");
+        OPB_REQUIRE(where >= 0 && where <= 2, "where: 0 pageable host, 1 device, 2 pinned host");
+        OPB_REQUIRE(n_hand_scales >= 1 && n_hand_scales <= kMaxScales, "1..8 hand scales");
+        every_submit(body_s, hand_s, imgs_bgr, where, n_frames, height, width, body_scales, n_body_scales, hand_scales,
+                     n_hand_scales);
+    });
+}
+int opb_pose_every_wait(opb_session* body_s, int* persons, int* frame_status) {
+    int rc = OPB_OK;
+    int g = guarded([&] {
+        OPB_REQUIRE(body_s && persons, "null argument");
+        rc = every_wait(body_s, persons, frame_status);
+    });
+    return g != OPB_OK ? g : rc;
+}
+int opb_pose_every_fetch(opb_session* body_s, double* records, int rows) {
+    return guarded([&] {
+        OPB_REQUIRE(body_s && body_s->every && body_s->every_persons >= 0, "no finished every-person batch");
+        const int T = body_s->every_persons;
+        if (rows < T) throw Error(OPB_ERR_CAPACITY, "records buffer smaller than the result");
+        if (T) {
+            OPB_REQUIRE(records != nullptr, "null records buffer");
+            memcpy(records, body_s->every->records_host, (size_t)T * 180 * sizeof(double));
+        }
+    });
 }
 
 int opb_hand_submit(opb_session* s, const uint8_t* crops, int img_is_device, int n, int H, int W, const double* scales, int ns) {
@@ -1978,6 +2188,53 @@ int opb_pose_select(opb_context* ctx, const double* host_candidates, int n_candi
             host_boxes8[k * 4 + 1] = hb[k].y;
             host_boxes8[k * 4 + 2] = hb[k].w;
             host_boxes8[k * 4 + 3] = hb[k].valid;
+        }
+    });
+}
+
+/* stage-level: rows and boxes of every person (pose.cu) on host-provided body results of one frame */
+int opb_pose_every_select(opb_context* ctx, const double* host_candidates, int n_candidates, const double* host_subset,
+                          int n_subset, int H, int W, double* host_records, int* host_boxes) {
+    return guarded([&] {
+        OPB_REQUIRE(ctx && n_candidates >= 0 && n_subset >= 0, "bad arguments");
+        OPB_REQUIRE(n_subset == 0 || (host_candidates && host_subset && host_records && host_boxes), "null argument");
+        OPB_CUDA(cudaSetDevice(ctx->device));
+        const int cap = std::max(n_subset, 1);
+        StagePost sp;
+        sp.create(std::max(n_candidates, 1), 1, 1, cap, nullptr, ctx->stream);
+        OPB_CUDA(cudaMemcpyAsync(sp.host.lb.subset_count, &n_subset, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+        if (n_candidates)
+            OPB_CUDA(cudaMemcpyAsync(sp.host.pb.candidates, host_candidates, (size_t)n_candidates * 32, cudaMemcpyHostToDevice, ctx->stream));
+        if (n_subset)
+            OPB_CUDA(cudaMemcpyAsync(sp.host.lb.subset, host_subset, (size_t)n_subset * 160, cudaMemcpyHostToDevice, ctx->stream));
+        DevPool pool;
+        double* records = pool.alloc_t<double>((size_t)cap * 180);
+        HandBox* list = pool.alloc_t<HandBox>((size_t)cap * 2);
+        int* list_rec = pool.alloc_t<int>((size_t)cap * 2);
+        int* counts = pool.alloc_t<int>(kEveryCounts);
+        every_rows_launch(sp.dev, 1, H, W, cap, records, list, list_rec, counts, ctx->stream);
+        ctx->launches += 1;
+        std::vector<HandBox> hb((size_t)cap * 2);
+        std::vector<int> hr((size_t)cap * 2);
+        int hc[kEveryCounts];
+        OPB_CUDA(cudaMemcpyAsync(hc, counts, sizeof(hc), cudaMemcpyDeviceToHost, ctx->stream));
+        OPB_CUDA(cudaMemcpyAsync(hb.data(), list, hb.size() * sizeof(HandBox), cudaMemcpyDeviceToHost, ctx->stream));
+        OPB_CUDA(cudaMemcpyAsync(hr.data(), list_rec, hr.size() * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+        if (n_subset)
+            OPB_CUDA(cudaMemcpyAsync(host_records, records, (size_t)n_subset * 180 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        OPB_CUDA(cudaStreamSynchronize(ctx->stream));
+        OPB_REQUIRE(hc[0] == n_subset && hc[1] <= 2 * n_subset, "every-person rows: unexpected counts");
+        for (int i = 0; i < 2 * n_subset; ++i) {
+            int* b = host_boxes + (size_t)i * 5;
+            if (i < hc[1]) {
+                b[0] = hb[i].x;
+                b[1] = hb[i].y;
+                b[2] = hb[i].w;
+                b[3] = hb[i].left;
+                b[4] = hr[i];
+            } else {
+                b[0] = b[1] = b[2] = b[3] = b[4] = -1;
+            }
         }
     });
 }

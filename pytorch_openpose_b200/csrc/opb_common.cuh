@@ -353,6 +353,31 @@ __host__ __device__ inline void pose_hand_boxes(const double* pose, int frame, i
                             pose[(j0 + 2) * 3 + 1], H, W, b);
     }
 }
+// the 18 body rows (x, y, score) of one subset row into body54: candidate[subset[k]][:3]; rows of missing joints (-1)
+// are left as they are (the callers zero them first)
+__device__ inline void person_rows(const double* cand, const double* row, double* body54) {
+    for (int k = 0; k < 18; ++k) {
+        const int idx = (int)row[k];
+        if (idx != -1) {
+            body54[k * 3 + 0] = cand[(size_t)idx * 4 + 0];
+            body54[k * 3 + 1] = cand[(size_t)idx * 4 + 1];
+            body54[k * 3 + 2] = cand[(size_t)idx * 4 + 2];
+        }
+    }
+}
+// util.handDetect (src/util.py:133-201) on one subset row: hand k (0 left: shoulder / elbow / wrist 5, 6, 7; 1 right:
+// 2, 3, 4).  Returns false, leaving b untouched, when one of the three joints is missing -- handDetect returns no box
+// then; otherwise fills x, y, w and valid (b.valid = w > 0: the reference's Hand raises on an empty crop).
+__device__ inline bool subset_hand_box(const double* cand, const double* row, int k, int H, int W, HandBox& b) {
+    const int j0 = k == 0 ? 5 : 2;
+    const int is = (int)row[j0], ie = (int)row[j0 + 1], iw = (int)row[j0 + 2];
+    if (is == -1 || ie == -1 || iw == -1) return false;
+    const double x1 = cand[(size_t)is * 4], y1 = cand[(size_t)is * 4 + 1];
+    const double x2 = cand[(size_t)ie * 4], y2 = cand[(size_t)ie * 4 + 1];
+    const double x3 = cand[(size_t)iw * 4], y3 = cand[(size_t)iw * 4 + 1];
+    hand_detect_box(x1, y1, x2, y2, x3, y3, H, W, b);
+    return true;
+}
 // the person with the largest left-shoulder x among the body results of one frame (srcmx/MotionEstimation.py:141-158,
 // srcmx/Batch_motion_Estimation.py:86-105): a missing shoulder (-1) indexes the LAST candidate, like candidate[-1];
 // np.argmax keeps the first maximum.  Writes the person's 18 body rows (x, y, score) into body54 -- rows of missing
@@ -375,14 +400,7 @@ __device__ inline const double* select_person_rows(const FramePost& fr, double* 
     }
     if (chosen < 0) return nullptr;
     const double* row = subset + (size_t)chosen * 20;
-    for (int k = 0; k < 18; ++k) {
-        const int idx = (int)row[k];
-        if (idx != -1) {
-            body54[k * 3 + 0] = cand[(size_t)idx * 4 + 0];
-            body54[k * 3 + 1] = cand[(size_t)idx * 4 + 1];
-            body54[k * 3 + 2] = cand[(size_t)idx * 4 + 2];
-        }
-    }
+    person_rows(cand, row, body54);
     return row;
 }
 
@@ -413,6 +431,20 @@ void hand_track_finish_launch(const HandBox* boxes_dev, const double* hand_peaks
 // [60][3] record (rows 18-59 zeroed) and both hand boxes derived from those rows as from a saved pose
 void batch_pose_select_launch(const FramePost* frames_dev, int n_frames, int H, int W, double* records_dev,
                               HandBox* boxes_dev, cudaStream_t stream);
+// every person of every frame (pose.cu).  Rows and boxes: one [60][3] record per subset row (body rows filled, hand
+// rows zero), records of frame f from the prefix of the person counts of frames 0..f-1; the boxes util.handDetect
+// returns, compacted in its order (frame, person, left before right) into `list` with their record in `list_rec`.
+// Records beyond `cap` and boxes beyond 2 * cap are not written.  counts: [0] persons T, [1] boxes V, [2] the chunk
+// cursor, reset to 0, [kEveryFrameCounts + f] persons of frame f.  n_frames <= 64.
+constexpr int kEveryFrameCounts = 4, kEveryCounts = kEveryFrameCounts + 64;
+void every_rows_launch(const FramePost* frames_dev, int n_frames, int H, int W, int cap, double* records, HandBox* list,
+                       int* list_rec, int* counts, cudaStream_t stream);
+// one hand chunk: slots [counts[2], counts[2] + C) of the list into boxes / dims / rec (invalid past V); after the hand
+// network, the finish scatters each slot's 21 key points into its record and advances counts[2] by C
+void every_stage_launch(const HandBox* list, const int* list_rec, const int* counts, int C, HandBox* boxes, int* dims, int* rec,
+                        cudaStream_t stream);
+void every_finish_launch(const HandBox* boxes, const int* rec, const double* hand_peaks_dev, int C, double* records,
+                         int* counts, cudaStream_t stream);
 
 // ---- gaussian taps shared by peaks.cu / hand.cu: scipy.ndimage.gaussian_filter(sigma=3) uses
 // radius int(4*3+0.5) = 12 and weights exp(-x^2/18) / sum (src/body.py:75, src/hand.py:62).  The

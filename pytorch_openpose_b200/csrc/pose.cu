@@ -29,18 +29,9 @@ __global__ void pose_select_kernel(const FramePost* __restrict__ frames, int n_f
         hb[k].valid = 0;
     }
     if (row) {
-        // util.handDetect on the chosen person (the caller blanks all other rows first, MotionEstimation.py:160-162):
-        // left hand from shoulder / elbow / wrist 5, 6, 7, right hand from 2, 3, 4
-        for (int k = 0; k < 2; ++k) {
-            const int j0 = k == 0 ? 5 : 2;
-            const int is = (int)row[j0], ie = (int)row[j0 + 1], iw = (int)row[j0 + 2];
-            if (is == -1 || ie == -1 || iw == -1) continue;
-            const double x1 = cand[(size_t)is * 4], y1 = cand[(size_t)is * 4 + 1];
-            const double x2 = cand[(size_t)ie * 4], y2 = cand[(size_t)ie * 4 + 1];
-            const double x3 = cand[(size_t)iw * 4], y3 = cand[(size_t)iw * 4 + 1];
-            // an empty box is invalid: the reference's Hand divides by the crop height, it raises there
-            hand_detect_box(x1, y1, x2, y2, x3, y3, H, W, hb[k]);
-        }
+        // util.handDetect on the chosen person (the caller blanks all other rows first, MotionEstimation.py:160-162);
+        // an empty box is invalid: the reference's Hand divides by the crop height, it raises there
+        for (int k = 0; k < 2; ++k) subset_hand_box(cand, row, k, H, W, hb[k]);
     }
     if (fixed_boxes) {                        // benchmarks / tests: random weights find nobody
         for (int k = 0; k < 2; ++k) {
@@ -58,8 +49,19 @@ __global__ void pose_select_kernel(const FramePost* __restrict__ frames, int n_f
     }
 }
 
-// hand key points of slot (frame, k) -> PoseMat rows (MotionEstimation.py:185-194): coordinate 0 means "missing" and
-// is not offset; left hands were mirrored: x -> w - x - 1 + x0
+// one hand key point p (x, y, score) of the crop of box b -> its PoseMat row (MotionEstimation.py:185-194): coordinate 0
+// means "missing" and is not offset; left hands were mirrored: x -> w - x - 1 + x0
+__device__ __forceinline__ void hand_point_to_frame(const HandBox& b, const double* p, double* out) {
+    double x = p[0], y = p[1];
+    if (b.left) x = x == 0 ? x : __dadd_rn(__dadd_rn((double)b.w - x, -1.0), (double)b.x);
+    else x = x == 0 ? x : __dadd_rn(x, (double)b.x);
+    y = y == 0 ? y : __dadd_rn(y, (double)b.y);
+    out[0] = x;
+    out[1] = y;
+    out[2] = p[2];
+}
+
+// hand key points of slot (frame, k) -> PoseMat rows
 __global__ void pose_finish_kernel(const HandBox* __restrict__ boxes, const double* __restrict__ peaks, int n_frames,
                                    double* __restrict__ pose) {
     const int slot = blockIdx.x;
@@ -69,14 +71,7 @@ __global__ void pose_finish_kernel(const HandBox* __restrict__ boxes, const doub
     const int f = slot >> 1;
     double* out = pose + (size_t)f * 180 + (size_t)((b.left ? 18 : 39) + j) * 3;
     if (!b.valid) return;                     // rows stay zero
-    const double* p = peaks + ((size_t)slot * 21 + j) * 3;
-    double x = p[0], y = p[1];
-    if (b.left) x = x == 0 ? x : __dadd_rn(__dadd_rn((double)b.w - x, -1.0), (double)b.x);
-    else x = x == 0 ? x : __dadd_rn(x, (double)b.x);
-    y = y == 0 ? y : __dadd_rn(y, (double)b.y);
-    out[0] = x;
-    out[1] = y;
-    out[2] = p[2];
+    hand_point_to_frame(b, peaks + ((size_t)slot * 21 + j) * 3, out);
 }
 
 // ---- the batched hand job (srcmx/Batch_motion_Estimation.py:19-63) on saved body poses
@@ -128,7 +123,123 @@ __global__ void batch_pose_select_kernel(const FramePost* __restrict__ frames, i
     boxes[2 * f + 1] = hb[1];
 }
 
+// ---- every person of every frame (the host loop Body -> util.handDetect -> Hand per box, src/util.py:133-201)
+// One block, one thread per frame (n <= 64): person and box counts of every frame, their prefixes, then each thread
+// writes its frame's records and boxes.  A frame holds a handful of persons; the loops are a few dozen scalar
+// operations per person.
+constexpr int kEveryMaxFrames = 64;
+__global__ void __launch_bounds__(kEveryMaxFrames) every_rows_kernel(const FramePost* __restrict__ frames, int n_frames,
+                                                                     int H, int W, int cap, double* __restrict__ records,
+                                                                     HandBox* __restrict__ list, int* __restrict__ list_rec,
+                                                                     int* __restrict__ counts) {
+    __shared__ int s_rec[kEveryMaxFrames + 1], s_box[kEveryMaxFrames + 1];
+    const int f = threadIdx.x;
+    int persons = 0, boxes = 0;
+    if (f < n_frames) {
+        const FramePost& fr = frames[f];
+        persons = min(*fr.lb.subset_count, fr.lb.subset_capacity);
+        for (int p = 0; p < persons; ++p) {
+            const double* row = fr.lb.subset + (size_t)p * 20;
+            for (int k = 0; k < 2; ++k) {
+                const int j0 = k == 0 ? 5 : 2;
+                boxes += (int)row[j0] != -1 && (int)row[j0 + 1] != -1 && (int)row[j0 + 2] != -1;
+            }
+        }
+    }
+    s_rec[f + 1] = persons;
+    s_box[f + 1] = boxes;
+    if (f < n_frames) counts[kEveryFrameCounts + f] = persons;
+    __syncthreads();
+    if (f == 0) {
+        s_rec[0] = s_box[0] = 0;
+        for (int i = 1; i <= n_frames; ++i) {
+            s_rec[i] += s_rec[i - 1];
+            s_box[i] += s_box[i - 1];
+        }
+        counts[0] = s_rec[n_frames];
+        counts[1] = s_box[n_frames];
+        counts[2] = 0;
+    }
+    __syncthreads();
+    if (f >= n_frames) return;
+    const FramePost& fr = frames[f];
+    const double* cand = fr.pb.candidates;
+    int v = s_box[f];
+    for (int p = 0; p < persons; ++p) {
+        const int r = s_rec[f] + p;
+        const double* row = fr.lb.subset + (size_t)p * 20;
+        if (r < cap) {
+            double* rec = records + (size_t)r * 180;
+            for (int i = 0; i < 180; ++i) rec[i] = 0.0;
+            person_rows(cand, row, rec);
+        }
+        for (int k = 0; k < 2; ++k) {
+            HandBox b;
+            b.frame = f;
+            b.left = k == 0;
+            if (!subset_hand_box(cand, row, k, H, W, b)) continue;
+            if (v < 2 * cap) {
+                list[v] = b;
+                list_rec[v] = r;
+            }
+            ++v;
+        }
+    }
+}
+
+// slot i of the chunk <- entry counts[2] + i of the list; past the box count an invalid box (grey crop, no rows)
+__global__ void every_stage_kernel(const HandBox* __restrict__ list, const int* __restrict__ list_rec,
+                                   const int* __restrict__ counts, int C, HandBox* __restrict__ boxes, int* __restrict__ dims,
+                                   int* __restrict__ rec) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= C) return;
+    const int v = counts[2] + i;
+    HandBox b{};
+    int r = -1;
+    if (v < counts[1]) {
+        b = list[v];
+        r = list_rec[v];
+    }
+    boxes[i] = b;
+    dims[i] = b.valid ? b.w : 0;
+    rec[i] = r;
+}
+
+// the 21 key points of slot `blockIdx.x` into its record (the pose_finish_kernel arithmetic); then the cursor moves on
+// to the next chunk -- only this thread touches it, and the next chunk's stage kernel runs after this kernel
+__global__ void every_finish_kernel(const HandBox* __restrict__ boxes, const int* __restrict__ rec,
+                                    const double* __restrict__ peaks, int C, double* __restrict__ records,
+                                    int* __restrict__ counts) {
+    const int slot = blockIdx.x;
+    const int j = threadIdx.x;
+    if (slot == 0 && j == 0) counts[2] += C;
+    if (j >= 21) return;
+    const HandBox b = boxes[slot];
+    if (!b.valid) return;                     // rows stay zero (no box, or a box of width <= 0)
+    double* out = records + (size_t)rec[slot] * 180 + (size_t)((b.left ? 18 : 39) + j) * 3;
+    hand_point_to_frame(b, peaks + ((size_t)slot * 21 + j) * 3, out);
+}
+
 }  // namespace
+
+void every_rows_launch(const FramePost* frames_dev, int n_frames, int H, int W, int cap, double* records, HandBox* list,
+                       int* list_rec, int* counts, cudaStream_t stream) {
+    OPB_REQUIRE(n_frames >= 1 && n_frames <= kEveryMaxFrames, "1..64 frames per batch");
+    every_rows_kernel<<<1, kEveryMaxFrames, 0, stream>>>(frames_dev, n_frames, H, W, cap, records, list, list_rec, counts);
+    OPB_CUDA(cudaGetLastError());
+}
+
+void every_stage_launch(const HandBox* list, const int* list_rec, const int* counts, int C, HandBox* boxes, int* dims, int* rec,
+                        cudaStream_t stream) {
+    every_stage_kernel<<<cdiv(C, 32), 32, 0, stream>>>(list, list_rec, counts, C, boxes, dims, rec);
+    OPB_CUDA(cudaGetLastError());
+}
+
+void every_finish_launch(const HandBox* boxes, const int* rec, const double* hand_peaks_dev, int C, double* records,
+                         int* counts, cudaStream_t stream) {
+    every_finish_kernel<<<C, 32, 0, stream>>>(boxes, rec, hand_peaks_dev, C, records, counts);
+    OPB_CUDA(cudaGetLastError());
+}
 
 void hand_track_boxes_host(const double* pose, int H, int W, HandBox* boxes) { pose_hand_boxes(pose, 0, H, W, boxes); }
 

@@ -43,6 +43,7 @@ extern "C" {
 typedef struct opb_context opb_context; /* one per (process, GPU): stream + workspace arena          */
 typedef struct opb_net opb_net;         /* weights of one CNN, repacked for the device               */
 typedef struct opb_session opb_session; /* per-caller state: plans + buffers for one frame in flight */
+typedef struct opb_tracker opb_tracker; /* person tracks of one video (opb_tracker_*)               */
 
 int opb_abi_version(void);
 const char* opb_last_error(void);
@@ -156,6 +157,28 @@ int opb_pose_every_submit(opb_session* body_s, opb_session* hand_s, const uint8_
                           const double* hand_scales, int n_hand_scales);
 int opb_pose_every_wait(opb_session* body_s, int* persons, int* frame_status);
 int opb_pose_every_fetch(opb_session* body_s, double* records, int rows);
+/* ---- person tracks across frames ----------------------------------------------------------------------------------
+ * A tracker links the persons of consecutive frames into tracks with the rule of motion.PersonLinker (its docstring is
+ * the specification; the ids are bit-identical): presence = score > 0, cost = mean joint distance over the >= min_joints
+ * body joints present in both, eligible when <= max_dist, greedy matching on (cost, track id, person), unmatched persons
+ * open new tracks (ids 0, 1, ... in creation order, never reused), a track unmatched for more than max_gap frames is
+ * dropped.  One tracker follows one video: frames are linked in the order the calls return.  Calls on one tracker are
+ * serialised by a mutex and each ends in a stream synchronise, so two session pairs may alternate on it.
+ * create: max_gap >= 1, max_dist finite >= 0, 1 <= min_joints <= 18.  reset: forget every track (next frame 0, next
+ * id 0).  state: live tracks, next id, frames linked so far (each pointer optional).
+ * wait_tracked: opb_pose_every_wait, then frames 0 .. n_link - 1 of the batch (0 <= n_link <= n) linked on the device
+ * in the same stream; frames past n_link (a padded batch) do not advance the tracker and get id -1.  A batch with a
+ * non-OK status is not linked.  fetch_ids: the ids of the last tracked wait, one per record, in record order.
+ * link_host: the same link launch on host records (persons_per_frame[f] records of 60 x 3 doubles for frame f, one
+ * frame after the other) -> ids, one per record (parity tests, foreign estimators).                               */
+int opb_tracker_create(opb_context* ctx, int max_gap, double max_dist, int min_joints, opb_tracker** out);
+int opb_tracker_destroy(opb_tracker* tracker);
+int opb_tracker_reset(opb_tracker* tracker);
+int opb_tracker_state(opb_tracker* tracker, int* live, int* next_id, int* frame);
+int opb_pose_every_wait_tracked(opb_session* body_s, opb_tracker* tracker, int n_link, int* persons, int* frame_status);
+int opb_pose_every_fetch_ids(opb_session* body_s, int* ids, int rows);
+int opb_tracker_link_host(opb_tracker* tracker, const double* records, const int* persons_per_frame, int n_frames,
+                          int* ids);
 
 /* ---- batched estimators: srcmx/Batch_model.py (the reference author's throughput path) ---------- */
 /* Batch_body.__call__ (srcmx/Batch_model.py:142-204): `frames` = (n, 3, height, width) float32 planar in

@@ -59,6 +59,13 @@ SIGNATURES = {
     "opb_pose_every_wait": (c_int, [c_void_p, POINTER(c_int), POINTER(c_int)]),
     "opb_pose_every_fetch": (c_int, [c_void_p, c_void_p, c_int]),
     "opb_pose_every_select": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "opb_tracker_create": (c_int, [c_void_p, c_int, c_double, c_int, POINTER(c_void_p)]),
+    "opb_tracker_destroy": (c_int, [c_void_p]),
+    "opb_tracker_reset": (c_int, [c_void_p]),
+    "opb_tracker_state": (c_int, [c_void_p, POINTER(c_int), POINTER(c_int), POINTER(c_int)]),
+    "opb_pose_every_wait_tracked": (c_int, [c_void_p, c_void_p, c_int, POINTER(c_int), POINTER(c_int)]),
+    "opb_pose_every_fetch_ids": (c_int, [c_void_p, c_void_p, c_int]),
+    "opb_tracker_link_host": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
     "opb_body_maps": (c_int, [c_void_p, c_void_p, c_void_p]),
     "opb_hand_maps": (c_int, [c_void_p, c_void_p]),
     "opb_batch_body_submit": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_double]),
@@ -243,6 +250,41 @@ class Session(object):
         try:
             if self.handle:
                 lib().opb_session_destroy(self.handle)
+                self.handle = None
+        except Exception:
+            pass
+
+
+class Tracker(object):
+    """Person tracks of one video on the device (opb_tracker_*): the rule of `motion.PersonLinker`, bit for bit."""
+
+    def __init__(self, ctx, max_gap, max_dist, min_joints=3):
+        self.handle = c_void_p()
+        check(lib().opb_tracker_create(ctx, int(max_gap), float(max_dist), int(min_joints), ctypes.byref(self.handle)))
+
+    def reset(self):
+        check(lib().opb_tracker_reset(self.handle))
+
+    def state(self):
+        """(live tracks, next id, frames linked so far)."""
+        live, nxt, frame = c_int(), c_int(), c_int()
+        check(lib().opb_tracker_state(self.handle, ctypes.byref(live), ctypes.byref(nxt), ctypes.byref(frame)))
+        return live.value, nxt.value, frame.value
+
+    def link_host(self, frames):
+        """frames: a list of (P_f, 60, 3) float64 record arrays -> list of (P_f,) int track ids, linked on the device."""
+        import numpy as np
+        counts = np.array([len(r) for r in frames], dtype=np.int32)
+        records = np.ascontiguousarray(np.concatenate([np.asarray(r, dtype=np.float64).reshape(-1, 60, 3) for r in frames])
+                                       if len(frames) else np.zeros((0, 60, 3)))
+        ids = np.empty(len(records), dtype=np.int32)
+        check(lib().opb_tracker_link_host(self.handle, records.ctypes.data, counts.ctypes.data, len(counts), ids.ctypes.data))
+        return np.split(ids.astype(np.int64), np.cumsum(counts)[:-1]) if len(counts) else []
+
+    def __del__(self):
+        try:
+            if self.handle:
+                lib().opb_tracker_destroy(self.handle)
                 self.handle = None
         except Exception:
             pass

@@ -17,8 +17,8 @@ BUILD = os.path.join(HERE, "build")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC"]
 # units whose float64 arithmetic must round exactly like numpy/scipy: no FMA contraction
-EXACT = {"peaks.cu", "paf.cu", "hand.cu", "prepost.cu", "pose.cu"}
-SOURCES = ["conv_tc.cu", "conv_patch.cu", "conv_pair.cu", "conv_tail.cu", "conv_simt.cu", "prepost.cu", "peaks.cu", "paf.cu", "hand.cu", "pose.cu", "net.cu", "api.cu"]
+EXACT = {"peaks.cu", "paf.cu", "hand.cu", "prepost.cu", "pose.cu", "track.cu"}
+SOURCES = ["conv_tc.cu", "conv_patch.cu", "conv_pair.cu", "conv_tail.cu", "conv_simt.cu", "prepost.cu", "peaks.cu", "paf.cu", "hand.cu", "pose.cu", "track.cu", "net.cu", "api.cu"]
 
 
 def _nvcc():

@@ -441,15 +441,19 @@ struct opb_session {
         int* chunk_rec = nullptr;        // [kEveryChunk]
         double* records_host = nullptr;  // pinned [cap][60][3]
         int* counts_host = nullptr;      // pinned [kEveryCounts]
+        int* ids = nullptr;              // [cap] track id of each record (opb_pose_every_wait_tracked)
+        int* ids_host = nullptr;         // pinned [cap]
         ~EveryBuffers() {
             if (records_host) cudaFreeHost(records_host);
             if (counts_host) cudaFreeHost(counts_host);
+            if (ids_host) cudaFreeHost(ids_host);
         }
     };
     std::unique_ptr<EveryBuffers> every;
     uint64_t every_allocs = 0;
     bool every_batch = false;            // the batch in flight is an opb_pose_every batch
     int every_persons = -1;              // persons of the last finished opb_pose_every batch; -1: none
+    bool every_linked = false;           // the last finished opb_pose_every batch was linked: ids_host holds its ids
     ~opb_session() {
         plans.clear();
         net_plans.clear();
@@ -460,6 +464,42 @@ struct opb_session {
         if (done) cudaEventDestroy(done);
         for (auto m : marks) if (m) cudaEventDestroy(m);
         if (stream) cudaStreamDestroy(stream);
+    }
+};
+
+// person tracks of one video (track.cu).  The host holds the authoritative (cur, live, next_id, frame); every link
+// passes it to the kernel and reads it back before it returns, under `mu`.
+struct opb_tracker {
+    opb_context* ctx = nullptr;
+    int max_gap = 1, min_joints = 3;
+    double max_dist = 0.0;
+    std::mutex mu;
+    int cur = 0, live = 0, next_id = 0, frame = 0;
+    // track slots (double-buffered), grown by doubling with the live tracks carried over
+    opb::DevPool tracks;
+    int cap = 0;
+    double* rows[2] = {nullptr, nullptr};
+    int* tid[2] = {nullptr, nullptr};
+    int* last[2] = {nullptr, nullptr};
+    int* track_taken = nullptr;
+    // per-frame scratch
+    opb::DevPool scratch;
+    int person_cap = 0, pair_cap = 0;
+    int* match = nullptr;
+    double* pair_cost = nullptr;
+    int* pair_k = nullptr;
+    int* pair_p = nullptr;
+    int* order = nullptr;
+    int* state = nullptr;             // [5] kernel output
+    int* state_host = nullptr;        // pinned [5]
+    // opb_tracker_link_host: the caller's records in device memory
+    opb::DevPool staging;
+    int staging_records = -1, staging_frames = -1;
+    double* records = nullptr;
+    int* persons = nullptr;
+    int* ids = nullptr;
+    ~opb_tracker() {
+        if (state_host) cudaFreeHost(state_host);
     }
 };
 
@@ -1397,6 +1437,8 @@ static void ensure_every_buffers(opb_session* bs, int persons) {
     e->chunk_rec = e->pool.alloc_t<int>(kEveryChunk);
     OPB_CUDA(cudaMallocHost((void**)&e->records_host, (size_t)cap * 180 * sizeof(double)));
     OPB_CUDA(cudaMallocHost((void**)&e->counts_host, kEveryCounts * sizeof(int)));
+    e->ids = e->pool.alloc_t<int>(cap);
+    OPB_CUDA(cudaMallocHost((void**)&e->ids_host, (size_t)cap * sizeof(int)));
     bs->every = std::move(e);
 }
 
@@ -1435,6 +1477,7 @@ static void every_submit(opb_session* bs, opb_session* hs, const uint8_t* imgs, 
     bs->batch_pose_box = 0;
     bs->every_batch = true;
     bs->every_persons = -1;
+    bs->every_linked = false;
     upload_image(bs, fp, imgs, where, (size_t)n * H * W * 3);
     // the hand plan of the chunks, with the hand session's work buffers sized for the largest crop
     OPB_CUDA(cudaStreamSynchronize(hs->stream));
@@ -1451,9 +1494,125 @@ static void every_submit(opb_session* bs, opb_session* hs, const uint8_t* imgs, 
     bs->net->ctx->launches += fp->launches_per_frame + 1;
 }
 
+// ------------------------------------------------------------------------------------------------
+// person tracks (opb_tracker_*): the link launch of track.cu on records in device memory
+// ------------------------------------------------------------------------------------------------
+// track slots for the live tracks plus every person of the frames to link, scratch for the largest frame and for its
+// pairs (at most live tracks x persons).  Grown by doubling; OPB_TEST_SMALL_BUFFERS starts tiny so that tests reach the
+// growth path.  Waits for `st` before it frees anything.
+static void tracker_reserve(opb_tracker* tr, const int* persons, int n, cudaStream_t st) {
+    static const bool tiny = getenv("OPB_TEST_SMALL_BUFFERS") != nullptr;
+    long long tracks = tr->live, pairs = 0;
+    int pmax = 0;
+    for (int f = 0; f < n; ++f) {
+        OPB_REQUIRE(persons[f] >= 0, "negative person count");
+        pairs = std::max(pairs, tracks * persons[f]);
+        tracks += persons[f];
+        pmax = std::max(pmax, persons[f]);
+    }
+    OPB_REQUIRE(tracks < (1LL << 30) && pairs < (1LL << 30), "tracker: too many tracks or pairs");
+    auto grown = [&](int have, long long need, int first) {
+        long long c = have ? have : (tiny ? 2 : first);
+        while (c < need) c *= 2;
+        return (int)c;
+    };
+    if (tracks > tr->cap) {
+        const int cap = grown(tr->cap, tracks, 256);
+        OPB_CUDA(cudaStreamSynchronize(st));
+        opb_tracker fresh;      // only its pool and pointers are used
+        for (int b = 0; b < 2; ++b) {
+            fresh.rows[b] = fresh.tracks.alloc_t<double>((size_t)cap * 54);
+            fresh.tid[b] = fresh.tracks.alloc_t<int>(cap);
+            fresh.last[b] = fresh.tracks.alloc_t<int>(cap);
+        }
+        fresh.track_taken = fresh.tracks.alloc_t<int>(cap);
+        if (tr->live) {
+            const int c = tr->cur, L = tr->live;
+            OPB_CUDA(cudaMemcpyAsync(fresh.rows[0], tr->rows[c], (size_t)L * 54 * sizeof(double), cudaMemcpyDeviceToDevice, st));
+            OPB_CUDA(cudaMemcpyAsync(fresh.tid[0], tr->tid[c], (size_t)L * sizeof(int), cudaMemcpyDeviceToDevice, st));
+            OPB_CUDA(cudaMemcpyAsync(fresh.last[0], tr->last[c], (size_t)L * sizeof(int), cudaMemcpyDeviceToDevice, st));
+            OPB_CUDA(cudaStreamSynchronize(st));
+        }
+        std::swap(tr->tracks.ptrs, fresh.tracks.ptrs);
+        std::swap(tr->tracks.bytes, fresh.tracks.bytes);
+        for (int b = 0; b < 2; ++b) {
+            tr->rows[b] = fresh.rows[b];
+            tr->tid[b] = fresh.tid[b];
+            tr->last[b] = fresh.last[b];
+        }
+        tr->track_taken = fresh.track_taken;
+        tr->cap = cap;
+        tr->cur = 0;
+    }
+    if (!tr->state || pmax > tr->person_cap || pairs > tr->pair_cap) {
+        const int person_cap = std::max(tr->person_cap, grown(tr->person_cap, pmax, 256));
+        const int pair_cap = std::max(tr->pair_cap, grown(tr->pair_cap, pairs, 4096));
+        OPB_CUDA(cudaStreamSynchronize(st));
+        tr->scratch.release();
+        tr->person_cap = person_cap;
+        tr->pair_cap = pair_cap;
+        tr->match = tr->scratch.alloc_t<int>(person_cap);
+        tr->pair_cost = tr->scratch.alloc_t<double>(pair_cap);
+        tr->pair_k = tr->scratch.alloc_t<int>(pair_cap);
+        tr->pair_p = tr->scratch.alloc_t<int>(pair_cap);
+        tr->order = tr->scratch.alloc_t<int>(pair_cap);
+        tr->state = tr->scratch.alloc_t<int>(5);
+        if (!tr->state_host) OPB_CUDA(cudaMallocHost((void**)&tr->state_host, 5 * sizeof(int)));
+    }
+}
+
+// links n frames (persons_dev / persons_host: the same counts) of records_dev; ids_dev gets one id per record.  The
+// state comes back to the pinned buffer; tracker_finish takes it once the stream has reached it.
+static void tracker_link_enqueue(opb_tracker* tr, const double* records_dev, const int* persons_dev, const int* persons_host,
+                                 int n, int* ids_dev, cudaStream_t st) {
+    tracker_reserve(tr, persons_host, n, st);
+    TrackLink a;
+    a.records = records_dev;
+    a.persons = persons_dev;
+    a.n_frames = n;
+    a.ids = ids_dev;
+    for (int b = 0; b < 2; ++b) {
+        a.rows[b] = tr->rows[b];
+        a.tid[b] = tr->tid[b];
+        a.last[b] = tr->last[b];
+    }
+    a.cap = tr->cap;
+    a.person_cap = tr->person_cap;
+    a.pair_cap = tr->pair_cap;
+    a.cur = tr->cur;
+    a.live = tr->live;
+    a.next_id = tr->next_id;
+    a.frame = tr->frame;
+    a.max_gap = tr->max_gap;
+    a.min_joints = tr->min_joints;
+    a.max_dist = tr->max_dist;
+    a.pair_cost = tr->pair_cost;
+    a.pair_k = tr->pair_k;
+    a.pair_p = tr->pair_p;
+    a.order = tr->order;
+    a.track_taken = tr->track_taken;
+    a.match = tr->match;
+    a.state = tr->state;
+    OPB_CUDA(cudaMemsetAsync(tr->state, 0, 5 * sizeof(int), st));
+    track_link_launch(a, st);
+    OPB_CUDA(cudaMemcpyAsync(tr->state_host, tr->state, 5 * sizeof(int), cudaMemcpyDeviceToHost, st));
+    tr->ctx->launches += 1;
+}
+
+static void tracker_finish(opb_tracker* tr) {
+    const int* s = tr->state_host;
+    if (s[4]) throw Error(OPB_ERR_INVALID, "tracker: link buffers too small (internal error)");
+    tr->cur = s[0];
+    tr->live = s[1];
+    tr->next_id = s[2];
+    tr->frame = s[3];
+}
+
 // Body overflow check (frames that overflowed are grown and redone, then the rows-and-boxes kernel runs again), records
-// grown to the person count, ceil(V / kEveryChunk) hand chunks, one copy of the T records.  persons: n ints.
-static int every_wait(opb_session* bs, int* persons, int* frame_status) {
+// grown to the person count, ceil(V / kEveryChunk) hand chunks, one copy of the T records.  persons: n ints.  With a
+// tracker, frames 0 .. n_link - 1 are linked after the hand chunks and their ids copied back with the records; a batch
+// whose Body raised IndexError is not linked.
+static int every_wait(opb_session* bs, int* persons, int* frame_status, opb_tracker* tr = nullptr, int n_link = 0) {
     OPB_REQUIRE(bs->active && bs->every && bs->every_batch && bs->pose_hand, "no every-person batch in flight");
     OPB_CUDA(cudaSetDevice(bs->net->ctx->device));
     cudaStream_t st = bs->stream;
@@ -1484,10 +1643,22 @@ static int every_wait(opb_session* bs, int* persons, int* frame_status) {
         const int nhs = rg.tabs.n_scales;
         bs->net->ctx->launches += (int64_t)cdiv(V, kEveryChunk) * (1 + nhs + hp->net->kernel_launches + (nhs + 1) + 6 + 1);
     }
+    std::unique_lock<std::mutex> lock;
+    const bool link = tr && rc == OPB_OK;
+    if (link) {
+        lock = std::unique_lock<std::mutex>(tr->mu);
+        bs->prof.mark(st, "hands");
+        if (T > 0) OPB_CUDA(cudaMemsetAsync(e.ids, 0xff, (size_t)T * sizeof(int), st));       // -1: not linked
+        tracker_link_enqueue(tr, e.records, e.counts + kEveryFrameCounts, e.counts_host + kEveryFrameCounts, n_link, e.ids, st);
+        bs->prof.mark(st, "track_link");
+        if (T > 0) OPB_CUDA(cudaMemcpyAsync(e.ids_host, e.ids, (size_t)T * sizeof(int), cudaMemcpyDeviceToHost, st));
+    }
     if (T > 0) OPB_CUDA(cudaMemcpyAsync(e.records_host, e.records, (size_t)T * 180 * sizeof(double), cudaMemcpyDeviceToHost, st));
     OPB_CUDA(cudaStreamSynchronize(st));
+    if (link) tracker_finish(tr);
     for (int f = 0; f < n; ++f) persons[f] = e.counts_host[kEveryFrameCounts + f];
     bs->every_persons = T;
+    bs->every_linked = link;
     return rc;
 }
 
@@ -1914,6 +2085,99 @@ int opb_pose_every_fetch(opb_session* body_s, double* records, int rows) {
             OPB_REQUIRE(records != nullptr, "null records buffer");
             memcpy(records, body_s->every->records_host, (size_t)T * 180 * sizeof(double));
         }
+    });
+}
+int opb_pose_every_wait_tracked(opb_session* body_s, opb_tracker* tracker, int n_link, int* persons, int* frame_status) {
+    int rc = OPB_OK;
+    int g = guarded([&] {
+        OPB_REQUIRE(body_s && tracker && persons, "null argument");
+        OPB_REQUIRE(tracker->ctx == body_s->net->ctx, "tracker and sessions must live on the same context");
+        OPB_REQUIRE(n_link >= 0 && n_link <= body_s->n_frames, "n_link: 0..frames of the batch");
+        rc = every_wait(body_s, persons, frame_status, tracker, n_link);
+    });
+    return g != OPB_OK ? g : rc;
+}
+int opb_pose_every_fetch_ids(opb_session* body_s, int* ids, int rows) {
+    return guarded([&] {
+        OPB_REQUIRE(body_s && body_s->every && body_s->every_persons >= 0 && body_s->every_linked,
+                    "no finished tracked every-person batch");
+        const int T = body_s->every_persons;
+        if (rows < T) throw Error(OPB_ERR_CAPACITY, "ids buffer smaller than the result");
+        if (T) {
+            OPB_REQUIRE(ids != nullptr, "null ids buffer");
+            memcpy(ids, body_s->every->ids_host, (size_t)T * sizeof(int));
+        }
+    });
+}
+
+/* ---- person tracks ----------------------------------------------------------------------------------------------- */
+int opb_tracker_create(opb_context* ctx, int max_gap, double max_dist, int min_joints, opb_tracker** out) {
+    return guarded([&] {
+        OPB_REQUIRE(ctx && out, "null argument");
+        OPB_REQUIRE(max_gap >= 1, "max_gap >= 1");
+        OPB_REQUIRE(std::isfinite(max_dist) && max_dist >= 0.0, "max_dist: finite, >= 0");
+        OPB_REQUIRE(min_joints >= 1 && min_joints <= 18, "min_joints: 1..18");
+        auto* t = new opb_tracker();
+        t->ctx = ctx;
+        t->max_gap = max_gap;
+        t->max_dist = max_dist;
+        t->min_joints = min_joints;
+        *out = t;
+    });
+}
+int opb_tracker_destroy(opb_tracker* tracker) {
+    return guarded([&] {
+        if (!tracker) return;
+        OPB_CUDA(cudaSetDevice(tracker->ctx->device));
+        delete tracker;
+    });
+}
+int opb_tracker_reset(opb_tracker* tracker) {
+    return guarded([&] {
+        OPB_REQUIRE(tracker, "null argument");
+        std::lock_guard<std::mutex> lock(tracker->mu);
+        tracker->cur = tracker->live = tracker->next_id = tracker->frame = 0;
+    });
+}
+int opb_tracker_state(opb_tracker* tracker, int* live, int* next_id, int* frame) {
+    return guarded([&] {
+        OPB_REQUIRE(tracker, "null argument");
+        std::lock_guard<std::mutex> lock(tracker->mu);
+        if (live) *live = tracker->live;
+        if (next_id) *next_id = tracker->next_id;
+        if (frame) *frame = tracker->frame;
+    });
+}
+int opb_tracker_link_host(opb_tracker* tracker, const double* records, const int* persons_per_frame, int n_frames, int* ids) {
+    return guarded([&] {
+        OPB_REQUIRE(tracker && persons_per_frame && n_frames >= 0, "bad arguments");
+        long long T = 0;
+        for (int f = 0; f < n_frames; ++f) {
+            OPB_REQUIRE(persons_per_frame[f] >= 0, "negative person count");
+            T += persons_per_frame[f];
+        }
+        OPB_REQUIRE(T < (1LL << 30), "too many records");
+        OPB_REQUIRE(T == 0 || (records && ids), "null argument");
+        opb_tracker* tr = tracker;
+        OPB_CUDA(cudaSetDevice(tr->ctx->device));
+        cudaStream_t st = tr->ctx->stream;
+        std::lock_guard<std::mutex> lock(tr->mu);
+        if (T > tr->staging_records || n_frames > tr->staging_frames) {
+            OPB_CUDA(cudaStreamSynchronize(st));
+            tr->staging.release();
+            tr->staging_records = (int)std::max<long long>(T, 2 * std::max(tr->staging_records, 0));
+            tr->staging_frames = std::max(n_frames, 2 * std::max(tr->staging_frames, 0));
+            tr->records = tr->staging.alloc_t<double>((size_t)std::max(tr->staging_records, 1) * 180);
+            tr->ids = tr->staging.alloc_t<int>(std::max(tr->staging_records, 1));
+            tr->persons = tr->staging.alloc_t<int>(std::max(tr->staging_frames, 1));
+        }
+        if (T) OPB_CUDA(cudaMemcpyAsync(tr->records, records, (size_t)T * 180 * sizeof(double), cudaMemcpyHostToDevice, st));
+        if (n_frames)
+            OPB_CUDA(cudaMemcpyAsync(tr->persons, persons_per_frame, (size_t)n_frames * sizeof(int), cudaMemcpyHostToDevice, st));
+        tracker_link_enqueue(tr, tr->records, tr->persons, persons_per_frame, n_frames, tr->ids, st);
+        if (T) OPB_CUDA(cudaMemcpyAsync(ids, tr->ids, (size_t)T * sizeof(int), cudaMemcpyDeviceToHost, st));
+        OPB_CUDA(cudaStreamSynchronize(st));
+        tracker_finish(tr);
     });
 }
 

@@ -446,6 +446,33 @@ void every_stage_launch(const HandBox* list, const int* list_rec, const int* cou
 void every_finish_launch(const HandBox* boxes, const int* rec, const double* hand_peaks_dev, int C, double* records,
                          int* counts, cudaStream_t stream);
 
+// person tracks across frames (track.cu): links n_frames frames of records (persons[f] records of frame f, one after
+// the other, [60][3] each; only rows 0-17 are read) in order, one block.  Track slot k of buffer b: body rows at
+// rows[b] + k * 54, id tid[b][k], last matched frame last[b][k]; slots hold ids ascending.  The state in (cur, live,
+// next_id, frame) comes as arguments and goes out to state[0..3]; state[4] is set non-zero if a capacity was short
+// (cap tracks after adding a frame's persons, person_cap persons per frame, pair_cap eligible pairs per frame).
+struct TrackLink {
+    const double* records;
+    const int* persons;
+    int n_frames;
+    int* ids;                                 // one per record
+    double* rows[2];
+    int* tid[2];
+    int* last[2];
+    int cap, person_cap, pair_cap;
+    int cur, live, next_id, frame;
+    int max_gap, min_joints;
+    double max_dist;
+    double* pair_cost;                        // [pair_cap]
+    int* pair_k;                              // [pair_cap] track slot
+    int* pair_p;                              // [pair_cap] person
+    int* order;                               // [pair_cap]
+    int* track_taken;                         // [cap]
+    int* match;                               // [person_cap] track slot of each person, -1: none
+    int* state;                               // [5]
+};
+void track_link_launch(const TrackLink& a, cudaStream_t stream);
+
 // ---- gaussian taps shared by peaks.cu / hand.cu: scipy.ndimage.gaussian_filter(sigma=3) uses
 // radius int(4*3+0.5) = 12 and weights exp(-x^2/18) / sum (src/body.py:75, src/hand.py:62).  The
 // constants are the exact float64 bit patterns numpy produces (w[d] = weight at distance d), so the

@@ -50,7 +50,7 @@ class FrameBatches(object):
     one thread each (seek with CAP_PROP_POS_FRAMES); batches then arrive in whatever order they are decoded -- every
     batch carries its first frame index -- and frames past the container's reported count are not read."""
 
-    def __init__(self, videopath, recpoint=None, batch=8, depth=4, pinned=False, workers=1, pad_last=False):
+    def __init__(self, videopath, recpoint=None, batch=8, depth=4, pinned=False, workers=1, pad_last=False, ordered=False):
         import cv2
         probe = cv2.VideoCapture(videopath)
         if not probe.isOpened():
@@ -63,7 +63,11 @@ class FrameBatches(object):
         self.pad_last = pad_last
         self.hold = max(depth - 2, 1)
         self.workers = max(1, int(workers))
+        # ordered: batches are yielded in frame order whatever the workers -- the segments one after the other, so a
+        # later segment decodes only as far as its ring of buffers reaches ahead
+        self.ordered = ordered
         self._q = queue.Queue()
+        self._qs = [queue.Queue() for _ in range(self.workers)] if ordered else [self._q] * self.workers
         n_batches = -(-self.count // batch)
         per = -(-n_batches // self.workers) * batch
         self._rings = []
@@ -71,7 +75,7 @@ class FrameBatches(object):
             lo = w * per
             hi = None if self.workers == 1 else min((w + 1) * per, self.count)
             if self.workers > 1 and lo >= self.count:
-                self._q.put(None)
+                self._qs[w].put(None)
                 self._rings.append(None)
                 continue
             ring = {"bufs": None, "free": queue.Queue(), "depth": self.hold + 2}
@@ -106,25 +110,34 @@ class FrameBatches(object):
                 fill += 1
                 index += 1
                 if fill == self.batch:
-                    self._q.put((w, cur, fill, first))
+                    self._qs[w].put((w, cur, fill, first))
                     cur = None
             if cur is not None and fill:
                 if self.pad_last:
                     ring["bufs"][cur][0][fill:] = ring["bufs"][cur][0][fill - 1]
-                self._q.put((w, cur, fill, first))
-            self._q.put(None)
+                self._qs[w].put((w, cur, fill, first))
+            self._qs[w].put(None)
         except BaseException as e:                     # surface decode errors in the consumer
-            self._q.put(e)
+            self._qs[w].put(e)
         finally:
             video.release()
 
-    def __iter__(self):
-        held, finished = [], 0
+    def _items(self):
+        if self.ordered:                               # each worker's batches arrive in order: take the workers in turn
+            for q in self._qs:
+                yield from iter(q.get, None)
+            return
+        finished = 0
         while finished < self.workers:
             item = self._q.get()
             if item is None:
                 finished += 1
                 continue
+            yield item
+
+    def __iter__(self):
+        held = []
+        for item in self._items():
             if isinstance(item, BaseException):
                 raise item
             w, cur, fill, first = item
@@ -314,15 +327,21 @@ def extract_motion_from_video(videopath, outpath, recpoint, body_estimation, han
     return mat
 
 
+def _pose_estimator(body_estimation, hand_estimation):
+    """The `PoseEstimator` of a Body / Hand pair, kept on the Body (its sessions are expensive to warm up)."""
+    from .motion import PoseEstimator
+    est = body_estimation.__dict__.setdefault("_pose_estimator", None)
+    if est is None or est.hand is not hand_estimation:
+        est = body_estimation.__dict__["_pose_estimator"] = PoseEstimator(body_estimation, hand_estimation)
+    return est
+
+
 def _extract_bodyhand_on_device(src, outpath, body_estimation, hand_estimation, sessions, pinned, log, stats):
     """mode='bodyhand' with the per-frame caller on the device: batches of frames in flight on `sessions` (body, hand)
     session pairs; every collect returns PoseMat rows for its batch."""
     import time
     import joblib
-    from .motion import PoseEstimator
-    est = body_estimation.__dict__.setdefault("_pose_estimator", None)
-    if est is None or est.hand is not hand_estimation:
-        est = body_estimation.__dict__["_pose_estimator"] = PoseEstimator(body_estimation, hand_estimation)
+    est = _pose_estimator(body_estimation, hand_estimation)
     pairs = est.sessions(sessions)
     mat = np.zeros((src.count, 60, 3))
     outname = os.path.split(outpath)[1]
@@ -362,6 +381,97 @@ def _extract_bodyhand_on_device(src, outpath, body_estimation, hand_estimation, 
     joblib.dump(mat, outpath)
     log("%s is saved!" % outpath)
     return mat
+
+
+# ---- every person, tracked ------------------------------------------------------------------------------------------
+def _write_tracks(outpath, count, frames):
+    """frames: [(first frame index, [(P_f, 60, 3) records], [(P_f,) ids])] in frame order -> the joblib file
+    {"count": count, "tracks": [(first_frame, posemat (L, 60, 3) float64), ...]} indexed by track id."""
+    import joblib
+    seen = {}
+    for first, recs, ids in frames:
+        for f, (r, i) in enumerate(zip(recs, ids)):
+            for p, tid in enumerate(i):
+                seen.setdefault(int(tid), []).append((first + f, r[p]))
+    tracks = []
+    for tid in range(len(seen)):
+        rows = seen[tid]
+        mat = np.zeros((rows[-1][0] - rows[0][0] + 1, 60, 3))
+        for t, r in rows:
+            mat[t - rows[0][0]] = r
+        tracks.append((rows[0][0], mat))
+    out = {"count": count, "tracks": tracks}
+    joblib.dump(out, outpath)
+    return out
+
+
+def extract_every_person_from_video(videopath, outpath, recpoint, body_estimation, hand_estimation, max_gap=15,
+                                    max_dist=None, min_joints=3, batch=8, sessions=2, decode_workers=1, log=print):
+    """Body and hands of every person of a video, linked into per-person tracks (`motion.PersonLinker`'s rule), dumped
+    with joblib to `outpath` as {"count": T, "tracks": [(first_frame, posemat (L, 60, 3) float64), ...]}, indexed by
+    track id.  A track's PoseMat runs from its first to its last matched frame; frames in between where it was not
+    matched are zero rows (the reference's "missing").  Coordinates are in ROI coordinates, like the other jobs.
+
+    max_dist=None means 0.1 x the ROI height: a choice that lets a person move a tenth of the picture between matched
+    frames, not a measured optimum.  max_gap: frames a track may go unmatched and still be picked up again.
+
+    With this package's `Body` and `Hand`, batches run on the device (`PoseEstimator.every_person` on `sessions`
+    session pairs in flight) and are linked there, in frame order, by one tracker.  With any other estimators the job
+    runs `motion.pose_mats_every_person` frame by frame and links with `PersonLinker`.  Both write the same file.
+    Frames are linked in order, so with decode_workers > 1 the later segments decode only a few batches ahead.  An
+    IndexError from Body is raised before anything is written."""
+    from .body import Body
+    from .hand import Hand
+    from .motion import PersonLinker, pose_mats_every_person
+    device = type(body_estimation) is Body and type(hand_estimation) is Hand
+    try:
+        src = FrameBatches(videopath, recpoint, batch=batch, depth=sessions + 3, pinned=device, workers=decode_workers,
+                           pad_last=device, ordered=True)
+    except FileNotFoundError as e:
+        log(str(e))
+        return None
+    outname = os.path.split(outpath)[1]
+    frames = []
+    if device:
+        est = _pose_estimator(body_estimation, hand_estimation)
+        pairs = est.sessions(sessions)
+        tracker = None
+        pending = []
+
+        def retire():
+            pair, first, nv = pending.pop(0)
+            n_link = max(0, min(nv, src.count - first))
+            recs, ids = est.collect_every_person(pair, tracker=tracker, n_link=n_link)
+            frames.append((first, recs[:n_link], ids[:n_link]))
+            if first % 100 < len(recs):
+                log("%s-%d/%d" % (outname, first, src.count))
+
+        for fr, first, n_valid in src:
+            if tracker is None:
+                height = fr.shape[1]
+                tracker = est.tracker(max_gap, 0.1 * height if max_dist is None else max_dist, min_joints)
+            if len(pending) == len(pairs):
+                retire()
+            pair = next(c for c in pairs if all(c is not p[0] for p in pending))
+            est.submit_every_person(fr, pair, where=2)
+            pending.append((pair, first, n_valid))
+        while pending:
+            retire()
+    else:
+        linker = None
+        for fr, first in src:
+            if linker is None:
+                linker = PersonLinker(max_gap, 0.1 * fr.shape[1] if max_dist is None else max_dist, min_joints)
+            recs, ids = [], []
+            for f in range(min(len(fr), src.count - first)):
+                recs.append(pose_mats_every_person(fr[f], body_estimation, hand_estimation))
+                ids.append(linker.link(recs[-1]))
+                if (first + f) % 100 == 0:
+                    log("%s-%d/%d" % (outname, first + f, src.count))
+            frames.append((first, recs, ids))
+    out = _write_tracks(outpath, src.count, frames)
+    log("%s is saved!" % outpath)
+    return out
 
 
 # ---- the batched jobs (srcmx/Batch_motion_Estimation.py) -----------------------------------------------------------

@@ -73,6 +73,83 @@ def pose_mats_every_person(oriImg, body_estimation, hand_estimation):
     return out
 
 
+class PersonLinker(object):
+    """Links the persons of consecutive frames into tracks: `link(records)` takes one frame's (P, 60, 3) records (as
+    `pose_mats_every_person` returns them) and returns P int track ids.  The rule, exactly (the device tracker,
+    `PoseEstimator.tracker`, is held to it bit for bit):
+
+      * Presence: joint j (0-17) of a record is present when its score column is > 0.
+      * Track state: each track keeps its id (assigned in creation order from 0, never reused), the 18 body rows of
+        the last person it was matched to, and the index of that frame.  A track is live for frame t when
+        t - last <= max_gap; a track that is not live at frame t is dropped for good.  Frame indices count every
+        linked frame, frames with nobody included.
+      * Cost of live track k against person p: J = the joints present in both, ascending.  If |J| < min_joints the
+        pair is not eligible.  Otherwise cost = (sum over j in J of sqrt(dx*dx + dy*dy)) / |J| in float64, with
+        dx = x_p - x_k, dy = y_p - y_k; every product, sum and the square root rounded separately (no FMA), the sum
+        starting at 0.0 and running in joint order.  The pair is eligible when cost <= max_dist.
+      * Matching: the eligible pairs sorted by (cost ascending, track id ascending, person index ascending), walked
+        greedily; a pair is accepted when neither its track nor its person is taken yet.
+      * New tracks: unmatched persons start new tracks, in person-index order.
+      * A matched track takes the person's body rows and the frame index.  Hand rows do not enter the cost."""
+
+    def __init__(self, max_gap, max_dist, min_joints=3):
+        if int(max_gap) != max_gap or max_gap < 1:
+            raise ValueError("max_gap: an int >= 1")
+        if not np.isfinite(max_dist) or max_dist < 0:
+            raise ValueError("max_dist: a finite number >= 0")
+        if int(min_joints) != min_joints or not 1 <= min_joints <= 18:
+            raise ValueError("min_joints: an int in 1..18")
+        self.max_gap, self.max_dist, self.min_joints = int(max_gap), float(max_dist), int(min_joints)
+        self.reset()
+
+    def reset(self):
+        """Forget every track: the next frame is frame 0 and the next id is 0."""
+        self._ids = np.zeros(0, dtype=np.int64)              # live tracks, ids ascending
+        self._rows = np.zeros((0, 18, 3))
+        self._last = np.zeros(0, dtype=np.int64)
+        self._next = 0
+        self._frame = 0
+
+    def link(self, records):
+        rec = np.asarray(records, dtype=np.float64)
+        if rec.ndim != 3 or rec.shape[1] < 18 or rec.shape[2] != 3:
+            raise ValueError("expected (P, 60, 3) records")
+        t = self._frame
+        live = t - self._last <= self.max_gap
+        self._ids, self._rows, self._last = self._ids[live], self._rows[live], self._last[live]
+        L, P = len(self._ids), len(rec)
+        body = rec[:, :18]
+        both = (self._rows[:, None, :, 2] > 0) & (body[None, :, :, 2] > 0)           # (L, P, 18)
+        dx = body[None, :, :, 0] - self._rows[:, None, :, 0]
+        dy = body[None, :, :, 1] - self._rows[:, None, :, 1]
+        dist = np.sqrt(dx * dx + dy * dy)
+        total = np.zeros((L, P))
+        for j in range(18):                                  # joint order; adding 0.0 for an absent joint is exact
+            total = total + np.where(both[:, :, j], dist[:, :, j], 0.0)
+        count = both.sum(axis=2)
+        ok = count >= self.min_joints
+        cost = np.where(ok, total / np.maximum(count, 1), np.inf)
+        k, p = np.nonzero(ok & (cost <= self.max_dist))
+        c = cost[k, p]
+        order = np.lexsort((p, self._ids[k], c))
+        ids = np.full(P, -1, dtype=np.int64)
+        track_taken = np.zeros(L, dtype=bool)
+        for i in order:
+            if not track_taken[k[i]] and ids[p[i]] < 0:
+                track_taken[k[i]] = True
+                ids[p[i]] = self._ids[k[i]]
+                self._rows[k[i]] = body[p[i]]
+                self._last[k[i]] = t
+        new = np.nonzero(ids < 0)[0]
+        ids[new] = self._next + np.arange(len(new))
+        self._ids = np.concatenate([self._ids, ids[new]])
+        self._rows = np.concatenate([self._rows, body[new]])
+        self._last = np.concatenate([self._last, np.full(len(new), t, dtype=np.int64)])
+        self._next += len(new)
+        self._frame = t + 1
+        return ids
+
+
 def _frame_batch(bs, frames, where):
     """(pointer, (n, H, W)) of a batch argument: (n, H, W, 3) uint8 host frames (kept alive on the session until the next
     submit) or, for where 1, (device pointer, (n, H, W))."""
@@ -152,23 +229,46 @@ class PoseEstimator(object):
         h_arr, nh = _lib.scales_array(self.hand.scale_search)
         _lib.check(_lib.lib().opb_pose_every_submit(bs.handle, hs.handle, ptr, where, n, H, W, b_arr, nb, h_arr, nh))
 
-    def collect_every_person(self, pair=None):
+    def collect_every_person(self, pair=None, tracker=None, n_link=None):
         """-> list of n arrays (P_f, 60, 3) float64, equal to `pose_mats_every_person` frame by frame.  Raises IndexError
-        like the reference's Body would (src/body.py:173)."""
+        like the reference's Body would (src/body.py:173).
+
+        With a `tracker` (`self.tracker(...)`), the first `n_link` frames of the batch (default: all) are linked on the
+        device after the hand half, and the result is (records, ids): ids[f] holds the (P_f,) int track ids of frame
+        f, -1 for frames past n_link (the padding of a short last batch, which does not advance the tracker).  Batches
+        are linked in the order their collects are called; a batch that raises IndexError is not linked."""
         import ctypes
         from . import _lib
         bs, hs = pair or self.sessions(1)[0]
         persons = (ctypes.c_int * bs._batch)()
         status = (ctypes.c_int * bs._batch)()
-        _lib.check(_lib.lib().opb_pose_every_wait(bs.handle, persons, status))
+        if tracker is None:
+            _lib.check(_lib.lib().opb_pose_every_wait(bs.handle, persons, status))
+        else:
+            n_link = bs._batch if n_link is None else int(n_link)
+            _lib.check(_lib.lib().opb_pose_every_wait_tracked(bs.handle, tracker.handle, n_link, persons, status))
         counts = list(persons)
         records = np.empty((sum(counts), 60, 3), dtype=np.float64)
         _lib.check(_lib.lib().opb_pose_every_fetch(bs.handle, records.ctypes.data, len(records)))
-        return np.split(records, np.cumsum(counts)[:-1])
+        split = np.cumsum(counts)[:-1]
+        if tracker is None:
+            return np.split(records, split)
+        ids = np.empty(len(records), dtype=np.int32)
+        _lib.check(_lib.lib().opb_pose_every_fetch_ids(bs.handle, ids.ctypes.data, len(ids)))
+        return np.split(records, split), np.split(ids.astype(np.int64), split)
 
-    def every_person(self, frames):
-        """One frame (H, W, 3) -> (P, 60, 3); a batch (n, H, W, 3) -> list of n such arrays."""
+    def every_person(self, frames, tracker=None):
+        """One frame (H, W, 3) -> (P, 60, 3); a batch (n, H, W, 3) -> list of n such arrays.  With a `tracker`:
+        (records, ids) of the same shapes, ids per frame as `collect_every_person` returns them."""
         single = np.ndim(frames) == 3
         self.submit_every_person(np.asarray(frames)[None] if single else frames)
-        out = self.collect_every_person()
-        return out[0] if single else out
+        out = self.collect_every_person(tracker=tracker)
+        if tracker is None:
+            return out[0] if single else out
+        return (out[0][0], out[1][0]) if single else out
+
+    def tracker(self, max_gap, max_dist, min_joints=3):
+        """A device tracker for one video (`PersonLinker`'s rule and arguments) on this estimator's GPU, for
+        `collect_every_person(..., tracker=)`.  It keeps its tracks until `reset()`."""
+        from . import _lib
+        return _lib.Tracker(self.body.net.ctx, max_gap, max_dist, min_joints)

@@ -151,7 +151,9 @@ int opb_pose_wait(opb_session* body_s, double* pose_mats, int* frame_status);
  * wait: runs the hand chunks, fills persons (n ints: records of each frame) and frame_status (optional: OPB_OK or
  * OPB_ERR_SUBSET_INDEX per frame), returns the first non-OK status like opb_body_wait_batch.
  * fetch: the records of the last wait, frame after frame (sum of persons x 60 x 3); rows = capacity of `records` in
- * records.                                                                                                        */
+ * records.
+ * wait, fetch, wait_tracked and fetch_ids below serve both opb_pose_every_submit and opb_batch_pose_every_submit: the
+ * wait runs the hand chunks of whichever submit put the batch in flight.                                          */
 int opb_pose_every_submit(opb_session* body_s, opb_session* hand_s, const uint8_t* imgs_bgr, int where, int n_frames,
                           int height, int width, const double* body_scales, int n_body_scales,
                           const double* hand_scales, int n_hand_scales);
@@ -238,6 +240,18 @@ int opb_batch_pose_submit(opb_session* body_s, opb_session* hand_s, const uint8_
                           int height, int width, double g_scale, int boxsize);
 int opb_batch_pose_wait(opb_session* body_s, double* motion_mats /* n x 18 x 3 */, double* hand_mats /* n x 42 x 3 */,
                         int* frame_status);
+/* ---- every person on the batched estimators -----------------------------------------------------------------------
+ * opb_batch_pose_submit's sequence for EVERY person Batch_body finds, not just the one with the largest left-shoulder x:
+ * per frame one 60 x 3 float64 record per subset row, in subset order -- rows 0-17 candidate[subset[p][k]][:3], rows
+ * 18-38 / 39-59 the left / right HandMat rows Batch_hand_extraction would derive from those body rows (boxes as
+ * HandImageDataset.__getitem__, crops cv2.resize(crop, (boxsize, boxsize), INTER_CUBIC), the left one mirrored, grey
+ * for a missing hand, Batch_hand, :41-56 back to ROI coordinates).  Every person gets both crops; a missing hand -- a
+ * missing joint, or a box of width <= 0 -- keeps the scores Batch_hand finds on its grey crop, with coordinates 0.
+ * Arguments and checks as opb_batch_pose_submit.  The crops run in fixed chunks through one Batch_hand plan, so memory
+ * does not depend on the number of persons.  Results: opb_pose_every_wait / _wait_tracked / _fetch / _fetch_ids.
+ * hand_s must not be used by other calls while a batch is in flight.                                               */
+int opb_batch_pose_every_submit(opb_session* body_s, opb_session* hand_s, const uint8_t* frames_bgr, int where,
+                                int n_frames, int height, int width, double g_scale, int boxsize);
 
 /* blurred heat maps of the last batched-estimator call: (n, 19 | 22, height, width) planar fp32; the
  * un-blurred maps and the PAFs come from opb_body_maps / opb_hand_maps.                             */
@@ -287,6 +301,12 @@ int opb_pose_select(opb_context* ctx, const double* host_candidates, int n_candi
  * record], the boxes util.handDetect returns in its order, rows past the box count all -1.                        */
 int opb_pose_every_select(opb_context* ctx, const double* host_candidates, int n_candidates, const double* host_subset,
                           int n_subset, int height, int width, double* host_records, int* host_boxes);
+/* The same for opb_batch_pose_every_*: host_boxes = 2 * n_subset x [x, y, w, valid, is_left, record], both slots of
+ * every person (left first) in person order; (0, 0, 0, 0) for a hand with a missing joint, valid 0 for a box of width
+ * <= 0.                                                                                                              */
+int opb_batch_pose_every_select(opb_context* ctx, const double* host_candidates, int n_candidates,
+                                const double* host_subset, int n_subset, int height, int width, double* host_records,
+                                int* host_boxes);
 /* src/hand.py:59-75 on a planar (>=21, h, w) fp32 device map -> 21x3 float64 host array.            */
 int opb_hand_peaks(opb_context* ctx, const float* dev_heat, int height, int width, double thre, double* host_peaks);
 

@@ -80,6 +80,9 @@ SIGNATURES = {
     "opb_debug_hand_track_taps": (c_int, [c_int, c_int, c_void_p, c_void_p]),
     "opb_batch_pose_submit": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_double, c_int]),
     "opb_batch_pose_wait": (c_int, [c_void_p, c_void_p, c_void_p, POINTER(c_int)]),
+    "opb_batch_pose_every_submit": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_double, c_int]),
+    "opb_batch_pose_every_select": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p,
+                                            c_void_p]),
     "opb_scale_dims": (c_int, [c_int, c_int, c_double, POINTER(c_int), POINTER(c_int), POINTER(c_int), POINTER(c_int)]),
     "opb_preprocess": (c_int, [c_void_p, c_void_p, c_int, c_int, c_double, c_void_p]),
     "opb_net_forward": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),

@@ -211,7 +211,10 @@ class BatchPoseEstimator(object):
     equal to what the two jobs write: MotionMat (n, 18, 3) and HandMat (n, 42, 3).
 
     `batch_body` / `batch_hand`: this package's `Batch_body` / `Batch_hand` (their scale_search, 0.5, is used).  A hand
-    box of width 0, on which the reference's cv2.resize raises, counts as a missing hand (as in `Batch_hand.track`)."""
+    box of width 0, on which the reference's cv2.resize raises, counts as a missing hand (as in `Batch_hand.track`).
+
+    `every_person` / `submit_every_person` / `collect_every_person` run the same sequence for every person of every
+    frame (`extract.batch_pose_mats_every_person` states the contract); `tracker` links them across batches."""
 
     MAX_BATCH = 32                                    # frames per submit: 64 hand crops, like Batch_hand.TRACK_BATCH
 
@@ -252,3 +255,54 @@ class BatchPoseEstimator(object):
             motion.append(m)
             hand.append(h)
         return np.concatenate(motion, 0), np.concatenate(hand, 0)
+
+    def submit_every_person(self, frames, pair=None, where=0, boxsize=368):
+        """Every person of every frame: frames as for `submit`.  Batch_body, the body rows of every subset row, both
+        hand crops of every person cut from the frames in device memory, Batch_hand on them in fixed chunks."""
+        bs, hs = pair or self.sessions(1)[0]
+        ptr, where, keep, (B, h, w) = _as_track_frames(frames, where)
+        bs._keepalive, bs._batch = keep, B
+        _lib.check(_lib.lib().opb_batch_pose_every_submit(bs.handle, hs.handle, ptr, where, B, h, w,
+                                                          float(self.body.scale_search), int(boxsize)))
+
+    def collect_every_person(self, pair=None, tracker=None, n_link=None):
+        """-> list of B arrays (P_f, 60, 3) float64, equal to `extract.batch_pose_mats_every_person` frame by frame:
+        record p of frame f is the [MotionMat | HandMat] row `collect` would return had its selection picked subset row
+        p.  Raises IndexError where the reference's Batch_body would (src/body.py:173).
+
+        With a `tracker` (`self.tracker(...)`): (records, ids), linked as `motion.PoseEstimator.collect_every_person`
+        links them (the first `n_link` frames, default all; -1 for the others; a batch that raises is not linked)."""
+        bs, hs = pair or self.sessions(1)[0]
+        persons = (ctypes.c_int * bs._batch)()
+        status = (ctypes.c_int * bs._batch)()
+        L = _lib.lib()
+        if tracker is None:
+            _lib.check(L.opb_pose_every_wait(bs.handle, persons, status))
+        else:
+            n_link = bs._batch if n_link is None else int(n_link)
+            _lib.check(L.opb_pose_every_wait_tracked(bs.handle, tracker.handle, n_link, persons, status))
+        counts = list(persons)
+        records = np.empty((sum(counts), 60, 3), dtype=np.float64)
+        _lib.check(L.opb_pose_every_fetch(bs.handle, records.ctypes.data, len(records)))
+        split = np.cumsum(counts)[:-1]
+        if tracker is None:
+            return np.split(records, split)
+        ids = np.empty(len(records), dtype=np.int32)
+        _lib.check(L.opb_pose_every_fetch_ids(bs.handle, ids.ctypes.data, len(ids)))
+        return np.split(records, split), np.split(ids.astype(np.int64), split)
+
+    def every_person(self, frames, tracker=None, boxsize=368):
+        """One frame (h, w, 3) -> (P, 60, 3); a batch (B, h, w, 3) of at most MAX_BATCH frames -> list of B such
+        arrays.  With a `tracker`: (records, ids) of the same shapes."""
+        frames = frames if hasattr(frames, "shape") else np.asarray(frames)
+        single = len(frames.shape) == 3
+        self.submit_every_person(frames[None] if single else frames, boxsize=boxsize)
+        out = self.collect_every_person(tracker=tracker)
+        if tracker is None:
+            return out[0] if single else out
+        return (out[0][0], out[1][0]) if single else out
+
+    def tracker(self, max_gap, max_dist, min_joints=3):
+        """A device tracker for one video (`motion.PersonLinker`'s rule and arguments) on this estimator's GPU, for
+        `collect_every_person(..., tracker=)`.  It keeps its tracks until `reset()`."""
+        return _lib.Tracker(self.body.net.ctx, max_gap, max_dist, min_joints)

@@ -256,7 +256,9 @@ struct FramePlan {
     uint64_t batch_pose_gen = 0;
     int batch_pose_uses = 0;
     // every person (opb_pose_every_*): the body sequence with the rows-and-boxes kernel, and one hand chunk (replayed
-    // once per kEveryChunk boxes) -- both on the body plan of the batch
+    // once per kEveryChunk boxes) -- both on the body plan of the batch.  opb_batch_pose_every_submit uses the same two
+    // slots of its Batch_body plan (a mode-2 plan, which no other every-person sequence shares), so it alternates with
+    // opb_batch_pose_submit (batch_pose_graph) on one session pair without re-capturing.
     cudaGraphExec_t every_graph = nullptr;
     uint64_t every_gen = 0;
     int every_uses = 0;
@@ -425,7 +427,7 @@ struct opb_session {
     opb_session* pose_hand = nullptr;    // hand session of the pose batch in flight
     std::vector<double> pose_hand_scales;
     bool pose_fixed = false;
-    int batch_pose_box = 0;              // boxsize of the opb_batch_pose batch in flight; 0: an opb_pose batch
+    int batch_pose_box = 0;              // boxsize of the opb_batch_pose(_every) batch in flight; 0: an opb_pose batch
     // every person of a batch (opb_pose_every_*), on a body session: the records and the compacted hand boxes, grown to
     // the largest person count seen, and the boxes of one hand chunk
     struct EveryBuffers {
@@ -436,9 +438,9 @@ struct opb_session {
         HandBox* list = nullptr;     // [2 cap] in util.handDetect's order
         int* list_rec = nullptr;     // [2 cap] record of each box
         int* counts = nullptr;       // [kEveryCounts] persons, boxes, chunk cursor
-        HandBox* chunk_boxes = nullptr;  // [kEveryChunk]
-        int* chunk_dims = nullptr;       // [kEveryChunk]
-        int* chunk_rec = nullptr;        // [kEveryChunk]
+        HandBox* chunk_boxes = nullptr;  // [kEveryChunkSlots]
+        int* chunk_dims = nullptr;       // [kEveryChunkSlots]
+        int* chunk_rec = nullptr;        // [kEveryChunkSlots]
         double* records_host = nullptr;  // pinned [cap][60][3]
         int* counts_host = nullptr;      // pinned [kEveryCounts]
         int* ids = nullptr;              // [cap] track id of each record (opb_pose_every_wait_tracked)
@@ -451,7 +453,7 @@ struct opb_session {
     };
     std::unique_ptr<EveryBuffers> every;
     uint64_t every_allocs = 0;
-    bool every_batch = false;            // the batch in flight is an opb_pose_every batch
+    bool every_batch = false;            // the batch in flight is an opb_pose_every or opb_batch_pose_every batch
     int every_persons = -1;              // persons of the last finished opb_pose_every batch; -1: none
     bool every_linked = false;           // the last finished opb_pose_every batch was linked: ids_host holds its ids
     ~opb_session() {
@@ -1416,6 +1418,11 @@ static void batch_pose_submit(opb_session* bs, opb_session* hs, const uint8_t* f
 // opb_pose_submit_batch holds at 8 frames (16 slots).  The CNN runs on every slot of a chunk, the empty ones of the
 // last chunk too, so a smaller chunk wastes less on a batch with few hands.
 constexpr int kEveryChunk = 8;
+// Crops per chunk of the batched estimators' every-person path (opb_batch_pose_every_*): boxsize-square crops through a
+// uint8 Batch_hand plan.  Measured on a B200 at 16, 32 and 64 (DESIGN.md section 7, N2): 16 is 3.5 % slower, 64 only
+// 0.3 % faster than 32 but doubles the plan's activations and the CNN slots wasted in a batch's last partial chunk.
+constexpr int kBatchEveryChunk = 32;
+constexpr int kEveryChunkSlots = kEveryChunk > kBatchEveryChunk ? kEveryChunk : kBatchEveryChunk;
 
 // records and box list for `persons` persons (grown by doubling; OPB_TEST_SMALL_BUFFERS starts tiny so that tests reach
 // the growth path of opb_pose_every_wait)
@@ -1432,9 +1439,9 @@ static void ensure_every_buffers(opb_session* bs, int persons) {
     e->list = e->pool.alloc_t<HandBox>((size_t)cap * 2);
     e->list_rec = e->pool.alloc_t<int>((size_t)cap * 2);
     e->counts = e->pool.alloc_t<int>(kEveryCounts, true);
-    e->chunk_boxes = e->pool.alloc_t<HandBox>(kEveryChunk);
-    e->chunk_dims = e->pool.alloc_t<int>(kEveryChunk);
-    e->chunk_rec = e->pool.alloc_t<int>(kEveryChunk);
+    e->chunk_boxes = e->pool.alloc_t<HandBox>(kEveryChunkSlots);
+    e->chunk_dims = e->pool.alloc_t<int>(kEveryChunkSlots);
+    e->chunk_rec = e->pool.alloc_t<int>(kEveryChunkSlots);
     OPB_CUDA(cudaMallocHost((void**)&e->records_host, (size_t)cap * 180 * sizeof(double)));
     OPB_CUDA(cudaMallocHost((void**)&e->counts_host, kEveryCounts * sizeof(int)));
     e->ids = e->pool.alloc_t<int>(cap);
@@ -1442,10 +1449,12 @@ static void ensure_every_buffers(opb_session* bs, int persons) {
     bs->every = std::move(e);
 }
 
-// rows and boxes of every person from the body results of the batch; the counts to pinned memory
+// rows and boxes of every person from the body results of the batch (the batched estimators' box rule for an
+// opb_batch_pose_every batch); the counts to pinned memory
 static void every_rows_enqueue(opb_session* bs, FramePlan* fp, int n) {
     opb_session::EveryBuffers& e = *bs->every;
-    every_rows_launch(fp->post_dev, n, fp->key.H, fp->key.W, e.cap, e.records, e.list, e.list_rec, e.counts, bs->stream);
+    every_rows_launch(fp->post_dev, n, fp->key.H, fp->key.W, e.cap, e.records, e.list, e.list_rec, e.counts,
+                      bs->batch_pose_box != 0, bs->stream);
     OPB_CUDA(cudaMemcpyAsync(e.counts_host, e.counts, kEveryCounts * sizeof(int), cudaMemcpyDeviceToHost, bs->stream));
 }
 
@@ -1487,6 +1496,67 @@ static void every_submit(opb_session* bs, opb_session* hs, const uint8_t* imgs, 
     const uint64_t gen = gen_key({bs->buffer_gen, bs->every->gen});
     run_or_replay_slot(bs, GraphSlot{fp->every_graph, fp->every_gen, fp->every_uses}, gen, [&] {
         run_front(bs, fp, n, H, W);
+        body_post_enqueue(bs, fp, n, H, W);
+        every_rows_enqueue(bs, fp, n);
+    });
+    OPB_CUDA(cudaEventRecord(bs->done, st));
+    bs->net->ctx->launches += fp->launches_per_frame + 1;
+}
+
+// ------------------------------------------------------------------------------------------------
+// every person on the batched estimators: Batch_body, the body rows of every subset row and both hand crops of every
+// person as Batch_hand_extraction derives them from a saved MotionMat row (grey crops for missing hands), Batch_hand on
+// every crop, _box_to_roi into the records.  The waits, fetches, growth and tracking are every_wait's.
+// ------------------------------------------------------------------------------------------------
+// one chunk of the hand half: the next kBatchEveryChunk slots of the list, their crops cut from the frames still in the
+// Batch_body plan's input buffer into the uint8 Batch_hand plan hp, Batch_hand on all of them, key points into records
+static void batch_every_chunk_enqueue(opb_session* bs, opb_session* hs, FramePlan* fp, FramePlan* hp, int boxsize) {
+    cudaStream_t st = bs->stream;
+    opb_session::EveryBuffers& e = *bs->every;
+    const int C = kBatchEveryChunk;
+    every_stage_launch(e.list, e.list_rec, e.counts, C, e.chunk_boxes, e.chunk_dims, e.chunk_rec, st);
+    preprocess_ragged_launch(fp->d_img, fp->key.H, fp->key.W, e.chunk_boxes, C, hp->d_img, boxsize, 0, hs->track->tabs, st);
+    batch_hand_enqueue(bs, hp, C, boxsize, boxsize);            // bs only lends its stream and profiler
+    batch_every_finish_launch(e.chunk_boxes, e.chunk_rec, hp->hb.peaks, C, boxsize, e.records, e.counts, st);
+}
+
+static void batch_every_submit(opb_session* bs, opb_session* hs, const uint8_t* frames, int where, int n, int H, int W,
+                               double g_scale, int boxsize) {
+    OPB_REQUIRE(bs->net->kind == OPB_NET_BODY && hs->net->kind == OPB_NET_HAND,
+                "batch every person: a body session and a hand session");
+    OPB_REQUIRE(bs->net->ctx == hs->net->ctx, "batch every person: both networks must live on the same context");
+    OPB_REQUIRE(n >= 1 && n <= 64, "1..64 frames per batch");
+    OPB_REQUIRE(H >= 1 && W >= 1, "empty frame");
+    OPB_REQUIRE(g_scale > 0, "scale must be positive");
+    OPB_REQUIRE(boxsize >= 8 && boxsize % 8 == 0, "boxsize must be a positive multiple of 8 (srcmx/Batch_model.py:377)");
+    OPB_CUDA(cudaSetDevice(bs->net->ctx->device));
+    cudaStream_t st = bs->stream;
+    // the records, the crop tables and the hand plan may still serve the previous batch of this pair, or work of the
+    // hand session's own stream
+    OPB_CUDA(cudaStreamSynchronize(st));
+    OPB_CUDA(cudaStreamSynchronize(hs->stream));
+    ensure_every_buffers(bs, 0);
+    track_with_tables(hs, boxsize, std::min(H, W));                 // crop tables of every side up to min(H, W)
+    FramePlan* fp = get_plan(bs, n, H, W, &g_scale, 1, 2);          // Batch_body on uint8 frames
+    ensure_host(bs, n, 0);
+    bs->active = fp;
+    bs->n_frames = n;
+    bs->pose_hand = hs;
+    bs->batch_pose_box = boxsize;
+    bs->every_batch = true;
+    bs->every_persons = -1;
+    bs->every_linked = false;
+    const double one = 1.0;
+    FramePlan* hp = get_plan(hs, kBatchEveryChunk, boxsize, boxsize, &one, 1, 2);   // uint8 Batch_hand on one chunk
+    hs->active = hp;
+    hs->hand_crops = kBatchEveryChunk;
+    bs->prof.reset();
+    bs->prof.mark(st, "start");
+    upload_image(bs, fp, frames, where, (size_t)n * H * W * 3);
+    bs->prof.mark(st, "h2d");
+    const uint64_t gen = gen_key({bs->buffer_gen, bs->every->gen});
+    run_or_replay_slot(bs, GraphSlot{fp->every_graph, fp->every_gen, fp->every_uses}, gen, [&] {
+        run_front_f32(bs, fp, n, H, W);
         body_post_enqueue(bs, fp, n, H, W);
         every_rows_enqueue(bs, fp, n);
     });
@@ -1609,9 +1679,10 @@ static void tracker_finish(opb_tracker* tr) {
 }
 
 // Body overflow check (frames that overflowed are grown and redone, then the rows-and-boxes kernel runs again), records
-// grown to the person count, ceil(V / kEveryChunk) hand chunks, one copy of the T records.  persons: n ints.  With a
-// tracker, frames 0 .. n_link - 1 are linked after the hand chunks and their ids copied back with the records; a batch
-// whose Body raised IndexError is not linked.
+// grown to the person count, the hand chunks -- ceil(V / kEveryChunk) Hand chunks, or for an opb_batch_pose_every batch
+// ceil(V / kBatchEveryChunk) Batch_hand chunks -- and one copy of the T records.  persons: n ints.  With a tracker,
+// frames 0 .. n_link - 1 are linked after the hand chunks and their ids copied back with the records; a batch whose
+// Body / Batch_body raised IndexError is not linked.
 static int every_wait(opb_session* bs, int* persons, int* frame_status, opb_tracker* tr = nullptr, int n_link = 0) {
     OPB_REQUIRE(bs->active && bs->every && bs->every_batch && bs->pose_hand, "no every-person batch in flight");
     OPB_CUDA(cudaSetDevice(bs->net->ctx->device));
@@ -1631,7 +1702,18 @@ static int every_wait(opb_session* bs, int* persons, int* frame_status, opb_trac
     }
     opb_session::EveryBuffers& e = *bs->every;
     const int T = e.counts_host[0], V = e.counts_host[1];
-    if (V > 0) {
+    if (V > 0 && bs->batch_pose_box) {
+        opb_session* hs = bs->pose_hand;
+        FramePlan* hp = hs->active;
+        const int boxsize = bs->batch_pose_box;
+        const uint64_t gen = gen_key({bs->buffer_gen, hs->buffer_gen, (uint64_t)(uintptr_t)hp, hs->track->gen, e.gen,
+                                      (uint64_t)(uintptr_t)fp->d_img, (uint64_t)fp->key.H, (uint64_t)fp->key.W,
+                                      (uint64_t)boxsize});
+        for (int base = 0; base < V; base += kBatchEveryChunk)
+            run_or_replay_slot(bs, GraphSlot{fp->every_hand_graph, fp->every_hand_gen, fp->every_hand_uses}, gen,
+                               [&] { batch_every_chunk_enqueue(bs, hs, fp, hp, boxsize); });
+        bs->net->ctx->launches += (int64_t)cdiv(V, kBatchEveryChunk) * (3 /* stage, crops, finish */ + hp->launches_per_frame);
+    } else if (V > 0) {
         opb_session* hs = bs->pose_hand;
         FramePlan* hp = hs->active;
         const opb_session::Ragged& rg = *hs->ragged;
@@ -2057,6 +2139,14 @@ int opb_batch_pose_wait(opb_session* body_s, double* motion_mats, double* hand_m
 }
 
 /* ---- every person of every frame ------------------------------------------------------------------------------- */
+int opb_batch_pose_every_submit(opb_session* body_s, opb_session* hand_s, const uint8_t* frames_bgr, int where,
+                                int n_frames, int height, int width, double g_scale, int boxsize) {
+    return guarded([&] {
+        OPB_REQUIRE(body_s && hand_s && frames_bgr, "null argument");
+        OPB_REQUIRE(where >= 0 && where <= 2, "where: 0 pageable host, 1 device, 2 pinned host");
+        batch_every_submit(body_s, hand_s, frames_bgr, where, n_frames, height, width, g_scale, boxsize);
+    });
+}
 int opb_pose_every_submit(opb_session* body_s, opb_session* hand_s, const uint8_t* imgs_bgr, int where, int n_frames,
                           int height, int width, const double* body_scales, int n_body_scales, const double* hand_scales,
                           int n_hand_scales) {
@@ -2457,49 +2547,62 @@ int opb_pose_select(opb_context* ctx, const double* host_candidates, int n_candi
 }
 
 /* stage-level: rows and boxes of every person (pose.cu) on host-provided body results of one frame */
+static void every_select(opb_context* ctx, const double* host_candidates, int n_candidates, const double* host_subset,
+                         int n_subset, int H, int W, double* host_records, int* host_boxes, bool batched) {
+    OPB_REQUIRE(ctx && n_candidates >= 0 && n_subset >= 0, "bad arguments");
+    OPB_REQUIRE(n_subset == 0 || (host_candidates && host_subset && host_records && host_boxes), "null argument");
+    OPB_CUDA(cudaSetDevice(ctx->device));
+    const int cap = std::max(n_subset, 1);
+    StagePost sp;
+    sp.create(std::max(n_candidates, 1), 1, 1, cap, nullptr, ctx->stream);
+    OPB_CUDA(cudaMemcpyAsync(sp.host.lb.subset_count, &n_subset, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+    if (n_candidates)
+        OPB_CUDA(cudaMemcpyAsync(sp.host.pb.candidates, host_candidates, (size_t)n_candidates * 32, cudaMemcpyHostToDevice, ctx->stream));
+    if (n_subset)
+        OPB_CUDA(cudaMemcpyAsync(sp.host.lb.subset, host_subset, (size_t)n_subset * 160, cudaMemcpyHostToDevice, ctx->stream));
+    DevPool pool;
+    double* records = pool.alloc_t<double>((size_t)cap * 180);
+    HandBox* list = pool.alloc_t<HandBox>((size_t)cap * 2);
+    int* list_rec = pool.alloc_t<int>((size_t)cap * 2);
+    int* counts = pool.alloc_t<int>(kEveryCounts);
+    every_rows_launch(sp.dev, 1, H, W, cap, records, list, list_rec, counts, batched, ctx->stream);
+    ctx->launches += 1;
+    std::vector<HandBox> hb((size_t)cap * 2);
+    std::vector<int> hr((size_t)cap * 2);
+    int hc[kEveryCounts];
+    OPB_CUDA(cudaMemcpyAsync(hc, counts, sizeof(hc), cudaMemcpyDeviceToHost, ctx->stream));
+    OPB_CUDA(cudaMemcpyAsync(hb.data(), list, hb.size() * sizeof(HandBox), cudaMemcpyDeviceToHost, ctx->stream));
+    OPB_CUDA(cudaMemcpyAsync(hr.data(), list_rec, hr.size() * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    if (n_subset)
+        OPB_CUDA(cudaMemcpyAsync(host_records, records, (size_t)n_subset * 180 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    OPB_CUDA(cudaStreamSynchronize(ctx->stream));
+    OPB_REQUIRE(hc[0] == n_subset && hc[1] <= 2 * n_subset && (!batched || hc[1] == 2 * n_subset),
+                "every-person rows: unexpected counts");
+    const int fields = batched ? 6 : 5;
+    for (int i = 0; i < 2 * n_subset; ++i) {
+        int* b = host_boxes + (size_t)i * fields;
+        if (i < hc[1]) {
+            b[0] = hb[i].x;
+            b[1] = hb[i].y;
+            b[2] = hb[i].w;
+            if (batched) b[3] = hb[i].valid;
+            b[fields - 2] = hb[i].left;
+            b[fields - 1] = hr[i];
+        } else {
+            for (int k = 0; k < fields; ++k) b[k] = -1;
+        }
+    }
+}
 int opb_pose_every_select(opb_context* ctx, const double* host_candidates, int n_candidates, const double* host_subset,
                           int n_subset, int H, int W, double* host_records, int* host_boxes) {
     return guarded([&] {
-        OPB_REQUIRE(ctx && n_candidates >= 0 && n_subset >= 0, "bad arguments");
-        OPB_REQUIRE(n_subset == 0 || (host_candidates && host_subset && host_records && host_boxes), "null argument");
-        OPB_CUDA(cudaSetDevice(ctx->device));
-        const int cap = std::max(n_subset, 1);
-        StagePost sp;
-        sp.create(std::max(n_candidates, 1), 1, 1, cap, nullptr, ctx->stream);
-        OPB_CUDA(cudaMemcpyAsync(sp.host.lb.subset_count, &n_subset, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-        if (n_candidates)
-            OPB_CUDA(cudaMemcpyAsync(sp.host.pb.candidates, host_candidates, (size_t)n_candidates * 32, cudaMemcpyHostToDevice, ctx->stream));
-        if (n_subset)
-            OPB_CUDA(cudaMemcpyAsync(sp.host.lb.subset, host_subset, (size_t)n_subset * 160, cudaMemcpyHostToDevice, ctx->stream));
-        DevPool pool;
-        double* records = pool.alloc_t<double>((size_t)cap * 180);
-        HandBox* list = pool.alloc_t<HandBox>((size_t)cap * 2);
-        int* list_rec = pool.alloc_t<int>((size_t)cap * 2);
-        int* counts = pool.alloc_t<int>(kEveryCounts);
-        every_rows_launch(sp.dev, 1, H, W, cap, records, list, list_rec, counts, ctx->stream);
-        ctx->launches += 1;
-        std::vector<HandBox> hb((size_t)cap * 2);
-        std::vector<int> hr((size_t)cap * 2);
-        int hc[kEveryCounts];
-        OPB_CUDA(cudaMemcpyAsync(hc, counts, sizeof(hc), cudaMemcpyDeviceToHost, ctx->stream));
-        OPB_CUDA(cudaMemcpyAsync(hb.data(), list, hb.size() * sizeof(HandBox), cudaMemcpyDeviceToHost, ctx->stream));
-        OPB_CUDA(cudaMemcpyAsync(hr.data(), list_rec, hr.size() * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-        if (n_subset)
-            OPB_CUDA(cudaMemcpyAsync(host_records, records, (size_t)n_subset * 180 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        OPB_CUDA(cudaStreamSynchronize(ctx->stream));
-        OPB_REQUIRE(hc[0] == n_subset && hc[1] <= 2 * n_subset, "every-person rows: unexpected counts");
-        for (int i = 0; i < 2 * n_subset; ++i) {
-            int* b = host_boxes + (size_t)i * 5;
-            if (i < hc[1]) {
-                b[0] = hb[i].x;
-                b[1] = hb[i].y;
-                b[2] = hb[i].w;
-                b[3] = hb[i].left;
-                b[4] = hr[i];
-            } else {
-                b[0] = b[1] = b[2] = b[3] = b[4] = -1;
-            }
-        }
+        every_select(ctx, host_candidates, n_candidates, host_subset, n_subset, H, W, host_records, host_boxes, false);
+    });
+}
+int opb_batch_pose_every_select(opb_context* ctx, const double* host_candidates, int n_candidates, const double* host_subset,
+                                int n_subset, int H, int W, double* host_records, int* host_boxes) {
+    return guarded([&] {
+        every_select(ctx, host_candidates, n_candidates, host_subset, n_subset, H, W, host_records, host_boxes, true);
     });
 }
 

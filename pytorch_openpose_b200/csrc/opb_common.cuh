@@ -436,15 +436,21 @@ void batch_pose_select_launch(const FramePost* frames_dev, int n_frames, int H, 
 // returns, compacted in its order (frame, person, left before right) into `list` with their record in `list_rec`.
 // Records beyond `cap` and boxes beyond 2 * cap are not written.  counts: [0] persons T, [1] boxes V, [2] the chunk
 // cursor, reset to 0, [kEveryFrameCounts + f] persons of frame f.  n_frames <= 64.
+// batched: the batched estimators' box rule instead (Batch_hand_extraction on each record's body rows, pose_hand_boxes):
+// always both boxes of every person, left then right, an invalid one for a missing hand, so V = 2T.
 constexpr int kEveryFrameCounts = 4, kEveryCounts = kEveryFrameCounts + 64;
 void every_rows_launch(const FramePost* frames_dev, int n_frames, int H, int W, int cap, double* records, HandBox* list,
-                       int* list_rec, int* counts, cudaStream_t stream);
+                       int* list_rec, int* counts, bool batched, cudaStream_t stream);
 // one hand chunk: slots [counts[2], counts[2] + C) of the list into boxes / dims / rec (invalid past V); after the hand
 // network, the finish scatters each slot's 21 key points into its record and advances counts[2] by C
 void every_stage_launch(const HandBox* list, const int* list_rec, const int* counts, int C, HandBox* boxes, int* dims, int* rec,
                         cudaStream_t stream);
 void every_finish_launch(const HandBox* boxes, const int* rec, const double* hand_peaks_dev, int C, double* records,
                          int* counts, cudaStream_t stream);
+// the batched estimators' finish: Batch_hand key points of a boxsize-square crop -> rows 18-59 of record rec[i]
+// (_box_to_roi); a slot with an invalid box keeps its scores with coordinates 0, slots with rec -1 are skipped
+void batch_every_finish_launch(const HandBox* boxes, const int* rec, const double* hand_peaks_dev, int C, int boxsize,
+                               double* records, int* counts, cudaStream_t stream);
 
 // person tracks across frames (track.cu): links n_frames frames of records (persons[f] records of frame f, one after
 // the other, [60][3] each; only rows 0-17 are read) in order, one block.  Track slot k of buffer b: body rows at

@@ -86,23 +86,28 @@ __global__ void hand_track_boxes_kernel(const double* __restrict__ poses, int n_
     boxes[2 * f + 1] = hb[1];
 }
 
-// Batch_hand key points of slot (frame, k) -> HandMat rows (_box_to_roi, Batch_motion_Estimation.py:41-56): scaled by
-// w / boxsize, shifted by the box origin, x un-mirrored for left hands; a coordinate of exactly 0 stays 0.  A slot
-// without a box has the box (0, 0, 0): its coordinates become 0 but its scores -- Batch_hand on the grey crop -- stay.
+// one Batch_hand key point p of the crop of box b -> its HandMat row (_box_to_roi, Batch_motion_Estimation.py:41-56):
+// scaled by w / boxsize, shifted by the box origin, x un-mirrored for left hands; a coordinate of exactly 0 stays 0.  A
+// slot without a box has the box (0, 0, 0): its coordinates become 0 but its score -- Batch_hand on the grey crop --
+// stays.
+__device__ __forceinline__ void hand_track_point(const HandBox& b, const double* p, int boxsize, double* out) {
+    const double bx = b.valid ? b.x : 0, by = b.valid ? b.y : 0, bw = b.valid ? b.w : 0;
+    const double px = __ddiv_rn(__dmul_rn(p[0], bw), (double)boxsize);
+    const double py = __ddiv_rn(__dmul_rn(p[1], bw), (double)boxsize);
+    out[0] = px == 0 ? px : (b.left ? __dadd_rn(__dsub_rn(__dsub_rn(bw, px), 1.0), bx) : __dadd_rn(px, bx));
+    out[1] = py == 0 ? py : __dadd_rn(py, by);
+    out[2] = p[2];
+}
+
+// Batch_hand key points of slot (frame, k) -> HandMat rows
 __global__ void hand_track_finish_kernel(const HandBox* __restrict__ boxes, const double* __restrict__ peaks, int boxsize,
                                          double* __restrict__ mats, int frame_stride) {
     const int slot = blockIdx.x;
     const int j = threadIdx.x;
     if (j >= 21) return;
     const HandBox b = boxes[slot];
-    const double bx = b.valid ? b.x : 0, by = b.valid ? b.y : 0, bw = b.valid ? b.w : 0;
-    const double* p = peaks + ((size_t)slot * 21 + j) * 3;
-    const double px = __ddiv_rn(__dmul_rn(p[0], bw), (double)boxsize);
-    const double py = __ddiv_rn(__dmul_rn(p[1], bw), (double)boxsize);
-    double* out = mats + (size_t)(slot >> 1) * frame_stride + (size_t)((b.left ? 0 : 21) + j) * 3;
-    out[0] = px == 0 ? px : (b.left ? __dadd_rn(__dsub_rn(__dsub_rn(bw, px), 1.0), bx) : __dadd_rn(px, bx));
-    out[1] = py == 0 ? py : __dadd_rn(py, by);
-    out[2] = p[2];
+    hand_track_point(b, peaks + ((size_t)slot * 21 + j) * 3, boxsize,
+                     mats + (size_t)(slot >> 1) * frame_stride + (size_t)((b.left ? 0 : 21) + j) * 3);
 }
 
 // ---- the one-pass body + hand job: Batch_body_extraction and Batch_hand_extraction (srcmx/Batch_motion_Estimation.py:
@@ -127,7 +132,12 @@ __global__ void batch_pose_select_kernel(const FramePost* __restrict__ frames, i
 // One block, one thread per frame (n <= 64): person and box counts of every frame, their prefixes, then each thread
 // writes its frame's records and boxes.  A frame holds a handful of persons; the loops are a few dozen scalar
 // operations per person.
+// kBatched: the box rule of the batched estimators (Batch_hand_extraction on the saved MotionMat, as
+// batch_pose_select_kernel): both boxes of every person, left then right, from pose_hand_boxes on the record's own body
+// rows -- a missing hand is an invalid box that stays in the list (Batch_hand runs on its grey crop), so V = 2T and the
+// boxes of record r are entries 2r and 2r + 1.
 constexpr int kEveryMaxFrames = 64;
+template <bool kBatched>
 __global__ void __launch_bounds__(kEveryMaxFrames) every_rows_kernel(const FramePost* __restrict__ frames, int n_frames,
                                                                      int H, int W, int cap, double* __restrict__ records,
                                                                      HandBox* __restrict__ list, int* __restrict__ list_rec,
@@ -138,7 +148,8 @@ __global__ void __launch_bounds__(kEveryMaxFrames) every_rows_kernel(const Frame
     if (f < n_frames) {
         const FramePost& fr = frames[f];
         persons = min(*fr.lb.subset_count, fr.lb.subset_capacity);
-        for (int p = 0; p < persons; ++p) {
+        if (kBatched) boxes = 2 * persons;
+        else for (int p = 0; p < persons; ++p) {
             const double* row = fr.lb.subset + (size_t)p * 20;
             for (int k = 0; k < 2; ++k) {
                 const int j0 = k == 0 ? 5 : 2;
@@ -172,17 +183,27 @@ __global__ void __launch_bounds__(kEveryMaxFrames) every_rows_kernel(const Frame
             double* rec = records + (size_t)r * 180;
             for (int i = 0; i < 180; ++i) rec[i] = 0.0;
             person_rows(cand, row, rec);
-        }
-        for (int k = 0; k < 2; ++k) {
-            HandBox b;
-            b.frame = f;
-            b.left = k == 0;
-            if (!subset_hand_box(cand, row, k, H, W, b)) continue;
-            if (v < 2 * cap) {
-                list[v] = b;
-                list_rec[v] = r;
+            if (kBatched) {                    // v = 2r < 2 cap
+                HandBox hb[2];
+                pose_hand_boxes(rec, f, H, W, hb);
+                for (int k = 0; k < 2; ++k) {
+                    list[2 * r + k] = hb[k];
+                    list_rec[2 * r + k] = r;
+                }
             }
-            ++v;
+        }
+        if (!kBatched) {
+            for (int k = 0; k < 2; ++k) {
+                HandBox b;
+                b.frame = f;
+                b.left = k == 0;
+                if (!subset_hand_box(cand, row, k, H, W, b)) continue;
+                if (v < 2 * cap) {
+                    list[v] = b;
+                    list_rec[v] = r;
+                }
+                ++v;
+            }
         }
     }
 }
@@ -220,12 +241,35 @@ __global__ void every_finish_kernel(const HandBox* __restrict__ boxes, const int
     hand_point_to_frame(b, peaks + ((size_t)slot * 21 + j) * 3, out);
 }
 
+// the batched estimators' chunk finish: slot i's 21 key points into rows 18-38 / 39-59 of record rec[i] with the
+// hand_track_finish_kernel arithmetic (_box_to_roi).  Unlike every_finish_kernel, a slot with an invalid box is written
+// too -- a missing hand keeps the scores Batch_hand finds on its grey crop, with coordinates 0; slots past V (rec -1)
+// are not.  Then the cursor moves on.
+__global__ void batch_every_finish_kernel(const HandBox* __restrict__ boxes, const int* __restrict__ rec,
+                                          const double* __restrict__ peaks, int C, int boxsize, double* __restrict__ records,
+                                          int* __restrict__ counts) {
+    const int slot = blockIdx.x;
+    const int j = threadIdx.x;
+    if (slot == 0 && j == 0) counts[2] += C;
+    if (j >= 21) return;
+    const int r = rec[slot];
+    if (r < 0) return;
+    const HandBox b = boxes[slot];
+    hand_track_point(b, peaks + ((size_t)slot * 21 + j) * 3, boxsize,
+                     records + (size_t)r * 180 + (size_t)((b.left ? 18 : 39) + j) * 3);
+}
+
 }  // namespace
 
 void every_rows_launch(const FramePost* frames_dev, int n_frames, int H, int W, int cap, double* records, HandBox* list,
-                       int* list_rec, int* counts, cudaStream_t stream) {
+                       int* list_rec, int* counts, bool batched, cudaStream_t stream) {
     OPB_REQUIRE(n_frames >= 1 && n_frames <= kEveryMaxFrames, "1..64 frames per batch");
-    every_rows_kernel<<<1, kEveryMaxFrames, 0, stream>>>(frames_dev, n_frames, H, W, cap, records, list, list_rec, counts);
+    if (batched)
+        every_rows_kernel<true><<<1, kEveryMaxFrames, 0, stream>>>(frames_dev, n_frames, H, W, cap, records, list, list_rec,
+                                                                   counts);
+    else
+        every_rows_kernel<false><<<1, kEveryMaxFrames, 0, stream>>>(frames_dev, n_frames, H, W, cap, records, list, list_rec,
+                                                                    counts);
     OPB_CUDA(cudaGetLastError());
 }
 
@@ -238,6 +282,12 @@ void every_stage_launch(const HandBox* list, const int* list_rec, const int* cou
 void every_finish_launch(const HandBox* boxes, const int* rec, const double* hand_peaks_dev, int C, double* records,
                          int* counts, cudaStream_t stream) {
     every_finish_kernel<<<C, 32, 0, stream>>>(boxes, rec, hand_peaks_dev, C, records, counts);
+    OPB_CUDA(cudaGetLastError());
+}
+
+void batch_every_finish_launch(const HandBox* boxes, const int* rec, const double* hand_peaks_dev, int C, int boxsize,
+                               double* records, int* counts, cudaStream_t stream) {
+    batch_every_finish_kernel<<<C, 32, 0, stream>>>(boxes, rec, hand_peaks_dev, C, boxsize, records, counts);
     OPB_CUDA(cudaGetLastError());
 }
 

@@ -681,10 +681,7 @@ def batch_bodyhand_extraction(videopath, body_outpath, hand_outpath, batch_size,
     except FileNotFoundError as e:
         log(str(e))
         return None
-    est = batch_body_model.__dict__.setdefault("_batch_pose_estimator", None)
-    if est is None or est.hand is not batch_hand_estimation:
-        est = batch_body_model.__dict__["_batch_pose_estimator"] = BatchPoseEstimator(batch_body_model,
-                                                                                      batch_hand_estimation)
+    est = _batch_pose_estimator(batch_body_model, batch_hand_estimation)
     pairs = est.sessions(sessions)
     outname = os.path.split(body_outpath)[1]
     motion = np.zeros((src.count, 18, 3))
@@ -720,6 +717,147 @@ def batch_bodyhand_extraction(videopath, body_outpath, hand_outpath, batch_size,
     joblib.dump(hand, hand_outpath)
     log("the %s file is saved" % hand_outpath)
     return motion, hand
+
+
+def _batch_pose_estimator(batch_body_model, batch_hand_estimation):
+    """The `BatchPoseEstimator` of a Batch_body / Batch_hand pair, kept on the Batch_body (its sessions are expensive to
+    warm up)."""
+    from .batch_model import BatchPoseEstimator
+    est = batch_body_model.__dict__.setdefault("_batch_pose_estimator", None)
+    if est is None or est.hand is not batch_hand_estimation:
+        est = batch_body_model.__dict__["_batch_pose_estimator"] = BatchPoseEstimator(batch_body_model,
+                                                                                      batch_hand_estimation)
+    return est
+
+
+# ---- every person on the batched estimators, tracked ----------------------------------------------------------------
+def _batch_hand_crops(frame, body, boxsize):
+    """`hand_crops_from_pose` on a record's body rows, except that a box of width 0 -- on which cv2.resize raises --
+    is a missing hand (grey crop, params 0), as in `Batch_hand.track`."""
+    pose = np.array(body, dtype=np.float64)
+    candidate, subset = pose_person(pose)
+    for x, y, w, is_left in util.handDetect(candidate, subset, frame):
+        if w <= 0:
+            pose[7 if is_left else 4] = 0                          # drop the wrist: that hand has no box
+    return hand_crops_from_pose(frame, pose, boxsize)
+
+
+def batch_pose_mats_every_person(frames_u8, batch_body_model, batch_hand_estimation, boxsize=368):
+    """Every person of every frame on the batched estimators: (n, h, w, 3) uint8 ROI-cropped frames -> list of n arrays
+    (P_f, 60, 3) float64, one record per subset row of `batch_body_model`'s result, in subset order.
+
+    Record p of frame f is the row of [MotionMat | HandMat] that `batch_bodyhand_extraction` would write for frame f had
+    its person selection picked subset row p:
+      * rows 0-17: candidate[subset[p][k]][:3], zero where the index is -1 (as `body_pose`);
+      * rows 18-38 (left hand) and 39-59 (right hand): `hand_crops_from_pose(frame, rows 0-17, boxsize)`,
+        `batch_hand_estimation` on the ToTensor-ed crops, `_box_to_roi` back to ROI coordinates.
+    Every person always gets both crops: a missing hand gets the grey crop and keeps the scores Batch_hand finds on it
+    (coordinates 0), as HandImageDataset does.  The records have PoseMat's layout, so `motion.PersonLinker` and the
+    tracks file of `extract_every_person_from_video` apply unchanged.
+
+    Deviation (as `Batch_hand.track`): a box of width 0, on which cv2.resize raises, is a missing hand.  A frame on which
+    Batch_body raises IndexError raises for the batch.  Works with any estimators: it is the host fallback of
+    `batch_every_person_extraction` and the oracle of `BatchPoseEstimator.every_person`."""
+    frames_u8 = np.asarray(frames_u8)
+    results = batch_body_model(to_tensor(frames_u8)) if len(frames_u8) else []
+    out, crops, slots = [], [], []                                 # slots: (frame, person, params, left)
+    for f, (candidate, subset) in enumerate(results):
+        recs = np.zeros((len(subset), 60, 3))
+        for p in range(len(subset)):
+            for k in range(18):
+                idx = int(subset[p][k])
+                if idx != -1:
+                    recs[p, k, :] = candidate[idx][:3]
+            left, leftparams, right, rightparams = _batch_hand_crops(frames_u8[f], recs[p, :18], boxsize)
+            crops += [left, right]
+            slots += [(f, p, leftparams, True), (f, p, rightparams, False)]
+        out.append(recs)
+    for lo in range(0, len(crops), 64):
+        peaks = batch_hand_estimation(to_tensor(np.stack(crops[lo:lo + 64])))
+        for (f, p, params, left), pk in zip(slots[lo:lo + 64], peaks):
+            row = 18 if left else 39
+            out[f][p, row:row + 21, :] = _box_to_roi(np.array(pk, dtype=np.float64), params, boxsize, mirrored=left)
+    return out
+
+
+def batch_every_person_extraction(videopath, outpath, batch_size, recpoint, batch_body_model, batch_hand_estimation,
+                                  max_gap=15, max_dist=None, min_joints=3, boxsize=368, log=print, decode_workers=1,
+                                  sessions=2):
+    """Body and hands of every person of a video on the batched estimators, linked into per-person tracks
+    (`motion.PersonLinker`'s rule), dumped with joblib to `outpath` in the format of `extract_every_person_from_video`:
+    {"count": frames, "tracks": [(first_frame, posemat (L, 60, 3) float64), ...]}, indexed by track id, with zero rows
+    where a track was not matched.  The records are those of `batch_pose_mats_every_person`, in ROI coordinates.
+    max_dist=None means 0.1 x the ROI height; max_gap as in `extract_every_person_from_video`.
+
+    With this package's `Batch_body` and `Batch_hand`, batches of at most `BatchPoseEstimator.MAX_BATCH` frames run on the
+    device (`BatchPoseEstimator.every_person`, `sessions` session pairs in flight, frames from a pinned ring) and are
+    linked there, in frame order, by one tracker.  With any other estimators the job runs `batch_pose_mats_every_person`
+    on batches of `batch_size` frames and links with `PersonLinker`.  Both write the same file and log lines.  Frames are
+    linked in order, so with decode_workers > 1 the later segments decode only a few batches ahead.  An IndexError from
+    Batch_body is raised before anything is written.
+
+    From `run_body_job`, one video per call:
+
+        body, hand = Batch_body(body_model_path), Batch_hand(hand_model_path)
+
+        def process_video(videopath, outpath):
+            batch_every_person_extraction(videopath, outpath, 32, recpoint, body, hand)
+        run_body_job(videofolder, datadir, recpoint, process_video, mode="tracks")
+
+    (create the two estimators once, outside the closure: their sessions are kept across videos)."""
+    from .batch_model import Batch_body, Batch_hand, BatchPoseEstimator
+    from .motion import PersonLinker
+    device = type(batch_body_model) is Batch_body and type(batch_hand_estimation) is Batch_hand
+    batch = min(batch_size, BatchPoseEstimator.MAX_BATCH) if device else batch_size
+    try:
+        src = FrameBatches(videopath, recpoint, batch=batch, depth=sessions + 3 if device else 4, pinned=device,
+                           workers=decode_workers, pad_last=device, ordered=True)
+    except FileNotFoundError as e:
+        log(str(e))
+        return None
+    outname = os.path.split(outpath)[1]
+    frames = []
+
+    def progress(first, n):
+        for t in range(first, first + n):
+            if t % 100 == 0:
+                log("%s-%d/%d" % (outname, t, src.count))
+
+    if device:
+        est = _batch_pose_estimator(batch_body_model, batch_hand_estimation)
+        pairs = est.sessions(sessions)
+        tracker = None
+        pending = []                                               # (pair, first, n_valid)
+
+        def retire():
+            pair, first, nv = pending.pop(0)
+            n_link = max(0, min(nv, src.count - first))
+            recs, ids = est.collect_every_person(pair, tracker=tracker, n_link=n_link)
+            frames.append((first, recs[:n_link], ids[:n_link]))
+            progress(first, n_link)
+
+        for fr, first, n_valid in src:
+            if tracker is None:
+                tracker = est.tracker(max_gap, 0.1 * fr.shape[1] if max_dist is None else max_dist, min_joints)
+            if len(pending) == len(pairs):
+                retire()
+            pair = next(c for c in pairs if all(c is not p[0] for p in pending))
+            est.submit_every_person(fr, pair, where=2, boxsize=boxsize)
+            pending.append((pair, first, n_valid))
+        while pending:
+            retire()
+    else:
+        linker = None
+        for fr, first in src:
+            if linker is None:
+                linker = PersonLinker(max_gap, 0.1 * fr.shape[1] if max_dist is None else max_dist, min_joints)
+            n = max(0, min(len(fr), src.count - first))
+            recs = batch_pose_mats_every_person(fr[:n], batch_body_model, batch_hand_estimation, boxsize)
+            frames.append((first, recs, [linker.link(r) for r in recs]))
+            progress(first, n)
+    out = _write_tracks(outpath, src.count, frames)
+    log("%s is saved!" % outpath)
+    return out
 
 
 # ---- resume ledger (srcmx/utilmx.py:190-208) ----------------------------------------------------------------------

@@ -321,6 +321,47 @@ int opb_smooth_debug(opb_context* ctx, const float* dev_heat, int parts, int hei
 int opb_conv2d(opb_context* ctx, const void* dev_in_bf16, int n, int h, int w, int cin, const float* weight,
                const float* bias, int cout, int k, int relu, int pool, int out_fp32, void* dev_out, int impl);
 
+/* Debug: one CNN execution plan, step by step (layer-by-layer tests).
+ * plan      : builds (or finds) the session's plan for n_scales input shapes, shapes[4 * i ..] = {n, hp, wp, in_elem}
+ *             (in_elem 1: uint8 pixels, 2: bf16 values as the batched estimators feed them); *n_steps = its steps.  Later
+ *             calls refer to this plan (it is looked up again by its shapes, so it may be rebuilt, never dangles).
+ * set_input : copies scale `scale`'s input, (n, hp, wp, 3) elements of in_elem bytes, from device memory.
+ * info      : what step i computes (no device work).
+ * step      : runs step i alone on the session's stream, waits for it, and fills *info.
+ * read      : copies a view of step i (problem p; which 0 = input, 1 = output) densely into dev_dst as (n, h, w, c)
+ *             elements of `elem` bytes, and waits for the copy.
+ * run       : runs every step back to back as opb_net_forward does, then waits once.                               */
+#define OPB_DEBUG_MAX_PROBLEMS 8
+#define OPB_STEP_CONV_FIRST 0  /* conv1_1 on the CUDA-core / mma.sync path                                    */
+#define OPB_STEP_CONV 1        /* a grouped tensor-core convolution launch                                    */
+#define OPB_STEP_TAIL 2        /* fused 1x1 -> ReLU -> 1x1 tail, 128-channel intermediate (Mconv6 -> Mconv7)  */
+#define OPB_STEP_TAIL_WIDE 3   /* fused tail with a 512-channel intermediate (conv5_4 -> conv5_5, conv6_1 -> conv6_2) */
+#define OPB_STEP_POOL 4        /* stand-alone 2x2 max-pool (OPB_NO_FUSE_POOL=1)                               */
+typedef struct opb_debug_view {
+    int n, h, w, c, cstride, coff, elem;
+} opb_debug_view;
+typedef struct opb_debug_step {
+    int kind;                  /* OPB_STEP_*                                                                   */
+    int n_problems;
+    int block_n;               /* N tile that runs (tensor-core launches)                                       */
+    int pool;                  /* fused 2x2 max-pool                                                            */
+    int wide;                  /* conv1_2 ran in the wide-pixel form (the views are those of the plain layer)   */
+    int pair;                  /* CTA-pair kernel                                                               */
+    int half_tiles;            /* CTA pair: 16 x 8 tiles                                                        */
+    int weights_resident;      /* CTA pair: one weight set kept in shared memory for the whole kernel          */
+    char name[64];             /* the step's profile name (conv_tc128:..., conv_tc64:..., conv_tail:..., ...) */
+    char layer[OPB_DEBUG_MAX_PROBLEMS][32];
+    char layer2[OPB_DEBUG_MAX_PROBLEMS][32];   /* second layer of a fused tail, else ""                       */
+    int scale[OPB_DEBUG_MAX_PROBLEMS];
+    opb_debug_view in[OPB_DEBUG_MAX_PROBLEMS], out[OPB_DEBUG_MAX_PROBLEMS];
+} opb_debug_step;
+int opb_net_debug_plan(opb_session* s, int n_scales, const int* shapes, int* n_steps);
+int opb_net_debug_set_input(opb_session* s, int scale, const void* dev_src);
+int opb_net_debug_info(opb_session* s, int i, opb_debug_step* info);
+int opb_net_debug_step(opb_session* s, int i, opb_debug_step* info);
+int opb_net_debug_read(opb_session* s, int i, int problem, int which, void* dev_dst);
+int opb_net_debug_run(opb_session* s);
+
 /* Host only (no device call): the wide-pixel weights of a 64 -> 64 channel 3x3 layer (src/model.py:36 conv1_2) as the
  * library packs them at opb_net_finalize.  weight: [64][64][3][3] fp32, bias [64]  ->  w_wide [128][9][128] bf16 bit
  * patterns (output column = parity_out * 64 + cout; K index = (dy * 3 + di) * 128 + parity_in * 64 + cin, di the tap in

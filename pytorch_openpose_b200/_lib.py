@@ -103,6 +103,12 @@ SIGNATURES = {
     "opb_debug_composite_taps": (c_int, [c_int, c_int, c_int, c_void_p, c_void_p]),
     "opb_debug_resize_dsize": (c_int, [c_int, ctypes.c_double]),
     "opb_debug_pair_tiles": (c_int, [c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_void_p]),
+    "opb_net_debug_plan": (c_int, [c_void_p, c_int, c_void_p, POINTER(c_int)]),
+    "opb_net_debug_set_input": (c_int, [c_void_p, c_int, c_void_p]),
+    "opb_net_debug_info": (c_int, [c_void_p, c_int, c_void_p]),
+    "opb_net_debug_step": (c_int, [c_void_p, c_int, c_void_p]),
+    "opb_net_debug_read": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p]),
+    "opb_net_debug_run": (c_int, [c_void_p]),
     "opb_conv2d": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_int,
                            c_int, c_int, c_void_p, c_int]),
 }

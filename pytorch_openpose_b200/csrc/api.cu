@@ -456,6 +456,7 @@ struct opb_session {
     bool every_batch = false;            // the batch in flight is an opb_pose_every or opb_batch_pose_every batch
     int every_persons = -1;              // persons of the last finished opb_pose_every batch; -1: none
     bool every_linked = false;           // the last finished opb_pose_every batch was linked: ids_host holds its ids
+    std::vector<NetShape> debug_shapes;  // the plan of the opb_net_debug_* calls (looked up by its shapes on every call)
     ~opb_session() {
         plans.clear();
         net_plans.clear();
@@ -2326,6 +2327,90 @@ int opb_net_forward(opb_session* s, const uint8_t* dev_in, int n, int hp, int wp
             OPB_CUDA(cudaMemcpyAsync(dev_paf, plan->out_paf[0], px * 40 * 4, cudaMemcpyDeviceToDevice, s->stream));
         }
         OPB_CUDA(cudaMemcpyAsync(dev_heat, plan->out_heat[0], px * 24 * 4, cudaMemcpyDeviceToDevice, s->stream));
+        s->net->ctx->launches += plan->kernel_launches;
+        OPB_CUDA(cudaStreamSynchronize(s->stream));
+    });
+}
+
+static NetPlan* debug_plan(opb_session* s) {
+    OPB_REQUIRE(s, "null session");
+    OPB_REQUIRE(!s->debug_shapes.empty(), "opb_net_debug_plan first");
+    OPB_CUDA(cudaSetDevice(s->net->ctx->device));
+    return get_net_plan(s, s->debug_shapes);
+}
+static void fill_debug_step(const NetPlan* plan, int i, opb_debug_step* info) {
+    OPB_REQUIRE(i >= 0 && i < (int)plan->steps.size(), "step index out of range");
+    if (!info) return;
+    const StepInfo& st = plan->step_info[i];
+    OPB_REQUIRE((int)st.probs.size() <= OPB_DEBUG_MAX_PROBLEMS, "too many problems in one step");
+    memset(info, 0, sizeof(*info));
+    info->kind = st.kind;
+    info->n_problems = (int)st.probs.size();
+    info->block_n = st.block_n;
+    info->pool = st.pool;
+    info->wide = st.wide;
+    info->pair = st.pair;
+    info->half_tiles = st.half_tiles;
+    info->weights_resident = st.weights_resident;
+    snprintf(info->name, sizeof info->name, "%s", plan->step_names[i].c_str());
+    auto view = [](const TensorView& t) { return opb_debug_view{t.n, t.h, t.w, t.c, t.cstride, t.coff, t.elem}; };
+    for (size_t p = 0; p < st.probs.size(); ++p) {
+        const StepProblem& q = st.probs[p];
+        snprintf(info->layer[p], sizeof info->layer[p], "%s", q.layer.c_str());
+        snprintf(info->layer2[p], sizeof info->layer2[p], "%s", q.layer2.c_str());
+        info->scale[p] = q.scale;
+        info->in[p] = view(q.in);
+        info->out[p] = view(q.out);
+    }
+}
+
+int opb_net_debug_plan(opb_session* s, int n_scales, const int* shapes, int* n_steps) {
+    return guarded([&] {
+        OPB_REQUIRE(s && shapes && n_steps && n_scales >= 1 && n_scales <= kMaxScales, "opb_net_debug_plan: bad argument");
+        std::vector<NetShape> v;
+        for (int i = 0; i < n_scales; ++i) v.push_back({shapes[4 * i], shapes[4 * i + 1], shapes[4 * i + 2], shapes[4 * i + 3]});
+        s->debug_shapes = v;
+        *n_steps = (int)debug_plan(s)->steps.size();
+    });
+}
+int opb_net_debug_set_input(opb_session* s, int scale, const void* dev_src) {
+    return guarded([&] {
+        NetPlan* plan = debug_plan(s);
+        OPB_REQUIRE(dev_src && scale >= 0 && scale < (int)plan->shapes.size(), "opb_net_debug_set_input: bad argument");
+        const NetShape& sh = plan->shapes[scale];
+        OPB_CUDA(cudaMemcpyAsync(plan->in_u8[scale], dev_src, (size_t)sh.n * sh.hp * sh.wp * 3 * sh.in_elem,
+                                 cudaMemcpyDeviceToDevice, s->stream));
+        OPB_CUDA(cudaStreamSynchronize(s->stream));
+    });
+}
+int opb_net_debug_info(opb_session* s, int i, opb_debug_step* info) {
+    return guarded([&] { fill_debug_step(debug_plan(s), i, info); });
+}
+int opb_net_debug_step(opb_session* s, int i, opb_debug_step* info) {
+    return guarded([&] {
+        NetPlan* plan = debug_plan(s);
+        fill_debug_step(plan, i, info);
+        plan->steps[i](s->stream);
+        s->net->ctx->launches += 1;
+        OPB_CUDA(cudaStreamSynchronize(s->stream));
+    });
+}
+int opb_net_debug_read(opb_session* s, int i, int problem, int which, void* dev_dst) {
+    return guarded([&] {
+        NetPlan* plan = debug_plan(s);
+        OPB_REQUIRE(dev_dst && i >= 0 && i < (int)plan->steps.size(), "opb_net_debug_read: bad argument");
+        const StepInfo& st = plan->step_info[i];
+        OPB_REQUIRE(problem >= 0 && problem < (int)st.probs.size() && (which == 0 || which == 1), "opb_net_debug_read: bad view");
+        const TensorView& t = which == 0 ? st.probs[problem].in : st.probs[problem].out;
+        OPB_CUDA(cudaMemcpy2DAsync(dev_dst, (size_t)t.c * t.elem, t.ptr(), (size_t)t.cstride * t.elem, (size_t)t.c * t.elem,
+                                   t.pixels(), cudaMemcpyDeviceToDevice, s->stream));
+        OPB_CUDA(cudaStreamSynchronize(s->stream));
+    });
+}
+int opb_net_debug_run(opb_session* s) {
+    return guarded([&] {
+        NetPlan* plan = debug_plan(s);
+        plan->run(s->stream);
         s->net->ctx->launches += plan->kernel_launches;
         OPB_CUDA(cudaStreamSynchronize(s->stream));
     });

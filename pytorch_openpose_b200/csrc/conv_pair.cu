@@ -736,6 +736,8 @@ ConvLaunch* conv_pair_plan(const std::vector<ConvOp>& ops, int block_n, int num_
     OPB_REQUIRE(order_pairs(P) == pairs, "conv_pair: pair order");
     P.total_pairs = pairs;
     L->tiles = pairs * 2;
+    L->half_tiles = small;
+    L->weights_resident = P.bres > 0;
     L->block_n = block_n;
     const int clusters = pairs < num_sms / 2 ? pairs : num_sms / 2;
     L->grid = clusters * 2;

@@ -290,7 +290,7 @@ struct Builder {
         return s;
     }
     // one grouped tensor-core launch; ins/outs parallel vectors, all with the same layer kernel size/block_n
-    void conv_group(const std::vector<std::string>& names, const std::vector<TensorView>& ins,
+    void conv_group(const std::vector<std::string>& names, const std::vector<int>& scales, const std::vector<TensorView>& ins,
                     const std::vector<TensorView>& outs, bool pool) {
         size_t i = 0;
         while (i < names.size()) {
@@ -315,6 +315,11 @@ struct Builder {
                 OPB_REQUIRE(op.in.c == d.cin_dev, "plan: input channel mismatch for " + names[i]);
                 ops.push_back(op);
             }
+            StepInfo info;
+            info.kind = kStepConv;
+            info.pool = pool;
+            for (size_t j = 0; j < ops.size(); ++j)
+                info.probs.push_back({names[first + j], "", scales[first + j], ops[j].in, ops[j].out});
             // 3x3 / 7x7 layers run patch-resident (conv_patch.cu); 1x1 layers (and OPB_CONV_IMPL=tap) per-tap tiles
             // Small problems (one 640x480 frame at scale 0.5 gives 4 super-tiles per stage layer) leave most SMs idle and
             // their latency is the depth of one tile's K loop: halve the N tile so that twice as many CTA pairs share
@@ -331,6 +336,7 @@ struct Builder {
                         ops[j] = wide_pool_op(ops[j], d.w_wide, d.bias_wide);
                     }
                     bn_run = 128;
+                    info.wide = true;
                 }
             }
             if (ops[0].ks > 1 && conv_impl == 2 && bn == 128 && getenv("OPB_NO_SMALL_BN") == nullptr) {
@@ -345,13 +351,18 @@ struct Builder {
             plan->launches.push_back(L);
             plan->steps.push_back([L](cudaStream_t s) { conv_tc_plan_run(L, s); });
             plan->step_names.push_back(std::string(bn_run == 128 ? "conv_tc128:" : "conv_tc64:") + names[first]);   // the N tile that runs
+            info.block_n = bn_run;
+            info.pair = ops[0].ks > 1 && conv_impl == 2;
+            info.half_tiles = L->half_tiles;
+            info.weights_resident = L->weights_resident;
+            plan->step_info.push_back(info);
             plan->step_gflop.push_back(gf);
             plan->kernel_launches += 1;
         }
     }
     // Mconv6 + Mconv7 of a refinement stage as one fused launch (conv_tail.cu); OPB_NO_FUSE_TAILS=1: two grouped launches.
-    bool tail_group(const std::vector<std::string>& n6, const std::vector<std::string>& n7, const std::vector<TensorView>& ins,
-                    const std::vector<TensorView>& outs) {
+    bool tail_group(const std::vector<std::string>& n6, const std::vector<std::string>& n7, const std::vector<int>& scales,
+                    const std::vector<TensorView>& ins, const std::vector<TensorView>& outs) {
         static const bool fuse = getenv("OPB_NO_FUSE_TAILS") == nullptr;
         if (!fuse) return false;
         std::vector<TailOp> ops;
@@ -383,11 +394,12 @@ struct Builder {
         plan->step_names.push_back("conv_tail:" + n6[0]);
         plan->step_gflop.push_back(gf);
         plan->kernel_launches += 1;
+        tail_info(kStepTail, n6, n7, scales, ins, outs);
         return true;
     }
     // conv5_4 + conv5_5 of stage 1 (hand: conv6_1 + conv6_2) as one fused launch with the 512-channel intermediate kept on
     // the SM (conv_tail.cu, wide variant); OPB_NO_FUSE_WIDE=1: two grouped launches through HBM.
-    bool wide_tail_group(const std::vector<std::string>& n4, const std::vector<std::string>& n5,
+    bool wide_tail_group(const std::vector<std::string>& n4, const std::vector<std::string>& n5, const std::vector<int>& scales,
                          const std::vector<TensorView>& ins, const std::vector<TensorView>& outs) {
         static const bool fuse = getenv("OPB_NO_FUSE_WIDE") == nullptr && getenv("OPB_NO_FUSE_TAILS") == nullptr;
         if (!fuse) return false;
@@ -420,7 +432,16 @@ struct Builder {
         plan->step_names.push_back("conv_tail:" + n4[0]);
         plan->step_gflop.push_back(gf);
         plan->kernel_launches += 1;
+        tail_info(kStepTailWide, n4, n5, scales, ins, outs);
         return true;
+    }
+    void tail_info(int kind, const std::vector<std::string>& n1, const std::vector<std::string>& n2, const std::vector<int>& scales,
+                   const std::vector<TensorView>& ins, const std::vector<TensorView>& outs) {
+        StepInfo info;
+        info.kind = kind;
+        info.block_n = 128;
+        for (size_t i = 0; i < n1.size(); ++i) info.probs.push_back({n1[i], n2[i], scales[i], ins[i], outs[i]});
+        plan->step_info.push_back(info);
     }
     // algorithmic FLOPs of one layer on one input (un-padded channel counts, SURVEY.md 8d)
     double add_flops(const std::string& name, const TensorView& in) {
@@ -468,8 +489,15 @@ std::unique_ptr<NetPlan> build_net_plan(opb_net* net, const std::vector<NetShape
         plan->step_names.push_back("conv_first:conv1_1");
         plan->step_gflop.push_back(B.add_flops("conv1_1", in));
         plan->kernel_launches += 1;
+        StepInfo info;
+        info.kind = kStepConvFirst;
+        info.probs.push_back({"conv1_1", "", s, in, out});
+        plan->step_info.push_back(info);
         cur[s] = out;
     }
+
+    std::vector<int> scale_ids(S), branch_scale_ids(2 * S);
+    for (int s = 0; s < S; ++s) scale_ids[s] = branch_scale_ids[2 * s] = branch_scale_ids[2 * s + 1] = s;
 
     // ---- VGG trunk on tensor cores, all scales grouped per layer ----
     auto trunk = [&](const std::string& name, int cout, bool pool, std::vector<TensorView>* into = nullptr) {
@@ -482,7 +510,7 @@ std::unique_ptr<NetPlan> build_net_plan(opb_net* net, const std::vector<NetShape
             else
                 outs[s] = B.act(cur[s].n, cur[s].h, cur[s].w, cout);
         }
-        B.conv_group(std::vector<std::string>(S, name), cur, outs, pool && B.fuse_pool);
+        B.conv_group(std::vector<std::string>(S, name), scale_ids, cur, outs, pool && B.fuse_pool);
         if (pool && !B.fuse_pool) {
             for (int s = 0; s < S; ++s) {
                 TensorView pooled = B.act(outs[s].n, outs[s].h / 2, outs[s].w / 2, cout);
@@ -491,6 +519,10 @@ std::unique_ptr<NetPlan> build_net_plan(opb_net* net, const std::vector<NetShape
                 plan->step_names.push_back("maxpool2");
                 plan->step_gflop.push_back(0.0);
                 plan->kernel_launches += 1;
+                StepInfo info;
+                info.kind = kStepPool;
+                info.probs.push_back({name, "", s, full, pooled});
+                plan->step_info.push_back(info);
                 outs[s] = pooled;
             }
         }
@@ -547,14 +579,14 @@ std::unique_ptr<NetPlan> build_net_plan(opb_net* net, const std::vector<NetShape
             std::vector<TensorView> i1, i2, o1, o2;
             const int bn0 = net->dev.at(names[0]).block_n, bn1 = net->dev.at(names[1]).block_n;
             if (bn0 == bn1) {
-                B.conv_group(names, ins, outs, false);
+                B.conv_group(names, branch_scale_ids, ins, outs, false);
             } else {
                 for (int s = 0; s < S; ++s) {
                     n1.push_back(names[2 * s]); i1.push_back(ins[2 * s]); o1.push_back(outs[2 * s]);
                     n2.push_back(names[2 * s + 1]); i2.push_back(ins[2 * s + 1]); o2.push_back(outs[2 * s + 1]);
                 }
-                B.conv_group(n1, i1, o1, false);
-                B.conv_group(n2, i2, o2, false);
+                B.conv_group(n1, scale_ids, i1, o1, false);
+                B.conv_group(n2, scale_ids, i2, o2, false);
             }
         };
         auto both = [&](const std::vector<TensorView>& per_scale) {
@@ -592,7 +624,7 @@ std::unique_ptr<NetPlan> build_net_plan(opb_net* net, const std::vector<NetShape
                     snprintf(buf, sizeof buf, "conv5_5_CPM_L%d", b + 1);
                     n5[2 * s + b] = buf;
                 }
-            if (!B.wide_tail_group(n4, n5, pa, slices(false))) {
+            if (!B.wide_tail_group(n4, n5, branch_scale_ids, pa, slices(false))) {
                 branch_layer("conv5_4_CPM_L%d", 0, pa, wide, false);
                 branch_layer("conv5_5_CPM_L%d", 0, wide, slices(false), false);
             }
@@ -612,7 +644,7 @@ std::unique_ptr<NetPlan> build_net_plan(opb_net* net, const std::vector<NetShape
                     snprintf(buf, sizeof buf, "Mconv7_stage%d_L%d", st, b + 1);
                     n7[2 * s + b] = buf;
                 }
-            if (!B.tail_group(n6, n7, pa, slices(st == 6))) {
+            if (!B.tail_group(n6, n7, branch_scale_ids, pa, slices(st == 6))) {
                 branch_layer("Mconv6_stage%d_L%d", st, pa, pb, true);
                 branch_layer("Mconv7_stage%d_L%d", st, pb, slices(st == 6), true);
             }
@@ -635,10 +667,10 @@ std::unique_ptr<NetPlan> build_net_plan(opb_net* net, const std::vector<NetShape
             wide[s] = B.act(cat[s].n, cat[s].h, cat[s].w, 512);
         }
         auto layer = [&](const std::string& name, const std::vector<TensorView>& ins, const std::vector<TensorView>& outs) {
-            B.conv_group(std::vector<std::string>(S, name), ins, outs, false);
+            B.conv_group(std::vector<std::string>(S, name), scale_ids, ins, outs, false);
         };
-        if (!B.wide_tail_group(std::vector<std::string>(S, "conv6_1_CPM"), std::vector<std::string>(S, "conv6_2_CPM"), feat,
-                               heat_slice)) {
+        if (!B.wide_tail_group(std::vector<std::string>(S, "conv6_1_CPM"), std::vector<std::string>(S, "conv6_2_CPM"), scale_ids,
+                               feat, heat_slice)) {
             layer("conv6_1_CPM", feat, wide);
             layer("conv6_2_CPM", wide, heat_slice);
         }
@@ -652,13 +684,14 @@ std::unique_ptr<NetPlan> build_net_plan(opb_net* net, const std::vector<NetShape
             layer(nm(3), pb, pa);
             layer(nm(4), pa, pb);
             layer(nm(5), pb, pa);
-            if (!B.tail_group(std::vector<std::string>(S, nm(6)), std::vector<std::string>(S, nm(7)), pa,
+            if (!B.tail_group(std::vector<std::string>(S, nm(6)), std::vector<std::string>(S, nm(7)), scale_ids, pa,
                               st == 6 ? final_out : heat_slice)) {
                 layer(nm(6), pa, pb);
                 layer(nm(7), pb, st == 6 ? final_out : heat_slice);
             }
         }
     }
+    OPB_REQUIRE(plan->step_info.size() == plan->steps.size(), "plan: step metadata out of step");
     return plan;
 }
 

@@ -111,6 +111,27 @@ struct Profiler {
     }
 };
 
+// What one step of a plan computes, for the layer-by-layer tests (opb_net_debug_*): host metadata only.
+enum StepKind {
+    kStepConvFirst = OPB_STEP_CONV_FIRST, kStepConv = OPB_STEP_CONV, kStepTail = OPB_STEP_TAIL,
+    kStepTailWide = OPB_STEP_TAIL_WIDE, kStepPool = OPB_STEP_POOL
+};
+struct StepProblem {
+    std::string layer, layer2;      // layer2: the second layer of a fused tail
+    int scale = 0;                  // index into NetPlan::shapes
+    TensorView in, out;             // conv1_2 in its wide-pixel form: the views of the plain layer
+};
+struct StepInfo {
+    int kind = kStepConv;
+    std::vector<StepProblem> probs;
+    int block_n = 0;                // N tile of a tensor-core launch
+    bool pool = false;              // fused 2x2 max-pool
+    bool wide = false;              // conv1_2 ran in the wide-pixel form
+    bool pair = false;              // CTA-pair kernel
+    bool half_tiles = false;        // CTA pair: 16 x 8 tiles
+    bool weights_resident = false;  // CTA pair: the weight set stays in shared memory (bres)
+};
+
 struct NetPlan {
     DevPool pool;
     std::vector<NetShape> shapes;
@@ -118,6 +139,7 @@ struct NetPlan {
     std::vector<float*> out_paf, out_heat;      // per scale: fp32 NHWC (cstride 40 / 24); hand: heat only
     std::vector<std::function<void(cudaStream_t)>> steps;
     std::vector<std::string> step_names;        // parallel to steps
+    std::vector<StepInfo> step_info;            // parallel to steps
     std::vector<double> step_gflop;
     std::vector<ConvLaunch*> launches;
     int kernel_launches = 0;

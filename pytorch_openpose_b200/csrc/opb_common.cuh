@@ -79,6 +79,8 @@ void conv_tc_launch(const std::vector<ConvOp>& ops, int block_n, cudaStream_t st
 // pre-encoded launch (tensor maps + tile list built once per plan, replayed per frame)
 struct ConvLaunch {
     int tiles = 0;
+    bool half_tiles = false;        // CTA pair: 16 x 8 tiles (plan metadata, for the layer tests)
+    bool weights_resident = false;  // CTA pair: bres
     virtual void run(cudaStream_t stream) const = 0;
     virtual ~ConvLaunch() {}
 };

@@ -37,8 +37,8 @@ def test_body_keypoints_vs_bf16_emulating_oracle():
     layers with ReLU amplify that like any other perturbation (measured: maps 1e-2 apart, half the bf16-vs-fp32
     distance).  So the check is relative: the device must be CLOSER to the bf16 emulation than the emulation is to
     fp32, for the maps and for the key points -- a kernel defect would add to the device's distance and not to the
-    emulation's.  (Per-layer exactness is established separately: tests/test_gpu_conv.py compares every kernel variant
-    with an fp64 convolution of the same bf16 inputs.)"""
+    emulation's.  (Per-layer exactness is established separately: tests/test_gpu_net_layers.py compares every launch of
+    the networks' execution plans, problem by problem, with an fp64 convolution of the device's own bf16 inputs.)"""
     from pytorch_openpose_b200 import Body
     sd, img, scales = _kaiming_scene()
     body = Body(sd, scale_search=list(scales))

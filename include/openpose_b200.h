@@ -120,6 +120,13 @@ int opb_body_maps(opb_session* s, float* host_heat, float* host_paf);
 int opb_hand_submit(opb_session* s, const uint8_t* crops_bgr, int img_is_device, int n_crops, int height,
                     int width, const double* scale_search, int n_scales);
 int opb_hand_wait(opb_session* s, double* peaks);
+/* n_crops square crops of any sides as one batch: crop i is the dense sides[i] x sides[i] x 3 uint8 BGR image at
+ * bytes [offsets[i], offsets[i + 1]) of `packed` (n_crops + 1 offsets, offsets[0] = 0, crops back to back; `where`
+ * as opb_body_submit for the whole packed buffer).  Row i of the peaks equals opb_hand_submit on crop i alone, bit
+ * for bit.  The scales must resize every square crop to a net input whose side is a multiple of 8 (the default
+ * 0.5, 1, 1.5, 2 do).  Results: opb_hand_wait; opb_hand_maps refuses such a batch (its maps have no common shape). */
+int opb_hand_submit_ragged(opb_session* s, const uint8_t* packed, const size_t* offsets, int where, int n_crops,
+                           const int* sides, const double* scale_search, int n_scales);
 /* heatmap_avg of the last hand batch: (n_crops, 22, h, w) planar fp32 (src/hand.py:33,57).             */
 int opb_hand_maps(opb_session* s, float* host_heat);
 

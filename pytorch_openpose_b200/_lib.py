@@ -49,6 +49,7 @@ SIGNATURES = {
     "opb_body_wait_batch": (c_int, [c_void_p, POINTER(c_int), POINTER(c_int), POINTER(c_int)]),
     "opb_body_fetch_frame": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int]),
     "opb_hand_submit": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, POINTER(c_double), c_int]),
+    "opb_hand_submit_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, POINTER(c_double), c_int]),
     "opb_hand_wait": (c_int, [c_void_p, c_void_p]),
     "opb_pose_submit_batch": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, POINTER(c_double), c_int,
                                       POINTER(c_double), c_int, c_void_p]),

@@ -265,7 +265,12 @@ struct FramePlan {
     cudaGraphExec_t every_hand_graph = nullptr;
     uint64_t every_hand_gen = 0;
     int every_hand_uses = 0;
+    // Hand()(list of square crops) (opb_hand_submit_ragged), on the hand plan of the list
+    cudaGraphExec_t crops_graph = nullptr;
+    uint64_t crops_gen = 0;
+    int crops_uses = 0;
     ~FramePlan() {
+        if (crops_graph) cudaGraphExecDestroy(crops_graph);
         if (graph) cudaGraphExecDestroy(graph);
         if (pose_graph) cudaGraphExecDestroy(pose_graph);
         if (track_graph) cudaGraphExecDestroy(track_graph);
@@ -385,6 +390,27 @@ struct opb_session {
         std::vector<int> net_side;   // net input side per scale (the same for every crop size)
     };
     std::unique_ptr<Ragged> ragged;
+    // Hand()(list of square crops of any sides) (opb_hand_submit_ragged), on a hand session: the same tables for sides
+    // up to the largest seen, kept apart from `ragged` (a pose batch of another stream may be reading those), and the
+    // per-crop boxes, sides and byte offsets into the packed crops, grown to the longest list seen
+    std::unique_ptr<Ragged> crop_tables;
+    struct CropList {
+        DevPool pool;
+        int cap = 0;
+        HandBox* boxes = nullptr;        // [cap] (x = y = 0, side, not mirrored)
+        int* sides = nullptr;            // [cap]
+        size_t* offsets = nullptr;       // [cap] byte offset of each crop in the packed input
+        HandBox* boxes_host = nullptr;   // pinned copies, uploaded inside the launch sequence
+        int* sides_host = nullptr;
+        size_t* offsets_host = nullptr;
+        ~CropList() {
+            if (boxes_host) cudaFreeHost(boxes_host);
+            if (sides_host) cudaFreeHost(sides_host);
+            if (offsets_host) cudaFreeHost(offsets_host);
+        }
+    };
+    std::unique_ptr<CropList> crop_list;
+    bool hand_ragged = false;            // the last hand batch was a crop list: its maps have one pitch per crop
     struct PoseBuffers {
         DevPool pool;
         int frames = 0;
@@ -1027,6 +1053,7 @@ static void hand_submit(opb_session* s, const uint8_t* img, int where, int n, in
     ensure_host(s, 1, (size_t)n * 63);
     s->active = fp;
     s->hand_crops = n;
+    s->hand_ragged = false;
     cudaStream_t st = s->stream;
     s->prof.reset();
     s->prof.mark(st, "start");
@@ -1066,6 +1093,7 @@ static void batch_hand_submit(opb_session* s, const void* crops, bool u8, int wh
     ensure_host(s, 1, (size_t)n * 63);
     s->active = fp;
     s->hand_crops = n;
+    s->hand_ragged = false;
     cudaStream_t st = s->stream;
     s->prof.reset();
     s->prof.mark(st, "start");
@@ -1153,6 +1181,7 @@ static void hand_track_submit(opb_session* s, const uint8_t* frames, int where, 
     FramePlan* fp = get_plan(s, slots, boxsize, boxsize, &one, 1, 2);
     s->active = fp;
     s->hand_crops = slots;
+    s->hand_ragged = false;
     t.plan = fp;
     s->prof.reset();
     upload_bytes(s, t.frames_dev, frames, where, bytes);
@@ -1175,7 +1204,7 @@ static void hand_track_submit(opb_session* s, const uint8_t* frames, int where, 
 // ------------------------------------------------------------------------------------------------
 // Tap tables for every square crop of side 1..wmax at the hand estimator's scales, built with the same host functions
 // as the single-size path (so a ragged slot is processed exactly like Hand()(crop) would process that crop).
-static void build_ragged_tables(opb_session* hs, const double* scales, int ns, int wmax) {
+static std::unique_ptr<opb_session::Ragged> build_ragged_tables(const double* scales, int ns, int wmax) {
     auto r = std::make_unique<opb_session::Ragged>();
     r->scales.assign(scales, scales + ns);
     TableSlab slab;
@@ -1207,7 +1236,7 @@ static void build_ragged_tables(opb_session* hs, const double* scales, int ns, i
     r->tabs.index = r->pool.upload(index);
     r->tabs.n_scales = ns;
     r->tabs.wmax = wmax;
-    hs->ragged = std::move(r);
+    return r;
 }
 
 // the hand session's ragged tables cover every crop of an H x W frame at these scales; returns their crop side limit, the
@@ -1216,7 +1245,7 @@ static int ensure_ragged_tables(opb_session* bs, opb_session* hs, int H, int W, 
     const int wmax = std::min(H, W);
     if (!hs->ragged || hs->ragged->tabs.wmax < wmax || hs->ragged->scales != std::vector<double>(hscales, hscales + nhs)) {
         OPB_CUDA(cudaStreamSynchronize(bs->stream));
-        build_ragged_tables(hs, hscales, nhs, wmax);
+        hs->ragged = build_ragged_tables(hscales, nhs, wmax);
     }
     return hs->ragged->tabs.wmax;
 }
@@ -1239,20 +1268,96 @@ static void ensure_pose_buffers(opb_session* bs, int n) {
 // Hand on `slots` boxes (dims: side of each valid box, else 0) of the frames `fp` holds, as one ragged batch on the hand
 // plan `hp` of hs: crops cut -- the left ones mirrored -- from the frames -> hand CNN -> ragged post-processing, the
 // key points of slot i at hp->hb.peaks + i * 63
+static void ragged_hand_net_post(cudaStream_t st, const opb_session::Ragged& rg, FramePlan* hp, const HandBox* boxes,
+                                 const int* dims, int slots);
 static void ragged_hand_enqueue(cudaStream_t st, opb_session* hs, FramePlan* fp, FramePlan* hp, const HandBox* boxes,
                                 const int* dims, int slots) {
     const opb_session::Ragged& rg = *hs->ragged;
+    for (int s = 0; s < rg.tabs.n_scales; ++s)
+        preprocess_ragged_launch(fp->d_img, fp->key.H, fp->key.W, boxes, slots, hp->net->in_u8[s], rg.net_side[s], s, rg.tabs, st);
+    ragged_hand_net_post(st, rg, hp, boxes, dims, slots);
+}
+// the rest of a ragged hand batch once every slot's crop is resized into the net inputs of hp
+static void ragged_hand_net_post(cudaStream_t st, const opb_session::Ragged& rg, FramePlan* hp, const HandBox* boxes,
+                                 const int* dims, int slots) {
     const int tw = rg.tabs.wmax, nhs = rg.tabs.n_scales;
     const float* src[kMaxScales];
     int ho[kMaxScales], wo[kMaxScales];
     for (int s = 0; s < nhs; ++s) {
-        preprocess_ragged_launch(fp->d_img, fp->key.H, fp->key.W, boxes, slots, hp->net->in_u8[s], rg.net_side[s], s, rg.tabs, st);
         src[s] = hp->net->out_heat[s];
         ho[s] = wo[s] = rg.net_side[s] / 8;
     }
     hp->net->run(st, nullptr);
     upsample_ragged_launch(src, ho, wo, nhs, 24, 22, boxes, slots, rg.tabs, tw, hp->up_scratch, hp->heat_avg, st);
     hand_peaks_ragged_launch(hp->heat_avg, slots, 22, dims, tw, 0.03, hp->hb, st);      // thre, src/hand.py:31
+}
+
+// Hand()(crop) for every crop of a list of square crops of any sides, as one ragged batch: crop i is the dense
+// sides[i] x sides[i] x 3 image at bytes [offsets[i], offsets[i + 1]) of `packed`.  The crops are uploaded as they are
+// into the input arena; the packed form of the ragged crop kernel resizes each one with the tables of its own side, and
+// from there on the batch is the hand half of the pose pipeline (one CNN plan per crop count and scales, upsample,
+// Gaussian, components and selection at each crop's own size).
+static uint64_t gen_key(std::initializer_list<uint64_t> parts);
+static void hand_submit_ragged(opb_session* s, const uint8_t* packed, const size_t* offsets, int where, int n,
+                               const int* sides, const double* scales, int ns) {
+    OPB_REQUIRE(s->net->kind == OPB_NET_HAND, "session was created on a body network");
+    OPB_REQUIRE(n >= 1 && n <= 1024, "1..1024 crops per batch");
+    OPB_REQUIRE(ns >= 1 && ns <= kMaxScales, "scale_search must hold 1..8 entries");
+    OPB_REQUIRE(offsets[0] == 0, "offsets[0] must be 0 (the crops are packed back to back)");
+    int wmax = 0;
+    for (int i = 0; i < n; ++i) {
+        OPB_REQUIRE(sides[i] >= 1, "empty crop (the reference divides by oriImg.shape[0], src/hand.py:32)");
+        OPB_REQUIRE(offsets[i + 1] >= offsets[i] && offsets[i + 1] - offsets[i] == (size_t)sides[i] * sides[i] * 3,
+                    "offsets[i + 1] - offsets[i] must be sides[i] * sides[i] * 3 bytes (crop " + std::to_string(i) + ")");
+        wmax = std::max(wmax, sides[i]);
+    }
+    OPB_CUDA(cudaSetDevice(s->net->ctx->device));
+    cudaStream_t st = s->stream;
+    OPB_CUDA(cudaStreamSynchronize(st));          // the pinned crop list and the tables may still serve the previous batch
+    const std::vector<double> sc(scales, scales + ns);
+    if (!s->crop_tables || s->crop_tables->tabs.wmax < wmax || s->crop_tables->scales != sc)
+        s->crop_tables = build_ragged_tables(scales, ns, wmax);
+    const opb_session::Ragged& rg = *s->crop_tables;
+    const int tw = rg.tabs.wmax;
+    if (!s->crop_list || s->crop_list->cap < n) {
+        auto cl = std::make_unique<opb_session::CropList>();
+        cl->boxes = cl->pool.alloc_t<HandBox>(n);
+        cl->sides = cl->pool.alloc_t<int>(n);
+        cl->offsets = cl->pool.alloc_t<size_t>(n);
+        OPB_CUDA(cudaMallocHost((void**)&cl->boxes_host, (size_t)n * sizeof(HandBox)));
+        OPB_CUDA(cudaMallocHost((void**)&cl->sides_host, (size_t)n * sizeof(int)));
+        OPB_CUDA(cudaMallocHost((void**)&cl->offsets_host, (size_t)n * sizeof(size_t)));
+        cl->cap = n;
+        s->crop_list = std::move(cl);
+    }
+    opb_session::CropList& cl = *s->crop_list;
+    for (int i = 0; i < n; ++i) {
+        cl.boxes_host[i] = HandBox{i, 0, 0, sides[i], 0, 1};
+        cl.sides_host[i] = sides[i];
+        cl.offsets_host[i] = offsets[i];
+    }
+    // the frame plan of n crops of the table side: its arenas hold n tw-square crops (more than the packed list needs)
+    // and its CNN plan is the one every n-crop batch of these scales shares
+    FramePlan* fp = get_plan(s, n, tw, tw, scales, ns);
+    ensure_host(s, 1, (size_t)n * 63);
+    s->active = fp;
+    s->hand_crops = n;
+    s->hand_ragged = true;
+    s->prof.reset();
+    upload_bytes(s, fp->d_img, packed, where, offsets[n]);
+    const uint64_t gen = gen_key({s->buffer_gen, (uint64_t)(uintptr_t)cl.boxes, (uint64_t)(uintptr_t)rg.tabs.slab,
+                                  (uint64_t)(uintptr_t)rg.tabs.index});
+    run_or_replay_slot(s, GraphSlot{fp->crops_graph, fp->crops_gen, fp->crops_uses}, gen, [&] {
+        OPB_CUDA(cudaMemcpyAsync(cl.boxes, cl.boxes_host, (size_t)n * sizeof(HandBox), cudaMemcpyHostToDevice, st));
+        OPB_CUDA(cudaMemcpyAsync(cl.sides, cl.sides_host, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, st));
+        OPB_CUDA(cudaMemcpyAsync(cl.offsets, cl.offsets_host, (size_t)n * sizeof(size_t), cudaMemcpyHostToDevice, st));
+        for (int i = 0; i < ns; ++i)
+            preprocess_packed_launch(fp->d_img, cl.offsets, cl.boxes, n, fp->net->in_u8[i], rg.net_side[i], i, rg.tabs, st);
+        ragged_hand_net_post(st, rg, fp, cl.boxes, cl.sides, n);
+        OPB_CUDA(cudaMemcpyAsync(s->hand_host, fp->hb.peaks, (size_t)n * 63 * sizeof(double), cudaMemcpyDeviceToHost, st));
+    });
+    OPB_CUDA(cudaEventRecord(s->done, st));
+    s->net->ctx->launches += ns + fp->net->kernel_launches + (ns + 1) + 6;
 }
 
 // the hand half of the pose pipeline, on the body session's stream: boxes from the body results (or the fixed ones already
@@ -1291,6 +1396,7 @@ static void pose_submit(opb_session* bs, opb_session* hs, const uint8_t* imgs, i
     FramePlan* hp = get_plan(hs, slots, tw, tw, hscales, nhs);
     hs->active = hp;
     hs->hand_crops = slots;
+    hs->hand_ragged = false;
     int* fixed_dev = nullptr;
     if (fixed_boxes) {
         OPB_CUDA(cudaStreamSynchronize(st));                   // the pinned copy of the previous batch's boxes is free
@@ -1391,6 +1497,7 @@ static void batch_pose_submit(opb_session* bs, opb_session* hs, const uint8_t* f
     FramePlan* hp = get_plan(hs, 2 * n, boxsize, boxsize, &one, 1, 2);      // uint8 Batch_hand on 2n crops
     hs->active = hp;
     hs->hand_crops = 2 * n;
+    hs->hand_ragged = false;
     t.plan = hp;
     bs->prof.reset();
     bs->prof.mark(st, "start");
@@ -1494,6 +1601,7 @@ static void every_submit(opb_session* bs, opb_session* hs, const uint8_t* imgs, 
     FramePlan* hp = get_plan(hs, kEveryChunk, tw, tw, hscales, nhs);
     hs->active = hp;
     hs->hand_crops = kEveryChunk;
+    hs->hand_ragged = false;
     const uint64_t gen = gen_key({bs->buffer_gen, bs->every->gen});
     run_or_replay_slot(bs, GraphSlot{fp->every_graph, fp->every_gen, fp->every_uses}, gen, [&] {
         run_front(bs, fp, n, H, W);
@@ -1551,6 +1659,7 @@ static void batch_every_submit(opb_session* bs, opb_session* hs, const uint8_t* 
     FramePlan* hp = get_plan(hs, kBatchEveryChunk, boxsize, boxsize, &one, 1, 2);   // uint8 Batch_hand on one chunk
     hs->active = hp;
     hs->hand_crops = kBatchEveryChunk;
+    hs->hand_ragged = false;
     bs->prof.reset();
     bs->prof.mark(st, "start");
     upload_image(bs, fp, frames, where, (size_t)n * H * W * 3);
@@ -1981,6 +2090,7 @@ int opb_body_maps(opb_session* s, float* host_heat, float* host_paf) {
 int opb_hand_maps(opb_session* s, float* host_heat) {
     return guarded([&] {
         OPB_REQUIRE(s && s->active && s->net->kind == OPB_NET_HAND && host_heat, "no finished hand batch");
+        OPB_REQUIRE(!s->hand_ragged, "the last hand batch was a list of crops of different sides: its maps have no common shape");
         OPB_CUDA(cudaEventSynchronize(s->done));
         const size_t px = (size_t)s->active->key.H * s->active->key.W;
         OPB_CUDA(cudaMemcpy(host_heat, s->active->heat_avg, px * 22 * 4 * s->active->key.n, cudaMemcpyDeviceToHost));
@@ -2276,6 +2386,13 @@ int opb_hand_submit(opb_session* s, const uint8_t* crops, int img_is_device, int
     return guarded([&] {
         OPB_REQUIRE(s && crops && scales, "null argument");
         hand_submit(s, crops, img_is_device, n, H, W, scales, ns);
+    });
+}
+int opb_hand_submit_ragged(opb_session* s, const uint8_t* packed, const size_t* offsets, int where, int n, const int* sides,
+                           const double* scales, int ns) {
+    return guarded([&] {
+        OPB_REQUIRE(s && packed && offsets && sides && scales, "null argument");
+        hand_submit_ragged(s, packed, offsets, where, n, sides, scales, ns);
     });
 }
 int opb_hand_wait(opb_session* s, double* peaks) {

@@ -413,6 +413,9 @@ struct RaggedTables {
 };
 void preprocess_ragged_launch(const uint8_t* frames, int H, int W, const HandBox* boxes, int n_slots, uint8_t* out, int S,
                               int scale, const RaggedTables& tabs, cudaStream_t stream);
+// the same resize with slot i read from its own dense boxes[i].w-square crop at byte offset offsets[i] of `packed`
+void preprocess_packed_launch(const uint8_t* packed, const size_t* offsets, const HandBox* boxes, int n_slots, uint8_t* out,
+                              int S, int scale, const RaggedTables& tabs, cudaStream_t stream);
 void upsample_ragged_launch(const float* const* src, const int* ho, const int* wo, int n_scales, int cstride, int C,
                             const HandBox* boxes, int n_slots, const RaggedTables& tabs, int wmax, float* scratch,
                             float* out_planar, cudaStream_t stream);

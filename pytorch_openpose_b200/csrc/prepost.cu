@@ -239,7 +239,11 @@ __device__ __forceinline__ const uint8_t* ragged_table(const RaggedTables& t, in
 
 // Hand.__call__'s cv2.resize of the crop (src/hand.py:38) for every slot, reading the crop -- mirrored for left hands,
 // cv2.flip(crop, 1) at srcmx/MotionEstimation.py:191 -- straight from the frame.  Arithmetic as preprocess_kernel.
+// kPacked: slot i's crop is its own dense w x w image at byte offset offsets[i] of `frames` (Hand()(list of crops));
+// the box then only carries the side (x = y = 0, not mirrored).
+template <bool kPacked>
 __global__ void __launch_bounds__(128) preprocess_ragged_kernel(const uint8_t* __restrict__ frames, int H, int W,
+                                                                const size_t* __restrict__ offsets,
                                                                 const HandBox* __restrict__ boxes, uint8_t* __restrict__ out,
                                                                 int S, int scale, const RaggedTables tabs) {
     const int x = blockIdx.x * blockDim.x + threadIdx.x;
@@ -254,7 +258,8 @@ __global__ void __launch_bounds__(128) preprocess_ragged_kernel(const uint8_t* _
     const int w = b.w;
     const int* xf = (const int*)ragged_table(tabs, w, scale, 0);
     const short* xc = (const short*)ragged_table(tabs, w, scale, 1);
-    const uint8_t* img = frames + (size_t)b.frame * H * W * 3;
+    const uint8_t* img = kPacked ? frames + offsets[blockIdx.z] : frames + (size_t)b.frame * H * W * 3;
+    const int pitch = kPacked ? w : W;
     const int x0 = xf[x], y0 = xf[y];                            // square crops: one table for both axes
     int cx[4], wx[4];
     const short4 xw4 = *(const short4*)(xc + x * 4);
@@ -267,7 +272,7 @@ __global__ void __launch_bounds__(128) preprocess_ragged_kernel(const uint8_t* _
     int hor[4][3];
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-        const uint8_t* row = img + (size_t)(b.y + clampi(y0 + k, 0, w - 1)) * W * 3;
+        const uint8_t* row = img + (size_t)(b.y + clampi(y0 + k, 0, w - 1)) * pitch * 3;
         int s0 = 0, s1 = 0, s2 = 0;
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
@@ -384,7 +389,14 @@ void preprocess_launch_batched(const uint8_t* img, int n, int H, int W, uint8_t*
 void preprocess_ragged_launch(const uint8_t* frames, int H, int W, const HandBox* boxes, int n_slots, uint8_t* out, int S,
                               int scale, const RaggedTables& tabs, cudaStream_t stream) {
     dim3 grid(cdiv(S, 128), S, n_slots);
-    preprocess_ragged_kernel<<<grid, 128, 0, stream>>>(frames, H, W, boxes, out, S, scale, tabs);
+    preprocess_ragged_kernel<false><<<grid, 128, 0, stream>>>(frames, H, W, nullptr, boxes, out, S, scale, tabs);
+    OPB_CUDA(cudaGetLastError());
+}
+
+void preprocess_packed_launch(const uint8_t* packed, const size_t* offsets, const HandBox* boxes, int n_slots, uint8_t* out,
+                              int S, int scale, const RaggedTables& tabs, cudaStream_t stream) {
+    dim3 grid(cdiv(S, 128), S, n_slots);
+    preprocess_ragged_kernel<true><<<grid, 128, 0, stream>>>(packed, 0, 0, offsets, boxes, out, S, scale, tabs);
     OPB_CUDA(cudaGetLastError());
 }
 

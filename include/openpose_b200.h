@@ -369,6 +369,19 @@ int opb_net_debug_step(opb_session* s, int i, opb_debug_step* info);
 int opb_net_debug_read(opb_session* s, int i, int problem, int which, void* dev_dst);
 int opb_net_debug_run(opb_session* s);
 
+/* Post-processing of Body (mode 0: scale_search, 1..8 scales) and Batch_body (mode 1: g_scale, one scale) on net
+ * outputs the caller supplies, through the frame plan a real call of that geometry uses: the same tile bounds, fused
+ * peak kernel, composite PAF sampling and grouping, only the upload, the front end and the CNN are skipped.
+ * post_dims (host only): ho_wo[2 * i], ho_wo[2 * i + 1] = the net output size of scale i; *fused = 1 when the peak
+ *   kernel evaluates the heat maps from the net outputs, 0 when the plan materialises them first.
+ * post_submit: heat[i] (n, ho, wo, 24) and paf[i] (n, ho, wo, 40) fp32 host arrays per scale (19 / 38 channels used).
+ *   Results through opb_body_wait_batch / opb_body_fetch_frame; the maps through opb_body_maps / opb_batch_maps.
+ * part_begin (after a wait, any body batch): first candidate row of each of the 18 parts of a frame, and the total. */
+int opb_body_debug_post_dims(int height, int width, const double* scales, int n_scales, int mode, int* ho_wo, int* fused);
+int opb_body_debug_post_submit(opb_session* s, int n_frames, int height, int width, const double* scales, int n_scales,
+                               int mode, const float* const* heat, const float* const* paf);
+int opb_body_debug_part_begin(opb_session* s, int frame, int* part_begin19);
+
 /* Host only (no device call): the wide-pixel weights of a 64 -> 64 channel 3x3 layer (src/model.py:36 conv1_2) as the
  * library packs them at opb_net_finalize.  weight: [64][64][3][3] fp32, bias [64]  ->  w_wide [128][9][128] bf16 bit
  * patterns (output column = parity_out * 64 + cout; K index = (dy * 3 + di) * 128 + parity_in * 64 + cin, di the tap in

@@ -110,6 +110,10 @@ SIGNATURES = {
     "opb_net_debug_step": (c_int, [c_void_p, c_int, c_void_p]),
     "opb_net_debug_read": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p]),
     "opb_net_debug_run": (c_int, [c_void_p]),
+    "opb_body_debug_post_dims": (c_int, [c_int, c_int, POINTER(c_double), c_int, c_int, c_void_p, POINTER(c_int)]),
+    "opb_body_debug_post_submit": (c_int, [c_void_p, c_int, c_int, c_int, POINTER(c_double), c_int, c_int,
+                                           POINTER(c_void_p), POINTER(c_void_p)]),
+    "opb_body_debug_part_begin": (c_int, [c_void_p, c_int, c_void_p]),
     "opb_conv2d": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_int,
                            c_int, c_int, c_void_p, c_int]),
 }

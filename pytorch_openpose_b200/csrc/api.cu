@@ -645,6 +645,25 @@ static void upload_post_table(FramePlan* fp, cudaStream_t st) {
     OPB_CUDA(cudaMemcpyAsync(fp->post_dev, fp->post.data(), fp->post.size() * sizeof(FramePost), cudaMemcpyHostToDevice, st));
 }
 
+// per-scale net output sizes of a plan: mode 0 Body (scale_search), mode >= 1 the batched estimators (one scale)
+static ScaleDims plan_dims(int H, int W, double scale, int mode, bool body) {
+    return mode >= 1 ? batch_dims(H, W, scale, body) : scale_dims(H, W, scale);
+}
+
+// do the heat maps of a body plan fit the fused peak kernel (peaks.cu), so that they need not be materialised?
+static bool plan_fits_fused(const std::vector<UpTables>& uptabs, const std::vector<ScaleDims>& dims, int H, int W) {
+    std::vector<std::vector<int>> xf, ybf, ybr;
+    std::vector<int> wo, rs;
+    for (size_t i = 0; i < dims.size(); ++i) {
+        xf.push_back(uptabs[i].h_xf);
+        ybf.push_back(uptabs[i].h_ybf);
+        ybr.push_back(uptabs[i].h_ybr);
+        wo.push_back(dims[i].wo);
+        rs.push_back(uptabs[i].yb_rs);
+    }
+    return composite_fits_fused(xf, ybf, ybr, wo, rs, H, W);
+}
+
 static FramePlan* get_plan(opb_session* s, int n, int H, int W, const double* scales, int n_scales, int mode = 0) {
     OPB_REQUIRE(n_scales >= 1 && n_scales <= kMaxScales, "scale_search must hold 1..8 entries");
     FrameKey key{n, H, W, std::vector<double>(scales, scales + n_scales), mode};
@@ -664,7 +683,7 @@ static FramePlan* get_plan(opb_session* s, int n, int H, int W, const double* sc
     std::vector<NetShape> shapes;
     const int C = body ? 57 : 22;
     for (int i = 0; i < n_scales; ++i) {
-        const ScaleDims d = mode >= 1 ? batch_dims(H, W, scales[i], body) : scale_dims(H, W, scales[i]);
+        const ScaleDims d = plan_dims(H, W, scales[i], mode, body);
         fp->dims.push_back(d);
         if (mode >= 1) fp->f32taps.push_back(make_f32_taps(fp->tables, H, W, d));
         else fp->u8taps.push_back(make_u8_taps(fp->tables, H, W, d));
@@ -681,17 +700,8 @@ static FramePlan* get_plan(opb_session* s, int n, int H, int W, const double* sc
     for (auto& t : fp->uptabs) t.relocate_to(dev_tables);
     fp->launches_per_frame = n_scales /*preprocess*/ + fp->net->kernel_launches;
     if (body) {
-        std::vector<std::vector<int>> xf, ybf, ybr;
-        std::vector<int> wo, rs;
-        for (int i = 0; i < n_scales; ++i) {
-            xf.push_back(fp->uptabs[i].h_xf);
-            ybf.push_back(fp->uptabs[i].h_ybf);
-            ybr.push_back(fp->uptabs[i].h_ybr);
-            wo.push_back(fp->dims[i].wo);
-            rs.push_back(fp->uptabs[i].yb_rs);
-        }
         static const bool no_fuse = getenv("OPB_NO_FUSED_PEAKS") != nullptr;      // A/B switch: materialised planes
-        fp->fused_ok = !no_fuse && composite_fits_fused(xf, ybf, ybr, wo, rs, H, W);
+        fp->fused_ok = !no_fuse && plan_fits_fused(fp->uptabs, fp->dims, H, W);
         // OPB_TEST_SMALL_BUFFERS: start with tiny result buffers so that tests exercise the growth path of body_wait
         static const bool tiny = getenv("OPB_TEST_SMALL_BUFFERS") != nullptr;
         fp->counters = fp->pool.alloc_t<int>((size_t)n * kCounterInts, true);
@@ -2530,6 +2540,61 @@ int opb_net_debug_run(opb_session* s) {
         plan->run(s->stream);
         s->net->ctx->launches += plan->kernel_launches;
         OPB_CUDA(cudaStreamSynchronize(s->stream));
+    });
+}
+
+// Body (mode 0) / Batch_body (mode 1) post-processing of a frame plan on caller-supplied net outputs
+static void check_debug_post(int n_scales, int mode) {
+    OPB_REQUIRE(mode == 0 || mode == 1, "mode 0 (Body) or 1 (Batch_body)");
+    OPB_REQUIRE(n_scales >= 1 && n_scales <= kMaxScales && (mode == 0 || n_scales == 1),
+                "Body takes 1..8 scales, Batch_body one");
+}
+int opb_body_debug_post_dims(int H, int W, const double* scales, int ns, int mode, int* ho_wo, int* fused) {
+    return guarded([&] {
+        OPB_REQUIRE(scales && ho_wo && fused, "null argument");
+        check_debug_post(ns, mode);
+        TableSlab slab;
+        std::vector<ScaleDims> dims;
+        std::vector<UpTables> tabs;
+        for (int i = 0; i < ns; ++i) {
+            dims.push_back(plan_dims(H, W, scales[i], mode, true));
+            tabs.push_back(make_up_tables(slab, H, W, dims[i], ns));
+            ho_wo[2 * i] = dims[i].ho;
+            ho_wo[2 * i + 1] = dims[i].wo;
+        }
+        *fused = plan_fits_fused(tabs, dims, H, W) ? 1 : 0;
+    });
+}
+int opb_body_debug_post_submit(opb_session* s, int n, int H, int W, const double* scales, int ns, int mode,
+                               const float* const* heat, const float* const* paf) {
+    return guarded([&] {
+        OPB_REQUIRE(s && scales && heat && paf, "null argument");
+        OPB_REQUIRE(s->net->kind == OPB_NET_BODY, "session was created on a hand network");
+        OPB_REQUIRE(n >= 1 && n <= 64, "1..64 frames per batch");
+        check_debug_post(ns, mode);
+        OPB_CUDA(cudaSetDevice(s->net->ctx->device));
+        FramePlan* fp = get_plan(s, n, H, W, scales, ns, mode == 0 ? 0 : 2);
+        ensure_host(s, n, 0);
+        s->active = fp;
+        s->n_frames = n;
+        s->prof.reset();
+        for (int i = 0; i < ns; ++i) {
+            OPB_REQUIRE(heat[i] && paf[i], "null net output");
+            const size_t px = (size_t)n * fp->dims[i].ho * fp->dims[i].wo;
+            OPB_CUDA(cudaMemcpyAsync(fp->net->out_heat[i], heat[i], px * 24 * sizeof(float), cudaMemcpyHostToDevice, s->stream));
+            OPB_CUDA(cudaMemcpyAsync(fp->net->out_paf[i], paf[i], px * 40 * sizeof(float), cudaMemcpyHostToDevice, s->stream));
+        }
+        body_post_enqueue(s, fp, n, H, W);
+        finish_submit(s, fp);
+        s->net->ctx->launches -= ns + fp->net->kernel_launches;        // no front end, no CNN
+        OPB_CUDA(cudaStreamSynchronize(s->stream));                     // the caller's arrays may be pageable
+    });
+}
+int opb_body_debug_part_begin(opb_session* s, int frame, int* part_begin19) {
+    return guarded([&] {
+        OPB_REQUIRE(s && part_begin19 && s->active && frame >= 0 && frame < (int)s->results.size(),
+                    "no finished frame with this index (opb_body_wait_batch first)");
+        memcpy(part_begin19, s->host[frame].counts + 1, 19 * sizeof(int));
     });
 }
 

@@ -316,6 +316,21 @@ int opb_batch_pose_every_select(opb_context* ctx, const double* host_candidates,
                                 int* host_boxes);
 /* src/hand.py:59-75 on a planar (>=21, h, w) fp32 device map -> 21x3 float64 host array.            */
 int opb_hand_peaks(opb_context* ctx, const float* dev_heat, int height, int width, double thre, double* host_peaks);
+/* Debug: the hand post-processing launches of one geometry on planar fp32 device maps, crop c's 21 key-point planes
+ * at dev_maps + c * chan_stride planes.  mode 0 (Hand, threshold 0.03 on the sigma=3 smoothing): sides == NULL runs
+ * the equal-size launch on n_crops maps of height x width; otherwise the list launch, crop c of side sides[c] (0 = no
+ * crop, zero key points), planes at pitch max(sides)^2 (height and width are ignored).  mode 1 (Batch_hand, threshold
+ * 0.035f on the maps as given).  Optional device outputs: dev_smoothed (mode 0 equal size) the float64 smoothed
+ * planes, dev_labels the component labels (root = smallest raster index of the component, -1 off the mask),
+ * dev_sums the sums plane, each n_crops * 21 planes at the geometry's pitch.  flags & 1: every component counts as a
+ * contender of the component choice, and dev_sums holds numpy's sum of each component at its root.
+ * host_peaks: n_crops * 21 * 3 doubles (x, y, score). */
+int opb_hand_debug_post(opb_context* ctx, const float* dev_maps, int n_crops, int chan_stride, const int* sides, int height,
+                        int width, int mode, int flags, double* dev_smoothed, int* dev_labels, double* dev_sums,
+                        double* host_peaks);
+/* Host only (no device call): np.sum of n contiguous float32 (is_f32) or float64 values, computed by the pairwise
+ * summation the device's component choice uses; *out = the result (float32 results widened). */
+int opb_debug_pairwise_sum(const void* values, long long n, int is_f32, double* out);
 
 /* Debug: the float64 Gaussian-smoothed maps (parts, H, W) the NMS compares, for bit-exactness tests. */
 int opb_smooth_debug(opb_context* ctx, const float* dev_heat, int parts, int height, int width, double* dev_smoothed);

@@ -96,6 +96,9 @@ SIGNATURES = {
     "opb_group_limbs": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, POINTER(c_int), c_double, c_void_p, c_int,
                                 POINTER(c_int), c_void_p, c_int, POINTER(c_int)]),
     "opb_hand_peaks": (c_int, [c_void_p, c_void_p, c_int, c_int, c_double, c_void_p]),
+    "opb_hand_debug_post": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_int, c_int, c_void_p,
+                                    c_void_p, c_void_p, c_void_p]),
+    "opb_debug_pairwise_sum": (c_int, [c_void_p, ctypes.c_longlong, c_int, POINTER(c_double)]),
     "opb_bench_grouping": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, POINTER(c_float), POINTER(c_int),
                                    POINTER(c_int)]),
     "opb_smooth_debug": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),

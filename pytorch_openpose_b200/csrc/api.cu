@@ -2873,19 +2873,59 @@ int opb_batch_pose_every_select(opb_context* ctx, const double* host_candidates,
     });
 }
 
+// The hand post-processing launches of one geometry on caller-supplied planar maps (opb_hand_peaks, opb_hand_debug_post)
+static void hand_post(opb_context* ctx, const float* dev_maps, int n_crops, int chan_stride, const int* sides, int H, int W,
+                      int mode, int flags, double thre, double* dev_smoothed, int* dev_labels, double* dev_sums,
+                      double* host_peaks) {
+    OPB_REQUIRE(ctx && dev_maps && host_peaks, "hand post-processing: null argument");
+    OPB_REQUIRE(n_crops >= 1 && chan_stride >= 21 && (mode == 0 || mode == 1) && (flags & ~1) == 0,
+                "hand post-processing: bad argument");
+    OPB_REQUIRE(!sides || mode == 0, "hand post-processing: per-crop sides are a mode-0 geometry");
+    OPB_REQUIRE(!dev_smoothed || (mode == 0 && !sides), "hand post-processing: smoothed planes are a mode-0 equal-size output");
+    if (sides) {
+        H = W = 0;
+        for (int c = 0; c < n_crops; ++c) {
+            OPB_REQUIRE(sides[c] >= 0, "hand post-processing: negative side");
+            H = W = std::max(W, sides[c]);
+        }
+    }
+    OPB_REQUIRE(H >= 1 && W >= 1, "hand post-processing: empty maps");
+    OPB_CUDA(cudaSetDevice(ctx->device));
+    const size_t planes = (size_t)n_crops * 21 * H * W;
+    DevPool pool;
+    HandBuffers hb;
+    hb.labels = dev_labels ? dev_labels : pool.alloc_t<int>(planes);
+    hb.sums = dev_sums ? dev_sums : pool.alloc_t<double>(planes);
+    hb.peaks = pool.alloc_t<double>((size_t)n_crops * 63, true);
+    hb.exact_all = flags & 1;
+    if (mode == 1)
+        hand_peaks_blurred_launch(dev_maps, n_crops, chan_stride, H, W, (float)thre, hb, ctx->stream);
+    else if (sides)
+        hand_peaks_ragged_launch(dev_maps, n_crops, chan_stride, pool.upload(std::vector<int>(sides, sides + n_crops)), W,
+                                 thre, hb, ctx->stream);
+    else
+        hand_peaks_launch2(dev_maps, n_crops, chan_stride, H, W, thre, hb, dev_smoothed, ctx->stream);
+    ctx->launches += 6;                  // smooth or mask, runs, merge, compress, flatten, select
+    OPB_CUDA(cudaMemcpyAsync(host_peaks, hb.peaks, (size_t)n_crops * 63 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    OPB_CUDA(cudaStreamSynchronize(ctx->stream));
+}
+
 int opb_hand_peaks(opb_context* ctx, const float* dev_heat, int H, int W, double thre, double* host_peaks) {
+    return guarded([&] { hand_post(ctx, dev_heat, 1, 21, nullptr, H, W, 0, 0, thre, nullptr, nullptr, nullptr, host_peaks); });
+}
+
+int opb_hand_debug_post(opb_context* ctx, const float* dev_maps, int n_crops, int chan_stride, const int* sides, int H, int W,
+                        int mode, int flags, double* dev_smoothed, int* dev_labels, double* dev_sums, double* host_peaks) {
     return guarded([&] {
-        OPB_REQUIRE(dev_heat && host_peaks, "null argument");
-        OPB_CUDA(cudaSetDevice(ctx->device));
-        DevPool pool;
-        HandBuffers hb;
-        hb.labels = pool.alloc_t<int>((size_t)21 * H * W);
-        hb.sums = pool.alloc_t<double>((size_t)21 * H * W);
-        hb.peaks = pool.alloc_t<double>(63, true);
-        hand_peaks_launch2(dev_heat, 1, 21, H, W, thre, hb, nullptr, ctx->stream);
-        ctx->launches += 4;
-        OPB_CUDA(cudaMemcpyAsync(host_peaks, hb.peaks, 63 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-        OPB_CUDA(cudaStreamSynchronize(ctx->stream));
+        hand_post(ctx, dev_maps, n_crops, chan_stride, sides, H, W, mode, flags, mode == 1 ? (double)0.035f : 0.03,
+                  dev_smoothed, dev_labels, dev_sums, host_peaks);
+    });
+}
+
+int opb_debug_pairwise_sum(const void* values, long long n, int is_f32, double* out) {
+    return guarded([&] {
+        OPB_REQUIRE(out && n >= 0 && (values || n == 0), "opb_debug_pairwise_sum: bad argument");
+        *out = is_f32 ? (double)numpy_sum((const float*)values, n) : numpy_sum((const double*)values, n);
     });
 }
 

@@ -282,8 +282,9 @@ void pack_results_launch(const FramePost* frames_dev, int n_frames, cudaStream_t
 // ---- hand peaks (hand.cu)
 struct HandBuffers {
     int* labels;              // [crops*21][h][w]
-    double* sums;             // [crops*21][h][w] per-root sums of raw values
-    double* peaks;            // [crops*21][3] output
+    double* sums;             // [crops*21][h][w] per-root sums of raw values; scratch of the exact component sums
+    double* peaks;            // [crops*21][3] output; [0] / [1] hold the map's sum of |value| and mask count until select
+    bool exact_all = false;   // opb_hand_debug_post flag 1: every component gets numpy's sum (sums plane: that sum at its root)
 };
 void hand_peaks_launch2(const float* heat_planar, int n_crops, int chan_stride_maps, int h, int w, double thre,
                         HandBuffers hb, double* smoothed_out, cudaStream_t stream);
@@ -313,6 +314,66 @@ __host__ __device__ inline double dmul_rn(double a, double b) {
     return a * b;
 #endif
 }
+// np.sum of a contiguous 1-D array of n values in the array's own type (float64 for Hand's raw maps, float32 for
+// Batch_hand's blurred maps): numpy's pairwise summation over all n elements, then added to the reduction's +0.0
+// (which turns a sum of -0.0s into +0.0).  Every addition rounds once and there are no products to contract, so the
+// host and the device produce the same bits.
+__host__ __device__ inline long long pairwise_split(long long n) {
+    long long n2 = n / 2;
+    return n2 - n2 % 8;
+}
+template <typename T>
+__host__ __device__ inline T pairwise_leaf(const T* a, long long n) {           // n <= 128
+    if (n < 8) {
+        T r = T(0);
+        for (long long i = 0; i < n; ++i) r = r + a[i];
+        return r;
+    }
+    T r[8];
+    for (int j = 0; j < 8; ++j) r[j] = a[j];
+    long long i = 8;
+    for (; i < n - n % 8; i += 8)
+        for (int j = 0; j < 8; ++j) r[j] = r[j] + a[i + j];
+    T res = ((r[0] + r[1]) + (r[2] + r[3])) + ((r[4] + r[5]) + (r[6] + r[7]));
+    for (; i < n; ++i) res = res + a[i];
+    return res;
+}
+// pw(a, n) = n <= 128 ? leaf : pw(a, n2) + pw(a + n2, n - n2), walked without recursion (the device stack stays
+// small and fixed): leaves are visited left to right; level k of the current path holds the length of its pending
+// right half and, once its left half is done, that half's sum.  A split leaves at most n / 2 + 8 values, so 32 levels
+// cover any n below 2^36.
+template <typename T>
+__host__ __device__ inline T pairwise_block(const T* a, long long n) {
+    T left[32];
+    long long right[32];
+    unsigned has_left = 0;                            // bit k: left[k] holds level k's left-half sum
+    int sp = 0;
+    long long pos = 0, len = n;
+    while (true) {
+        while (len > 128) {                           // descend along left halves
+            const long long n2 = pairwise_split(len);
+            right[sp] = len - n2;
+            has_left &= ~(1u << sp);
+            ++sp;
+            len = n2;
+        }
+        T val = pairwise_leaf(a + pos, len);
+        pos += len;
+        while (sp > 0 && (has_left >> (sp - 1) & 1)) {   // both halves done: combine and go up
+            --sp;
+            val = left[sp] + val;
+        }
+        if (sp == 0) return val;
+        left[sp - 1] = val;                           // left half of level sp - 1 done: its right half is next
+        has_left |= 1u << (sp - 1);
+        len = right[sp - 1];
+    }
+}
+template <typename T>
+__host__ __device__ inline T numpy_sum(const T* a, long long n) {
+    return T(0) + pairwise_block(a, n);
+}
+
 // util.handDetect (src/util.py:133-201) for one arm of one person: shoulder (x1, y1), elbow (x2, y2), wrist (x3, y3) in
 // an H x W image -> square box (x, y, w); valid = w > 0 (the reference's crop of an empty box raises)
 __host__ __device__ inline void hand_detect_box(double x1, double y1, double x2, double y2, double x3, double y3, int H, int W,

@@ -84,6 +84,9 @@ int opb_session_profile_get(opb_session* s, int i, const char** name, float* ms_
 int opb_session_progress(opb_session* s, int* last_done, int* total, const char** name_done, const char** name_next);
 int opb_session_mark(opb_session* s, int slot);
 int opb_session_elapsed(opb_session* a, int slot_a, opb_session* b, int slot_b, float* ms);
+/* debug: how many launch sequences of the session were captured into a CUDA graph and launched, and how many replayed
+ * an already captured graph (the first uses of a job, profiled runs and OPB_NO_GRAPH=1 runs count in neither).      */
+int opb_session_graph_stats(opb_session* s, long long* captures, long long* replays);
 
 /* ---- Body.__call__ (src/body.py:24-212) --------------------------------------------------------
  * submit: enqueue the whole frame (H2D of the image when img_is_device == 0, preprocessing at every

@@ -42,6 +42,7 @@ SIGNATURES = {
     "opb_session_progress": (c_int, [c_void_p, POINTER(c_int), POINTER(c_int), POINTER(c_char_p), POINTER(c_char_p)]),
     "opb_session_mark": (c_int, [c_void_p, c_int]),
     "opb_session_elapsed": (c_int, [c_void_p, c_int, c_void_p, c_int, POINTER(c_float)]),
+    "opb_session_graph_stats": (c_int, [c_void_p, POINTER(ctypes.c_longlong), POINTER(ctypes.c_longlong)]),
     "opb_body_submit": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, POINTER(c_double), c_int]),
     "opb_body_wait": (c_int, [c_void_p, POINTER(c_int), POINTER(c_int)]),
     "opb_body_fetch": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_int]),

@@ -4,6 +4,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <algorithm>
+#include <atomic>
 #include <cmath>
 #include <initializer_list>
 #include <mutex>
@@ -235,48 +236,39 @@ struct FrameKey {
     }
 };
 
+// Values of one process-wide counter: a session's `gen` names one state of its buffers, a plan's `serial` one plan.
+// Neither repeats, so a graph key built from them cannot match a state or a plan it was not captured on.
+static std::atomic<uint64_t> g_gen_counter{0};
+static uint64_t next_gen() { return ++g_gen_counter; }
+
+static uint64_t gen_key(std::initializer_list<uint64_t> parts) {      // FNV-1a over the words
+    uint64_t h = 14695981039346656037ull;
+    for (uint64_t v : parts) h = (h ^ v) * 1099511628211ull;
+    return h;
+}
+
+// The launch sequences a submit or wait replays as a CUDA graph, one graph per job on the plan it runs on.
+//   Frame      Body / Batch_body / Hand / Batch_hand on the plan of the batch
+//   Crops      Hand()(list of square crops) (opb_hand_submit_ragged) on the hand plan of the list
+//   HandTrack  opb_hand_track_submit: crop kernel into a uint8 Batch_hand plan
+//   Pose       opb_pose_submit_batch: body + hands on the body plan
+//   BatchPose  opb_batch_pose_submit: Batch_body + Batch_hand on the Batch_body plan
+//   Every      opb_pose_every_submit / opb_batch_pose_every_submit: body + rows-and-boxes kernel
+//   EveryHand  the hand chunk of an every-person wait (replayed once per chunk)
+enum class Job { Frame, Crops, HandTrack, Pose, BatchPose, Every, EveryHand, kCount };
+
 struct FramePlan {
     DevPool pool;
     FrameKey key;
-    // the device work of one submit (everything between the input upload and the "done" event) as a CUDA graph:
-    // captured on the third use of the plan, re-captured when a session buffer it points into has moved
-    cudaGraphExec_t graph = nullptr;
-    uint64_t graph_gen = 0;
-    int uses = 0;
-    // the same for the body + hands sequence of opb_pose_submit_batch (a different launch list over the same buffers)
-    cudaGraphExec_t pose_graph = nullptr;
-    uint64_t pose_gen = 0;
-    int pose_uses = 0;
-    // the same for the hand-track sequence of opb_hand_track_submit (a uint8 Batch_hand plan fed by the crop kernel)
-    cudaGraphExec_t track_graph = nullptr;
-    uint64_t track_gen = 0;
-    int track_uses = 0;
-    // the same for the one-pass body + hand sequence of opb_batch_pose_submit (on the Batch_body plan)
-    cudaGraphExec_t batch_pose_graph = nullptr;
-    uint64_t batch_pose_gen = 0;
-    int batch_pose_uses = 0;
-    // every person (opb_pose_every_*): the body sequence with the rows-and-boxes kernel, and one hand chunk (replayed
-    // once per kEveryChunk boxes) -- both on the body plan of the batch.  opb_batch_pose_every_submit uses the same two
-    // slots of its Batch_body plan (a mode-2 plan, which no other every-person sequence shares), so it alternates with
-    // opb_batch_pose_submit (batch_pose_graph) on one session pair without re-capturing.
-    cudaGraphExec_t every_graph = nullptr;
-    uint64_t every_gen = 0;
-    int every_uses = 0;
-    cudaGraphExec_t every_hand_graph = nullptr;
-    uint64_t every_hand_gen = 0;
-    int every_hand_uses = 0;
-    // Hand()(list of square crops) (opb_hand_submit_ragged), on the hand plan of the list
-    cudaGraphExec_t crops_graph = nullptr;
-    uint64_t crops_gen = 0;
-    int crops_uses = 0;
+    const uint64_t serial = next_gen();
+    struct Graph {
+        cudaGraphExec_t exec = nullptr;
+        uint64_t key = 0;
+        int uses = 0;
+    } graphs[(int)Job::kCount];
     ~FramePlan() {
-        if (crops_graph) cudaGraphExecDestroy(crops_graph);
-        if (graph) cudaGraphExecDestroy(graph);
-        if (pose_graph) cudaGraphExecDestroy(pose_graph);
-        if (track_graph) cudaGraphExecDestroy(track_graph);
-        if (batch_pose_graph) cudaGraphExecDestroy(batch_pose_graph);
-        if (every_graph) cudaGraphExecDestroy(every_graph);
-        if (every_hand_graph) cudaGraphExecDestroy(every_hand_graph);
+        for (auto& g : graphs)
+            if (g.exec) cudaGraphExecDestroy(g.exec);
     }
     std::vector<ScaleDims> dims;
     std::vector<U8Taps> u8taps;
@@ -380,7 +372,16 @@ struct opb_session {
     // size-dependent work buffers, grown to the largest frame seen and shared by all plans of the session
     enum { AR_IMG, AR_SCRATCH, AR_HEAT, AR_PAF, AR_LABELS, AR_SUMS, AR_PEAKS, AR_BLUR, AR_COUNT };
     struct Arena { void* p = nullptr; size_t cap = 0; } arena[AR_COUNT];
-    uint64_t buffer_gen = 1;         // bumped whenever an arena or a pinned result buffer is reallocated
+    // A new next_gen() value whenever memory that a captured launch sequence of this session may read is freed or
+    // moved, or its captured launch parameters change (see bump).  Every graph key holds it.
+    uint64_t gen = next_gen();
+    long long captures = 0, replays = 0;     // graph launches that captured / replayed (opb_session_graph_stats)
+    // the batch in flight: its job and, for a body + hand job, the hand session, Batch_hand boxsize (0: none) and
+    // whether the hand boxes were given
+    Job job = Job::kCount;
+    opb_session* pair_hand = nullptr;
+    int pair_box = 0;
+    bool pair_fixed = false;
     // per-frame caller on the device (opb_pose_*): a hand session carries the tap tables of every crop size, a body
     // session the per-batch pose / box buffers
     struct Ragged {
@@ -410,7 +411,6 @@ struct opb_session {
         }
     };
     std::unique_ptr<CropList> crop_list;
-    bool hand_ragged = false;            // the last hand batch was a crop list: its maps have one pitch per crop
     struct PoseBuffers {
         DevPool pool;
         int frames = 0;
@@ -441,8 +441,7 @@ struct opb_session {
         double* mats = nullptr;      // [frames][42][3]
         double* poses_host = nullptr;   // pinned
         double* mats_host = nullptr;    // pinned
-        uint64_t gen = 1;            // bumped whenever a buffer, the tables or the frame size change
-        int H = 0, W = 0, n = 0;     // last batch
+        int n = 0;                   // frames of the last batch
         FramePlan* plan = nullptr;   // uint8 Batch_hand plan of the last batch (its input buffer holds the crops)
         ~HandTrack() {
             if (poses_host) cudaFreeHost(poses_host);
@@ -450,16 +449,11 @@ struct opb_session {
         }
     };
     std::unique_ptr<HandTrack> track;
-    opb_session* pose_hand = nullptr;    // hand session of the pose batch in flight
-    std::vector<double> pose_hand_scales;
-    bool pose_fixed = false;
-    int batch_pose_box = 0;              // boxsize of the opb_batch_pose(_every) batch in flight; 0: an opb_pose batch
     // every person of a batch (opb_pose_every_*), on a body session: the records and the compacted hand boxes, grown to
     // the largest person count seen, and the boxes of one hand chunk
     struct EveryBuffers {
         DevPool pool;
         int cap = 0;                 // records; the box list holds 2 * cap
-        uint64_t gen = 0;            // unique per allocation (graph keys)
         double* records = nullptr;   // [cap][60][3]
         HandBox* list = nullptr;     // [2 cap] in util.handDetect's order
         int* list_rec = nullptr;     // [2 cap] record of each box
@@ -478,8 +472,6 @@ struct opb_session {
         }
     };
     std::unique_ptr<EveryBuffers> every;
-    uint64_t every_allocs = 0;
-    bool every_batch = false;            // the batch in flight is an opb_pose_every or opb_batch_pose_every batch
     int every_persons = -1;              // persons of the last finished opb_pose_every batch; -1: none
     bool every_linked = false;           // the last finished opb_pose_every batch was linked: ids_host holds its ids
     std::vector<NetShape> debug_shapes;  // the plan of the opb_net_debug_* calls (looked up by its shapes on every call)
@@ -534,20 +526,25 @@ struct opb_tracker {
 
 namespace opb {
 
+// Every captured graph of the session is re-captured on its next replay: called wherever memory that a captured launch
+// sequence may read is freed or moved, or its captured launch parameters change -- only on paths that reallocate, so
+// the steady state replays.
+static void bump(opb_session* s) { s->gen = next_gen(); }
+
 static void ensure_host(opb_session* s, int frames, size_t hand_doubles) {
     const size_t need = sizeof(HostResults) * (size_t)frames;
     if (s->host_bytes < need) {
         if (s->host) cudaFreeHost(s->host);
         OPB_CUDA(cudaMallocHost((void**)&s->host, need));
         s->host_bytes = need;
-        ++s->buffer_gen;
+        bump(s);
     }
     const size_t hneed = hand_doubles * sizeof(double);
     if (s->hand_host_bytes < hneed) {
         if (s->hand_host) cudaFreeHost(s->hand_host);
         OPB_CUDA(cudaMallocHost((void**)&s->hand_host, hneed));
         s->hand_host_bytes = hneed;
-        ++s->buffer_gen;
+        bump(s);
     }
 }
 static void ensure_staging(opb_session* s, size_t bytes) {
@@ -564,6 +561,7 @@ static void drop_plans(opb_session* s) {
     OPB_CUDA(cudaStreamSynchronize(s->stream));
     s->plans.clear();
     s->active = nullptr;
+    bump(s);
 }
 
 // Plan construction allocates with cudaMalloc, uploads with synchronous copies and zero-fills through DevPool (which
@@ -590,6 +588,7 @@ static NetPlan* get_net_plan(opb_session* s, const std::vector<NetShape>& shapes
             }
         }
         s->net_plans.erase(victim);
+        bump(s);
     }
     auto plan = build_net_plan(s->net, shapes);
     NetPlan* raw = plan.get();
@@ -609,7 +608,7 @@ static void* arena_get(opb_session* s, int which, size_t bytes) {
         const size_t want = bytes + bytes / 4 + 256;
         OPB_CUDA(cudaMalloc(&a.p, want));
         a.cap = want;
-        ++s->buffer_gen;
+        bump(s);
     }
     return a.p;
 }
@@ -724,27 +723,25 @@ static FramePlan* get_plan(opb_session* s, int n, int H, int W, const double* sc
     return raw;
 }
 
-// Runs `enqueue` (kernel launches, memsets and result copies on the session's stream) either directly or, once the plan
-// has been used a few times, as one CUDA graph launch: a frame is ~70 small dependent launches, and for the small
-// default configuration (640x480, one scale) the launch gaps, not the kernels, are most of the latency.
-struct GraphSlot {
-    cudaGraphExec_t& graph;
-    uint64_t& gen;
-    int& uses;
-};
+// Runs `enqueue` (kernel launches, memsets and result copies on the session's stream) either directly or, once the job
+// has run a few times on the plan, as one CUDA graph launch: a frame is ~70 small dependent launches, and for the small
+// default configuration (640x480, one scale) the launch gaps, not the kernels, are most of the latency.  The graph is
+// re-captured when `key` changes: gen_key over the running session's gen, for a body + hand job the hand session's gen
+// and the hand plan's serial, and the launch parameters that the plan's FrameKey does not fix.
 template <typename F>
-static void run_or_replay_slot(opb_session* s, GraphSlot g, uint64_t want_gen, F&& enqueue) {
+static void run_job(opb_session* s, FramePlan* fp, Job job, uint64_t key, F&& enqueue) {
     static const bool no_graph = getenv("OPB_NO_GRAPH") != nullptr;
     cudaStream_t st = s->stream;
+    FramePlan::Graph& g = fp->graphs[(int)job];
     ++g.uses;
     if (no_graph || s->prof.on || g.uses < 3) {         // first uses run eagerly (lazy module loading, attributes)
         enqueue();
         return;
     }
-    if (!g.graph || g.gen != want_gen) {
-        if (g.graph) {
-            cudaGraphExecDestroy(g.graph);
-            g.graph = nullptr;
+    if (!g.exec || g.key != key) {
+        if (g.exec) {
+            cudaGraphExecDestroy(g.exec);
+            g.exec = nullptr;
         }
         cudaGraph_t cg = nullptr;
         OPB_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
@@ -756,16 +753,15 @@ static void run_or_replay_slot(opb_session* s, GraphSlot g, uint64_t want_gen, F
             throw;
         }
         OPB_CUDA(cudaStreamEndCapture(st, &cg));
-        const cudaError_t e = cudaGraphInstantiate(&g.graph, cg, 0);
+        const cudaError_t e = cudaGraphInstantiate(&g.exec, cg, 0);
         cudaGraphDestroy(cg);
         OPB_CUDA(e);
-        g.gen = want_gen;
+        g.key = key;
+        ++s->captures;
+    } else {
+        ++s->replays;
     }
-    OPB_CUDA(cudaGraphLaunch(g.graph, st));
-}
-template <typename F>
-static void run_or_replay(opb_session* s, FramePlan* fp, F&& enqueue) {
-    run_or_replay_slot(s, GraphSlot{fp->graph, fp->graph_gen, fp->uses}, s->buffer_gen, enqueue);
+    OPB_CUDA(cudaGraphLaunch(g.exec, st));
 }
 
 static void upload_bytes(opb_session* s, void* dst, const void* img, int where, size_t bytes) {
@@ -880,7 +876,7 @@ static void body_post_enqueue(opb_session* s, FramePlan* fp, int n, int H, int W
 
 // A frame produced more peaks / scored limb pairs / connections / person rows than its buffers hold (the reference has
 // no such limits): give that frame larger buffers, repeat its post-processing from the net outputs that are still on
-// the device, and make the plan re-capture its graph.  Returns false when nothing can grow any further.
+// the device, and make the session re-capture its graphs.  Returns false when nothing can grow any further.
 static bool grow_and_redo(opb_session* s, FramePlan* fp, int f, int appended, int status) {
     FramePost& bp = fp->post[f];
     int peak_cap = bp.pb.capacity, pair_cap = bp.lb.pair_capacity, conn_cap = bp.lb.conn_capacity;
@@ -910,28 +906,29 @@ static bool grow_and_redo(opb_session* s, FramePlan* fp, int f, int appended, in
                     conn_cap, subset_cap);
     bp = bigger;                                         // the old buffers stay in the plan's pool until it dies
     upload_post_table(fp, s->stream);
-    if (fp->graph) {
-        cudaGraphExecDestroy(fp->graph);
-        fp->graph = nullptr;
-    }
-    if (fp->pose_graph) {
-        cudaGraphExecDestroy(fp->pose_graph);
-        fp->pose_graph = nullptr;
-    }
-    if (fp->batch_pose_graph) {
-        cudaGraphExecDestroy(fp->batch_pose_graph);
-        fp->batch_pose_graph = nullptr;
-    }
-    if (fp->every_graph) {
-        cudaGraphExecDestroy(fp->every_graph);
-        fp->every_graph = nullptr;
-    }
+    bump(s);                                             // the captured launches carry the old capacities
     const bool prof = s->prof.on;
     s->prof.on = false;
     body_post_range(s, fp, f, 1, fp->key.H, fp->key.W);
     s->prof.on = prof;
     OPB_CUDA(cudaStreamSynchronize(s->stream));
     return true;
+}
+
+static bool frame_overflowed(const FramePost& bp, const HostResults* h) {
+    return h->counts[0] > bp.pb.capacity || (h->counts[21] & (kStPairOverflow | kStConnOverflow | kStSubsetOverflow));
+}
+
+// Grows and redoes frame f of the finished batch until its results fit or nothing can grow any further; returns whether
+// anything grew.  The caller checks frame_overflowed afterwards.
+static bool fit_frame(opb_session* s, FramePlan* fp, int f) {
+    const HostResults* h = s->host + f;
+    bool grew = false;
+    for (int attempt = 0; attempt < 12 && frame_overflowed(fp->post[f], h); ++attempt) {
+        if (!grow_and_redo(s, fp, f, h->counts[0], h->counts[21])) break;
+        grew = true;
+    }
+    return grew;
 }
 
 static void finish_submit(opb_session* s, FramePlan* fp) {
@@ -947,12 +944,13 @@ static void body_submit(opb_session* s, const uint8_t* img, int where, int n, in
     ensure_host(s, n, 0);
     s->active = fp;
     s->n_frames = n;
+    s->job = Job::Frame;
     cudaStream_t st = s->stream;
     s->prof.reset();
     s->prof.mark(st, "start");
     upload_image(s, fp, img, where, (size_t)n * H * W * 3);
     s->prof.mark(st, "h2d");
-    run_or_replay(s, fp, [&] {
+    run_job(s, fp, Job::Frame, gen_key({s->gen}), [&] {
         run_front(s, fp, n, H, W);
         body_post_enqueue(s, fp, n, H, W);
     });
@@ -979,12 +977,13 @@ static void batch_body_submit(opb_session* s, const void* frames, bool u8, int w
     ensure_host(s, n, 0);
     s->active = fp;
     s->n_frames = n;
+    s->job = Job::Frame;
     cudaStream_t st = s->stream;
     s->prof.reset();
     s->prof.mark(st, "start");
     upload_image(s, fp, (const uint8_t*)frames, where, (size_t)n * H * W * 3 * (u8 ? 1 : sizeof(float)));
     s->prof.mark(st, "h2d");
-    run_or_replay(s, fp, [&] {
+    run_job(s, fp, Job::Frame, gen_key({s->gen}), [&] {
         run_front_f32(s, fp, n, H, W);
         body_post_enqueue(s, fp, n, H, W);              // 5x5 blur (utilmx.py:261-263) inside the peak kernel
     });
@@ -1003,14 +1002,9 @@ static int body_wait(opb_session* s, int* n_cand, int* n_subset, int* frame_stat
         HostResults* h = s->host + f;
         FramePost& bp = fp->post[f];
         FrameResult& r = s->results[f];
-        int appended = h->counts[0];
-        int status = h->counts[21];
-        for (int attempt = 0; attempt < 12; ++attempt) {
-            if (appended <= bp.pb.capacity && !(status & (kStPairOverflow | kStConnOverflow | kStSubsetOverflow))) break;
-            if (!grow_and_redo(s, fp, f, appended, status)) break;
-            appended = h->counts[0];
-            status = h->counts[21];
-        }
+        fit_frame(s, fp, f);
+        const int appended = h->counts[0];
+        const int status = h->counts[21];
         if (appended > bp.pb.capacity)
             throw Error(OPB_ERR_CAPACITY, "more than " + std::to_string(bp.pb.capacity) + " heat-map peaks in one frame");
         if (status & (kStPairOverflow | kStConnOverflow | kStSubsetOverflow))
@@ -1063,13 +1057,13 @@ static void hand_submit(opb_session* s, const uint8_t* img, int where, int n, in
     ensure_host(s, 1, (size_t)n * 63);
     s->active = fp;
     s->hand_crops = n;
-    s->hand_ragged = false;
+    s->job = Job::Frame;
     cudaStream_t st = s->stream;
     s->prof.reset();
     s->prof.mark(st, "start");
     upload_image(s, fp, img, where, (size_t)n * H * W * 3);
     s->prof.mark(st, "h2d");
-    run_or_replay(s, fp, [&] {
+    run_job(s, fp, Job::Frame, gen_key({s->gen}), [&] {
         run_front(s, fp, n, H, W);
         run_upsample(fp, false, n, 22, 24, H, W, fp->heat_avg, st);
         s->prof.mark(st, "upsample_avg");
@@ -1103,13 +1097,13 @@ static void batch_hand_submit(opb_session* s, const void* crops, bool u8, int wh
     ensure_host(s, 1, (size_t)n * 63);
     s->active = fp;
     s->hand_crops = n;
-    s->hand_ragged = false;
+    s->job = Job::Frame;
     cudaStream_t st = s->stream;
     s->prof.reset();
     s->prof.mark(st, "start");
     upload_image(s, fp, (const uint8_t*)crops, where, (size_t)n * H * W * 3 * (u8 ? 1 : sizeof(float)));
     s->prof.mark(st, "h2d");
-    run_or_replay(s, fp, [&] {
+    run_job(s, fp, Job::Frame, gen_key({s->gen}), [&] {
         batch_hand_enqueue(s, fp, n, H, W);
         OPB_CUDA(cudaMemcpyAsync(s->hand_host, fp->hb.peaks, (size_t)n * 63 * sizeof(double), cudaMemcpyDeviceToHost, st));
         s->prof.mark(st, "d2h");
@@ -1139,13 +1133,15 @@ static void build_track_tables(opb_session::HandTrack& t, int boxsize, int wmax)
     t.tabs.n_scales = 1;
     t.tabs.wmax = wmax;
     t.boxsize = boxsize;
-    ++t.gen;
 }
 // the hand session's HandTrack with tables for `boxsize` and crops of up to wmax pixels (nothing may still use them)
 static opb_session::HandTrack& track_with_tables(opb_session* s, int boxsize, int wmax) {
     if (!s->track) s->track = std::make_unique<opb_session::HandTrack>();
     opb_session::HandTrack& t = *s->track;
-    if (t.boxsize != boxsize || t.tabs.wmax < wmax) build_track_tables(t, boxsize, wmax);
+    if (t.boxsize != boxsize || t.tabs.wmax < wmax) {
+        build_track_tables(t, boxsize, wmax);
+        bump(s);
+    }
     return t;
 }
 
@@ -1171,18 +1167,15 @@ static void hand_track_submit(opb_session* s, const uint8_t* frames, int where, 
         OPB_CUDA(cudaMallocHost((void**)&t.poses_host, (size_t)n * 54 * sizeof(double)));
         OPB_CUDA(cudaMallocHost((void**)&t.mats_host, (size_t)n * 126 * sizeof(double)));
         t.frames = n;
-        ++t.gen;
+        bump(s);
     }
     const size_t bytes = (size_t)n * H * W * 3;
     if (t.frame_bytes < bytes) {
         t.frame_pool.release();
         t.frames_dev = (uint8_t*)t.frame_pool.alloc(bytes);
         t.frame_bytes = bytes;
-        ++t.gen;
+        bump(s);
     }
-    if (t.H != H || t.W != W) ++t.gen;           // the captured launches carry the frame size
-    t.H = H;
-    t.W = W;
     t.n = n;
     memcpy(t.poses_host, poses, (size_t)n * 54 * sizeof(double));
     // the crops go straight into the input buffer of the uint8 Batch_hand plan of 2n boxsize-square crops
@@ -1191,12 +1184,11 @@ static void hand_track_submit(opb_session* s, const uint8_t* frames, int where, 
     FramePlan* fp = get_plan(s, slots, boxsize, boxsize, &one, 1, 2);
     s->active = fp;
     s->hand_crops = slots;
-    s->hand_ragged = false;
+    s->job = Job::HandTrack;
     t.plan = fp;
     s->prof.reset();
     upload_bytes(s, t.frames_dev, frames, where, bytes);
-    const uint64_t gen = (s->buffer_gen << 32) ^ t.gen;
-    run_or_replay_slot(s, GraphSlot{fp->track_graph, fp->track_gen, fp->track_uses}, gen, [&] {
+    run_job(s, fp, Job::HandTrack, gen_key({s->gen, (uint64_t)H, (uint64_t)W}), [&] {
         OPB_CUDA(cudaMemcpyAsync(t.poses, t.poses_host, (size_t)n * 54 * sizeof(double), cudaMemcpyHostToDevice, st));
         hand_track_boxes_launch(t.poses, n, H, W, t.boxes, st);
         preprocess_ragged_launch(t.frames_dev, H, W, t.boxes, slots, fp->d_img, boxsize, 0, t.tabs, st);
@@ -1256,6 +1248,7 @@ static int ensure_ragged_tables(opb_session* bs, opb_session* hs, int H, int W, 
     if (!hs->ragged || hs->ragged->tabs.wmax < wmax || hs->ragged->scales != std::vector<double>(hscales, hscales + nhs)) {
         OPB_CUDA(cudaStreamSynchronize(bs->stream));
         hs->ragged = build_ragged_tables(hscales, nhs, wmax);
+        bump(hs);
     }
     return hs->ragged->tabs.wmax;
 }
@@ -1273,6 +1266,7 @@ static void ensure_pose_buffers(opb_session* bs, int n) {
     OPB_CUDA(cudaMallocHost((void**)&pb->host, (size_t)n * 180 * sizeof(double)));
     OPB_CUDA(cudaMallocHost((void**)&pb->fixed_host, (size_t)n * 6 * sizeof(int)));
     bs->pose = std::move(pb);
+    bump(bs);
 }
 
 // Hand on `slots` boxes (dims: side of each valid box, else 0) of the frames `fp` holds, as one ragged batch on the hand
@@ -1307,7 +1301,6 @@ static void ragged_hand_net_post(cudaStream_t st, const opb_session::Ragged& rg,
 // into the input arena; the packed form of the ragged crop kernel resizes each one with the tables of its own side, and
 // from there on the batch is the hand half of the pose pipeline (one CNN plan per crop count and scales, upsample,
 // Gaussian, components and selection at each crop's own size).
-static uint64_t gen_key(std::initializer_list<uint64_t> parts);
 static void hand_submit_ragged(opb_session* s, const uint8_t* packed, const size_t* offsets, int where, int n,
                                const int* sides, const double* scales, int ns) {
     OPB_REQUIRE(s->net->kind == OPB_NET_HAND, "session was created on a body network");
@@ -1325,8 +1318,10 @@ static void hand_submit_ragged(opb_session* s, const uint8_t* packed, const size
     cudaStream_t st = s->stream;
     OPB_CUDA(cudaStreamSynchronize(st));          // the pinned crop list and the tables may still serve the previous batch
     const std::vector<double> sc(scales, scales + ns);
-    if (!s->crop_tables || s->crop_tables->tabs.wmax < wmax || s->crop_tables->scales != sc)
+    if (!s->crop_tables || s->crop_tables->tabs.wmax < wmax || s->crop_tables->scales != sc) {
         s->crop_tables = build_ragged_tables(scales, ns, wmax);
+        bump(s);
+    }
     const opb_session::Ragged& rg = *s->crop_tables;
     const int tw = rg.tabs.wmax;
     if (!s->crop_list || s->crop_list->cap < n) {
@@ -1339,6 +1334,7 @@ static void hand_submit_ragged(opb_session* s, const uint8_t* packed, const size
         OPB_CUDA(cudaMallocHost((void**)&cl->offsets_host, (size_t)n * sizeof(size_t)));
         cl->cap = n;
         s->crop_list = std::move(cl);
+        bump(s);
     }
     opb_session::CropList& cl = *s->crop_list;
     for (int i = 0; i < n; ++i) {
@@ -1352,12 +1348,10 @@ static void hand_submit_ragged(opb_session* s, const uint8_t* packed, const size
     ensure_host(s, 1, (size_t)n * 63);
     s->active = fp;
     s->hand_crops = n;
-    s->hand_ragged = true;
+    s->job = Job::Crops;
     s->prof.reset();
     upload_bytes(s, fp->d_img, packed, where, offsets[n]);
-    const uint64_t gen = gen_key({s->buffer_gen, (uint64_t)(uintptr_t)cl.boxes, (uint64_t)(uintptr_t)rg.tabs.slab,
-                                  (uint64_t)(uintptr_t)rg.tabs.index});
-    run_or_replay_slot(s, GraphSlot{fp->crops_graph, fp->crops_gen, fp->crops_uses}, gen, [&] {
+    run_job(s, fp, Job::Crops, gen_key({s->gen}), [&] {
         OPB_CUDA(cudaMemcpyAsync(cl.boxes, cl.boxes_host, (size_t)n * sizeof(HandBox), cudaMemcpyHostToDevice, st));
         OPB_CUDA(cudaMemcpyAsync(cl.sides, cl.sides_host, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, st));
         OPB_CUDA(cudaMemcpyAsync(cl.offsets, cl.offsets_host, (size_t)n * sizeof(size_t), cudaMemcpyHostToDevice, st));
@@ -1368,6 +1362,34 @@ static void hand_submit_ragged(opb_session* s, const uint8_t* packed, const size
     });
     OPB_CUDA(cudaEventRecord(s->done, st));
     s->net->ctx->launches += ns + fp->net->kernel_launches + (ns + 1) + 6;
+}
+
+// ------------------------------------------------------------------------------------------------
+// body + hand jobs on a session pair (opb_pose_submit_batch, opb_batch_pose_submit, opb_pose_every_submit,
+// opb_batch_pose_every_submit): the whole batch runs on the body session's stream, with the hand session's plan and
+// work buffers
+// ------------------------------------------------------------------------------------------------
+static void pair_check(opb_session* bs, opb_session* hs, int n, int H, int W, const char* job) {
+    OPB_REQUIRE(bs->net->kind == OPB_NET_BODY && hs->net->kind == OPB_NET_HAND,
+                std::string(job) + ": a body session and a hand session");
+    OPB_REQUIRE(bs->net->ctx == hs->net->ctx, std::string(job) + ": both networks must live on the same context");
+    OPB_REQUIRE(n >= 1 && n <= 64, "1..64 frames per batch");
+    OPB_REQUIRE(H >= 1 && W >= 1, "empty frame");
+}
+// the batch of body plan fp and hand plan hp becomes the one in flight on both sessions
+static void pair_begin(opb_session* bs, opb_session* hs, Job job, FramePlan* fp, FramePlan* hp, int boxsize, bool fixed) {
+    bs->active = fp;
+    bs->n_frames = fp->key.n;
+    bs->job = hs->job = job;
+    bs->pair_hand = hs;
+    bs->pair_box = boxsize;
+    bs->pair_fixed = fixed;
+    hs->active = hp;
+    hs->hand_crops = hp->key.n;
+    if (job == Job::Every) {
+        bs->every_persons = -1;
+        bs->every_linked = false;
+    }
 }
 
 // the hand half of the pose pipeline, on the body session's stream: boxes from the body results (or the fixed ones already
@@ -1384,9 +1406,7 @@ static void pose_hand_enqueue(opb_session* bs, opb_session* hs, FramePlan* fp, F
 
 static void pose_submit(opb_session* bs, opb_session* hs, const uint8_t* imgs, int where, int n, int H, int W,
                         const double* bscales, int nbs, const double* hscales, int nhs, const int* fixed_boxes) {
-    OPB_REQUIRE(bs->net->kind == OPB_NET_BODY && hs->net->kind == OPB_NET_HAND, "pose: a body session and a hand session");
-    OPB_REQUIRE(bs->net->ctx == hs->net->ctx, "pose: both networks must live on the same context");
-    OPB_REQUIRE(n >= 1 && n <= 64, "1..64 frames per batch");
+    pair_check(bs, hs, n, H, W, "pose");
     OPB_CUDA(cudaSetDevice(bs->net->ctx->device));
     const int slots = 2 * n;
     const int tw = ensure_ragged_tables(bs, hs, H, W, hscales, nhs);
@@ -1394,35 +1414,22 @@ static void pose_submit(opb_session* bs, opb_session* hs, const uint8_t* imgs, i
     // body part: as opb_body_submit_batch
     FramePlan* fp = get_plan(bs, n, H, W, bscales, nbs);
     ensure_host(bs, n, 0);
-    bs->active = fp;
-    bs->n_frames = n;
-    bs->pose_hand = hs;
-    bs->batch_pose_box = 0;
-    bs->every_batch = false;
     cudaStream_t st = bs->stream;
     upload_image(bs, fp, imgs, where, (size_t)n * H * W * 3);
     // hand part on the same stream, with the hand session's CNN plan and work buffers (sized for the largest crop)
     OPB_CUDA(cudaStreamSynchronize(hs->stream));               // nothing of the hand session's own stream may still use them
     FramePlan* hp = get_plan(hs, slots, tw, tw, hscales, nhs);
-    hs->active = hp;
-    hs->hand_crops = slots;
-    hs->hand_ragged = false;
-    int* fixed_dev = nullptr;
-    if (fixed_boxes) {
+    const bool fixed = fixed_boxes != nullptr;
+    pair_begin(bs, hs, Job::Pose, fp, hp, 0, fixed);
+    if (fixed) {
         OPB_CUDA(cudaStreamSynchronize(st));                   // the pinned copy of the previous batch's boxes is free
         memcpy(bs->pose->fixed_host, fixed_boxes, (size_t)n * 6 * sizeof(int));
-        fixed_dev = bs->pose->fixed;
     }
-    // everything between the frame upload and the PoseMat copy is one launch sequence on one stream: replayed as a CUDA
-    // graph from the third use on (re-captured when a buffer of either session, the hand plan or the box source changed)
-    const uint64_t gen = bs->buffer_gen * 1000003ull + hs->buffer_gen * 7919ull + (uint64_t)(uintptr_t)hp +
-                         (uint64_t)(uintptr_t)hs->ragged->tabs.slab + (fixed_dev ? 1 : 0);
-    bs->pose_hand_scales.assign(hscales, hscales + nhs);
-    bs->pose_fixed = fixed_dev != nullptr;
-    run_or_replay_slot(bs, GraphSlot{fp->pose_graph, fp->pose_gen, fp->pose_uses}, gen, [&] {
+    // everything between the frame upload and the PoseMat copy is one launch sequence on one stream
+    run_job(bs, fp, Job::Pose, gen_key({bs->gen, hs->gen, hp->serial, fixed}), [&] {
         run_front(bs, fp, n, H, W);
         body_post_enqueue(bs, fp, n, H, W);
-        pose_hand_enqueue(bs, hs, fp, hp, n, H, W, fixed_dev != nullptr);
+        pose_hand_enqueue(bs, hs, fp, hp, n, H, W, fixed);
     });
     OPB_CUDA(cudaEventRecord(bs->done, st));
     bs->net->ctx->launches += fp->launches_per_frame + nhs + hp->net->kernel_launches + (nhs + 1) + 6 + 2;
@@ -1437,14 +1444,9 @@ static int pose_batch_status(opb_session* bs, int* frame_status, bool& grew) {
     FramePlan* fp = bs->active;
     for (int f = 0; f < bs->n_frames; ++f) {
         const HostResults* h = bs->host + f;
-        for (int attempt = 0; attempt < 12; ++attempt) {
-            const FramePost& bp = fp->post[f];
-            if (h->counts[0] <= bp.pb.capacity && !(h->counts[21] & (kStPairOverflow | kStConnOverflow | kStSubsetOverflow))) break;
-            if (!grow_and_redo(bs, fp, f, h->counts[0], h->counts[21])) break;
-            grew = true;
-        }
+        if (fit_frame(bs, fp, f)) grew = true;
         const int status = h->counts[21];
-        if (h->counts[0] > fp->post[f].pb.capacity || (status & (kStPairOverflow | kStConnOverflow | kStSubsetOverflow)))
+        if (frame_overflowed(fp->post[f], h))
             throw Error(OPB_ERR_CAPACITY, "a frame overflowed the body result buffers (status " + std::to_string(status) + ")");
         const int st = (status & kStIndexError) ? OPB_ERR_SUBSET_INDEX : OPB_OK;
         if (frame_status) frame_status[f] = st;
@@ -1473,19 +1475,9 @@ static void batch_pose_hand_enqueue(opb_session* bs, opb_session* hs, FramePlan*
     OPB_CUDA(cudaMemcpyAsync(pb.host, pb.pose, (size_t)n * 180 * sizeof(double), cudaMemcpyDeviceToHost, st));
 }
 
-static uint64_t gen_key(std::initializer_list<uint64_t> parts) {      // FNV-1a over the words
-    uint64_t h = 14695981039346656037ull;
-    for (uint64_t v : parts) h = (h ^ v) * 1099511628211ull;
-    return h;
-}
-
 static void batch_pose_submit(opb_session* bs, opb_session* hs, const uint8_t* frames, int where, int n, int H, int W,
                               double g_scale, int boxsize) {
-    OPB_REQUIRE(bs->net->kind == OPB_NET_BODY && hs->net->kind == OPB_NET_HAND,
-                "batch pose: a body session and a hand session");
-    OPB_REQUIRE(bs->net->ctx == hs->net->ctx, "batch pose: both networks must live on the same context");
-    OPB_REQUIRE(n >= 1 && n <= 64, "1..64 frames per batch");
-    OPB_REQUIRE(H >= 1 && W >= 1, "empty frame");
+    pair_check(bs, hs, n, H, W, "batch pose");
     OPB_REQUIRE(g_scale > 0, "scale must be positive");
     OPB_REQUIRE(boxsize >= 8 && boxsize % 8 == 0, "boxsize must be a positive multiple of 8 (srcmx/Batch_model.py:377)");
     OPB_CUDA(cudaSetDevice(bs->net->ctx->device));
@@ -1498,28 +1490,16 @@ static void batch_pose_submit(opb_session* bs, opb_session* hs, const uint8_t* f
     opb_session::HandTrack& t = track_with_tables(hs, boxsize, std::min(H, W));
     FramePlan* fp = get_plan(bs, n, H, W, &g_scale, 1, 2);          // Batch_body on uint8 frames
     ensure_host(bs, n, 0);
-    bs->active = fp;
-    bs->n_frames = n;
-    bs->pose_hand = hs;
-    bs->batch_pose_box = boxsize;
-    bs->every_batch = false;
     const double one = 1.0;
     FramePlan* hp = get_plan(hs, 2 * n, boxsize, boxsize, &one, 1, 2);      // uint8 Batch_hand on 2n crops
-    hs->active = hp;
-    hs->hand_crops = 2 * n;
-    hs->hand_ragged = false;
+    pair_begin(bs, hs, Job::BatchPose, fp, hp, boxsize, false);
     t.plan = hp;
     bs->prof.reset();
     bs->prof.mark(st, "start");
     upload_image(bs, fp, frames, where, (size_t)n * H * W * 3);
     bs->prof.mark(st, "h2d");
-    // one launch sequence from the uploaded frames to the records copy, replayed as a CUDA graph from the third use on;
-    // re-captured when a buffer of either session, the hand plan, the crop tables, the records or the frame size change
-    const opb_session::PoseBuffers& pb = *bs->pose;
-    const uint64_t gen = gen_key({bs->buffer_gen, hs->buffer_gen, (uint64_t)(uintptr_t)hp, t.gen,
-                                  (uint64_t)(uintptr_t)pb.pose, (uint64_t)(uintptr_t)pb.boxes, (uint64_t)(uintptr_t)pb.host,
-                                  (uint64_t)H, (uint64_t)W, (uint64_t)boxsize});
-    run_or_replay_slot(bs, GraphSlot{fp->batch_pose_graph, fp->batch_pose_gen, fp->batch_pose_uses}, gen, [&] {
+    // one launch sequence from the uploaded frames to the records copy
+    run_job(bs, fp, Job::BatchPose, gen_key({bs->gen, hs->gen, hp->serial, (uint64_t)boxsize}), [&] {
         run_front_f32(bs, fp, n, H, W);
         body_post_enqueue(bs, fp, n, H, W);
         batch_pose_hand_enqueue(bs, hs, fp, hp, n, boxsize);
@@ -1552,7 +1532,6 @@ static void ensure_every_buffers(opb_session* bs, int persons) {
     OPB_CUDA(cudaStreamSynchronize(bs->stream));
     auto e = std::make_unique<opb_session::EveryBuffers>();
     e->cap = cap;
-    e->gen = ++bs->every_allocs;
     e->records = e->pool.alloc_t<double>((size_t)cap * 180);
     e->list = e->pool.alloc_t<HandBox>((size_t)cap * 2);
     e->list_rec = e->pool.alloc_t<int>((size_t)cap * 2);
@@ -1565,14 +1544,15 @@ static void ensure_every_buffers(opb_session* bs, int persons) {
     e->ids = e->pool.alloc_t<int>(cap);
     OPB_CUDA(cudaMallocHost((void**)&e->ids_host, (size_t)cap * sizeof(int)));
     bs->every = std::move(e);
+    bump(bs);
 }
 
-// rows and boxes of every person from the body results of the batch (the batched estimators' box rule for an
-// opb_batch_pose_every batch); the counts to pinned memory
+// rows and boxes of every person from the body results of the batch (the batched estimators' box rule on a Batch_body
+// plan); the counts to pinned memory
 static void every_rows_enqueue(opb_session* bs, FramePlan* fp, int n) {
     opb_session::EveryBuffers& e = *bs->every;
     every_rows_launch(fp->post_dev, n, fp->key.H, fp->key.W, e.cap, e.records, e.list, e.list_rec, e.counts,
-                      bs->batch_pose_box != 0, bs->stream);
+                      fp->key.mode >= 1, bs->stream);
     OPB_CUDA(cudaMemcpyAsync(e.counts_host, e.counts, kEveryCounts * sizeof(int), cudaMemcpyDeviceToHost, bs->stream));
 }
 
@@ -1588,32 +1568,19 @@ static void every_chunk_enqueue(opb_session* bs, opb_session* hs, FramePlan* fp,
 
 static void every_submit(opb_session* bs, opb_session* hs, const uint8_t* imgs, int where, int n, int H, int W,
                          const double* bscales, int nbs, const double* hscales, int nhs) {
-    OPB_REQUIRE(bs->net->kind == OPB_NET_BODY && hs->net->kind == OPB_NET_HAND, "every person: a body session and a hand session");
-    OPB_REQUIRE(bs->net->ctx == hs->net->ctx, "every person: both networks must live on the same context");
-    OPB_REQUIRE(n >= 1 && n <= 64, "1..64 frames per batch");
-    OPB_REQUIRE(H >= 1 && W >= 1, "empty frame");
+    pair_check(bs, hs, n, H, W, "every person");
     OPB_CUDA(cudaSetDevice(bs->net->ctx->device));
     cudaStream_t st = bs->stream;
     const int tw = ensure_ragged_tables(bs, hs, H, W, hscales, nhs);
     ensure_every_buffers(bs, 0);
     FramePlan* fp = get_plan(bs, n, H, W, bscales, nbs);
     ensure_host(bs, n, 0);
-    bs->active = fp;
-    bs->n_frames = n;
-    bs->pose_hand = hs;
-    bs->batch_pose_box = 0;
-    bs->every_batch = true;
-    bs->every_persons = -1;
-    bs->every_linked = false;
     upload_image(bs, fp, imgs, where, (size_t)n * H * W * 3);
     // the hand plan of the chunks, with the hand session's work buffers sized for the largest crop
     OPB_CUDA(cudaStreamSynchronize(hs->stream));
     FramePlan* hp = get_plan(hs, kEveryChunk, tw, tw, hscales, nhs);
-    hs->active = hp;
-    hs->hand_crops = kEveryChunk;
-    hs->hand_ragged = false;
-    const uint64_t gen = gen_key({bs->buffer_gen, bs->every->gen});
-    run_or_replay_slot(bs, GraphSlot{fp->every_graph, fp->every_gen, fp->every_uses}, gen, [&] {
+    pair_begin(bs, hs, Job::Every, fp, hp, 0, false);
+    run_job(bs, fp, Job::Every, gen_key({bs->gen}), [&] {
         run_front(bs, fp, n, H, W);
         body_post_enqueue(bs, fp, n, H, W);
         every_rows_enqueue(bs, fp, n);
@@ -1641,11 +1608,7 @@ static void batch_every_chunk_enqueue(opb_session* bs, opb_session* hs, FramePla
 
 static void batch_every_submit(opb_session* bs, opb_session* hs, const uint8_t* frames, int where, int n, int H, int W,
                                double g_scale, int boxsize) {
-    OPB_REQUIRE(bs->net->kind == OPB_NET_BODY && hs->net->kind == OPB_NET_HAND,
-                "batch every person: a body session and a hand session");
-    OPB_REQUIRE(bs->net->ctx == hs->net->ctx, "batch every person: both networks must live on the same context");
-    OPB_REQUIRE(n >= 1 && n <= 64, "1..64 frames per batch");
-    OPB_REQUIRE(H >= 1 && W >= 1, "empty frame");
+    pair_check(bs, hs, n, H, W, "batch every person");
     OPB_REQUIRE(g_scale > 0, "scale must be positive");
     OPB_REQUIRE(boxsize >= 8 && boxsize % 8 == 0, "boxsize must be a positive multiple of 8 (srcmx/Batch_model.py:377)");
     OPB_CUDA(cudaSetDevice(bs->net->ctx->device));
@@ -1658,24 +1621,14 @@ static void batch_every_submit(opb_session* bs, opb_session* hs, const uint8_t* 
     track_with_tables(hs, boxsize, std::min(H, W));                 // crop tables of every side up to min(H, W)
     FramePlan* fp = get_plan(bs, n, H, W, &g_scale, 1, 2);          // Batch_body on uint8 frames
     ensure_host(bs, n, 0);
-    bs->active = fp;
-    bs->n_frames = n;
-    bs->pose_hand = hs;
-    bs->batch_pose_box = boxsize;
-    bs->every_batch = true;
-    bs->every_persons = -1;
-    bs->every_linked = false;
     const double one = 1.0;
     FramePlan* hp = get_plan(hs, kBatchEveryChunk, boxsize, boxsize, &one, 1, 2);   // uint8 Batch_hand on one chunk
-    hs->active = hp;
-    hs->hand_crops = kBatchEveryChunk;
-    hs->hand_ragged = false;
+    pair_begin(bs, hs, Job::Every, fp, hp, boxsize, false);
     bs->prof.reset();
     bs->prof.mark(st, "start");
     upload_image(bs, fp, frames, where, (size_t)n * H * W * 3);
     bs->prof.mark(st, "h2d");
-    const uint64_t gen = gen_key({bs->buffer_gen, bs->every->gen});
-    run_or_replay_slot(bs, GraphSlot{fp->every_graph, fp->every_gen, fp->every_uses}, gen, [&] {
+    run_job(bs, fp, Job::Every, gen_key({bs->gen}), [&] {
         run_front_f32(bs, fp, n, H, W);
         body_post_enqueue(bs, fp, n, H, W);
         every_rows_enqueue(bs, fp, n);
@@ -1804,7 +1757,7 @@ static void tracker_finish(opb_tracker* tr) {
 // frames 0 .. n_link - 1 are linked after the hand chunks and their ids copied back with the records; a batch whose
 // Body / Batch_body raised IndexError is not linked.
 static int every_wait(opb_session* bs, int* persons, int* frame_status, opb_tracker* tr = nullptr, int n_link = 0) {
-    OPB_REQUIRE(bs->active && bs->every && bs->every_batch && bs->pose_hand, "no every-person batch in flight");
+    OPB_REQUIRE(bs->active && bs->job == Job::Every, "no every-person batch in flight");
     OPB_CUDA(cudaSetDevice(bs->net->ctx->device));
     cudaStream_t st = bs->stream;
     FramePlan* fp = bs->active;
@@ -1822,27 +1775,19 @@ static int every_wait(opb_session* bs, int* persons, int* frame_status, opb_trac
     }
     opb_session::EveryBuffers& e = *bs->every;
     const int T = e.counts_host[0], V = e.counts_host[1];
-    if (V > 0 && bs->batch_pose_box) {
-        opb_session* hs = bs->pose_hand;
-        FramePlan* hp = hs->active;
-        const int boxsize = bs->batch_pose_box;
-        const uint64_t gen = gen_key({bs->buffer_gen, hs->buffer_gen, (uint64_t)(uintptr_t)hp, hs->track->gen, e.gen,
-                                      (uint64_t)(uintptr_t)fp->d_img, (uint64_t)fp->key.H, (uint64_t)fp->key.W,
-                                      (uint64_t)boxsize});
+    opb_session* hs = bs->pair_hand;
+    FramePlan* hp = hs->active;
+    const int boxsize = bs->pair_box;
+    if (V > 0 && boxsize) {
+        const uint64_t key = gen_key({bs->gen, hs->gen, hp->serial, (uint64_t)boxsize});
         for (int base = 0; base < V; base += kBatchEveryChunk)
-            run_or_replay_slot(bs, GraphSlot{fp->every_hand_graph, fp->every_hand_gen, fp->every_hand_uses}, gen,
-                               [&] { batch_every_chunk_enqueue(bs, hs, fp, hp, boxsize); });
+            run_job(bs, fp, Job::EveryHand, key, [&] { batch_every_chunk_enqueue(bs, hs, fp, hp, boxsize); });
         bs->net->ctx->launches += (int64_t)cdiv(V, kBatchEveryChunk) * (3 /* stage, crops, finish */ + hp->launches_per_frame);
     } else if (V > 0) {
-        opb_session* hs = bs->pose_hand;
-        FramePlan* hp = hs->active;
-        const opb_session::Ragged& rg = *hs->ragged;
-        const uint64_t gen = gen_key({bs->buffer_gen, hs->buffer_gen, (uint64_t)(uintptr_t)hp, (uint64_t)(uintptr_t)rg.tabs.slab,
-                                      (uint64_t)rg.tabs.wmax, e.gen, (uint64_t)(uintptr_t)fp->d_img});
+        const uint64_t key = gen_key({bs->gen, hs->gen, hp->serial});
         for (int base = 0; base < V; base += kEveryChunk)
-            run_or_replay_slot(bs, GraphSlot{fp->every_hand_graph, fp->every_hand_gen, fp->every_hand_uses}, gen,
-                               [&] { every_chunk_enqueue(bs, hs, fp, hp); });
-        const int nhs = rg.tabs.n_scales;
+            run_job(bs, fp, Job::EveryHand, key, [&] { every_chunk_enqueue(bs, hs, fp, hp); });
+        const int nhs = hs->ragged->tabs.n_scales;
         bs->net->ctx->launches += (int64_t)cdiv(V, kEveryChunk) * (1 + nhs + hp->net->kernel_launches + (nhs + 1) + 6 + 1);
     }
     std::unique_lock<std::mutex> lock;
@@ -2023,6 +1968,13 @@ int opb_body_fetch_frame(opb_session* s, int frame, double* candidate, int cand_
     return guarded([&] { body_fetch(s, frame, candidate, cand_rows, subset, subset_rows); });
 }
 
+int opb_session_graph_stats(opb_session* s, long long* captures, long long* replays) {
+    return guarded([&] {
+        OPB_REQUIRE(s && captures && replays, "null argument");
+        *captures = s->captures;
+        *replays = s->replays;
+    });
+}
 int opb_session_set_profiling(opb_session* s, int on) {
     return guarded([&] {
         OPB_REQUIRE(s != nullptr, "null session");
@@ -2100,7 +2052,7 @@ int opb_body_maps(opb_session* s, float* host_heat, float* host_paf) {
 int opb_hand_maps(opb_session* s, float* host_heat) {
     return guarded([&] {
         OPB_REQUIRE(s && s->active && s->net->kind == OPB_NET_HAND && host_heat, "no finished hand batch");
-        OPB_REQUIRE(!s->hand_ragged, "the last hand batch was a list of crops of different sides: its maps have no common shape");
+        OPB_REQUIRE(s->job != Job::Crops, "the last hand batch was a list of crops of different sides: its maps have no common shape");
         OPB_CUDA(cudaEventSynchronize(s->done));
         const size_t px = (size_t)s->active->key.H * s->active->key.W;
         OPB_CUDA(cudaMemcpy(host_heat, s->active->heat_avg, px * 22 * 4 * s->active->key.n, cudaMemcpyDeviceToHost));
@@ -2212,15 +2164,14 @@ int opb_pose_submit_batch(opb_session* body_s, opb_session* hand_s, const uint8_
 int opb_pose_wait(opb_session* body_s, double* pose_mats, int* frame_status) {
     int rc = OPB_OK;
     int g = guarded([&] {
-        OPB_REQUIRE(body_s && pose_mats && body_s->pose && body_s->active && !body_s->batch_pose_box && !body_s->every_batch,
-                    "no pose batch in flight");
+        OPB_REQUIRE(body_s && pose_mats && body_s->active && body_s->job == Job::Pose, "no pose batch in flight");
         // body results first: they report the overflow / IndexError conditions of every frame
         bool grew = false;
         rc = pose_batch_status(body_s, frame_status, grew);
         if (grew) {
             FramePlan* fp = body_s->active;
-            opb_session* hs = body_s->pose_hand;
-            pose_hand_enqueue(body_s, hs, fp, hs->active, body_s->n_frames, fp->key.H, fp->key.W, body_s->pose_fixed);
+            opb_session* hs = body_s->pair_hand;
+            pose_hand_enqueue(body_s, hs, fp, hs->active, body_s->n_frames, fp->key.H, fp->key.W, body_s->pair_fixed);
             OPB_CUDA(cudaStreamSynchronize(body_s->stream));
         }
         memcpy(pose_mats, body_s->pose->host, (size_t)body_s->n_frames * 180 * sizeof(double));
@@ -2240,14 +2191,14 @@ int opb_batch_pose_submit(opb_session* body_s, opb_session* hand_s, const uint8_
 int opb_batch_pose_wait(opb_session* body_s, double* motion_mats, double* hand_mats, int* frame_status) {
     int rc = OPB_OK;
     int g = guarded([&] {
-        OPB_REQUIRE(body_s && motion_mats && hand_mats && body_s->pose && body_s->active && body_s->batch_pose_box &&
-                        !body_s->every_batch, "no batch-pose batch in flight");
+        OPB_REQUIRE(body_s && motion_mats && hand_mats && body_s->active && body_s->job == Job::BatchPose,
+                    "no batch-pose batch in flight");
         OPB_CUDA(cudaSetDevice(body_s->net->ctx->device));
         bool grew = false;
         rc = pose_batch_status(body_s, frame_status, grew);
         if (grew) {                                   // the hand half again, on the grown frames' new body results
-            opb_session* hs = body_s->pose_hand;
-            batch_pose_hand_enqueue(body_s, hs, body_s->active, hs->active, body_s->n_frames, body_s->batch_pose_box);
+            opb_session* hs = body_s->pair_hand;
+            batch_pose_hand_enqueue(body_s, hs, body_s->active, hs->active, body_s->n_frames, body_s->pair_box);
             OPB_CUDA(cudaStreamSynchronize(body_s->stream));
         }
         const double* rec = body_s->pose->host;
@@ -2407,7 +2358,7 @@ int opb_hand_submit_ragged(opb_session* s, const uint8_t* packed, const size_t* 
 }
 int opb_hand_wait(opb_session* s, double* peaks) {
     return guarded([&] {
-        OPB_REQUIRE(s && s->active && peaks, "no frame in flight");
+        OPB_REQUIRE(s && s->active && peaks && (s->job == Job::Frame || s->job == Job::Crops), "no frame in flight");
         OPB_CUDA(cudaEventSynchronize(s->done));
         memcpy(peaks, s->hand_host, (size_t)s->hand_crops * 63 * sizeof(double));
     });
@@ -2577,6 +2528,7 @@ int opb_body_debug_post_submit(opb_session* s, int n, int H, int W, const double
         ensure_host(s, n, 0);
         s->active = fp;
         s->n_frames = n;
+        s->job = Job::Frame;
         s->prof.reset();
         for (int i = 0; i < ns; ++i) {
             OPB_REQUIRE(heat[i] && paf[i], "null net output");

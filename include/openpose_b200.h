@@ -426,6 +426,38 @@ int opb_debug_resize_dsize(int n, double f);
  * the tiling (every pixel stored exactly once, both tiles of a pair share one orientation).  *written = entries.     */
 int opb_debug_pair_tiles(int n, int h, int w, int n_tiles_n, int small, int* out, int cap, int* written);
 
+/* ---- MJPG frames decoded on the device ------------------------------------------------------------------------
+ * A decoded frame equals cv2.imdecode(packet, cv2.IMREAD_COLOR) bit for bit (libjpeg-turbo's ISLOW IDCT, fancy
+ * upsampling and YCbCr -> BGR tables), cropped like numpy's frame[y0:y1, x0:x1].  Baseline / extended sequential
+ * Huffman JPEG, 8-bit, one scan: grey, or YCbCr 4:4:4, 4:2:2, 4:2:0.  Other packets are not decoded here
+ * (OPB_JPEG_FALLBACK): the caller decodes them and puts the frame in place with opb_jpeg_upload.
+ *
+ * opb_jpeg_submit: n packets, packet i = packed[offsets[i] .. offsets[i + 1]) in host memory (where 0 pageable or 2
+ *   pinned: both are read the same way -- the host parses and destuffs every packet into the session's own pinned
+ *   buffer and uploads from there, so pinned packets gain nothing), are parsed on the host and decoded on the session's
+ *   stream, so the session's next submit with where = 1
+ *   reads them in stream order.  roi = {x0, y0, x1, y1} (Python slice ends) or NULL for the whole frame; every packet
+ *   of a batch must have the same frame size.  flags[n] gets what the host already knows: OPB_JPEG_FALLBACK, or
+ *   OPB_JPEG_CORRUPT for restart markers that do not match the header.  *dev_frames: (n, height, width, 3) uint8 BGR
+ *   device frames, valid until the session's next opb_jpeg_submit.  The call does not wait for the stream; it waits
+ *   only for the upload of the session's previous batch before reusing its pinned buffers.
+ * opb_jpeg_upload: copies the host frame (height, width, 3) of a packet decoded elsewhere into slot `index`.
+ * opb_jpeg_fetch: waits for the stream and copies the n frames to host memory.
+ * opb_jpeg_status: waits for the decode and gives flags[n]: the submit's flags | OPB_JPEG_CORRUPT for entropy data
+ *   the device could not decode consistently (a bad Huffman code, a segment that runs out or has data left over).
+ * opb_jpeg_decode_host (host only): the same decoder on the CPU, for one packet.  *height / *width / *status are set
+ *   first (0 x 0 when no frame header was read); the frame is written when out != NULL and *status == 0 after
+ *   parsing (OPB_ERR_CAPACITY when out_bytes is short).  Malformed headers return OPB_ERR_INVALID.             */
+#define OPB_JPEG_FALLBACK 1
+#define OPB_JPEG_CORRUPT 2
+int opb_jpeg_submit(opb_session* s, const uint8_t* packed, const int64_t* offsets, int where, int n, const int* roi,
+                    int* flags, uint8_t** dev_frames, int* height, int* width);
+int opb_jpeg_upload(opb_session* s, int index, const uint8_t* host_frame);
+int opb_jpeg_fetch(opb_session* s, uint8_t* host_out);
+int opb_jpeg_status(opb_session* s, int* flags);
+int opb_jpeg_decode_host(const uint8_t* packet, int64_t size, const int* roi, uint8_t* out, int64_t out_bytes,
+                         int* height, int* width, int* status);
+
 #ifdef __cplusplus
 }
 #endif

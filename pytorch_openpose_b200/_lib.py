@@ -18,6 +18,7 @@ OPB_ERR_CAPACITY = -4
 OPB_ERR_SUBSET_INDEX = -5
 OPB_ERR_NO_DEVICE = -6
 NET_BODY, NET_HAND = 0, 1
+JPEG_FALLBACK, JPEG_CORRUPT = 1, 2
 
 # name -> (restype, argtypes); every symbol include/openpose_b200.h declares
 SIGNATURES = {
@@ -118,6 +119,13 @@ SIGNATURES = {
     "opb_body_debug_post_submit": (c_int, [c_void_p, c_int, c_int, c_int, POINTER(c_double), c_int, c_int,
                                            POINTER(c_void_p), POINTER(c_void_p)]),
     "opb_body_debug_part_begin": (c_int, [c_void_p, c_int, c_void_p]),
+    "opb_jpeg_submit": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, POINTER(c_void_p),
+                                POINTER(c_int), POINTER(c_int)]),
+    "opb_jpeg_upload": (c_int, [c_void_p, c_int, c_void_p]),
+    "opb_jpeg_fetch": (c_int, [c_void_p, c_void_p]),
+    "opb_jpeg_status": (c_int, [c_void_p, c_void_p]),
+    "opb_jpeg_decode_host": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_int64, POINTER(c_int), POINTER(c_int),
+                                     POINTER(c_int)]),
     "opb_conv2d": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_int,
                            c_int, c_int, c_void_p, c_int]),
 }

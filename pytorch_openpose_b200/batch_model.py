@@ -15,7 +15,11 @@ from .body import _load_checkpoint
 
 
 def _as_frames_u8(frames, where):
-    """Decoded frames (B, h, w, 3) uint8 as they come out of cv2 -> (pointer, keepalive, (B, h, w))."""
+    """Decoded frames (B, h, w, 3) uint8 as they come out of cv2, or (device pointer, (B, h, w)) with where=1 ->
+    (pointer, keepalive, (B, h, w))."""
+    if where == 1 and isinstance(frames, tuple):
+        ptr, shape = frames
+        return ptr, None, tuple(shape)
     arr = np.ascontiguousarray(frames, dtype=np.uint8)
     if arr.ndim != 4 or arr.shape[3] != 3:
         raise ValueError("expected (B, h, w, 3) uint8 frames")
@@ -24,7 +28,8 @@ def _as_frames_u8(frames, where):
 
 def _as_track_frames(frames, where):
     """-> (pointer, where, keepalive, (B, h, w)) of (B, h, w, 3) uint8 frames: torch CUDA tensors are read in place
-    (where=1), pinned CPU tensors straight from their pages (where=2); anything else as `where` says."""
+    (where=1), pinned CPU tensors straight from their pages (where=2), (device pointer, (B, h, w)) with where=1;
+    anything else as `where` says."""
     if hasattr(frames, "detach"):
         import torch
         t = frames.detach()

@@ -1,6 +1,7 @@
 // extern "C" surface of libopenpose_b200.so (include/openpose_b200.h) and the per-frame pipelines behind
 // Body.__call__ (src/body.py:24-212) and Hand.__call__ (src/hand.py:25-75).
 #include "net.cuh"
+#include "jpeg.cuh"
 #include <cstdlib>
 #include <cstring>
 #include <algorithm>
@@ -475,7 +476,9 @@ struct opb_session {
     int every_persons = -1;              // persons of the last finished opb_pose_every batch; -1: none
     bool every_linked = false;           // the last finished opb_pose_every batch was linked: ids_host holds its ids
     std::vector<NetShape> debug_shapes;  // the plan of the opb_net_debug_* calls (looked up by its shapes on every call)
+    JpegBatch* jpeg = nullptr;           // packets decoded for this session's next batch (opb_jpeg_*)
     ~opb_session() {
+        jpeg_batch_free(jpeg);
         plans.clear();
         net_plans.clear();
         for (auto& a : arena) if (a.p) cudaFree(a.p);
@@ -2974,6 +2977,41 @@ int opb_conv2d(opb_context* ctx, const void* dev_in, int n, int h, int w, int ci
         ctx->launches += 1;
         OPB_CUDA(cudaStreamSynchronize(ctx->stream));
     });
+}
+
+// ---- MJPG frames decoded on the device (jpeg.cu) ----
+int opb_jpeg_submit(opb_session* s, const uint8_t* packed, const int64_t* offsets, int where, int n, const int* roi,
+                    int* flags, uint8_t** dev_frames, int* height, int* width) {
+    return guarded([&] {
+        OPB_REQUIRE(s, "null session");
+        OPB_REQUIRE(where == 0 || where == 2, "where: 0 pageable host, 2 pinned host (the host parses the packets)");
+        s->net->ctx->launches += jpeg_submit(s->jpeg, s->net->ctx->device, s->stream, packed, offsets, n, roi, flags,
+                                             dev_frames, height, width);
+    });
+}
+int opb_jpeg_upload(opb_session* s, int index, const uint8_t* host_frame) {
+    return guarded([&] {
+        OPB_REQUIRE(s, "null session");
+        OPB_CUDA(cudaSetDevice(s->net->ctx->device));
+        jpeg_upload(s->jpeg, s->stream, index, host_frame);
+    });
+}
+int opb_jpeg_fetch(opb_session* s, uint8_t* host_out) {
+    return guarded([&] {
+        OPB_REQUIRE(s, "null session");
+        OPB_CUDA(cudaSetDevice(s->net->ctx->device));
+        jpeg_fetch(s->jpeg, s->stream, host_out);
+    });
+}
+int opb_jpeg_status(opb_session* s, int* flags) {
+    return guarded([&] {
+        OPB_REQUIRE(s, "null session");
+        jpeg_status(s->jpeg, flags);
+    });
+}
+int opb_jpeg_decode_host(const uint8_t* packet, int64_t size, const int* roi, uint8_t* out, int64_t out_bytes,
+                         int* height, int* width, int* status) {
+    return guarded([&] { jpeg_decode_host(packet, size, roi, out, out_bytes, height, width, status); });
 }
 
 }  // extern "C"

@@ -48,14 +48,31 @@ class FrameBatches(object):
     workers=1 reads the file front to back like the reference (`video.read()` until it fails) and yields batches in
     order.  workers=k splits the frame range into k contiguous, batch-aligned segments, one `cv2.VideoCapture` and
     one thread each (seek with CAP_PROP_POS_FRAMES); batches then arrive in whatever order they are decoded -- every
-    batch carries its first frame index -- and frames past the container's reported count are not read."""
+    batch carries its first frame index -- and frames past the container's reported count are not read.
 
-    def __init__(self, videopath, recpoint=None, batch=8, depth=4, pinned=False, workers=1, pad_last=False, ordered=False):
+    decode="device": the frames are not decoded here.  One thread reads the raw JPEG packets of an MJPG video
+    (CAP_PROP_FORMAT = -1) into a ring of buffers (pageable: the library parses the packets on the host and copies
+    what it uploads into its own pinned buffer, so `pinned` does not apply), and every batch is a `jpeg.Packets` (with `recpoint`) for
+    `jpeg.DeviceFrames` to decode on the session that consumes it; pad_last repeats the last packet, batches come in
+    order, `workers` is ignored.  A video that is not MJPG raises ValueError."""
+
+    def __init__(self, videopath, recpoint=None, batch=8, depth=4, pinned=False, workers=1, pad_last=False, ordered=False,
+                 decode="cv2"):
         import cv2
+        if decode not in ("cv2", "device"):
+            raise ValueError("decode must be 'cv2' or 'device', not %r" % (decode,))
         probe = cv2.VideoCapture(videopath)
         if not probe.isOpened():
             raise FileNotFoundError("the file %s is not exist" % videopath)
         self.count = int(probe.get(cv2.CAP_PROP_FRAME_COUNT))
+        self.device = decode == "device"
+        if self.device:
+            fourcc = int(probe.get(cv2.CAP_PROP_FOURCC)) & 0xFFFFFFFF
+            if fourcc.to_bytes(4, "little").upper() != b"MJPG":
+                probe.release()
+                raise ValueError("%s: decode='device' reads MJPG video, this one is %r"
+                                 % (videopath, fourcc.to_bytes(4, "little")))
+            workers = 1
         probe.release()
         self.videopath, self.recpoint, self.batch, self.pinned = videopath, recpoint, batch, pinned
         # pad_last: a short final batch is filled up with copies of its last frame and yielded at full size as
@@ -80,7 +97,8 @@ class FrameBatches(object):
                 continue
             ring = {"bufs": None, "free": queue.Queue(), "depth": self.hold + 2}
             self._rings.append(ring)
-            threading.Thread(target=self._run, args=(w, ring, lo, hi), daemon=True).start()
+            threading.Thread(target=self._run_packets if self.device else self._run, args=(w, ring, lo, hi),
+                             daemon=True).start()
 
     def _crop(self, frame):
         if self.recpoint is None:
@@ -122,6 +140,51 @@ class FrameBatches(object):
         finally:
             video.release()
 
+    def _run_packets(self, w, ring, lo, hi):
+        import cv2
+        from .jpeg import Packets
+        video = cv2.VideoCapture(self.videopath)
+        try:
+            video.set(cv2.CAP_PROP_FORMAT, -1)         # raw packets, not decoded frames
+            ring["bufs"] = [None] * ring["depth"]
+            ring["packets"] = [None] * ring["depth"]
+            for i in range(ring["depth"]):
+                ring["free"].put(i)
+            index, parts, first = 0, [], 0
+
+            def put(parts, fill, first):
+                cur = ring["free"].get()
+                if self.pad_last:
+                    parts = parts + [parts[-1]] * (self.batch - fill)
+                offsets = np.zeros(len(parts) + 1, np.int64)
+                offsets[1:] = np.cumsum([len(p) for p in parts])
+                if ring["bufs"][cur] is None or len(ring["bufs"][cur][0]) < offsets[-1]:
+                    ring["bufs"][cur] = _alloc((int(offsets[-1]) * 5 // 4 + 4096,), np.uint8, False)
+                data = ring["bufs"][cur][0]
+                for p, o in zip(parts, offsets):
+                    data[o:o + len(p)] = p
+                ring["packets"][cur] = Packets(data, offsets, self.recpoint)
+                self._qs[w].put((w, cur, fill, first))
+
+            while True:
+                ret, pkt = video.read()
+                if ret is False:
+                    break
+                if not parts:
+                    first = index
+                parts.append(np.asarray(pkt, np.uint8).ravel())
+                index += 1
+                if len(parts) == self.batch:
+                    put(parts, len(parts), first)
+                    parts = []
+            if parts:
+                put(parts, len(parts), first)
+            self._qs[w].put(None)
+        except BaseException as e:
+            self._qs[w].put(e)
+        finally:
+            video.release()
+
     def _items(self):
         if self.ordered:                               # each worker's batches arrive in order: take the workers in turn
             for q in self._qs:
@@ -145,10 +208,38 @@ class FrameBatches(object):
             if len(held) > self.hold:                  # the consumer is done with the oldest buffer
                 ow, oc = held.pop(0)
                 self._rings[ow]["free"].put(oc)
-            if self.pad_last:
+            if self.device:
+                batch = self._rings[w]["packets"][cur]
+                yield (batch, first, fill) if self.pad_last else (batch, first)
+            elif self.pad_last:
                 yield self._rings[w]["bufs"][cur][0], first, fill
             else:
                 yield self._rings[w]["bufs"][cur][0][:fill], first
+
+
+def _check_decode(decode, native):
+    if decode not in ("cv2", "device"):
+        raise ValueError("decode must be 'cv2' or 'device', not %r" % (decode,))
+    if decode == "device" and not native:
+        raise ValueError("decode='device' decodes on the sessions of this package's estimators; these are not")
+
+
+def _decoded(session, frames, first, where):
+    """A FrameBatches batch as the submits take it: packets (decode='device') are decoded on `session`, the one that
+    consumes them -> ((device pointer, (n, h, w)), 1, jpeg.DeviceFrames); host frames pass through -> (frames, where,
+    None)."""
+    from .jpeg import DeviceFrames, Packets
+    if isinstance(frames, Packets):
+        d = DeviceFrames(session, frames, first)
+        return d.where1, 1, d
+    return frames, where, None
+
+
+def _rerun_corrupt(dec, resubmit):
+    """Before a batch's results are read: frames whose entropy data the device found corrupt are decoded with
+    cv2.imdecode, put in place, and the batch runs again."""
+    if dec is not None and dec.repair():
+        resubmit()
 
 
 def _job_sessions(estimator, n):
@@ -234,19 +325,29 @@ def _hands_into(pose60, frame, candidate, subset, chosen, hand_estimation):
 
 
 def extract_motion_from_video(videopath, outpath, recpoint, body_estimation, hand_estimation=None, mode="body",
-                              batch=8, sessions=2, pinned=None, log=print, decode_workers=1, stats=None):
+                              batch=8, sessions=2, pinned=None, log=print, decode_workers=1, stats=None, decode="cv2"):
     """`Extract_MotionData_from_Video` (srcmx/MotionEstimation.py:25-77): MotionMat (count, 18 | 60, 3) float64, dumped
     with joblib to `outpath`.  `body_estimation` is a `Body`: batches of frames are kept in flight on `sessions` of its
-    sessions; any other callable `frame -> (candidate, subset)` is called frame by frame."""
+    sessions; any other callable `frame -> (candidate, subset)` is called frame by frame.
+
+    decode="device" (MJPG video, this package's `Body`, and in mode 'bodyhand' its `Hand` on the device path): the
+    JPEG packets go up and are decoded on the session that consumes them (`jpeg.DeviceFrames`); the frames equal
+    cv2.imdecode's, which differ from cv2.VideoCapture's by a few LSB (DESIGN.md section 2)."""
     import joblib
     if mode == "bodyhand" and hand_estimation is None:
         raise ValueError("mode='bodyhand' needs a hand estimator")
     pipelined = hasattr(body_estimation, "submit_batch")
     if pinned is None:
         pinned = pipelined
+    native_hand = mode == "bodyhand" and pipelined and hasattr(hand_estimation, "submit") and hasattr(hand_estimation, "net")
+    from .body import Body
+    from .hand import Hand
+    on_device = (native_hand and type(body_estimation) is Body and type(hand_estimation) is Hand
+                 and os.environ.get("OPB_HOST_HANDS") is None)
+    _check_decode(decode, on_device or (mode == "body" and type(body_estimation) is Body))
     try:
         src = FrameBatches(videopath, recpoint, batch=batch, depth=sessions + 3, pinned=pinned, workers=decode_workers,
-                           pad_last=pipelined)
+                           pad_last=pipelined, decode=decode)
     except FileNotFoundError as e:
         log(str(e))
         return None
@@ -255,11 +356,7 @@ def extract_motion_from_video(videopath, outpath, recpoint, body_estimation, han
     outname = os.path.split(outpath)[1]
     done = 0
     hand_pool = None
-    native_hand = mode == "bodyhand" and pipelined and hasattr(hand_estimation, "submit") and hasattr(hand_estimation, "net")
-    from .body import Body
-    from .hand import Hand
-    if (native_hand and type(body_estimation) is Body and type(hand_estimation) is Hand
-            and os.environ.get("OPB_HOST_HANDS") is None):
+    if on_device:
         # both estimators are this package's: person selection, hand boxes, crops and the hand network stay on the
         # device, PoseMat is the only thing that comes back (motion.PoseEstimator)
         return _extract_bodyhand_on_device(src, outpath, body_estimation, hand_estimation, sessions, pinned, log, stats)
@@ -290,8 +387,9 @@ def extract_motion_from_video(videopath, outpath, recpoint, body_estimation, han
         pending = []                                                   # (session, frames, first)
 
         def retire():
-            s, fr, fi, nv = pending.pop(0)
+            s, fr, fi, nv, dec, arg, wh = pending.pop(0)
             t = time.perf_counter()
+            _rerun_corrupt(dec, lambda: body_estimation.submit_batch(arg, s, where=wh))
             res = body_estimation.collect_batch(s)
             clock["collect_wait"] += time.perf_counter() - t
             t = time.perf_counter()
@@ -310,9 +408,10 @@ def extract_motion_from_video(videopath, outpath, recpoint, body_estimation, han
                 retire()
             s = next(c for c in ss if all(c is not p[0] for p in pending))
             t = time.perf_counter()
-            body_estimation.submit_batch(frames, s, where=2 if pinned else 0)
+            arg, wh, dec = _decoded(s, frames, first, 2 if pinned else 0)
+            body_estimation.submit_batch(arg, s, where=wh)
             clock["submit"] += time.perf_counter() - t
-            pending.append((s, frames, first, n_valid))
+            pending.append((s, frames, first, n_valid, dec, arg, wh))
         while pending:
             retire()
         if stats is not None:
@@ -349,8 +448,9 @@ def _extract_bodyhand_on_device(src, outpath, body_estimation, hand_estimation, 
     pending = []
 
     def retire():
-        pair, first, nv = pending.pop(0)
+        pair, first, nv, dec, arg, wh = pending.pop(0)
         t = time.perf_counter()
+        _rerun_corrupt(dec, lambda: est.submit_batch(arg, pair, where=wh))
         pose = est.collect(pair)
         clock["collect_wait"] += time.perf_counter() - t
         hi = min(first + nv, len(mat))
@@ -371,9 +471,10 @@ def _extract_bodyhand_on_device(src, outpath, body_estimation, hand_estimation, 
             retire()
         pair = next(c for c in pairs if all(c is not p[0] for p in pending))
         t = time.perf_counter()
-        est.submit_batch(frames, pair, where=2 if pinned else 0)
+        arg, wh, dec = _decoded(pair[0], frames, first, 2 if pinned else 0)
+        est.submit_batch(arg, pair, where=wh)
         clock["submit"] += time.perf_counter() - t
-        pending.append((pair, first, n_valid))
+        pending.append((pair, first, n_valid, dec, arg, wh))
     while pending:
         retire()
     if stats is not None:
@@ -406,7 +507,8 @@ def _write_tracks(outpath, count, frames):
 
 
 def extract_every_person_from_video(videopath, outpath, recpoint, body_estimation, hand_estimation, max_gap=15,
-                                    max_dist=None, min_joints=3, batch=8, sessions=2, decode_workers=1, log=print):
+                                    max_dist=None, min_joints=3, batch=8, sessions=2, decode_workers=1, log=print,
+                                    decode="cv2"):
     """Body and hands of every person of a video, linked into per-person tracks (`motion.PersonLinker`'s rule), dumped
     with joblib to `outpath` as {"count": T, "tracks": [(first_frame, posemat (L, 60, 3) float64), ...]}, indexed by
     track id.  A track's PoseMat runs from its first to its last matched frame; frames in between where it was not
@@ -419,14 +521,16 @@ def extract_every_person_from_video(videopath, outpath, recpoint, body_estimatio
     session pairs in flight) and are linked there, in frame order, by one tracker.  With any other estimators the job
     runs `motion.pose_mats_every_person` frame by frame and links with `PersonLinker`.  Both write the same file.
     Frames are linked in order, so with decode_workers > 1 the later segments decode only a few batches ahead.  An
-    IndexError from Body is raised before anything is written."""
+    IndexError from Body is raised before anything is written.  decode="device" (MJPG video, the device path): the
+    JPEG packets are decoded on the consuming session, as in `extract_motion_from_video`."""
     from .body import Body
     from .hand import Hand
     from .motion import PersonLinker, pose_mats_every_person
     device = type(body_estimation) is Body and type(hand_estimation) is Hand
+    _check_decode(decode, device)
     try:
         src = FrameBatches(videopath, recpoint, batch=batch, depth=sessions + 3, pinned=device, workers=decode_workers,
-                           pad_last=device, ordered=True)
+                           pad_last=device, ordered=True, decode=decode)
     except FileNotFoundError as e:
         log(str(e))
         return None
@@ -439,22 +543,24 @@ def extract_every_person_from_video(videopath, outpath, recpoint, body_estimatio
         pending = []
 
         def retire():
-            pair, first, nv = pending.pop(0)
+            pair, first, nv, dec, arg, wh = pending.pop(0)
             n_link = max(0, min(nv, src.count - first))
+            _rerun_corrupt(dec, lambda: est.submit_every_person(arg, pair, where=wh))
             recs, ids = est.collect_every_person(pair, tracker=tracker, n_link=n_link)
             frames.append((first, recs[:n_link], ids[:n_link]))
             if first % 100 < len(recs):
                 log("%s-%d/%d" % (outname, first, src.count))
 
         for fr, first, n_valid in src:
-            if tracker is None:
-                height = fr.shape[1]
-                tracker = est.tracker(max_gap, 0.1 * height if max_dist is None else max_dist, min_joints)
             if len(pending) == len(pairs):
                 retire()
             pair = next(c for c in pairs if all(c is not p[0] for p in pending))
-            est.submit_every_person(fr, pair, where=2)
-            pending.append((pair, first, n_valid))
+            arg, wh, dec = _decoded(pair[0], fr, first, 2)
+            if tracker is None:
+                height = dec.shape[1] if dec is not None else fr.shape[1]
+                tracker = est.tracker(max_gap, 0.1 * height if max_dist is None else max_dist, min_joints)
+            est.submit_every_person(arg, pair, where=wh)
+            pending.append((pair, first, n_valid, dec, arg, wh))
         while pending:
             retire()
     else:
@@ -481,15 +587,19 @@ def to_tensor(frames_u8):
 
 
 def batch_body_extraction(videopath, outpath, batch_size, recpoint, batch_body_model, log=print, decode_workers=1,
-                          sessions=2):
+                          sessions=2, decode="cv2"):
     """`Batch_body_extraction` (srcmx/Batch_motion_Estimation.py:66-112) -> MotionMat (COUNTS, 18, 3).  A `Batch_body`
     of this package is fed the decoded uint8 frames directly (`submit_frames`: ToTensor's /255 on the device) on
-    `sessions` sessions; any other callable gets `ToTensor`-ed float batches like the reference's DataLoader yields."""
+    `sessions` sessions; any other callable gets `ToTensor`-ed float batches like the reference's DataLoader yields.
+    decode="device" (MJPG video, this package's `Batch_body`): the JPEG packets are decoded on the consuming session
+    (`jpeg.DeviceFrames`); frames equal cv2.imdecode's (DESIGN.md section 2)."""
     import joblib
+    from .batch_model import Batch_body
     pipelined = hasattr(batch_body_model, "submit_frames")
+    _check_decode(decode, type(batch_body_model) is Batch_body)
     try:
         src = FrameBatches(videopath, recpoint, batch=batch_size, depth=sessions + 3 if pipelined else 4, pinned=pipelined,
-                           workers=decode_workers, pad_last=pipelined)
+                           workers=decode_workers, pad_last=pipelined, decode=decode)
     except FileNotFoundError as e:
         log(str(e))
         return None
@@ -509,15 +619,20 @@ def batch_body_extraction(videopath, outpath, batch_size, recpoint, batch_body_m
     if pipelined:
         ss = _job_sessions(batch_body_model, sessions)
         pending = []
+        def retire():
+            s, fi, nv, dec, arg, wh = pending.pop(0)
+            _rerun_corrupt(dec, lambda: batch_body_model.submit_frames(arg, s, where=wh))
+            finish(fi, batch_body_model.collect(s)[:nv])
+
         for frames, first, n_valid in src:
             if len(pending) == sessions:
-                s, fi, nv = pending.pop(0)
-                finish(fi, batch_body_model.collect(s)[:nv])
+                retire()
             s = next(c for c in ss if all(c is not p[0] for p in pending))
-            batch_body_model.submit_frames(frames, s, where=2)
-            pending.append((s, first, n_valid))
-        for s, fi, nv in pending:
-            finish(fi, batch_body_model.collect(s)[:nv])
+            arg, wh, dec = _decoded(s, frames, first, 2)
+            batch_body_model.submit_frames(arg, s, where=wh)
+            pending.append((s, first, n_valid, dec, arg, wh))
+        while pending:
+            retire()
     else:
         for frames, first in src:
             finish(first, batch_body_model(to_tensor(frames)))
@@ -570,7 +685,7 @@ def _box_to_roi(peaks, box, boxsize, mirrored):
 
 
 def batch_hand_extraction(videopath, motiondata, recpoints, outpath, batch_hand_estimation, boxsize=368, batchsize=32,
-                          log=print, decode_workers=1, sessions=2):
+                          log=print, decode_workers=1, sessions=2, decode="cv2"):
     """`Batch_hand_extraction` (srcmx/Batch_motion_Estimation.py:19-63) -> HandMat (COUNTS, 42, 3): rows 0-20 left hand,
     21-41 right hand, in ROI coordinates; a coordinate of exactly 0 means "missing" and is not offset.
 
@@ -579,12 +694,15 @@ def batch_hand_extraction(videopath, motiondata, recpoints, outpath, batch_hand_
     batches are in flight on `sessions` sessions and HandMat rows are the only thing that comes back (batches of at
     most 32 frames; `decode_workers` as in `batch_body_extraction`).  One deviation from the host path: a hand box of
     width 0, on which the reference's cv2.resize raises, is treated as a missing hand.  OPB_HOST_HANDS=1, or any other
-    estimator, takes the host path: crops cut with cv2 and `batch_hand_estimation` called on ToTensor-ed batches."""
+    estimator, takes the host path: crops cut with cv2 and `batch_hand_estimation` called on ToTensor-ed batches.
+    decode="device" (MJPG video, the device path): the JPEG packets are decoded on the consuming session."""
     import joblib
     from .batch_model import Batch_hand
-    if type(batch_hand_estimation) is Batch_hand and os.environ.get("OPB_HOST_HANDS") is None:
+    on_device = type(batch_hand_estimation) is Batch_hand and os.environ.get("OPB_HOST_HANDS") is None
+    _check_decode(decode, on_device)
+    if on_device:
         return _batch_hand_on_device(videopath, motiondata, recpoints, outpath, batch_hand_estimation, boxsize,
-                                     min(batchsize, Batch_hand.TRACK_BATCH), log, decode_workers, sessions)
+                                     min(batchsize, Batch_hand.TRACK_BATCH), log, decode_workers, sessions, decode)
     src = FrameBatches(videopath, recpoints, batch=batchsize, depth=4, pinned=False)
     assert src.count == len(motiondata)
     mat = np.zeros((len(motiondata), 42, 3))
@@ -605,10 +723,10 @@ def batch_hand_extraction(videopath, motiondata, recpoints, outpath, batch_hand_
 
 
 def _batch_hand_on_device(videopath, motiondata, recpoints, outpath, est, boxsize, batchsize, log, decode_workers,
-                          sessions):
+                          sessions, decode="cv2"):
     import joblib
     src = FrameBatches(videopath, recpoints, batch=batchsize, depth=sessions + 3, pinned=True, workers=decode_workers,
-                       pad_last=True)
+                       pad_last=True, decode=decode)
     assert src.count == len(motiondata)
     motiondata = np.asarray(motiondata, dtype=np.float64)
     mat = np.zeros((len(motiondata), 42, 3))
@@ -618,7 +736,8 @@ def _batch_hand_on_device(videopath, motiondata, recpoints, outpath, est, boxsiz
 
     def retire():
         nonlocal count
-        s, first, nv = pending.pop(0)
+        s, first, nv, dec, arg, wh, poses = pending.pop(0)
+        _rerun_corrupt(dec, lambda: est.submit_track(arg, poses, s, where=wh, boxsize=boxsize))
         hi = min(first + nv, len(mat))
         mat[first:hi] = est.collect_track(s)[:hi - first]
         for _ in range(hi - first):
@@ -634,8 +753,9 @@ def _batch_hand_on_device(videopath, motiondata, recpoints, outpath, est, boxsiz
         if len(pending) == sessions:
             retire()
         s = next(c for c in ss if all(c is not p[0] for p in pending))
-        est.submit_track(frames, poses, s, where=2, boxsize=boxsize)
-        pending.append((s, first, nv))
+        arg, wh, dec = _decoded(s, frames, first, 2)
+        est.submit_track(arg, poses, s, where=wh, boxsize=boxsize)
+        pending.append((s, first, nv, dec, arg, wh, poses))
     while pending:
         retire()
     joblib.dump(mat, outpath)
@@ -644,7 +764,7 @@ def _batch_hand_on_device(videopath, motiondata, recpoints, outpath, est, boxsiz
 
 
 def batch_bodyhand_extraction(videopath, body_outpath, hand_outpath, batch_size, recpoint, batch_body_model,
-                              batch_hand_estimation, boxsize=368, log=print, decode_workers=1, sessions=2):
+                              batch_hand_estimation, boxsize=368, log=print, decode_workers=1, sessions=2, decode="cv2"):
     """`Batch_body_extraction` and then `Batch_hand_extraction` on its track (srcmx/Batch_motion_Estimation.py:19-112)
     -> (MotionMat (COUNTS, 18, 3), HandMat (COUNTS, 42, 3)), written to `body_outpath` / `hand_outpath` with the same
     shapes, dtypes and log lines as `batch_body_extraction` and `batch_hand_extraction`.
@@ -663,9 +783,12 @@ def batch_bodyhand_extraction(videopath, body_outpath, hand_outpath, batch_size,
                                       Batch_body(body_model_path), Batch_hand(hand_model_path))
         run_body_job(videofolder, datadir, recpoint, process_video)
 
-    (create the two estimators once, outside the closure: their sessions are kept across videos)."""
+    (create the two estimators once, outside the closure: their sessions are kept across videos).  decode="device"
+    (MJPG video, this package's estimators): the JPEG packets are decoded on the consuming session."""
     from .batch_model import Batch_body, Batch_hand, BatchPoseEstimator
-    if type(batch_body_model) is not Batch_body or type(batch_hand_estimation) is not Batch_hand:
+    native = type(batch_body_model) is Batch_body and type(batch_hand_estimation) is Batch_hand
+    _check_decode(decode, native)
+    if not native:
         motion = batch_body_extraction(videopath, body_outpath, batch_size, recpoint, batch_body_model, log=log,
                                        decode_workers=decode_workers, sessions=sessions)
         if motion is None:
@@ -677,7 +800,7 @@ def batch_bodyhand_extraction(videopath, body_outpath, hand_outpath, batch_size,
     batch = min(batch_size, BatchPoseEstimator.MAX_BATCH)
     try:
         src = FrameBatches(videopath, recpoint, batch=batch, depth=sessions + 3, pinned=True, workers=decode_workers,
-                           pad_last=True)
+                           pad_last=True, decode=decode)
     except FileNotFoundError as e:
         log(str(e))
         return None
@@ -690,7 +813,8 @@ def batch_bodyhand_extraction(videopath, body_outpath, hand_outpath, batch_size,
     counts = [0, 0]                                                # frames retired: body job, hand job
 
     def retire():
-        pair, first, nv = pending.pop(0)
+        pair, first, nv, dec, arg, wh = pending.pop(0)
+        _rerun_corrupt(dec, lambda: est.submit(arg, pair, where=wh, boxsize=boxsize))
         m, h = est.collect(pair)
         hi = min(first + nv, len(motion))
         motion[first:hi] = m[:hi - first]
@@ -708,8 +832,9 @@ def batch_bodyhand_extraction(videopath, body_outpath, hand_outpath, batch_size,
         if len(pending) == len(pairs):
             retire()
         pair = next(c for c in pairs if all(c is not p[0] for p in pending))
-        est.submit(frames, pair, where=2, boxsize=boxsize)
-        pending.append((pair, first, n_valid))
+        arg, wh, dec = _decoded(pair[0], frames, first, 2)
+        est.submit(arg, pair, where=wh, boxsize=boxsize)
+        pending.append((pair, first, n_valid, dec, arg, wh))
     while pending:
         retire()
     joblib.dump(motion, body_outpath)
@@ -782,7 +907,7 @@ def batch_pose_mats_every_person(frames_u8, batch_body_model, batch_hand_estimat
 
 def batch_every_person_extraction(videopath, outpath, batch_size, recpoint, batch_body_model, batch_hand_estimation,
                                   max_gap=15, max_dist=None, min_joints=3, boxsize=368, log=print, decode_workers=1,
-                                  sessions=2):
+                                  sessions=2, decode="cv2"):
     """Body and hands of every person of a video on the batched estimators, linked into per-person tracks
     (`motion.PersonLinker`'s rule), dumped with joblib to `outpath` in the format of `extract_every_person_from_video`:
     {"count": frames, "tracks": [(first_frame, posemat (L, 60, 3) float64), ...]}, indexed by track id, with zero rows
@@ -804,14 +929,16 @@ def batch_every_person_extraction(videopath, outpath, batch_size, recpoint, batc
             batch_every_person_extraction(videopath, outpath, 32, recpoint, body, hand)
         run_body_job(videofolder, datadir, recpoint, process_video, mode="tracks")
 
-    (create the two estimators once, outside the closure: their sessions are kept across videos)."""
+    (create the two estimators once, outside the closure: their sessions are kept across videos).  decode="device"
+    (MJPG video, this package's estimators): the JPEG packets are decoded on the consuming session."""
     from .batch_model import Batch_body, Batch_hand, BatchPoseEstimator
     from .motion import PersonLinker
     device = type(batch_body_model) is Batch_body and type(batch_hand_estimation) is Batch_hand
+    _check_decode(decode, device)
     batch = min(batch_size, BatchPoseEstimator.MAX_BATCH) if device else batch_size
     try:
         src = FrameBatches(videopath, recpoint, batch=batch, depth=sessions + 3 if device else 4, pinned=device,
-                           workers=decode_workers, pad_last=device, ordered=True)
+                           workers=decode_workers, pad_last=device, ordered=True, decode=decode)
     except FileNotFoundError as e:
         log(str(e))
         return None
@@ -830,20 +957,23 @@ def batch_every_person_extraction(videopath, outpath, batch_size, recpoint, batc
         pending = []                                               # (pair, first, n_valid)
 
         def retire():
-            pair, first, nv = pending.pop(0)
+            pair, first, nv, dec, arg, wh = pending.pop(0)
             n_link = max(0, min(nv, src.count - first))
+            _rerun_corrupt(dec, lambda: est.submit_every_person(arg, pair, where=wh, boxsize=boxsize))
             recs, ids = est.collect_every_person(pair, tracker=tracker, n_link=n_link)
             frames.append((first, recs[:n_link], ids[:n_link]))
             progress(first, n_link)
 
         for fr, first, n_valid in src:
-            if tracker is None:
-                tracker = est.tracker(max_gap, 0.1 * fr.shape[1] if max_dist is None else max_dist, min_joints)
             if len(pending) == len(pairs):
                 retire()
             pair = next(c for c in pairs if all(c is not p[0] for p in pending))
-            est.submit_every_person(fr, pair, where=2, boxsize=boxsize)
-            pending.append((pair, first, n_valid))
+            arg, wh, dec = _decoded(pair[0], fr, first, 2)
+            if tracker is None:
+                height = dec.shape[1] if dec is not None else fr.shape[1]
+                tracker = est.tracker(max_gap, 0.1 * height if max_dist is None else max_dist, min_joints)
+            est.submit_every_person(arg, pair, where=wh, boxsize=boxsize)
+            pending.append((pair, first, n_valid, dec, arg, wh))
         while pending:
             retire()
     else:

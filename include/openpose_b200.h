@@ -266,6 +266,9 @@ int opb_batch_pose_every_submit(opb_session* body_s, opb_session* hand_s, const 
 /* blurred heat maps of the last batched-estimator call: (n, 19 | 22, height, width) planar fp32; the
  * un-blurred maps and the PAFs come from opb_body_maps / opb_hand_maps.                             */
 int opb_batch_maps(opb_session* s, float* host_blurred_heat);
+/* Debug: the bf16 net input of the last batched-estimator call, (n, hp, wp, 3) bit patterns: the resized frames (a
+ * Batch_hand crop is not resized) minus 0.5, zero padding to multiples of 8 (hp, wp as O.batch_size_pad gives them).  */
+int opb_batch_debug_input(opb_session* s, uint16_t* host_dst);
 
 /* ---- stage-level entry points on DEVICE buffers (parity tests, per-stage benches) ------------- */
 /* src/body.py:38-41 + src/util.py:12-32: cubic resize by `multiplier`, pad right/bottom with 128 to a
@@ -418,6 +421,13 @@ int opb_debug_resize_taps(int src, int dst, double scale, int* first, float* coe
 int opb_debug_hand_track_taps(int side, int boxsize, int* first, float* coef4);
 int opb_debug_composite_taps(int n_net, int n_resized, int n_orig, int* first, float* w6);
 int opb_debug_resize_dsize(int n, double f);
+/* The same for Batch_body / Batch_hand, whose resizes are torch's F.interpolate(mode="bicubic") on float32:
+ * opb_debug_batch_resize_taps: the front end's taps, F.interpolate(scale_factor=scale_factor), or size mode (dst
+ *   given) when scale_factor <= 0.
+ * opb_debug_batch_composite_taps: the map side, F.interpolate(scale_factor=8), crop to n_resized,
+ *   F.interpolate(size=n_orig).                                                                                     */
+int opb_debug_batch_resize_taps(int src, int dst, double scale_factor, int* first, float* coef4);
+int opb_debug_batch_composite_taps(int n_net, int n_resized, int n_orig, int* first, float* w6);
 
 /* Host only (no device call): the tile list of the CTA-pair convolution kernel for one problem of n images of h x w
  * pixels, exactly as the kernel decodes it -- 8 ints per (pair, cluster rank): image, x0, y0, n0, real (0 = padding tile,

@@ -76,6 +76,7 @@ SIGNATURES = {
     "opb_batch_body_submit_u8": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_double]),
     "opb_batch_hand_submit_u8": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int]),
     "opb_batch_maps": (c_int, [c_void_p, c_void_p]),
+    "opb_batch_debug_input": (c_int, [c_void_p, c_void_p]),
     "opb_hand_track_submit": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int]),
     "opb_hand_track_wait": (c_int, [c_void_p, c_void_p]),
     "opb_hand_track_crops": (c_int, [c_void_p, c_void_p]),
@@ -108,6 +109,8 @@ SIGNATURES = {
     "opb_debug_resize_taps": (c_int, [c_int, c_int, ctypes.c_double, c_void_p, c_void_p]),
     "opb_debug_composite_taps": (c_int, [c_int, c_int, c_int, c_void_p, c_void_p]),
     "opb_debug_resize_dsize": (c_int, [c_int, ctypes.c_double]),
+    "opb_debug_batch_resize_taps": (c_int, [c_int, c_int, ctypes.c_double, c_void_p, c_void_p]),
+    "opb_debug_batch_composite_taps": (c_int, [c_int, c_int, c_int, c_void_p, c_void_p]),
     "opb_debug_pair_tiles": (c_int, [c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_void_p]),
     "opb_net_debug_plan": (c_int, [c_void_p, c_int, c_void_p, POINTER(c_int)]),
     "opb_net_debug_set_input": (c_int, [c_void_p, c_int, c_void_p]),

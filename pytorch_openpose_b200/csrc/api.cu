@@ -132,14 +132,14 @@ static ScaleDims batch_dims(int H, int W, double g_scale, bool body) {
     return d;
 }
 
-// float tap tables of the torch bicubic resize (batched estimators' front end)
+// float tap tables of the torch bicubic resize (batched estimators' front end, F.interpolate(scale_factor=mult))
 struct F32Taps {
     int *xf, *yf;
     float *xc, *yc;
     void relocate_to(uint8_t* b) { relocate(xf, b); relocate(yf, b); relocate(xc, b); relocate(yc, b); }
 };
 static F32Taps make_f32_taps(TableSlab& pool, int H, int W, const ScaleDims& d) {
-    const CubicTaps tx = cubic_taps(W, d.w, 1.0 / d.mult), ty = cubic_taps(H, d.h, 1.0 / d.mult);
+    const CubicTaps tx = torch_cubic_taps(W, d.w, d.mult), ty = torch_cubic_taps(H, d.h, d.mult);
     F32Taps u;
     u.xf = pool.add(tx.first);
     u.yf = pool.add(ty.first);
@@ -162,11 +162,12 @@ struct UpTables {
         relocate(ybf, b); relocate(ybr, b); relocate(ybw, b);
     }
 };
-static UpTables make_up_tables(TableSlab& pool, int H, int W, const ScaleDims& d, int n_scales) {
+// torch: the batched estimators' map resizes (F.interpolate(scale_factor=8), then F.interpolate(size=(H, W)))
+static UpTables make_up_tables(TableSlab& pool, int H, int W, const ScaleDims& d, int n_scales, bool torch) {
     std::vector<int> fx, fy;
     std::vector<float> wx, wy;
-    composite_taps(d.wo, d.w, W, fx, wx);
-    composite_taps(d.ho, d.h, H, fy, wy);
+    composite_taps(d.wo, d.w, W, fx, wx, torch);
+    composite_taps(d.ho, d.h, H, fy, wy, torch);
     // the cross-scale average (heatmap / len(multiplier), src/body.py:67-68) is folded into the row weights
     for (auto& v : wy) v = v / (float)n_scales;
     UpTables t;
@@ -689,7 +690,7 @@ static FramePlan* get_plan(opb_session* s, int n, int H, int W, const double* sc
         fp->dims.push_back(d);
         if (mode >= 1) fp->f32taps.push_back(make_f32_taps(fp->tables, H, W, d));
         else fp->u8taps.push_back(make_u8_taps(fp->tables, H, W, d));
-        fp->uptabs.push_back(make_up_tables(fp->tables, H, W, d, n_scales));
+        fp->uptabs.push_back(make_up_tables(fp->tables, H, W, d, n_scales, mode >= 1));
         shapes.push_back({n, d.hp, d.wp, mode >= 1 ? 2 : 1});
         fp->scratch_floats += (size_t)n * C * d.ho * W;
     }
@@ -2105,6 +2106,19 @@ int opb_batch_maps(opb_session* s, float* host_blurred_heat) {
     });
 }
 
+int opb_batch_debug_input(opb_session* s, uint16_t* host_dst) {
+    return guarded([&] {
+        OPB_REQUIRE(s && s->active && s->active->key.mode >= 1 && host_dst, "no finished batched-estimator call");
+        OPB_CUDA(cudaSetDevice(s->net->ctx->device));
+        OPB_CUDA(cudaEventSynchronize(s->done));
+        const FramePlan* fp = s->active;
+        const ScaleDims& d = fp->dims[0];
+        const size_t bytes = (size_t)fp->key.n * d.hp * d.wp * 3 * sizeof(__nv_bfloat16);
+        OPB_CUDA(cudaMemcpyAsync(host_dst, fp->net->in_u8[0], bytes, cudaMemcpyDeviceToHost, s->stream));
+        OPB_CUDA(cudaStreamSynchronize(s->stream));
+    });
+}
+
 /* ---- the batched hand job on the device ------------------------------------------------------------------------- */
 int opb_hand_track_submit(opb_session* hand_s, const uint8_t* frames_bgr, int where, int n_frames, int height, int width,
                           const double* host_poses, int boxsize) {
@@ -2512,7 +2526,7 @@ int opb_body_debug_post_dims(int H, int W, const double* scales, int ns, int mod
         std::vector<UpTables> tabs;
         for (int i = 0; i < ns; ++i) {
             dims.push_back(plan_dims(H, W, scales[i], mode, true));
-            tabs.push_back(make_up_tables(slab, H, W, dims[i], ns));
+            tabs.push_back(make_up_tables(slab, H, W, dims[i], ns, mode >= 1));
             ho_wo[2 * i] = dims[i].ho;
             ho_wo[2 * i + 1] = dims[i].wo;
         }
@@ -2565,7 +2579,7 @@ int opb_upsample_avg(opb_context* ctx, const float* const* dev_maps, const doubl
         size_t scratch = 0;
         for (int i = 0; i < ns; ++i) {
             dims.push_back(scale_dims(H, W, scales[i]));
-            tabs.push_back(make_up_tables(slab, H, W, dims[i], ns));
+            tabs.push_back(make_up_tables(slab, H, W, dims[i], ns, false));
             scratch += (size_t)C * dims[i].ho * W;
         }
         uint8_t* base = commit_tables(pool, slab, ctx->stream);
@@ -2909,6 +2923,27 @@ int opb_debug_composite_taps(int n_net, int n_resized, int n_orig, int* first, f
         std::vector<int> f;
         std::vector<float> w;
         composite_taps(n_net, n_resized, n_orig, f, w);
+        memcpy(first, f.data(), sizeof(int) * n_orig);
+        memcpy(w6, w.data(), sizeof(float) * 6 * n_orig);
+    });
+}
+
+int opb_debug_batch_resize_taps(int src, int dst, double scale_factor, int* first, float* coef4) {
+    return guarded([&] {
+        OPB_REQUIRE(first && coef4 && src >= 1 && dst >= 1, "opb_debug_batch_resize_taps: bad argument");
+        const CubicTaps t = torch_cubic_taps(src, dst, scale_factor);
+        memcpy(first, t.first.data(), sizeof(int) * dst);
+        memcpy(coef4, t.coef.data(), sizeof(float) * 4 * dst);
+    });
+}
+
+int opb_debug_batch_composite_taps(int n_net, int n_resized, int n_orig, int* first, float* w6) {
+    return guarded([&] {
+        OPB_REQUIRE(first && w6 && n_net >= 1 && n_resized >= 1 && n_resized <= 8 * n_net && n_orig >= 1,
+                    "opb_debug_batch_composite_taps: bad argument");
+        std::vector<int> f;
+        std::vector<float> w;
+        composite_taps(n_net, n_resized, n_orig, f, w, true);
         memcpy(first, f.data(), sizeof(int) * n_orig);
         memcpy(w6, w.data(), sizeof(float) * 6 * n_orig);
     });

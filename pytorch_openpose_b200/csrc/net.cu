@@ -741,10 +741,48 @@ CubicTaps cubic_taps(int src, int dst, double scale) {
     return t;
 }
 
-// composite 1-D operator: x8 cubic upsample of n_net samples -> crop to n_resized -> cubic resize to n_orig
-void composite_taps(int n_net, int n_resized, int n_orig, std::vector<int>& first, std::vector<float>& w6) {
-    const CubicTaps up = cubic_taps(n_net, n_net * 8, 1.0 / 8.0);
-    const CubicTaps down = cubic_taps(n_resized, n_orig, 1.0 / ((double)n_orig / (double)n_resized));
+// F.interpolate(mode="bicubic", align_corners=False) of float32 tensors: ATen's compute_indices_weights_cubic,
+// guard_index_and_lambda and get_cubic_upsample_coefficients (the Batch_body / Batch_hand resizes).  Unlike cv2 the
+// step is a float32 value (1 / scale_factor rounded once, or float(src) / float(dst) in size mode, scale_factor <= 0),
+// the source coordinate is one float32 fused multiply-add, and c3 is a polynomial of its own.  ATen's compiled CPU
+// kernel fuses the first multiply-add of cc1 and the first two of cc2 and rounds the rest separately; this order
+// reproduces the installed torch's weights bit for bit (tests/test_batch_resize_host.py).
+CubicTaps torch_cubic_taps(int src, int dst, double scale_factor) {
+    CubicTaps t;
+    t.first.resize(dst);
+    t.coef.resize((size_t)dst * 4);
+    const float A = -0.75f;
+    const float s = scale_factor > 0 ? (float)(1.0 / scale_factor) : (float)src / (float)dst;
+    auto cc1 = [A](float x) {                         // ((A + 2) x - (A + 3)) x x + 1
+        volatile float p = std::fmaf(A + 2.0f, x, -(A + 3.0f));
+        volatile float q = p * x;
+        volatile float r = q * x;
+        return r + 1.0f;
+    };
+    auto cc2 = [A](float x) {                         // ((A x - 5 A) x + 8 A) x - 4 A
+        volatile float p = std::fmaf(std::fmaf(A, x, -5.0f * A), x, 8.0f * A);
+        volatile float q = p * x;
+        return q - 4.0f * A;
+    };
+    for (int d = 0; d < dst; ++d) {
+        const float r = std::fmaf(s, (float)d + 0.5f, -0.5f);
+        const int i = std::min((int)std::floor(r), src - 1);
+        const float l = std::min(std::max(r - (float)i, 0.0f), 1.0f);
+        t.first[d] = i - 1;
+        t.coef[(size_t)d * 4 + 0] = cc2(l + 1.0f);
+        t.coef[(size_t)d * 4 + 1] = cc1(l);
+        t.coef[(size_t)d * 4 + 2] = cc1(1.0f - l);
+        t.coef[(size_t)d * 4 + 3] = cc2((1.0f - l) + 1.0f);
+    }
+    return t;
+}
+
+// composite 1-D operator: x8 cubic upsample of n_net samples -> crop to n_resized -> cubic resize to n_orig, with
+// cv2's taps (Body) or torch's (Batch_body / Batch_hand, size mode for the resize)
+void composite_taps(int n_net, int n_resized, int n_orig, std::vector<int>& first, std::vector<float>& w6, bool torch) {
+    const CubicTaps up = torch ? torch_cubic_taps(n_net, n_net * 8, 8.0) : cubic_taps(n_net, n_net * 8, 1.0 / 8.0);
+    const CubicTaps down = torch ? torch_cubic_taps(n_resized, n_orig, 0.0)
+                                 : cubic_taps(n_resized, n_orig, 1.0 / ((double)n_orig / (double)n_resized));
     first.assign(n_orig, 0);
     w6.assign((size_t)n_orig * kUpTaps, 0.f);
     std::vector<double> acc(n_net);

@@ -168,7 +168,10 @@ struct CubicTaps {
     std::vector<float> coef;      // [dst][4] float32 coefficients
 };
 CubicTaps cubic_taps(int src, int dst, double scale);
+// torch's bicubic taps; scale_factor <= 0: size mode (dst given, step float(src) / float(dst))
+CubicTaps torch_cubic_taps(int src, int dst, double scale_factor);
 int resize_dsize(int n, double f);                 // cv2: saturate_cast<int>(n*f), round half to even
-void composite_taps(int n_net, int n_resized, int n_orig, std::vector<int>& first, std::vector<float>& w6);
+void composite_taps(int n_net, int n_resized, int n_orig, std::vector<int>& first, std::vector<float>& w6,
+                    bool torch = false);
 
 }  // namespace opb

@@ -484,9 +484,10 @@ void upsample_avg_launch2(const UpsampleScale* scales, int n_scales, int n_img, 
 namespace {
 
 // Front end of Batch_body.__call__ (Batch_model.py:153-155) and Batch_hand.__call__ (:373): float frames in [0,1],
-// planar (n,3,H,W); bicubic resize (torch semantics: A = -0.75, half-pixel centres, clamped taps, no antialias) to
-// (h,w); minus 0.5; zero padding to (hp,wp).  Output: bf16 HWC3, the input format of conv1_1's bf16 variant.  With
-// identical sizes the taps degenerate to (0,1,0,0) and the frame is copied exactly.
+// planar (n,3,H,W); bicubic resize to (h,w) with the tables of net.cu::torch_cubic_taps (torch's own weights bit for
+// bit: A = -0.75, half-pixel centres, clamped taps, no antialias, float32 step 1 / scale_factor); minus 0.5; zero
+// padding to (hp,wp).  Output: bf16 HWC3, the input format of conv1_1's bf16 variant.  With identical sizes the taps
+// are (0,1,0,0) and the output is bf16(x - 0.5) exactly.
 // sample (c, y, x) of frame `img`: planar float, or decoded uint8 HWC pixels with ToTensor's division by 255 applied here
 __device__ __forceinline__ float frame_at(const float* in, size_t img, int c, int y, int x, int H, int W) {
     return __ldg(in + ((img * 3 + c) * (size_t)H + y) * W + x);

@@ -31,9 +31,10 @@ from oracle import openpose_oracle as O
 U = 2.0 ** -24
 
 
-def bound_factor(n_scales):
-    """c of the per-element bound c * 2^-24 * sum |w_y||w_x||v| (module docstring)."""
-    return 1.02 * (6 * n_scales + 9)
+def bound_factor(n_scales, extra=0):
+    """c of the per-element bound c * 2^-24 * sum |w_y||w_x||v| (module docstring); `extra` roundings by which the
+    reference operator itself may differ from the one the tables were built from (tests/batch_resize_ref.py)."""
+    return 1.02 * (6 * n_scales + 9 + extra)
 
 
 def axis_operators(H, W, dims):
@@ -53,18 +54,18 @@ def reference(nets, ops):
     return ref, mag
 
 
-def excess(planes, nets, ops):
+def excess(planes, nets, ops, extra=0):
     """max over elements of |planes - ref| / bound (<= 1 passes).  planes: (C, H, W) float32 device maps."""
     ref, mag = reference(nets, ops)
     err = np.abs(np.asarray(planes, dtype=np.float64) - ref)
-    bound = bound_factor(len(nets)) * (U * mag + 2.0 ** -149)
+    bound = bound_factor(len(nets), extra) * (U * mag + 2.0 ** -149)
     with np.errstate(divide="ignore", invalid="ignore"):
         r = np.where(err == 0, 0.0, err / bound)
     return float(r.max())
 
 
-def assert_within_bound(planes, nets, ops, what=""):
-    e = excess(planes, nets, ops)
+def assert_within_bound(planes, nets, ops, what="", extra=0):
+    e = excess(planes, nets, ops, extra)
     assert e <= 1.0, "%s: device maps exceed the float64 bound by %.3g x" % (what, e)
     return e
 
